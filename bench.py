@@ -9,8 +9,12 @@ ncclAllGather + a device merge give every rank the global top-K -- all inside th
 stocs_b200_score_sharded_device.  The weak-scaling figure (10^6 per GPU) is reported under `extra`.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload s1|s2]
+                  [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for how each field is produced.
+--dump-outputs DIR writes what the last timed step returned to its caller as DIR/<name>.npy
+(rank 0; integers widened to float64, which holds them exactly).  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -26,6 +30,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: nothing is cached in it
 
 N_SCENE = 1 << 20
 N_MODEL = 512
@@ -39,6 +44,23 @@ def algorithmic_bytes_per_hypothesis(M):
     # SURVEY.md section 8(d): 64 B per NN query (8 cell descriptors x 4 B + one 16 B candidate
     # position + one 16 B attribute record) x |M| queries + 48 B transform in + 8 B results out.
     return 56 + 64 * M
+
+
+def dump_outputs(dirname, arrays):
+    """--dump-outputs: each array as <dirname>/<name>.npy, float32 / float64 only."""
+    if not dirname:
+        return
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        if a.dtype not in (np.float32, np.float64):
+            a = a.astype(np.float64)
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
+def record_arrays(rec, prefix=""):
+    """the fields of a RECORD array (the top-K a scoring call returns), one array per field"""
+    return {f"{prefix}topk_{f}": rec[f] for f in ("index", "lcp", "inliers", "T")}
 
 
 def workload(rank, H):
@@ -431,9 +453,10 @@ def run_reference(args):
         n = min(1000 * cores, 10000)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            for e, T in zip(ests, Ts):
-                e.score(T[:n], threads=cores)
+            last = [e.score(T[:n], threads=cores) for e, T in zip(ests, Ts)]
         dt = time.perf_counter() - t0
+        dump_outputs(args.dump_outputs, {f"obj{k}_{name}": a for k, (lcp, inl) in enumerate(last)
+                                         for name, a in (("lcp", lcp), ("inliers", inl))})
         v = n * len(ests) * args.steps / dt
         cfg, sample = s2_config(args.gpus), f"{n} hypotheses of each of 2 of the 8 objects per step, {cores} threads"
     else:
@@ -445,8 +468,9 @@ def run_reference(args):
         t0 = time.perf_counter()
         for k in range(args.steps):
             off = (k * n) % (len(T) - n)
-            est.score(T[off:off + n], threads=cores)
+            lcp, inl = est.score(T[off:off + n], threads=cores)
         dt = time.perf_counter() - t0
+        dump_outputs(args.dump_outputs, {"lcp": lcp, "inliers": inl})
         v = n * args.steps / dt
         cfg, sample = s1_config(args.gpus), f"{n} hypotheses per step ({args.steps} steps) of the S1 list, {cores} threads"
     out = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus,
@@ -523,6 +547,7 @@ def main():
     ap.add_argument("--hyp", type=int, default=H_TOTAL, help="hypotheses in the list (default: the named config)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip S1-fit, weak scaling and pose latency")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)
@@ -621,6 +646,8 @@ def main():
     clocks = sampler.stop(t_begin, t_end) if sampler else None
     value = H * args.steps / (ms_total * 1e-3)
     rec = drec.cpu().numpy().view(RECORD).copy()
+    if rank == 0:
+        dump_outputs(args.dump_outputs, record_arrays(rec))
 
     # ---- merged result == single-GPU result of the whole list (asserted on every run)
     dTf = torch.from_numpy(T).to(dev) if world > 1 else dT
@@ -868,6 +895,8 @@ def run_s2(args, env):
     ms_total, kernel_ms, t_begin, t_end = timed_steps(step, args.steps, ctxs)
     clocks = sampler.stop(t_begin, t_end) if sampler else None
     recs = [dr.cpu().numpy().view(RECORD).copy() for dr in drecs]
+    if rank == 0:
+        dump_outputs(args.dump_outputs, {k: a for i, r in enumerate(recs) for k, a in record_arrays(r, f"obj{i}_").items()})
     if world > 1:
         allrec = [None] * world
         dist.all_gather_object(allrec, b"".join(r.tobytes() for r in recs))

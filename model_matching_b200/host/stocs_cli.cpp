@@ -5,8 +5,9 @@
 //
 // argv, the files read and written, and the progress lines on stdout are those of the reference's
 // src/stocs_match_one_object.cpp and src/model_preprocess.cpp (whose sources, unmodified, also
-// compile and link against this directory: tests/ref_callers).  Everything goes through the
-// public stocs::stocs_estimator / stocs::pre_process_model interface of stocs.hpp.
+// compile and link against this directory; tests/test_ref_callers.py pins what they write).
+// Everything goes through the public stocs::stocs_estimator / stocs::pre_process_model interface
+// of stocs.hpp.
 //
 // The reference keeps its tunables as compile-time globals ("edit and recompile", README.md:47-69);
 // here they live in one Settings record whose defaults are the reference's values and which the
