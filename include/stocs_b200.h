@@ -285,7 +285,10 @@ int stocs_b200_group_score_best(stocs_b200_group* g, const float* T16, int64_t H
 /* ---- diagnostics ---------------------------------------------------------------------------
  * [0] score kernels launched and [1] NN queries resolved by the kd-tree tie path, both accumulated
  * over the lifetime of the context; [2] grid cells and [3] replicated candidate records of the
- * current scene index. */
+ * current scene index; [4] / [5] hypotheses the device top-K path (score_sharded_device,
+ * group_score_best without per-hypothesis outputs) left unscored because they provably cannot
+ * enter the top K, rejected after the coarse test / before a queue drain, accumulated over the
+ * lifetime of the context. */
 int stocs_b200_get_counters(stocs_b200_ctx* ctx, int64_t* counters, int n);
 /* Data-dependent work of ONE scoring launch over H device-resident transforms, counted exactly by a
  * counting instantiation of the scoring kernel (results discarded, not for timing).  counters (up

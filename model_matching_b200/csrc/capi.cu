@@ -1,6 +1,7 @@
 // capi.cu -- the C ABI of libstocs_b200.so (include/stocs_b200.h): context, uploads, host-buffer
 // wrappers around the kernels.  No CPU fallback anywhere: every compute entry point launches
 // sm_100a kernels, and stocs_b200_create refuses to run without a compute-capability-10 device.
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -31,6 +32,18 @@ bool stocs_is_host_memory(const void* p) {
   cudaPointerAttributes pa{};
   if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) { cudaGetLastError(); return false; }
   return pa.type == cudaMemoryTypeHost;
+}
+
+// Largest class weight of the scene.  The top-K pruning bound of the scoring kernel (score.cu) needs
+// every weight of the scene in [0, w_max]; whatever replaces the weights calls this again.
+void stocs_set_weight_bound(stocs_b200_ctx* ctx, const float* cls, int S) {
+  ctx->w_max = 0.f;
+  ctx->prune_ok = true;
+  for (int i = 0; i < S; ++i) {
+    const float w = cls[i];
+    if (!(w >= 0.f && w <= FLT_MAX)) { ctx->prune_ok = false; break; }   // negative, NaN or infinite
+    if (w > ctx->w_max) ctx->w_max = w;
+  }
 }
 
 extern "C" {
@@ -222,6 +235,7 @@ int stocs_b200_upload_scene(stocs_b200_ctx* ctx, const float* pos3, const float*
   if (pixel_rc) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_spix.p, pixel_rc, (size_t)S * 8, cudaMemcpyHostToDevice, st));
   else STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_spix.p, 0, (size_t)S * 8, st));
   ctx->has_pixels = pixel_rc != nullptr;
+  stocs_set_weight_bound(ctx, class_probability, S);
   ctx->pix_min[0] = ctx->pix_min[1] = 0; ctx->pix_max[0] = ctx->pix_max[1] = 0;
   if (pixel_rc) {  // range of the pixel coordinates: instance sampling indexes images with them
     ctx->pix_min[0] = ctx->pix_max[0] = pixel_rc[0]; ctx->pix_min[1] = ctx->pix_max[1] = pixel_rc[1];
@@ -461,11 +475,13 @@ int stocs_b200_reduce_best(stocs_b200_ctx* ctx, const float* lcp, int64_t H, int
 int stocs_b200_get_counters(stocs_b200_ctx* ctx, int64_t* counters, int n) {
   if (!ctx || !counters) return STOCS_E_ARG;
   cudaSetDevice(ctx->device);
-  if (ctx->d_small.p) {
-    unsigned long long t = 0;
+  if (ctx->d_small.p) {   // tie counter at 200, top-K rejections at 208 and 216 (score.cu)
+    unsigned long long t[3] = {0, 0, 0};
     STOCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    STOCS_CUDA(ctx, cudaMemcpy(&t, ctx->d_small.as<char>() + 200, 8, cudaMemcpyDeviceToHost));
-    ctx->counters[1] = (int64_t)t;
+    STOCS_CUDA(ctx, cudaMemcpy(t, ctx->d_small.as<char>() + 200, 24, cudaMemcpyDeviceToHost));
+    ctx->counters[1] = (int64_t)t[0];
+    ctx->counters[4] = (int64_t)t[1];
+    ctx->counters[5] = (int64_t)t[2];
   }
   for (int i = 0; i < n && i < 8; ++i) counters[i] = ctx->counters[i];
   return STOCS_OK;

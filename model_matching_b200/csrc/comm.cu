@@ -120,10 +120,13 @@ __global__ void __launch_bounds__(1024) merge_records_kernel(const stocs_b200_re
 }
 
 // local block -> K packed records in d_send (device).  Enqueues on st.
+// prune: the caller reads nothing of d_lcp / d_inl but the K records, so hypotheses that provably
+// cannot enter the top K may be left unscored (lcp 0, see kPrune in score.cu)
 int enqueue_local_topk(stocs_b200_ctx* ctx, const float* d_T, int64_t H_local, int64_t index_offset, int K,
-                       float* d_lcp, int32_t* d_inl, stocs_b200_record* d_send, cudaStream_t st, bool time_it) {
+                       float* d_lcp, int32_t* d_inl, stocs_b200_record* d_send, cudaStream_t st, bool time_it, bool prune) {
   if (H_local > 0) {
-    int rc = stocs_launch_score(ctx, d_T, H_local, d_lcp, d_inl, st, time_it, 0, nullptr, stocs_is_host_memory(d_T));
+    int rc = stocs_launch_score(ctx, d_T, H_local, d_lcp, d_inl, st, time_it, 0, nullptr, stocs_is_host_memory(d_T),
+                                nullptr, 0, prune ? K : 0);
     if (rc) return rc;
   }
   // H_local == 0: the top-K kernels run over an empty array and emit K empty records
@@ -200,11 +203,11 @@ int stocs_b200_score_sharded_device(stocs_b200_ctx* ctx, const float* d_T16_loca
   const int nranks = ctx->comm ? ctx->comm_nranks : 1;
   if (nranks == 1)  // no collective: the local top-K is the global one
     return enqueue_local_topk(ctx, d_T16_local, H_local, index_offset, K, b_lcp.as<float>(), b_inl.as<int32_t>(),
-                              d_topk_out, st, true);
+                              d_topk_out, st, true, true);
   STOCS_CUDA(ctx, b_send.ensure((size_t)K * sizeof(stocs_b200_record)));
   STOCS_CUDA(ctx, b_recv.ensure((size_t)K * nranks * sizeof(stocs_b200_record)));
   int rc = enqueue_local_topk(ctx, d_T16_local, H_local, index_offset, K, b_lcp.as<float>(), b_inl.as<int32_t>(),
-                              b_send.as<stocs_b200_record>(), st, true);
+                              b_send.as<stocs_b200_record>(), st, true, true);
   if (rc) return rc;
   // the path's one collective
   STOCS_NCCL(ctx, g_nccl.AllGather(b_send.p, b_recv.p, (size_t)K * sizeof(stocs_b200_record), ncclInt8,
@@ -408,7 +411,8 @@ int stocs_b200_group_score_best(stocs_b200_group* g, const float* T16, int64_t H
       e = cudaMemcpyAsync(b_T.p, T16 + 16 * lo[i], (size_t)hl * 64, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) { c->err = std::string("group_score_best: ") + cudaGetErrorString(e); return group_fail(g, i, STOCS_E_CUDA); }
     int rc = enqueue_local_topk(c, b_T.as<float>(), hl, lo[i], K, b_lcp.as<float>(), b_inl.as<int32_t>(),
-                                n > 1 ? b_send.as<stocs_b200_record>() : b_out.as<stocs_b200_record>(), st, false);
+                                n > 1 ? b_send.as<stocs_b200_record>() : b_out.as<stocs_b200_record>(), st, false,
+                                !lcp && !inliers);
     if (rc) return group_fail(g, i, rc);
   }
   // 2. ONE all-gather (grouped: one call per device of this process)

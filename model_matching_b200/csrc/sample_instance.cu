@@ -329,6 +329,9 @@ int stocs_launch_sample_instance(stocs_b200_ctx* ctx, uint64_t seed, int base_nu
   a.S = ctx->S;
   a.ppf = stocs_ppf_view(ctx);
   a.seed = seed; a.base_num = base_num; a.dispersion = dispersion;
+  // the prior decay rewrites weights in place as fl(dispersion * w): inside [0, w_max] only for a
+  // dispersion in [0, 1], so any other value turns off the top-K pruning bound for this scene
+  if (!(dispersion >= 0.f && dispersion <= 1.f)) ctx->prune_ok = false;
   a.edge = ctx->d_edge.as<uint8_t>();
   a.prev_mask = ctx->d_inst_state.as<uint8_t>();
   a.seg_buffer = a.prev_mask + n;
@@ -391,8 +394,10 @@ int stocs_b200_set_class_probability(stocs_b200_ctx* ctx, const float* cls) {
   if (!ctx || !cls) return STOCS_E_ARG;
   if (ctx->S <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "no scene");
   cudaSetDevice(ctx->device);
+  ctx->prune_ok = false;   // until the new weights are in place and bounded
   STOCS_CUDA(ctx, cudaMemcpy2DAsync(ctx->d_sattr.as<char>() + 12, 16, cls, 4, 4, (size_t)ctx->S, cudaMemcpyHostToDevice, ctx->stream));
   STOCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  stocs_set_weight_bound(ctx, cls, ctx->S);
   return STOCS_OK;
 }
 

@@ -299,7 +299,7 @@ extern "C" int stocs_b200_build_scene_cloud(stocs_b200_ctx* ctx, const uint16_t*
   SC(cudaMemcpyAsync(&h_len[0], d_nvox, 4, cudaMemcpyDeviceToHost, st));
   SC(cudaMemcpyAsync(&h_len[1], d_scan.as<int>() + n, 4, cudaMemcpyDeviceToHost, st));
   const bool have_out = pos3 && nrm3 && pixel_rc && class_p;
-  long long guess = have_out ? ctx->counters[5] : 0;
+  long long guess = have_out ? ctx->counters[7] : 0;
   if (guess > out_cap) guess = out_cap;
   auto fetch = [&](long long from, long long to) -> cudaError_t {
     const size_t c = (size_t)(to - from);
@@ -315,7 +315,7 @@ extern "C" int stocs_b200_build_scene_cloud(stocs_b200_ctx* ctx, const uint16_t*
   SC(cudaStreamSynchronize(st));
   const long long nvox = (long long)h_len[0], n_emit = (long long)h_len[1];
   *n_out = n_emit;
-  ctx->counters[5] = nvox;
+  ctx->counters[7] = nvox;
   if (n_emit > cap) { cleanup(); STOCS_FAIL(ctx, STOCS_E_CAPACITY, "build_scene_cloud: output capacity too small"); }
   if (n_emit > 0 && !have_out) { cleanup(); STOCS_FAIL(ctx, STOCS_E_ARG, "build_scene_cloud: output pointer is NULL"); }
   if (n_emit > guess) {

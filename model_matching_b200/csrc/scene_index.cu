@@ -619,7 +619,7 @@ int stocs_build_scene_index(stocs_b200_ctx* ctx) {
     cap = (size_t)total + 1024;
   }
   ctx->ncand = total;
-  ctx->counters[4] = n_occ;
+  ctx->counters[6] = n_occ;
   tr.mark("index build");
   ctx->counters[2] = g.ncells;
   ctx->counters[3] = total;

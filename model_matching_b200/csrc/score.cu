@@ -6,11 +6,11 @@
 //
 // One warp per hypothesis, persistent CTAs, dynamic work counter.  Model points live in shared
 // memory as float4.
-//   Phase A (per block of 256 model points), two loops:
+//   Phase A (per block of 256 model points; the top-K instantiation: over the whole model), two loops:
 //     1. the test every point takes: fused affine map "transform o world->grid" (9 FMAs), floor,
 //        block coordinates clamped to the always-empty border block (no bounds test, no branch),
 //        one bit of a multi-resolution occupancy bitmap held in shared memory; survivors (~35 %)
-//        are compacted, in model-point order, into a per-warp byte list;
+//        are compacted, in model-point order, into a per-warp byte list (top-K: a survivor mask);
 //     2. survivors only, 32 at a time: one bit of the per-brick bitmap, then -- occupied bricks
 //        only -- ONE 16-byte brick record of the eps-dilated voxel grid (64-bit occupancy mask +
 //        rank base); lanes whose cell is occupied are compacted (ballot + popc rank) into a
@@ -27,6 +27,10 @@
 //     LCP bit-identical to the reference's sequential fp32 sum.
 // All memory-dependent steps are batched 32 wide, so the latency chain
 // brick -> offsets -> candidates -> attributes is paid once per drain, not once per model point.
+// The top-K instantiation (kPrune) also skips every hypothesis whose LCP provably stays below a
+// value K other hypotheses of the launch reach: see prune_reject / prune_publish.
+#include <cstring>
+
 #include "stocs_ctx.h"
 
 using namespace stocsm;
@@ -73,6 +77,14 @@ struct ScoreArgs {
   unsigned long long* tie_counter;
   unsigned long long* cnt;   // counting variant only (stocs_b200_score_counters): see ScoreCounter
   const int* __restrict__ order;   // claim number -> hypothesis (heavy-first schedule, see probe_order_kernel) or NULL
+  // top-K pruning (kPrune only, see prune_publish): theta bucket + histogram of this launch, the
+  // context's two rejection counters, and the scene's bound constants
+  unsigned* prune;                 // [0] theta bucket, [kBucketBase..] per-bucket counts; zeroed with the work counter
+  unsigned long long* rejected;    // [0] after loop 1, [1] before a drain (accumulated over the context's lifetime)
+  float w_max;                     // largest class weight of the scene
+  float bound_scale;               // 1 + (M+2) 2^-23 (exact in fp32)
+  unsigned key_lo;                 // bucket b >= 1 holds LCPs whose bit pattern >> 19 equals key_lo + b
+  int K;
   long long H;
   const long long* __restrict__ H_dev;   // optional: the count lives on the device (H is then an upper bound)
   GridDesc g;
@@ -204,8 +216,15 @@ struct WarpQueue {   // one per warp, shared memory (single base register, const
 #else
   unsigned long long best[32];  // drain: min over hits of (d^2 bit pattern << 32 | scene index), atomicMin
 #endif
-  uint8_t plist[256];    // phase A: survivors of the coarse test within the current 256-point block
+  union {
+    uint8_t plist[256];  // phase A: survivors of the coarse test within the current 256-point block
+    uint32_t wincl[32];  // kPrune, loop 2: inclusive prefix of the survivor counts of a window of 32 mask words
+  };
+  float thr_M;           // kPrune: theta * M rounded down (0: nothing to reject against)
+  int later;             // kPrune: survivors in the windows after the current one
+  unsigned rej[2];       // kPrune: hypotheses this warp rejected after loop 1 / before a drain
 };
+// (after the WarpQueues, kPrune: one survivor mask of Mpad/32 words per warp, bit = coarse-test survivor)
 
 struct Acc { float acc; int inl; unsigned ties; };
 
@@ -388,7 +407,78 @@ __device__ __forceinline__ int claim_hypothesis(const ScoreArgs& a) {
   return a.order ? __ldg(a.order + c) : (int)c;
 }
 
-template <bool kCount>
+// position of the (r+1)-th set bit of w (r < popc(w))
+__device__ __forceinline__ unsigned nth_set_bit(unsigned w, unsigned r) {
+  unsigned pos = 0;
+#pragma unroll
+  for (int s = 16; s >= 1; s >>= 1) {
+    const unsigned c = __popc(w & ((1u << s) - 1u));
+    if (r >= c) { r -= c; w >>= s; pos += s; }
+  }
+  return pos;
+}
+
+// ---- Top-K pruning (kPrune: the caller receives nothing but the K best records) ----------------
+// Bound.  The LCP is fl(S/M), S the fp32 sequential sum of the weights of the matched model points.
+// When `acc` has been summed and at most n further weights, each in [0, w_max], can follow, then
+// S <= (acc + n w_max)(1 + u)^n and fl(S/M) <= (S/M)(1 + u), u = 2^-24; for n <= M <= 5120,
+// (1 + u)^(M+1) < 1 + (M+2) 2^-23 = bound_scale.  B below is evaluated with upward rounding, theta*M
+// with downward rounding, so  B < theta*M  =>  lcp < theta  STRICTLY.  theta is a value that at least
+// K fully scored hypotheses of this launch reach, so the hypothesis's key is below the K-th key and it
+// cannot enter the top K; a hypothesis that could tie theta is never rejected, so ties are still
+// decided by index.  theta > 0 whenever anything is rejected, and topk_kernel ignores lcp == 0, so the
+// 0 written for a rejected hypothesis never displaces a record.
+__device__ __forceinline__ bool prune_reject(const ScoreArgs& a, float acc, int n, float thr_M) {
+  const float B = __fmul_ru(__fmaf_ru((float)n, a.w_max, acc), a.bound_scale);
+  return B < thr_M;
+}
+
+// theta.  Buckets of the LCP's bit pattern >> 19 (16 per octave), the top one just above w_max, 8
+// octaves deep; anything lower is bucket 0, which is never counted.  Bucket b >= 1 holds only values
+// >= its lower edge, an exact float, so "K hypotheses counted in buckets >= b" means "K hypotheses
+// reach edge(b)".  prune[0] is the highest such b found so far: it only grows, every value it takes
+// is valid, and a warp that reads a stale one only rejects less.  (A per-CTA threshold would not do:
+// a CTA sees a few dozen strong hypotheses in the whole launch, its K-th arrives too late.)
+constexpr int kBuckets = 128;
+constexpr int kBucketBase = 32;   // prune[] index of bucket 0 (theta sits alone in the first 128 bytes)
+__device__ __forceinline__ float theta_M(const ScoreArgs& a, unsigned tb) {
+  return tb ? __fmul_rd(__uint_as_float((a.key_lo + tb) << 19), (float)a.M) : 0.f;
+}
+// the current theta bucket, read by lane 0 and broadcast: every lane takes the same branch on it even
+// when another warp raises theta meanwhile
+__device__ __forceinline__ unsigned theta_bucket(const ScoreArgs& a, int lane) {
+  return __reduce_max_sync(0xffffffffu, lane == 0 ? __ldcg(a.prune) : 0u);
+}
+__device__ __forceinline__ unsigned lcp_bucket(const ScoreArgs& a, float v) {
+  const unsigned k = __float_as_uint(v) >> 19;
+  return k <= a.key_lo ? 0u : min(k - a.key_lo, (unsigned)kBuckets - 1u);
+}
+// a fully scored hypothesis in bucket b (>= 1, >= tb, the theta bucket this warp read) counts itself,
+// then walks down from the top bucket, 32 buckets at a time, to the highest bucket that holds >= K
+__device__ __forceinline__ void prune_publish(const ScoreArgs& a, unsigned b, unsigned tb, int lane) {
+  unsigned* hist = a.prune + kBucketBase;
+  if (lane == 0) atomicAdd(hist + b, 1u);
+  __syncwarp();
+  unsigned cum = 0;
+  for (int top = kBuckets - 32; top >= 0 && (unsigned)(top + 31) > tb; top -= 32) {
+    unsigned s = __ldcg(hist + top + lane);
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {   // suffix sum: buckets >= top + lane
+      const unsigned dn = __shfl_down_sync(0xffffffffu, s, o);
+      if (lane + o < 32) s += dn;
+    }
+    s += cum;
+    const unsigned ok = __ballot_sync(0xffffffffu, s >= (unsigned)a.K);
+    if (ok) {
+      const unsigned nb = (unsigned)top + 31u - __clz(ok);
+      if (lane == 0 && nb > tb) atomicMax(a.prune, nb);
+      return;
+    }
+    cum = __shfl_sync(0xffffffffu, s, 0);
+  }
+}
+
+template <bool kCount, bool kPrune>
 __global__ void __launch_bounds__(kWarps * 32, SCORE_MIN_BLOCKS) score_lcp_kernel(ScoreArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   float* s_model = reinterpret_cast<float*>(smem_raw);
@@ -406,7 +496,10 @@ __global__ void __launch_bounds__(kWarps * 32, SCORE_MIN_BLOCKS) score_lcp_kerne
 #endif
   uint32_t* s_coarse = reinterpret_cast<uint32_t*>(s_model + kModelFloats * Mpad);   // Mpad % 64 == 0: 16-byte aligned
   for (int i = threadIdx.x; i < a.coarse_words; i += blockDim.x) s_coarse[i] = a.coarse[i];
-  WarpQueue& q = reinterpret_cast<WarpQueue*>(s_coarse + ((a.coarse_words + 3) & ~3))[warp];
+  WarpQueue* queues = reinterpret_cast<WarpQueue*>(s_coarse + ((a.coarse_words + 3) & ~3));
+  WarpQueue& q = queues[warp];
+  uint32_t* smask = reinterpret_cast<uint32_t*>(queues + kWarps) + warp * (Mpad >> 5);   // survivor mask
+  if (kPrune && lane == 0) { q.rej[0] = 0u; q.rej[1] = 0u; }
   __syncthreads();
 #ifndef SCORE_AOS
   ModelPts mp4; mp4.x = s_model; mp4.Mpad = Mpad;                // positions as x[] y[] z[] (NaN beyond M)
@@ -417,6 +510,7 @@ __global__ void __launch_bounds__(kWarps * 32, SCORE_MIN_BLOCKS) score_lcp_kerne
 
   const unsigned lt_mask = lanemask_lt();
   const int M = a.M;
+  const int nw = (M + 31) >> 5;   // survivor-mask words (32 model points each)
   // shared-window address of the coarse bitmap, made warp-uniform through redux so that it lives in a
   // uniform register for the whole kernel
   const unsigned coarse_sa = __reduce_max_sync(0xffffffffu, (unsigned)__cvta_generic_to_shared(s_coarse));
@@ -454,107 +548,192 @@ __global__ void __launch_bounds__(kWarps * 32, SCORE_MIN_BLOCKS) score_lcp_kerne
     r.acc = 0.f;
     r.inl = 0;
     int qn = 0;
-    // Phase A runs over blocks of 256 model points in two loops.  Loop 1 is the cheap test every
-    // point takes: fused affine map -> cell -> one bit of the shared-memory coarse occupancy map;
-    // the survivors' indices are compacted, in model-point order, into a byte list.  Loop 2 visits
-    // only the survivors, 32 at a time: brick record, exact cell bit, enqueue.  (Explicit FMAs: the
-    // map only selects a cell, the eps-dilation margin of the index absorbs its rounding; the exact
-    // point is recomputed for queued queries.  Float->int floor saturates; NaN -- padding points,
-    // rejected fits -- gives cell 0, whose queries find no candidate because every distance is NaN.)
-    for (int blk = 0; blk < M; blk += 256) {
-      int nl = 0;
-      const int rounds = min(8, (M - blk + 31) >> 5);
-      for (int rr = 0; rr < rounds; ++rr) {
-        const float4 mp = mp4[blk + rr * 32 + lane];
-        const float fx = __fmaf_rn(g0, mp.x, __fmaf_rn(g3, mp.y, __fmaf_rn(g6, mp.z, g9)));
-        const float fy = __fmaf_rn(g1, mp.x, __fmaf_rn(g4, mp.y, __fmaf_rn(g7, mp.z, g10)));
-        const float fz = __fmaf_rn(g2, mp.x, __fmaf_rn(g5, mp.y, __fmaf_rn(g8, mp.z, g11)));
-        const unsigned ix = (unsigned)__float2int_rd(fx), iy = (unsigned)__float2int_rd(fy), iz = (unsigned)__float2int_rd(fz);
-        // block coordinates clamped to the always-empty border block (index = number of real
-        // blocks): no bounds test, no branch; blocks left of the grid are huge as unsigned
-        const unsigned cx = min(ix, (unsigned)a.coarse_nx), cy = min(iy, (unsigned)a.coarse_ny),
-                       cz = min(iz, (unsigned)a.coarse_nz);
-        const uint32_t cidx = (cz * (unsigned)a.coarse_sy + cy) * (unsigned)a.coarse_sx + cx;
-        // The bitmap word is loaded through its shared-window address held in a uniform register, and
-        // the ballot is written in PTX on ONE predicate: as plain C++ the compiler re-derived the
-        // address (S2UR + UMOV + 2 ULEA) and a second predicate (ISETP) in every iteration -- 40 -> 35
-        // SASS instructions per 32 points (profiles/r02_score_loop1_sass.txt).
-        unsigned cw;
-        asm("ld.shared.u32 %0, [%1];" : "=r"(cw) : "r"(coarse_sa + ((cidx >> 5) << 2)));
-        const unsigned bitv = (cw >> (cidx & 31)) & 1u;
+    // Phase A, two loops.  Loop 1 is the cheap test every point takes: fused affine map -> cell -> one
+    // bit of the shared-memory coarse occupancy map.  Loop 2 visits only the survivors, 32 at a time in
+    // model-point order: brick record, exact cell bit, enqueue.  (Explicit FMAs: the map only selects a
+    // cell, the eps-dilation margin of the index absorbs its rounding; the exact point is recomputed
+    // for queued queries.  Float->int floor saturates; NaN -- padding points, rejected fits -- gives
+    // cell 0, whose queries find no candidate because every distance is NaN.)
+    // loop 1 for model points p .. p+31: this lane's bit, and the warp's ballot in pm
+    auto coarse_test = [&](int p, unsigned& pm) -> unsigned {
+      const float4 mp = mp4[p + lane];
+      const float fx = __fmaf_rn(g0, mp.x, __fmaf_rn(g3, mp.y, __fmaf_rn(g6, mp.z, g9)));
+      const float fy = __fmaf_rn(g1, mp.x, __fmaf_rn(g4, mp.y, __fmaf_rn(g7, mp.z, g10)));
+      const float fz = __fmaf_rn(g2, mp.x, __fmaf_rn(g5, mp.y, __fmaf_rn(g8, mp.z, g11)));
+      const unsigned ix = (unsigned)__float2int_rd(fx), iy = (unsigned)__float2int_rd(fy), iz = (unsigned)__float2int_rd(fz);
+      // block coordinates clamped to the always-empty border block (index = number of real
+      // blocks): no bounds test, no branch; blocks left of the grid are huge as unsigned
+      const unsigned cx = min(ix, (unsigned)a.coarse_nx), cy = min(iy, (unsigned)a.coarse_ny),
+                     cz = min(iz, (unsigned)a.coarse_nz);
+      const uint32_t cidx = (cz * (unsigned)a.coarse_sy + cy) * (unsigned)a.coarse_sx + cx;
+      // The bitmap word is loaded through its shared-window address held in a uniform register, and
+      // the ballot is written in PTX on ONE predicate: as plain C++ the compiler re-derived the
+      // address (S2UR + UMOV + 2 ULEA) and a second predicate (ISETP) in every iteration -- 40 -> 35
+      // SASS instructions per 32 points (profiles/r02_score_loop1_sass.txt).
+      unsigned cw;
+      asm("ld.shared.u32 %0, [%1];" : "=r"(cw) : "r"(coarse_sa + ((cidx >> 5) << 2)));
+      const unsigned bitv = (cw >> (cidx & 31)) & 1u;
+      asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %1, 0;\n\tvote.sync.ballot.b32 %0, p, 0xffffffff;\n\t}" : "=r"(pm) : "r"(bitv));
+      return bitv;
+    };
+    // loop 2 for the survivor model point i of this lane (valid lanes only); drains the queue when it
+    // passes kQueue - 32.  kPrune: false = rejected before that drain (`unvisited` survivors of the
+    // current window, and q.later of later windows, are still to come after this group)
+    auto visit = [&](int i, bool valid, int unvisited) -> bool {
+      const float4 mp = mp4[i];
+      const float fx = __fmaf_rn(g0, mp.x, __fmaf_rn(g3, mp.y, __fmaf_rn(g6, mp.z, g9)));
+      const float fy = __fmaf_rn(g1, mp.x, __fmaf_rn(g4, mp.y, __fmaf_rn(g7, mp.z, g10)));
+      const float fz = __fmaf_rn(g2, mp.x, __fmaf_rn(g5, mp.y, __fmaf_rn(g8, mp.z, g11)));
+      const unsigned ix = (unsigned)__float2int_rd(fx * a.to_cell), iy = (unsigned)__float2int_rd(fy * a.to_cell),
+                     iz = (unsigned)__float2int_rd(fz * a.to_cell);
+      uint4 br = make_uint4(0u, 0u, 0u, 0u);
+      const unsigned bidx = ((iz >> 2) * (unsigned)a.g.nby + (iy >> 2)) * (unsigned)a.g.nbx + (ix >> 2);
+#ifdef SCORE_BRICK_OCC
+      // second-level filter: 1 bit per brick (L2-resident, 1/128 of the brick table) before the
+      // 16 B brick record, which for an empty brick would be a wasted DRAM access
+      if (valid && ((__ldg(a.brick_occ + (bidx >> 5)) >> (bidx & 31u)) & 1u)) br = LD_BRICK(a.bricks + bidx);
+#else
+      if (valid) br = LD_BRICK(a.bricks + bidx);
+#endif
+      if (kCount) {
+#ifdef SCORE_BRICK_OCC
+        const bool fetched = valid && ((__ldg(a.brick_occ + (bidx >> 5)) >> (bidx & 31u)) & 1u);
+#else
+        const bool fetched = valid;
+#endif
+        count<kCount>(a, lane, SC_BRICK_RECORDS, __popc(__ballot_sync(0xffffffffu, fetched)));
+      }
+      const unsigned bit = ((iz & 3u) << 4) | ((iy & 3u) << 2) | (ix & 3u);
+      const unsigned half = (bit & 32u) ? br.y : br.x;      // 64-bit occupancy mask as two words
+      const bool has = (half >> (bit & 31u)) & 1u;
+      const unsigned hm = __ballot_sync(0xffffffffu, has);
+      if (hm) {
+        if (has) {
+          const int slot = qn + __popc(hm & lt_mask);
+          const unsigned below = __popc(half & ((1u << (bit & 31u)) - 1u)) + ((bit & 32u) ? __popc(br.x) : 0u);
+          q.a0[slot] = br.z + below;
+          q.pi[slot] = (uint32_t)i;
+        }
+        qn += __popc(hm);
+        count<kCount>(a, lane, SC_QUEUED, __popc(hm));
+      }
+      if (qn > kQueue - 32) {
+        // at most the queued queries and the survivors not yet visited can still add a weight
+        if (kPrune && prune_reject(a, r.acc, qn + q.later + max(unvisited, 0), q.thr_M)) return false;
+        // drain whole groups of 32 only; the (in-order) remainder stays at the front of the queue,
+        // so a hypothesis pays for a partly filled group once, at its end (S1 2.098 -> 2.082 ms,
+        // S1-fit 3.660 -> 3.611 ms)
+        const int full = qn & ~31;
+        drain_queue<kCount>(a, q, full, lane, mp4, mn4, r);
+        const int rem = qn - full;
+        uint32_t ca = 0, cp = 0;
+        if (lane < rem) { ca = q.a0[full + lane]; cp = q.pi[full + lane]; }
+        __syncwarp();
+        if (lane < rem) { q.a0[lane] = ca; q.pi[lane] = cp; }
+        __syncwarp();
+        qn = rem;
+        // the map is re-read after a drain so that it is not live (in registers) across it
+        gr0 = q.G[0]; gr1 = q.G[1]; gr2 = q.G[2];
+        g0 = gr0.x; g3 = gr0.y; g6 = gr0.z; g9 = gr0.w; g1 = gr1.x; g4 = gr1.y; g7 = gr1.z; g10 = gr1.w;
+        g2 = gr2.x; g5 = gr2.y; g8 = gr2.z; g11 = gr2.w;
+      }
+      return true;
+    };
+    if (!kPrune) {
+      // per block of 256 model points: loop 1 compacts the survivors' indices, in model-point order,
+      // into a per-warp byte list, loop 2 walks it
+      for (int blk = 0; blk < M; blk += 256) {
+        int nl = 0;
+        const int rounds = min(8, (M - blk + 31) >> 5);
+        for (int rr = 0; rr < rounds; ++rr) {
+          unsigned pm;
+          const bool pass = coarse_test(blk + rr * 32, pm) != 0u;
+          if (pass) q.plist[nl + __popc(pm & lt_mask)] = (uint8_t)(rr * 32 + lane);
+          nl += __popc(pm);
+        }
+        count<kCount>(a, lane, SC_SURVIVORS, (unsigned)nl);
+        __syncwarp();
+        for (int e0 = 0; e0 < nl; e0 += 32) {
+          const bool valid = e0 + lane < nl;
+          visit(blk + (valid ? (int)q.plist[e0 + lane] : 0), valid, 0);
+        }
+        __syncwarp();
+      }
+    } else {
+      // kPrune: loop 1 runs over the WHOLE model first, so that the survivor count is known before the
+      // first brick lookup; the ballot of every 32 points is one word of the warp's survivor mask
+      for (int rr = 0; rr < nw; ++rr) {
         unsigned pm;
-        asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.u32 p, %1, 0;\n\tvote.sync.ballot.b32 %0, p, 0xffffffff;\n\t}" : "=r"(pm) : "r"(bitv));
-        const bool pass = bitv != 0u;
-        if (pass) q.plist[nl + __popc(pm & lt_mask)] = (uint8_t)(rr * 32 + lane);
-        nl += __popc(pm);
+        coarse_test(rr * 32, pm);
+        if (lane == 0) smask[rr] = pm;
       }
-      count<kCount>(a, lane, SC_SURVIVORS, (unsigned)nl);
       __syncwarp();
-      for (int e0 = 0; e0 < nl; e0 += 32) {
-        const bool valid = e0 + lane < nl;
-        const int i = blk + (valid ? (int)q.plist[e0 + lane] : 0);
-        const float4 mp = mp4[i];
-        const float fx = __fmaf_rn(g0, mp.x, __fmaf_rn(g3, mp.y, __fmaf_rn(g6, mp.z, g9)));
-        const float fy = __fmaf_rn(g1, mp.x, __fmaf_rn(g4, mp.y, __fmaf_rn(g7, mp.z, g10)));
-        const float fz = __fmaf_rn(g2, mp.x, __fmaf_rn(g5, mp.y, __fmaf_rn(g8, mp.z, g11)));
-        const unsigned ix = (unsigned)__float2int_rd(fx * a.to_cell), iy = (unsigned)__float2int_rd(fy * a.to_cell),
-                       iz = (unsigned)__float2int_rd(fz * a.to_cell);
-        uint4 br = make_uint4(0u, 0u, 0u, 0u);
-        const unsigned bidx = ((iz >> 2) * (unsigned)a.g.nby + (iy >> 2)) * (unsigned)a.g.nbx + (ix >> 2);
-#ifdef SCORE_BRICK_OCC
-        // second-level filter: 1 bit per brick (L2-resident, 1/128 of the brick table) before the
-        // 16 B brick record, which for an empty brick would be a wasted DRAM access
-        if (valid && ((__ldg(a.brick_occ + (bidx >> 5)) >> (bidx & 31u)) & 1u)) br = LD_BRICK(a.bricks + bidx);
-#else
-        if (valid) br = LD_BRICK(a.bricks + bidx);
-#endif
-        if (kCount) {
-#ifdef SCORE_BRICK_OCC
-          const bool fetched = valid && ((__ldg(a.brick_occ + (bidx >> 5)) >> (bidx & 31u)) & 1u);
-#else
-          const bool fetched = valid;
-#endif
-          count<kCount>(a, lane, SC_BRICK_RECORDS, __popc(__ballot_sync(0xffffffffu, fetched)));
-        }
-        const unsigned bit = ((iz & 3u) << 4) | ((iy & 3u) << 2) | (ix & 3u);
-        const unsigned half = (bit & 32u) ? br.y : br.x;      // 64-bit occupancy mask as two words
-        const bool has = (half >> (bit & 31u)) & 1u;
-        const unsigned hm = __ballot_sync(0xffffffffu, has);
-        if (hm) {
-          if (has) {
-            const int slot = qn + __popc(hm & lt_mask);
-            const unsigned below = __popc(half & ((1u << (bit & 31u)) - 1u)) + ((bit & 32u) ? __popc(br.x) : 0u);
-            q.a0[slot] = br.z + below;
-            q.pi[slot] = (uint32_t)i;
+      unsigned ns = 0;   // survivors of the whole model
+      for (int j = 0; j < nw; j += 32) ns += j + lane < nw ? __popc(smask[j + lane]) : 0u;
+      ns = __reduce_add_sync(0xffffffffu, ns);
+      const float thr = theta_M(a, theta_bucket(a, lane));
+      if (prune_reject(a, 0.f, (int)ns, thr)) {
+        if (lane == 0) q.rej[0]++;
+        goto rejected;
+      }
+      if (lane == 0) { q.thr_M = thr; q.later = (int)ns; }
+      __syncwarp();
+      // loop 2 over windows of 32 mask words (1024 model points)
+      for (int wb = 0; wb < nw; wb += 32) {
+        {  // inclusive prefix of the window's survivor counts
+          unsigned s = wb + lane < nw ? __popc(smask[wb + lane]) : 0u;
+#pragma unroll
+          for (int o = 1; o < 32; o <<= 1) {
+            const unsigned up = __shfl_up_sync(0xffffffffu, s, o);
+            if (lane >= o) s += up;
           }
-          qn += __popc(hm);
-          count<kCount>(a, lane, SC_QUEUED, __popc(hm));
+          q.wincl[lane] = s;
+          if (lane == 31) q.later -= (int)s;   // survivors in later windows
         }
-        if (qn > kQueue - 32) {
-          // drain whole groups of 32 only; the (in-order) remainder stays at the front of the queue,
-          // so a hypothesis pays for a partly filled group once, at its end (S1 2.098 -> 2.082 ms,
-          // S1-fit 3.660 -> 3.611 ms)
-          const int full = qn & ~31;
-          drain_queue<kCount>(a, q, full, lane, mp4, mn4, r);
-          const int rem = qn - full;
-          uint32_t ca = 0, cp = 0;
-          if (lane < rem) { ca = q.a0[full + lane]; cp = q.pi[full + lane]; }
-          __syncwarp();
-          if (lane < rem) { q.a0[lane] = ca; q.pi[lane] = cp; }
-          __syncwarp();
-          qn = rem;
-          // the map is re-read after a drain so that it is not live (in registers) across it
-          gr0 = q.G[0]; gr1 = q.G[1]; gr2 = q.G[2];
-          g0 = gr0.x; g3 = gr0.y; g6 = gr0.z; g9 = gr0.w; g1 = gr1.x; g4 = gr1.y; g7 = gr1.z; g10 = gr1.w;
-          g2 = gr2.x; g5 = gr2.y; g8 = gr2.z; g11 = gr2.w;
+        __syncwarp();
+        const int wn = (int)q.wincl[31];
+        for (int e0 = 0; e0 < wn; e0 += 32) {
+          // survivor k of the window: its word is the first whose inclusive prefix exceeds k
+          const bool valid = e0 + lane < wn;
+          const unsigned k = (unsigned)min(e0 + lane, wn - 1);
+          unsigned wj = 0;
+#pragma unroll
+          for (int st = 16; st >= 1; st >>= 1)
+            if (q.wincl[wj + st - 1] <= k) wj += st;
+          const unsigned word = smask[wb + wj];
+          const int i = valid ? (int)((wb + wj) * 32u + nth_set_bit(word, k - (q.wincl[wj] - __popc(word)))) : 0;
+          if (!visit(i, valid, wn - e0 - 32)) {
+            if (lane == 0) q.rej[1]++;
+            goto rejected;
+          }
         }
+        __syncwarp();
       }
-      __syncwarp();
     }
-    if (qn > 0) drain_queue<kCount>(a, q, qn, lane, mp4, mn4, r);
-    if (lane == 0) {
-      a.lcp[h] = r.acc / (float)M;
-      if (a.inl) a.inl[h] = r.inl;
+    if (qn > 0) {
+      if (kPrune && prune_reject(a, r.acc, qn, q.thr_M)) {
+        if (lane == 0) q.rej[1]++;
+        goto rejected;
+      }
+      drain_queue<kCount>(a, q, qn, lane, mp4, mn4, r);
+    }
+    {
+      const float v = r.acc / (float)M;
+      if (lane == 0) {
+        a.lcp[h] = v;
+        if (a.inl) a.inl[h] = r.inl;
+      }
+      if (kPrune) {
+        const unsigned b = lcp_bucket(a, v), tb = theta_bucket(a, lane);
+        if (b != 0u && b >= tb) prune_publish(a, b, tb, lane);
+      }
+    }
+    if (false) {
+    rejected:   // (kPrune only) lcp 0: topk_kernel never selects it
+      if (lane == 0) {
+        a.lcp[h] = 0.f;
+        if (a.inl) a.inl[h] = 0;
+      }
     }
     h = 0;
     if (lane == 0) h = claim_hypothesis(a);
@@ -562,6 +741,10 @@ __global__ void __launch_bounds__(kWarps * 32, SCORE_MIN_BLOCKS) score_lcp_kerne
     __syncwarp();
   }
   if (r.ties) atomicAdd(a.tie_counter, (unsigned long long)r.ties);
+  if (kPrune && lane == 0) {
+    if (q.rej[0]) atomicAdd(a.rejected, (unsigned long long)q.rej[0]);
+    if (q.rej[1]) atomicAdd(a.rejected + 1, (unsigned long long)q.rej[1]);
+  }
 }
 
 // Heavy-first schedule.  The cost of a hypothesis varies by an order of magnitude (a pose that lands
@@ -644,7 +827,7 @@ bool stocs_fmad_selftest(stocs_b200_ctx* ctx) {
 
 int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl,
                        cudaStream_t st, bool time_it, int slot, unsigned long long* d_counters, bool T_in_host_memory,
-                       const long long* d_H, long long grid_hint) {
+                       const long long* d_H, long long grid_hint, int prune_K) {
   if (H <= 0) return STOCS_OK;
   if (H >= (1ll << 31)) STOCS_FAIL(ctx, STOCS_E_ARG, "score: at most 2^31-1 hypotheses per call");
   // the kd-tree of a freshly uploaded scene may still be under construction on a host thread: collect
@@ -683,10 +866,33 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   a.dot_thr = ctx->dot_thr;
   a.to_block = 1.0f / (float)(1u << ctx->coarse_shift);
   a.to_cell = (float)(1u << ctx->coarse_shift);
-  size_t smem = (size_t)kModelFloats * ctx->Mpad * 4 + (size_t)((a.coarse_words + 3) & ~3) * 4 + (size_t)kWarps * sizeof(WarpQueue);
+  // top-K pruning: only for a caller that receives nothing but the K best records (prune_K = K), and
+  // only on a scene whose class weights are all finite and >= 0 (the bound needs w_max)
+  // (and with the lowest bucket edge a normal float, see lcp_bucket)
+  unsigned wbits;
+  memcpy(&wbits, &ctx->w_max, 4);
+  const int key_lo = (int)(wbits >> 19) + 1 - (kBuckets - 1);
+  const bool prune = prune_K > 0 && ctx->prune_ok && key_lo >= 16 && !d_counters && !d_H && slot == 0;
+  a.prune = nullptr;
+  a.rejected = (unsigned long long*)(ctx->d_small.as<char>() + 208);
+  a.w_max = ctx->w_max;
+  a.bound_scale = 1.0f + (float)(ctx->M + 2) * 0x1p-23f;   // exact: M + 2 < 2^13
+  a.key_lo = (unsigned)key_lo;
+  a.K = prune_K;
+  if (prune) {
+    // [0, 8) work counter, [128, 132) theta bucket, [256, 768) bucket counts: one memset per launch
+    DevBuf& b = ctx->pool[POOL_SCORE_PRUNE];
+    STOCS_CUDA(ctx, b.ensure(256 + kBuckets * 4));
+    wctr = b.as<unsigned long long>();
+    a.work_counter = wctr;
+    a.prune = (unsigned*)(b.as<char>() + 128);
+  }
+  size_t smem = (size_t)kModelFloats * ctx->Mpad * 4 + (size_t)((a.coarse_words + 3) & ~3) * 4 +
+                (size_t)kWarps * (sizeof(WarpQueue) + (prune ? (size_t)(ctx->Mpad / 32) * 4 : 0));   // + survivor masks
   // static (per-warp queues) + dynamic (model, coarse bitmap) may exceed the 48 KB default
   // d_counters != NULL selects the counting variant (same code + one global atomic per warp event)
-  void (*kernel)(ScoreArgs) = d_counters ? score_lcp_kernel<true> : score_lcp_kernel<false>;
+  void (*kernel)(ScoreArgs) = d_counters ? score_lcp_kernel<true, false>
+                                         : (prune ? score_lcp_kernel<false, true> : score_lcp_kernel<false, false>);
   STOCS_CUDA(ctx, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   STOCS_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kWarps * 32, smem));
@@ -694,7 +900,7 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   long long want = ((d_H && grid_hint > 0 && grid_hint < H ? grid_hint : H) + kWarps - 1) / kWarps;
   long long grid = (long long)ctx->num_sms * per_sm;
   if (grid > want) grid = want;
-  STOCS_CUDA(ctx, cudaMemsetAsync(wctr, 0, 8, st));  // work counter only; tie counter accumulates
+  STOCS_CUDA(ctx, cudaMemsetAsync(wctr, 0, prune ? 256 + kBuckets * 4 : 8, st));  // tie counter accumulates
   // Heavy-first schedule for MID-SIZE launches only.  Measured on B200 (S1 hypotheses, kernel + probe):
   // 125 000 hypotheses (the per-GPU share of the named config on 8 GPUs) 0.347 -> 0.312 ms; 10^6
   // hypotheses 2.100 -> 2.139 ms (the probe costs 64 us per 10^6, the tail it removes is ~0.09 ms

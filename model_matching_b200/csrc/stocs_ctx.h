@@ -93,6 +93,8 @@ enum PoolSlot : int {
   POOL_CONG_CONE = 50,
   // congruent.cu: bucket number of every Q entry; bucket starts; {Q index, cell} records in bucket order
   POOL_CONG_NEXT = 51, POOL_CONG_BSTART = 52, POOL_CONG_BUCKET = 53,
+  // score.cu: work counter, theta and bucket counts of a top-K-pruned scoring launch
+  POOL_SCORE_PRUNE = 54,
   POOL_COUNT = 56
 };
 
@@ -160,6 +162,8 @@ struct stocs_b200_ctx {
   DevBuf d_edge, d_inst_state, d_mask_store, d_frontier;
   int img_w = 0, img_h = 0;
   GridDesc grid{};
+  float w_max = 0.f;                   // largest class weight of the scene (top-K pruning bound, score.cu)
+  bool prune_ok = false;               // every class weight finite and >= 0: top-K pruning allowed
   DevBuf d_brick_occ;                  // 1 bit per brick: brick has an occupied cell
   DevBuf d_coarse;                     // 1 bit per block of 2^coarse_shift cells/axis (>= brick): block has an occupied cell
   int coarse_shift = 2, coarse_nx = 0, coarse_ny = 0, coarse_nz = 0, coarse_words = 0;
@@ -238,8 +242,9 @@ int stocs_pack_scene_attr(stocs_b200_ctx* ctx, const float* d_nrm3, const float*
 int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp,
                        int32_t* d_inl, cudaStream_t st, bool time_it, int slot = 0,
                        unsigned long long* d_counters = nullptr, bool T_in_host_memory = false,
-                       const long long* d_H = nullptr, long long grid_hint = 0);  // score.cu (d_H: the count lives on
-                                                                                  // the device, H bounds it, grid_hint sizes the launch)
+                       const long long* d_H = nullptr, long long grid_hint = 0,
+                       int prune_K = 0);  // score.cu (d_H: the count lives on the device, H bounds it, grid_hint sizes
+                                          // the launch; prune_K > 0: only the K best will be read, see kPrune)
 int stocs_launch_backproject(stocs_b200_ctx* ctx, const uint16_t* d_depth, const uint8_t* d_bgr,
                              int W, int H, float fx, float cx, float fy, float cy, float scale,
                              float* d_xyz, uint32_t* d_rgb, cudaStream_t st);  // backproject.cu
@@ -247,6 +252,8 @@ int stocs_launch_backproject(stocs_b200_ctx* ctx, const uint16_t* d_depth, const
 int stocs_kd_finish(stocs_b200_ctx* ctx, cudaStream_t st, bool upload = true);  // scene_index.cu
 bool stocs_fmad_selftest(stocs_b200_ctx* ctx);                             // score.cu
 bool stocs_is_host_memory(const void* p);                                  // capi.cu
+// w_max / prune_ok of the scene from its class weights (capi.cu; every writer of the weights calls it)
+void stocs_set_weight_bound(stocs_b200_ctx* ctx, const float* cls, int S);
 // top-K of a device lcp array (reduce.cu); d_idx/d_val may be NULL when only records are wanted
 int stocs_launch_topk(stocs_b200_ctx* ctx, const float* d_lcp, int64_t H, int K, int64_t index_offset,
                       int64_t* d_idx, float* d_val, cudaStream_t st, const float* d_T16 = nullptr,
