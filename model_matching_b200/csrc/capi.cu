@@ -26,12 +26,19 @@ float stocs_angle_threshold_dot() {
 
 static thread_local std::string g_create_err;
 
-// a "device pointer" handed to the *_device entry points may be page-locked host memory mapped into
-// the device address space (the zero-copy path): such transforms must not be read twice
-bool stocs_is_host_memory(const void* p) {
+// Page-locked host memory (cudaHostAlloc / cudaHostRegister, e.g. a pinned torch tensor) is mapped
+// into the device address space; this is its device alias, NULL for any other pointer.
+const void* stocs_host_alias(const void* p) {
   cudaPointerAttributes pa{};
-  if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) { cudaGetLastError(); return false; }
-  return pa.type == cudaMemoryTypeHost;
+  if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) { cudaGetLastError(); return nullptr; }
+  return pa.type == cudaMemoryTypeHost ? pa.devicePointer : nullptr;
+}
+
+// The host-buffer scoring calls read page-locked transforms in place through their device alias;
+// NULL: stage them through HBM (pageable memory, or STOCS_NO_ZERO_COPY set).
+const float* stocs_zero_copy_transforms(const float* T16) {
+  if (getenv("STOCS_NO_ZERO_COPY")) return nullptr;
+  return (const float*)stocs_host_alias(T16);
 }
 
 // Largest class weight of the scene.  The top-K pruning bound of the scoring kernel (score.cu) needs
@@ -286,7 +293,7 @@ int stocs_b200_score_lcp_device(stocs_b200_ctx* ctx, const float* d_T16, int64_t
   if (H < 0 || (H > 0 && (!d_T16 || !d_lcp))) STOCS_FAIL(ctx, STOCS_E_ARG, "score_lcp: bad argument");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-  return stocs_launch_score(ctx, d_T16, H, d_lcp, d_inliers, st, true, 0, nullptr, H > 0 && stocs_is_host_memory(d_T16));
+  return stocs_launch_score(ctx, d_T16, H, d_lcp, d_inliers, st, true, 0, nullptr, H > 0 && stocs_host_alias(d_T16));
 }
 
 // Top-32 of the resident lcp array into the page-locked cache, on stream st (no synchronize).
@@ -319,35 +326,29 @@ int stocs_b200_score_lcp(stocs_b200_ctx* ctx, const float* T16, int64_t H, float
   // hypothesis is trivially rejected the reads become the bound (1.56 ms per 10^6, 41 GB/s), still
   // no slower than the staged path.  Results are written to HBM and copied back once: letting the
   // kernel also write to host memory puts its reads behind the posted writes (3.98 ms).
-  {
-    cudaPointerAttributes pa{};
-    const bool mapped = cudaPointerGetAttributes(&pa, T16) == cudaSuccess && pa.type == cudaMemoryTypeHost &&
-                        pa.devicePointer != nullptr;
-    if (!mapped) cudaGetLastError();
-    if (mapped && !getenv("STOCS_NO_ZERO_COPY")) {
-      int rc = stocs_launch_score(ctx, (const float*)pa.devicePointer, H, ctx->d_lcp.as<float>(),
-                                  ctx->d_inl.as<int32_t>(), ctx->stream, true, 0, nullptr, /*T_in_host_memory=*/true);
-      if (rc != STOCS_OK) return rc;
-      ctx->last_T_dev = (const float*)pa.devicePointer;
-      // the top-32 reduction (what stocs_b200_reduce_best returns for the resident array) runs on
-      // the second stream while the copy engine returns the results
-      cudaError_t e = cudaEventRecord(ctx->join_ev[0], ctx->stream);
-      if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->aux_stream, ctx->join_ev[0], 0);
-      if (e == cudaSuccess) e = cudaMemcpyAsync(lcp, ctx->d_lcp.p, (size_t)H * 4, cudaMemcpyDeviceToHost, ctx->stream);
-      if (e == cudaSuccess && inliers)
-        e = cudaMemcpyAsync(inliers, ctx->d_inl.p, (size_t)H * 4, cudaMemcpyDeviceToHost, ctx->stream);
-      if (e == cudaSuccess) rc = enqueue_resident_topk(ctx, H, ctx->aux_stream);
-      cudaError_t e2 = cudaEventRecord(ctx->join_ev[1], ctx->aux_stream);
-      if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(ctx->stream, ctx->join_ev[1], 0);
-      if (e == cudaSuccess) e = e2;
-      e2 = cudaStreamSynchronize(ctx->stream);
-      if (e == cudaSuccess) e = e2;
-      if (e != cudaSuccess) { ctx->err = std::string("score_lcp: ") + cudaGetErrorString(e); return STOCS_E_CUDA; }
-      if (rc != STOCS_OK) return rc;
-      ctx->last_H = H;
-      ctx->top_valid = true;
-      return STOCS_OK;
-    }
+  if (const float* d_T = stocs_zero_copy_transforms(T16)) {
+    int rc = stocs_launch_score(ctx, d_T, H, ctx->d_lcp.as<float>(), ctx->d_inl.as<int32_t>(), ctx->stream, true, 0,
+                                nullptr, /*T_in_host_memory=*/true);
+    if (rc != STOCS_OK) return rc;
+    ctx->last_T_dev = d_T;
+    // the top-32 reduction (what stocs_b200_reduce_best returns for the resident array) runs on
+    // the second stream while the copy engine returns the results
+    cudaError_t e = cudaEventRecord(ctx->join_ev[0], ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->aux_stream, ctx->join_ev[0], 0);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(lcp, ctx->d_lcp.p, (size_t)H * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess && inliers)
+      e = cudaMemcpyAsync(inliers, ctx->d_inl.p, (size_t)H * 4, cudaMemcpyDeviceToHost, ctx->stream);
+    if (e == cudaSuccess) rc = enqueue_resident_topk(ctx, H, ctx->aux_stream);
+    cudaError_t e2 = cudaEventRecord(ctx->join_ev[1], ctx->aux_stream);
+    if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(ctx->stream, ctx->join_ev[1], 0);
+    if (e == cudaSuccess) e = e2;
+    e2 = cudaStreamSynchronize(ctx->stream);
+    if (e == cudaSuccess) e = e2;
+    if (e != cudaSuccess) { ctx->err = std::string("score_lcp: ") + cudaGetErrorString(e); return STOCS_E_CUDA; }
+    if (rc != STOCS_OK) return rc;
+    ctx->last_H = H;
+    ctx->top_valid = true;
+    return STOCS_OK;
   }
   // Pageable transforms are staged through HBM in chunks:
   STOCS_CUDA(ctx, ctx->d_T.ensure((size_t)H * 64));
@@ -360,13 +361,8 @@ int stocs_b200_score_lcp(stocs_b200_ctx* ctx, const float* T16, int64_t H, float
   // own stream behind its kernel.  (H2D from pageable memory is staged by the driver through its
   // own pinned buffer and returns early; D2H into pageable memory does not -- see below.)
   std::vector<int64_t> bounds;
-  int nequal = 0;
-  if (const char* e = getenv("STOCS_SCORE_CHUNKS")) nequal = atoi(e);
-  if (nequal > stocs_b200_ctx::kMaxChunks) nequal = stocs_b200_ctx::kMaxChunks;
-  if (H <= (1 << 16) || nequal == 1) {
+  if (H <= (1 << 16)) {
     bounds = {0, H};
-  } else if (nequal > 1) {
-    for (int c = 0; c <= nequal; ++c) bounds.push_back(H * c / nequal);
   } else {
     const int64_t e8 = (H + 7) / 8;
     bounds = {0, e8, 2 * e8, 4 * e8, H};
@@ -475,15 +471,15 @@ int stocs_b200_reduce_best(stocs_b200_ctx* ctx, const float* lcp, int64_t H, int
 int stocs_b200_get_counters(stocs_b200_ctx* ctx, int64_t* counters, int n) {
   if (!ctx || !counters) return STOCS_E_ARG;
   cudaSetDevice(ctx->device);
-  if (ctx->d_small.p) {   // tie counter at 200, top-K rejections at 208 and 216 (score.cu)
-    unsigned long long t[3] = {0, 0, 0};
+  if (ctx->d_small.p) {
+    DevScratch::ScoreTotals t{};
     STOCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    STOCS_CUDA(ctx, cudaMemcpy(t, ctx->d_small.as<char>() + 200, 24, cudaMemcpyDeviceToHost));
-    ctx->counters[1] = (int64_t)t[0];
-    ctx->counters[4] = (int64_t)t[1];
-    ctx->counters[5] = (int64_t)t[2];
+    STOCS_CUDA(ctx, cudaMemcpy(&t, &ctx->scratch()->score_totals, sizeof(t), cudaMemcpyDeviceToHost));
+    ctx->counters[CTR_TIES] = (int64_t)t.ties;
+    ctx->counters[CTR_REJECTED_LOOP1] = (int64_t)t.rejected[0];
+    ctx->counters[CTR_REJECTED_DRAIN] = (int64_t)t.rejected[1];
   }
-  for (int i = 0; i < n && i < 8; ++i) counters[i] = ctx->counters[i];
+  for (int i = 0; i < n && i < CTR_COUNT; ++i) counters[i] = ctx->counters[i];
   return STOCS_OK;
 }
 
@@ -497,12 +493,12 @@ int stocs_b200_score_counters(stocs_b200_ctx* ctx, const float* d_T16, int64_t H
   DevBuf &d_lcp = ctx->pool[POOL_SHARD_LCP], &d_inl = ctx->pool[POOL_SHARD_INL];
   STOCS_CUDA(ctx, d_lcp.ensure((size_t)H * 4));
   STOCS_CUDA(ctx, d_inl.ensure((size_t)H * 4));
-  unsigned long long* d_cnt = (unsigned long long*)(ctx->d_small.as<char>() + 3072);
-  STOCS_CUDA(ctx, cudaMemsetAsync(d_cnt, 0, 128, st));
+  unsigned long long* d_cnt = ctx->scratch()->score_counts;
+  unsigned long long h[sizeof(DevScratch::score_counts) / 8] = {0};
+  STOCS_CUDA(ctx, cudaMemsetAsync(d_cnt, 0, sizeof(h), st));
   int rc = stocs_launch_score(ctx, d_T16, H, d_lcp.as<float>(), d_inl.as<int32_t>(), st, false, 0, d_cnt);
   if (rc) return rc;
-  unsigned long long h[16] = {0};
-  STOCS_CUDA(ctx, cudaMemcpyAsync(h, d_cnt, 128, cudaMemcpyDeviceToHost, st));
+  STOCS_CUDA(ctx, cudaMemcpyAsync(h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
   STOCS_CUDA(ctx, cudaStreamSynchronize(st));
   int64_t out[9] = {H * (int64_t)ctx->M, (int64_t)h[0], (int64_t)h[1], (int64_t)h[2], (int64_t)h[3],
                     (int64_t)h[4], (int64_t)h[5], (int64_t)h[6], H};

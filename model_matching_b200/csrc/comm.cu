@@ -125,12 +125,33 @@ __global__ void __launch_bounds__(1024) merge_records_kernel(const stocs_b200_re
 int enqueue_local_topk(stocs_b200_ctx* ctx, const float* d_T, int64_t H_local, int64_t index_offset, int K,
                        float* d_lcp, int32_t* d_inl, stocs_b200_record* d_send, cudaStream_t st, bool time_it, bool prune) {
   if (H_local > 0) {
-    int rc = stocs_launch_score(ctx, d_T, H_local, d_lcp, d_inl, st, time_it, 0, nullptr, stocs_is_host_memory(d_T),
+    int rc = stocs_launch_score(ctx, d_T, H_local, d_lcp, d_inl, st, time_it, 0, nullptr, stocs_host_alias(d_T) != nullptr,
                                 nullptr, 0, prune ? K : 0);
     if (rc) return rc;
   }
   // H_local == 0: the top-K kernels run over an empty array and emit K empty records
   return stocs_launch_topk(ctx, d_lcp, H_local, K, index_offset, nullptr, nullptr, st, d_T, d_inl, d_send);
+}
+
+// the buffers of the collective: K local records (POOL_COMM_SEND), nranks*K gathered records
+// (POOL_COMM_RECV) and K merged records (POOL_COMM_OUT)
+cudaError_t ensure_record_buffers(stocs_b200_ctx* ctx, int K, int nranks) {
+  const size_t rec_bytes = (size_t)K * sizeof(stocs_b200_record);
+  cudaError_t e = ctx->pool[POOL_COMM_SEND].ensure(rec_bytes);
+  if (e == cudaSuccess) e = ctx->pool[POOL_COMM_RECV].ensure(rec_bytes * nranks);
+  if (e == cudaSuccess) e = ctx->pool[POOL_COMM_OUT].ensure(rec_bytes);
+  return e;
+}
+
+// ONE all-gather of the K records every rank left in POOL_COMM_SEND, then their merge into `out`
+// (K records), on stream st
+int gather_merge_records(stocs_b200_ctx* ctx, int K, stocs_b200_record* out, cudaStream_t st) {
+  DevBuf &b_send = ctx->pool[POOL_COMM_SEND], &b_recv = ctx->pool[POOL_COMM_RECV];
+  STOCS_NCCL(ctx, g_nccl.AllGather(b_send.p, b_recv.p, (size_t)K * sizeof(stocs_b200_record), ncclInt8,
+                                   (ncclComm_t)ctx->comm, st));
+  merge_records_kernel<<<1, 1024, 0, st>>>(b_recv.as<stocs_b200_record>(), K * ctx->comm_nranks, K, out);
+  STOCS_CUDA(ctx, cudaGetLastError());
+  return STOCS_OK;
 }
 
 }  // namespace
@@ -197,24 +218,17 @@ int stocs_b200_score_sharded_device(stocs_b200_ctx* ctx, const float* d_T16_loca
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
   DevBuf &b_lcp = ctx->pool[POOL_SHARD_LCP], &b_inl = ctx->pool[POOL_SHARD_INL];
-  DevBuf &b_send = ctx->pool[POOL_COMM_SEND], &b_recv = ctx->pool[POOL_COMM_RECV];
   STOCS_CUDA(ctx, b_lcp.ensure((size_t)(H_local ? H_local : 1) * 4));
   STOCS_CUDA(ctx, b_inl.ensure((size_t)(H_local ? H_local : 1) * 4));
   const int nranks = ctx->comm ? ctx->comm_nranks : 1;
   if (nranks == 1)  // no collective: the local top-K is the global one
     return enqueue_local_topk(ctx, d_T16_local, H_local, index_offset, K, b_lcp.as<float>(), b_inl.as<int32_t>(),
                               d_topk_out, st, true, true);
-  STOCS_CUDA(ctx, b_send.ensure((size_t)K * sizeof(stocs_b200_record)));
-  STOCS_CUDA(ctx, b_recv.ensure((size_t)K * nranks * sizeof(stocs_b200_record)));
+  STOCS_CUDA(ctx, ensure_record_buffers(ctx, K, nranks));
   int rc = enqueue_local_topk(ctx, d_T16_local, H_local, index_offset, K, b_lcp.as<float>(), b_inl.as<int32_t>(),
-                              b_send.as<stocs_b200_record>(), st, true, true);
+                              ctx->pool[POOL_COMM_SEND].as<stocs_b200_record>(), st, true, true);
   if (rc) return rc;
-  // the path's one collective
-  STOCS_NCCL(ctx, g_nccl.AllGather(b_send.p, b_recv.p, (size_t)K * sizeof(stocs_b200_record), ncclInt8,
-                                   (ncclComm_t)ctx->comm, st));
-  merge_records_kernel<<<1, 1024, 0, st>>>(b_recv.as<stocs_b200_record>(), K * nranks, K, d_topk_out);
-  STOCS_CUDA(ctx, cudaGetLastError());
-  return STOCS_OK;
+  return gather_merge_records(ctx, K, d_topk_out, st);
 }
 
 int stocs_b200_score_sharded(stocs_b200_ctx* ctx, const float* T16_local, int64_t H_local, int64_t index_offset, int K,
@@ -238,51 +252,38 @@ int stocs_b200_score_sharded(stocs_b200_ctx* ctx, const float* T16_local, int64_
     lcp_local = (float*)ctx->h_pinned;
   }
   const int nranks = ctx->comm ? ctx->comm_nranks : 1;
-  DevBuf &b_send = ctx->pool[POOL_COMM_SEND], &b_recv = ctx->pool[POOL_COMM_RECV], &b_out = ctx->pool[POOL_COMM_OUT];
-  STOCS_CUDA(ctx, b_send.ensure((size_t)K * sizeof(stocs_b200_record)));
-  STOCS_CUDA(ctx, b_recv.ensure((size_t)K * nranks * sizeof(stocs_b200_record)));
-  STOCS_CUDA(ctx, b_out.ensure((size_t)K * sizeof(stocs_b200_record)));
-  stocs_b200_record* d_local = nranks > 1 ? b_send.as<stocs_b200_record>() : b_out.as<stocs_b200_record>();
+  STOCS_CUDA(ctx, ensure_record_buffers(ctx, K, nranks));
+  DevBuf& b_out = ctx->pool[POOL_COMM_OUT];
+  stocs_b200_record* d_local = nranks > 1 ? ctx->pool[POOL_COMM_SEND].as<stocs_b200_record>() : b_out.as<stocs_b200_record>();
   // Page-locked, device-mapped transforms: ONE pass with ONE synchronisation.  The kernel reads the
   // transforms in place over PCIe; then the per-hypothesis results go back on the context stream
   // while, on the second stream, the K best are packed, all-gathered and merged.  (Going through
   // stocs_b200_score_lcp first costs its own top-32 reduction and a second synchronisation:
   // 0.58 -> 0.50 ms per step at 125 000 hypotheses per rank on 8 GPUs.)
-  if (H_local > 0 && !getenv("STOCS_NO_ZERO_COPY")) {
-    cudaPointerAttributes pa{};
-    const bool mapped = cudaPointerGetAttributes(&pa, T16_local) == cudaSuccess && pa.type == cudaMemoryTypeHost &&
-                        pa.devicePointer != nullptr;
-    if (!mapped) cudaGetLastError();
-    if (mapped) {
-      const float* d_T = (const float*)pa.devicePointer;
-      STOCS_CUDA(ctx, ctx->d_lcp.ensure((size_t)H_local * 4));
-      STOCS_CUDA(ctx, ctx->d_inl.ensure((size_t)H_local * 4));
-      ctx->top_valid = false;
-      int rc = stocs_launch_score(ctx, d_T, H_local, ctx->d_lcp.as<float>(), ctx->d_inl.as<int32_t>(), st, true, 0, nullptr, true);
-      if (rc) return rc;
-      ctx->last_H = H_local;
-      ctx->last_T_dev = d_T;
-      cudaStream_t aux = ctx->aux_stream;
-      STOCS_CUDA(ctx, cudaEventRecord(ctx->join_ev[0], st));
-      STOCS_CUDA(ctx, cudaStreamWaitEvent(aux, ctx->join_ev[0], 0));
-      STOCS_CUDA(ctx, cudaMemcpyAsync(lcp_local, ctx->d_lcp.p, (size_t)H_local * 4, cudaMemcpyDeviceToHost, st));
-      if (inliers_local)
-        STOCS_CUDA(ctx, cudaMemcpyAsync(inliers_local, ctx->d_inl.p, (size_t)H_local * 4, cudaMemcpyDeviceToHost, st));
-      rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H_local, K, index_offset, nullptr, nullptr, aux, d_T,
-                             ctx->d_inl.as<int32_t>(), d_local);
-      if (rc) return rc;
-      if (nranks > 1) {
-        STOCS_NCCL(ctx, g_nccl.AllGather(b_send.p, b_recv.p, (size_t)K * sizeof(stocs_b200_record), ncclInt8,
-                                         (ncclComm_t)ctx->comm, aux));
-        merge_records_kernel<<<1, 1024, 0, aux>>>(b_recv.as<stocs_b200_record>(), K * nranks, K, b_out.as<stocs_b200_record>());
-        STOCS_CUDA(ctx, cudaGetLastError());
-      }
-      STOCS_CUDA(ctx, cudaMemcpyAsync(topk_out, b_out.p, (size_t)K * sizeof(stocs_b200_record), cudaMemcpyDeviceToHost, aux));
-      STOCS_CUDA(ctx, cudaEventRecord(ctx->join_ev[1], aux));
-      STOCS_CUDA(ctx, cudaStreamWaitEvent(st, ctx->join_ev[1], 0));
-      STOCS_CUDA(ctx, cudaStreamSynchronize(st));
-      return STOCS_OK;
-    }
+  if (const float* d_T = H_local > 0 ? stocs_zero_copy_transforms(T16_local) : nullptr) {
+    STOCS_CUDA(ctx, ctx->d_lcp.ensure((size_t)H_local * 4));
+    STOCS_CUDA(ctx, ctx->d_inl.ensure((size_t)H_local * 4));
+    ctx->top_valid = false;
+    int rc = stocs_launch_score(ctx, d_T, H_local, ctx->d_lcp.as<float>(), ctx->d_inl.as<int32_t>(), st, true, 0, nullptr, true);
+    if (rc) return rc;
+    ctx->last_H = H_local;
+    ctx->last_T_dev = d_T;
+    cudaStream_t aux = ctx->aux_stream;
+    STOCS_CUDA(ctx, cudaEventRecord(ctx->join_ev[0], st));
+    STOCS_CUDA(ctx, cudaStreamWaitEvent(aux, ctx->join_ev[0], 0));
+    STOCS_CUDA(ctx, cudaMemcpyAsync(lcp_local, ctx->d_lcp.p, (size_t)H_local * 4, cudaMemcpyDeviceToHost, st));
+    if (inliers_local)
+      STOCS_CUDA(ctx, cudaMemcpyAsync(inliers_local, ctx->d_inl.p, (size_t)H_local * 4, cudaMemcpyDeviceToHost, st));
+    rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H_local, K, index_offset, nullptr, nullptr, aux, d_T,
+                           ctx->d_inl.as<int32_t>(), d_local);
+    if (rc) return rc;
+    if (nranks > 1) rc = gather_merge_records(ctx, K, b_out.as<stocs_b200_record>(), aux);
+    if (rc) return rc;
+    STOCS_CUDA(ctx, cudaMemcpyAsync(topk_out, b_out.p, (size_t)K * sizeof(stocs_b200_record), cudaMemcpyDeviceToHost, aux));
+    STOCS_CUDA(ctx, cudaEventRecord(ctx->join_ev[1], aux));
+    STOCS_CUDA(ctx, cudaStreamWaitEvent(st, ctx->join_ev[1], 0));
+    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
+    return STOCS_OK;
   }
   if (H_local > 0) {
     int rc = stocs_b200_score_lcp(ctx, T16_local, H_local, lcp_local, inliers_local);
@@ -293,12 +294,8 @@ int stocs_b200_score_sharded(stocs_b200_ctx* ctx, const float* T16_local, int64_
   int rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H_local, K, index_offset, nullptr, nullptr, st,
                              H_local > 0 ? ctx->last_T_dev : nullptr, H_local > 0 ? ctx->d_inl.as<int32_t>() : nullptr, d_local);
   if (rc) return rc;
-  if (nranks > 1) {
-    STOCS_NCCL(ctx, g_nccl.AllGather(b_send.p, b_recv.p, (size_t)K * sizeof(stocs_b200_record), ncclInt8,
-                                     (ncclComm_t)ctx->comm, st));
-    merge_records_kernel<<<1, 1024, 0, st>>>(b_recv.as<stocs_b200_record>(), K * nranks, K, b_out.as<stocs_b200_record>());
-    STOCS_CUDA(ctx, cudaGetLastError());
-  }
+  if (nranks > 1) rc = gather_merge_records(ctx, K, b_out.as<stocs_b200_record>(), st);
+  if (rc) return rc;
   STOCS_CUDA(ctx, cudaMemcpyAsync(topk_out, b_out.p, (size_t)K * sizeof(stocs_b200_record), cudaMemcpyDeviceToHost, st));
   STOCS_CUDA(ctx, cudaStreamSynchronize(st));
   return STOCS_OK;
@@ -400,18 +397,15 @@ int stocs_b200_group_score_best(stocs_b200_group* g, const float* T16, int64_t H
     cudaSetDevice(c->device);
     cudaStream_t st = c->stream;
     DevBuf &b_T = c->pool[POOL_SHARD_T], &b_lcp = c->pool[POOL_SHARD_LCP], &b_inl = c->pool[POOL_SHARD_INL];
-    DevBuf &b_send = c->pool[POOL_COMM_SEND], &b_recv = c->pool[POOL_COMM_RECV], &b_out = c->pool[POOL_COMM_OUT];
     cudaError_t e = b_T.ensure((size_t)(hl ? hl : 1) * 64);
     if (e == cudaSuccess) e = b_lcp.ensure((size_t)(hl ? hl : 1) * 4);
     if (e == cudaSuccess) e = b_inl.ensure((size_t)(hl ? hl : 1) * 4);
-    if (e == cudaSuccess) e = b_send.ensure(rec_bytes);
-    if (e == cudaSuccess) e = b_recv.ensure(rec_bytes * n);
-    if (e == cudaSuccess) e = b_out.ensure(rec_bytes);
+    if (e == cudaSuccess) e = ensure_record_buffers(c, K, n);
     if (e == cudaSuccess && hl > 0)
       e = cudaMemcpyAsync(b_T.p, T16 + 16 * lo[i], (size_t)hl * 64, cudaMemcpyHostToDevice, st);
     if (e != cudaSuccess) { c->err = std::string("group_score_best: ") + cudaGetErrorString(e); return group_fail(g, i, STOCS_E_CUDA); }
     int rc = enqueue_local_topk(c, b_T.as<float>(), hl, lo[i], K, b_lcp.as<float>(), b_inl.as<int32_t>(),
-                                n > 1 ? b_send.as<stocs_b200_record>() : b_out.as<stocs_b200_record>(), st, false,
+                                c->pool[n > 1 ? POOL_COMM_SEND : POOL_COMM_OUT].as<stocs_b200_record>(), st, false,
                                 !lcp && !inliers);
     if (rc) return group_fail(g, i, rc);
   }

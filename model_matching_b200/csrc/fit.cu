@@ -334,8 +334,8 @@ static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, in
     // 4. score + 5. best
     rc = stocs_launch_score(ctx, d_Tc, cap_items, d_lcp, d_inl, st, true, 0, nullptr, false, &d_state->n_items, guess);
     if (rc) return rc;
-    long long* d_bi = (long long*)(ctx->d_small.as<char>() + 512);
-    float* d_bv = (float*)(ctx->d_small.as<char>() + 512 + 256);
+    long long* d_bi = &ctx->scratch()->pipe_best_idx;
+    float* d_bv = &ctx->scratch()->pipe_best_lcp;
     // lists the closing block can scan itself (every online frame) skip the general top-K launch
     const bool small_list = cap_items <= (1ll << 20);
     if (!small_list) {

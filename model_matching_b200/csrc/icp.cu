@@ -182,6 +182,6 @@ extern "C" int stocs_b200_icp_point_to_plane(stocs_b200_ctx* ctx, const float* s
     for (int it = 0; it < max_iterations; ++it) pairs_per_iteration[it] = hs.n_pairs[it];
   if (iterations_done) *iterations_done = hs.iterations;
   if (converged) *converged = hs.failed ? 0 : 1;
-  ctx->counters[0] += 2 * max_iterations + 2;
+  ctx->counters[CTR_SCORE_LAUNCHES] += 2 * max_iterations + 2;
   return STOCS_OK;
 }

@@ -187,7 +187,7 @@ static int build_ppf_table(stocs_b200_ctx* ctx, const int* d_keys4, const int* d
   STOCS_CUDA(ctx, cudaMemsetAsync(counts, 0, (size_t)(nbins + 1) * 4, st));
   STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_ppf_keybits.p, 0, (size_t)((nkeybits + 31) / 32) * 4, st));
   if (list_n >= 0) {
-    unsigned long long* d_bad = (unsigned long long*)(ctx->d_small.as<char>() + 272);
+    unsigned long long* d_bad = &ctx->scratch()->ppf_bad;
     STOCS_CUDA(ctx, cudaMemsetAsync(d_bad, 0, 8, st));
     STOCS_CUDA(ctx, cudaMemsetAsync(keys_a.p, 0xff, (size_t)MM * 8, st));
     if (list_n > 0)
@@ -214,7 +214,7 @@ static int build_ppf_table(stocs_b200_ctx* ctx, const int* d_keys4, const int* d
   STOCS_CUDA(ctx, ctx->d_ppf_pairs.ensure((size_t)(npairs ? npairs : 1) * 4));
   if (npairs)
     ppf_strip_kernel<<<(npairs + 255) / 256, 256, 0, st>>>(keys_b.as<unsigned long long>(), npairs, ctx->d_ppf_pairs.as<uint32_t>());
-  unsigned long long* d_nkeys = (unsigned long long*)(ctx->d_small.as<char>() + 256);
+  unsigned long long* d_nkeys = &ctx->scratch()->ppf_nkeys;
   STOCS_CUDA(ctx, cudaMemsetAsync(d_nkeys, 0, 8, st));
   ppf_keybits_kernel<<<(unsigned)((nbins + 255) / 256), 256, 0, st>>>(ctx->d_ppf_bin_start.as<uint32_t>(), n1, na, tr,
                                                                        ctx->d_ppf_keybits.as<uint32_t>(), d_nkeys);
@@ -317,7 +317,7 @@ int stocs_b200_ppf_lookup(stocs_b200_ctx* ctx, const int32_t* key4, int32_t* pai
   DevBuf a, b, tmp;
   STOCS_CUDA(ctx, a.ensure((size_t)maxn * 4));
   STOCS_CUDA(ctx, b.ensure((size_t)maxn * 4));
-  long long* d_n = (long long*)(ctx->d_small.as<char>() + 264);
+  long long* d_n = &ctx->scratch()->ppf_lookup_n;
   ppf_gather_kernel<<<1, 128, 0, st>>>(stocs_ppf_view(ctx), key, a.as<uint32_t>(), maxn, d_n);
   long long n = 0;
   STOCS_CUDA(ctx, cudaMemcpyAsync(&n, d_n, 8, cudaMemcpyDeviceToHost, st));

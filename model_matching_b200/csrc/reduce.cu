@@ -219,7 +219,7 @@ int stocs_launch_topk(stocs_b200_ctx* ctx, const float* d_lcp, int64_t H, int K,
   const int which = (st == ctx->aux_stream) ? 1 : 0;
   DevBuf& lists = which ? ctx->pool[POOL_TOPK_LISTS_AUX] : ctx->d_work;
   STOCS_CUDA(ctx, lists.ensure((size_t)blocks * 32 * 8));
-  unsigned* ticket = (unsigned*)(ctx->d_small.as<char>() + 3344) + which;   // zero at creation, reset by the last CTA
+  unsigned* ticket = &ctx->scratch()->topk_ticket[which];   // zero at creation, reset by the last CTA
   topk_kernel<<<blocks, 256, 0, st>>>(d_lcp, H, lists.as<unsigned long long>(), ticket, K, index_offset,
                                       (long long*)d_idx, d_val, d_T16, d_inl, d_rec, d_H);
   STOCS_CUDA(ctx, cudaGetLastError());

@@ -359,9 +359,9 @@ int stocs_b200_sample_instance_base(stocs_b200_ctx* ctx, uint64_t seed, int base
   if (!base_idx4 || !inv2 || !valid) STOCS_FAIL(ctx, STOCS_E_ARG, "sample_instance_base: bad argument");
   cudaSetDevice(ctx->device);
   cudaStream_t st = ctx->stream;
-  int* d_ids = (int*)(ctx->d_small.as<char>() + 1024);
-  float* d_inv = (float*)(d_ids + 4);
-  uint8_t* d_valid = (uint8_t*)(d_inv + 2);
+  int* d_ids = ctx->scratch()->inst_ids;
+  float* d_inv = ctx->scratch()->inst_inv;
+  uint8_t* d_valid = &ctx->scratch()->inst_valid;
   int rc = stocs_launch_sample_instance(ctx, seed, base_num, dispersion, d_ids, d_inv, d_valid, st);
   if (rc) return rc;
   const size_t n = (size_t)ctx->img_w * ctx->img_h;

@@ -230,8 +230,8 @@ extern "C" int stocs_b200_build_scene_cloud(stocs_b200_ctx* ctx, const uint16_t*
   if (edge) { SC(d_edge.ensure((size_t)n)); SC(cudaMemcpyAsync(d_edge.p, edge, (size_t)n, cudaMemcpyHostToDevice, st)); }
   int rc = stocs_launch_backproject(ctx, d_depth.as<uint16_t>(), nullptr, W, H, fx, cx, fy, cy, depth_scale, d_xyz.as<float>(), nullptr, st);
   if (rc) { cleanup(); return rc; }
-  // counters in d_small: [300] first_zero, [301] n_zero, [302] n_valid
-  int* d_cnt = (int*)(ctx->d_small.as<char>() + 1200);
+  // device counters: first_zero, n_zero, n_valid, n_vox
+  int* d_cnt = ctx->scratch()->cloud;
   int init[3] = {0x7fffffff, 0, 0};
   SC(cudaMemcpyAsync(d_cnt, init, 12, cudaMemcpyHostToDevice, st));
   first_zero_kernel<<<nb, 256, 0, st>>>(d_depth.as<uint16_t>(), n, d_cnt, d_cnt + 1);
@@ -299,7 +299,7 @@ extern "C" int stocs_b200_build_scene_cloud(stocs_b200_ctx* ctx, const uint16_t*
   SC(cudaMemcpyAsync(&h_len[0], d_nvox, 4, cudaMemcpyDeviceToHost, st));
   SC(cudaMemcpyAsync(&h_len[1], d_scan.as<int>() + n, 4, cudaMemcpyDeviceToHost, st));
   const bool have_out = pos3 && nrm3 && pixel_rc && class_p;
-  long long guess = have_out ? ctx->counters[7] : 0;
+  long long guess = have_out ? ctx->counters[CTR_CLOUD_VOXELS] : 0;
   if (guess > out_cap) guess = out_cap;
   auto fetch = [&](long long from, long long to) -> cudaError_t {
     const size_t c = (size_t)(to - from);
@@ -315,7 +315,7 @@ extern "C" int stocs_b200_build_scene_cloud(stocs_b200_ctx* ctx, const uint16_t*
   SC(cudaStreamSynchronize(st));
   const long long nvox = (long long)h_len[0], n_emit = (long long)h_len[1];
   *n_out = n_emit;
-  ctx->counters[7] = nvox;
+  ctx->counters[CTR_CLOUD_VOXELS] = nvox;
   if (n_emit > cap) { cleanup(); STOCS_FAIL(ctx, STOCS_E_CAPACITY, "build_scene_cloud: output capacity too small"); }
   if (n_emit > 0 && !have_out) { cleanup(); STOCS_FAIL(ctx, STOCS_E_ARG, "build_scene_cloud: output pointer is NULL"); }
   if (n_emit > guess) {

@@ -410,9 +410,8 @@ static int kd_start(stocs_b200_ctx* ctx, int S) {
 int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4* d_out4,
                         float* d_out3, float* h_centroid3, float* h_aabb6, const float* h_pos3, float* h_centred3) {
   cudaStream_t st = ctx->stream;
-  STOCS_CUDA(ctx, ctx->d_small.ensure(256));
-  float* d_c = ctx->d_small.as<float>();
-  int* d_aabb = (int*)(d_c + 4);
+  float* d_c = ctx->scratch()->centroid;
+  int* d_aabb = ctx->scratch()->aabb;
   if (h_pos3) {
     float sx = 0.f, sy = 0.f, sz = 0.f;   // same order, same binary32 adds as the kernel (no contraction: no multiply)
     for (int i = 0; i < n; ++i) { sx += h_pos3[3 * (size_t)i]; sy += h_pos3[3 * (size_t)i + 1]; sz += h_pos3[3 * (size_t)i + 2]; }
@@ -619,10 +618,10 @@ int stocs_build_scene_index(stocs_b200_ctx* ctx) {
     cap = (size_t)total + 1024;
   }
   ctx->ncand = total;
-  ctx->counters[6] = n_occ;
+  ctx->counters[CTR_OCCUPIED_CELLS] = n_occ;
   tr.mark("index build");
-  ctx->counters[2] = g.ncells;
-  ctx->counters[3] = total;
+  ctx->counters[CTR_GRID_CELLS] = g.ncells;
+  ctx->counters[CTR_CANDIDATES] = total;
   return STOCS_OK;
 }
 

@@ -117,6 +117,24 @@ struct StocsPipeState {
   float best_Tc[16], best_Tw[16];
 };
 
+// Slots of stocs_b200_ctx::counters.  [0]-[5] are public: stocs_b200_get_counters returns them, and
+// include/stocs_b200.h documents what they count.  [6] and [7] are internal.
+enum CtxCounter : int {
+  CTR_SCORE_LAUNCHES = 0,   // score kernels launched (icp.cu adds the launches of its iterations)
+  CTR_TIES,                 // NN queries resolved by the kd-tree tie path (DevScratch::score_totals)
+  CTR_GRID_CELLS,           // grid cells of the current scene index
+  CTR_CANDIDATES,           // replicated candidate records of the current scene index
+  CTR_REJECTED_LOOP1,       // top-K hypotheses rejected after the coarse test (DevScratch::score_totals)
+  CTR_REJECTED_DRAIN,       // top-K hypotheses rejected before a queue drain (DevScratch::score_totals)
+  CTR_OCCUPIED_CELLS,       // occupied cells of the current scene index
+  // STATE, not a diagnostic: voxels of the last build_scene_cloud, which the next call takes as its
+  // guess of how many points to read back in the same queue as the list lengths (scene_cloud.cu)
+  CTR_CLOUD_VOXELS,
+  CTR_COUNT
+};
+
+struct DevScratch;
+
 struct stocs_b200_ctx {
   int device = 0;
   int num_sms = 0;
@@ -128,7 +146,7 @@ struct stocs_b200_ctx {
   static constexpr int kEvRing = 512;
   cudaEvent_t ev_ring[2 * kEvRing] = {};
   int64_t ev_count = 0;
-  static constexpr int kMaxChunks = 16;
+  static constexpr int kMaxChunks = 4;    // chunks of score_lcp's geometric plan
   cudaEvent_t chunk_ev[kMaxChunks] = {};  // H2D-complete events of score_lcp's chunks
   cudaEvent_t join_ev[2] = {nullptr, nullptr};
   std::string err;
@@ -188,8 +206,9 @@ struct stocs_b200_ctx {
   // counter arrays that every run leaves ZEROED (tracked by index_counts_clean / cong_bcount_clean),
   // so that the next run need not clear tens of megabytes first.
   DevBuf pool[POOL_COUNT];
-  // scratch
+  // scratch (d_small: 4 KB, laid out by DevScratch)
   DevBuf d_T, d_lcp, d_inl, d_work, d_tmp, d_tmp2, d_small;
+  DevScratch* scratch() const { return d_small.as<DevScratch>(); }
   void* h_pinned = nullptr;
   size_t h_pinned_bytes = 0;
 
@@ -213,13 +232,52 @@ struct stocs_b200_ctx {
   struct TopCache { int64_t idx[32]; float val[32]; };
   TopCache* h_top = nullptr;   // page-locked
   bool top_valid = false;
-  int64_t counters[8] = {0};
+  int64_t counters[CTR_COUNT] = {0};
   bool timing_valid = false;
 
   // multi-GPU (comm.cu): one NCCL communicator per context; ncclComm_t kept opaque here
   void* comm = nullptr;
   int comm_rank = 0, comm_nranks = 1;
 };
+
+// Small device values of the stages, in the context's 4 KB scratch (stocs_b200_ctx::d_small).
+// stocs_b200_create zeroes it once.  Fields marked ZERO-RELIANT count on that and are never cleared
+// again; every other field is written by its stage before it is read.
+struct DevScratch {
+  // score.cu: work counter of a scoring launch per slot (slot 0 by default, score_lcp's chunks use
+  // their chunk number so that concurrent chunks do not share one); cleared before each launch
+  unsigned long long work[stocs_b200_ctx::kMaxChunks];
+  // score.cu, ZERO-RELIANT: NN queries resolved by the kd-tree tie path, and top-K hypotheses
+  // rejected after the coarse test / before a drain, accumulated over the context's lifetime;
+  // stocs_b200_get_counters reads the three in one copy
+  struct ScoreTotals { unsigned long long ties, rejected[2]; } score_totals;
+  // capi.cu (stocs_b200_score_counters): the counting variant's ScoreCounter slots (score.cu)
+  unsigned long long score_counts[8];
+  // reduce.cu, ZERO-RELIANT: top-K ticket of the context stream [0] and of its second stream [1];
+  // the last CTA of a launch resets it
+  unsigned topk_ticket[2];
+  // score.cu: heavy-first schedule, next position from the front (heavy) and from the back (light)
+  unsigned lpt_fill[2];
+  // score.cu (stocs_fmad_selftest): written after the creation memset, so shared with no other field
+  float fmad_selftest;
+  // scene_index.cu (stocs_centre_points): centroid, and the bounding box as ordered ints (min xyz, max xyz)
+  float centroid[4];
+  int aabb[6];
+  // ppf_table.cu: occupied keys of the table build, entries of a lookup, entries an upload rejected
+  unsigned long long ppf_nkeys;
+  long long ppf_lookup_n;
+  unsigned long long ppf_bad;
+  // fit.cu: best transform of the pipeline's top-1 reduction (index, lcp)
+  long long pipe_best_idx;
+  float pipe_best_lcp;
+  // sample_instance.cu (stocs_b200_sample_instance_base): base point ids, inverse distances, valid flag
+  int inst_ids[4];
+  float inst_inv[2];
+  uint8_t inst_valid;
+  // scene_cloud.cu (build_scene_cloud): first zero-depth pixel, zero-depth pixels, valid pixels, voxels
+  int cloud[4];
+};
+static_assert(sizeof(DevScratch) <= 4096, "DevScratch must fit the 4 KB d_small allocation");
 
 #define STOCS_CUDA(ctx, call)                                                            \
   do {                                                                                   \
@@ -251,7 +309,11 @@ int stocs_launch_backproject(stocs_b200_ctx* ctx, const uint16_t* d_depth, const
 // joins the kd-tree build started by upload_scene (if any) and, with upload = true, queues its upload on st
 int stocs_kd_finish(stocs_b200_ctx* ctx, cudaStream_t st, bool upload = true);  // scene_index.cu
 bool stocs_fmad_selftest(stocs_b200_ctx* ctx);                             // score.cu
-bool stocs_is_host_memory(const void* p);                                  // capi.cu
+// device alias of page-locked host memory, NULL for any other pointer (capi.cu)
+const void* stocs_host_alias(const void* p);
+// device alias through which a host-buffer scoring call reads its transforms in place, NULL when
+// they are staged instead: pageable memory, or STOCS_NO_ZERO_COPY set (capi.cu)
+const float* stocs_zero_copy_transforms(const float* T16);
 // w_max / prune_ok of the scene from its class weights (capi.cu; every writer of the weights calls it)
 void stocs_set_weight_bound(stocs_b200_ctx* ctx, const float* cls, int S);
 // top-K of a device lcp array (reduce.cu); d_idx/d_val may be NULL when only records are wanted
