@@ -288,7 +288,9 @@ int stocs_b200_group_score_best(stocs_b200_group* g, const float* T16, int64_t H
  * current scene index; [4] / [5] hypotheses the device top-K path (score_sharded_device,
  * group_score_best without per-hypothesis outputs) left unscored because they provably cannot
  * enter the top K, rejected after the coarse test / before a queue drain, accumulated over the
- * lifetime of the context. */
+ * lifetime of the context; [6] and [7] are internal; [8] hypotheses of the same path rejected
+ * after the brick-bit refinement of the coarse survivors, which runs between the two, accumulated
+ * likewise. */
 int stocs_b200_get_counters(stocs_b200_ctx* ctx, int64_t* counters, int n);
 /* Data-dependent work of ONE scoring launch over H device-resident transforms, counted exactly by a
  * counting instantiation of the scoring kernel (results discarded, not for timing).  counters (up

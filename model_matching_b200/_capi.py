@@ -441,8 +441,8 @@ class Context:
         return r
 
     def counters(self):
-        c = np.zeros(8, np.int64)
-        self._check(self._L.stocs_b200_get_counters(self.h, _ptr(c), 8))
+        c = np.zeros(9, np.int64)
+        self._check(self._L.stocs_b200_get_counters(self.h, _ptr(c), 9))
         return c
 
     SCORE_COUNTER_NAMES = ("queries", "coarse_survivors", "brick_records", "queued", "candidates", "hits",

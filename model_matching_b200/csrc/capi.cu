@@ -478,6 +478,7 @@ int stocs_b200_get_counters(stocs_b200_ctx* ctx, int64_t* counters, int n) {
     ctx->counters[CTR_TIES] = (int64_t)t.ties;
     ctx->counters[CTR_REJECTED_LOOP1] = (int64_t)t.rejected[0];
     ctx->counters[CTR_REJECTED_DRAIN] = (int64_t)t.rejected[1];
+    ctx->counters[CTR_REJECTED_BRICK] = (int64_t)t.rejected[2];
   }
   for (int i = 0; i < n && i < CTR_COUNT; ++i) counters[i] = ctx->counters[i];
   return STOCS_OK;

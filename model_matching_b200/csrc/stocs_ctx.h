@@ -117,8 +117,8 @@ struct StocsPipeState {
   float best_Tc[16], best_Tw[16];
 };
 
-// Slots of stocs_b200_ctx::counters.  [0]-[5] are public: stocs_b200_get_counters returns them, and
-// include/stocs_b200.h documents what they count.  [6] and [7] are internal.
+// Slots of stocs_b200_ctx::counters.  [0]-[5] and [8] are public: stocs_b200_get_counters returns
+// them, and include/stocs_b200.h documents what they count.  [6] and [7] are internal.
 enum CtxCounter : int {
   CTR_SCORE_LAUNCHES = 0,   // score kernels launched (icp.cu adds the launches of its iterations)
   CTR_TIES,                 // NN queries resolved by the kd-tree tie path (DevScratch::score_totals)
@@ -130,6 +130,7 @@ enum CtxCounter : int {
   // STATE, not a diagnostic: voxels of the last build_scene_cloud, which the next call takes as its
   // guess of how many points to read back in the same queue as the list lengths (scene_cloud.cu)
   CTR_CLOUD_VOXELS,
+  CTR_REJECTED_BRICK,       // top-K hypotheses rejected after the brick-bit refinement (DevScratch::score_totals)
   CTR_COUNT
 };
 
@@ -248,9 +249,9 @@ struct DevScratch {
   // their chunk number so that concurrent chunks do not share one); cleared before each launch
   unsigned long long work[stocs_b200_ctx::kMaxChunks];
   // score.cu, ZERO-RELIANT: NN queries resolved by the kd-tree tie path, and top-K hypotheses
-  // rejected after the coarse test / before a drain, accumulated over the context's lifetime;
-  // stocs_b200_get_counters reads the three in one copy
-  struct ScoreTotals { unsigned long long ties, rejected[2]; } score_totals;
+  // rejected after the coarse test / before a drain / after the brick-bit refinement, accumulated
+  // over the context's lifetime; stocs_b200_get_counters reads the four in one copy
+  struct ScoreTotals { unsigned long long ties, rejected[3]; } score_totals;
   // capi.cu (stocs_b200_score_counters): the counting variant's ScoreCounter slots (score.cu)
   unsigned long long score_counts[8];
   // reduce.cu, ZERO-RELIANT: top-K ticket of the context stream [0] and of its second stream [1];
