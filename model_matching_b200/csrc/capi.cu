@@ -53,6 +53,118 @@ void stocs_set_weight_bound(stocs_b200_ctx* ctx, const float* cls, int S) {
   }
 }
 
+// Top-32 of the resident lcp array into the page-locked cache, on stream st (no synchronize).
+static int enqueue_resident_topk(stocs_b200_ctx* ctx, int64_t H, cudaStream_t st) {
+  DevBuf& d_top = ctx->pool[POOL_TOPK_RESIDENT];
+  STOCS_CUDA(ctx, d_top.ensure(32 * 12));
+  TopkRequest rq;
+  rq.idx = d_top.as<int64_t>();
+  rq.val = (float*)(rq.idx + 32);
+  int rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H, 32, 0, st, rq);
+  if (rc) return rc;
+  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_top->idx, rq.idx, 32 * 8, cudaMemcpyDeviceToHost, st));
+  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_top->val, rq.val, 32 * 4, cudaMemcpyDeviceToHost, st));
+  return STOCS_OK;
+}
+
+int stocs_score_host(stocs_b200_ctx* ctx, const char* who, const float* T16, int64_t H, float* lcp, int32_t* inliers,
+                     const ScoreTail& tail) {
+  cudaStream_t st = ctx->stream, aux = ctx->aux_stream;
+  int rc = STOCS_OK;
+  cudaError_t e = cudaSuccess;
+  auto ok = [&]() { return rc == STOCS_OK && e == cudaSuccess; };
+  // The second stream starts behind whatever is queued on the context stream; once forked, it is
+  // joined back even after an error, so that no work is left queued behind the context stream
+  // (the one callers order against).
+  bool forked = false;
+  auto fork = [&]() {
+    forked = true;
+    e = cudaEventRecord(ctx->join_ev[0], st);
+    if (e == cudaSuccess) e = cudaStreamWaitEvent(aux, ctx->join_ev[0], 0);
+  };
+  auto join = [&]() {
+    cudaError_t e2 = cudaEventRecord(ctx->join_ev[1], aux);
+    if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(st, ctx->join_ev[1], 0);
+    if (e == cudaSuccess) e = e2;
+  };
+  if (H == 0) {
+    rc = tail(st, nullptr);
+  } else {
+    ctx->top_valid = false;
+    e = ctx->d_lcp.ensure((size_t)H * 4);
+    if (e == cudaSuccess) e = ctx->d_inl.ensure((size_t)H * 4);
+    float* d_lcp = ctx->d_lcp.as<float>();
+    int32_t* d_inl = ctx->d_inl.as<int32_t>();
+    // Page-locked, device-mapped transforms (cudaHostAlloc / cudaHostRegister, e.g. a pinned torch
+    // tensor) are read by the kernel in place: each warp fetches its 48 B over PCIe while the SM's
+    // other 63 warps compute, so no staging copy and a single launch (one straggler tail instead of
+    // one per chunk).  Measured on S1: 2.98 ms against 2.94 ms with the transforms in HBM; when every
+    // hypothesis is trivially rejected the reads become the bound (1.56 ms per 10^6, 41 GB/s), still
+    // no slower than the staged path.  Results are written to HBM and copied back once: letting the
+    // kernel also write to host memory puts its reads behind the posted writes (3.98 ms).
+    if (const float* d_T = ok() ? stocs_zero_copy_transforms(T16) : nullptr) {
+      ScoreRequest rq;
+      rq.time_it = true;
+      rc = stocs_launch_score(ctx, d_T, H, d_lcp, d_inl, st, rq);
+      // the tail runs on the second stream while the copy engine returns the results
+      if (ok()) fork();
+      if (ok() && lcp) e = cudaMemcpyAsync(lcp, d_lcp, (size_t)H * 4, cudaMemcpyDeviceToHost, st);
+      if (ok() && inliers) e = cudaMemcpyAsync(inliers, d_inl, (size_t)H * 4, cudaMemcpyDeviceToHost, st);
+      if (ok()) rc = tail(aux, d_T);
+      if (forked) join();
+    } else {
+      // Pageable transforms are staged through HBM in chunks: the H2D copy of chunk k+1 (copy
+      // stream) overlaps the scoring of chunk k.  Chunks grow geometrically (H/8, H/8, H/4, H/2) so
+      // that scoring starts early and most of the work runs in large launches.  Consecutive chunks
+      // alternate between two compute streams, each launch with its own work counter, so the CTAs
+      // of chunk k+1 move in as the straggler warps of chunk k retire (a launch's tail is 0.1-0.2 ms
+      // on the S1 workload); each chunk's results go back on its own stream behind its kernel.
+      // (H2D from pageable memory is staged by the driver through its own pinned buffer and returns
+      // early; D2H into pageable memory does not -- see below.)
+      if (ok()) e = ctx->d_T.ensure((size_t)H * 64);
+      float* d_stage = ctx->d_T.as<float>();
+      std::vector<int64_t> bounds;
+      if (H <= (1 << 16)) {
+        bounds = {0, H};
+      } else {
+        const int64_t e8 = (H + 7) / 8;
+        bounds = {0, e8, 2 * e8, 4 * e8, H};
+        for (auto& b : bounds) if (b > H) b = H;
+      }
+      const int64_t nchunks = (int64_t)bounds.size() - 1;
+      cudaStream_t cs[2] = {st, aux};
+      if (ok() && nchunks > 1) fork();
+      for (int64_t c = 0; c < nchunks && ok(); ++c) {
+        const int64_t off = bounds[c], n = bounds[c + 1] - bounds[c];
+        if (n <= 0) continue;
+        e = cudaMemcpyAsync(d_stage + off * 16, T16 + off * 16, (size_t)n * 64, cudaMemcpyHostToDevice, ctx->copy_stream);
+        if (e == cudaSuccess) e = cudaEventRecord(ctx->chunk_ev[c], ctx->copy_stream);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(cs[c & 1], ctx->chunk_ev[c], 0);
+        ScoreRequest rq;
+        rq.slot = (int)c;
+        if (e == cudaSuccess) rc = stocs_launch_score(ctx, d_stage + off * 16, n, d_lcp + off, d_inl + off, cs[c & 1], rq);
+      }
+      // Result copies are enqueued only after EVERY chunk's H2D copy and kernel: a cudaMemcpyAsync
+      // into pageable memory returns when the copy is done, so issuing it inside the loop above would
+      // hold back the enqueue of chunk k+1's H2D until chunk k's kernel has finished (no overlap at all).
+      for (int64_t c = 0; c < nchunks && ok(); ++c) {
+        const int64_t off = bounds[c], n = bounds[c + 1] - bounds[c];
+        if (n <= 0) continue;
+        if (lcp) e = cudaMemcpyAsync(lcp + off, d_lcp + off, (size_t)n * 4, cudaMemcpyDeviceToHost, cs[c & 1]);
+        if (e == cudaSuccess && inliers)
+          e = cudaMemcpyAsync(inliers + off, d_inl + off, (size_t)n * 4, cudaMemcpyDeviceToHost, cs[c & 1]);
+      }
+      if (forked) join();
+      if (ok()) rc = tail(st, d_stage);
+    }
+  }
+  const cudaError_t es = cudaStreamSynchronize(st);
+  if (e == cudaSuccess) e = es;
+  if (rc == STOCS_OK && e != cudaSuccess) { ctx->err = std::string(who) + ": " + cudaGetErrorString(e); rc = STOCS_E_CUDA; }
+  if (H > 0) ctx->last_H = rc == STOCS_OK ? H : 0;
+  return rc;
+}
+
 extern "C" {
 
 int stocs_b200_abi_version(void) { return STOCS_B200_ABI_VERSION; }
@@ -121,7 +233,6 @@ void stocs_b200_destroy(stocs_b200_ctx* ctx) {
                     &ctx->d_frontier};
   for (DevBuf* b : bufs) b->release();
   for (DevBuf& b : ctx->pool) b.release();
-  if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
   for (cudaEvent_t e : ctx->ev_ring) if (e) cudaEventDestroy(e);
   for (int i = 0; i < stocs_b200_ctx::kMaxChunks; ++i) if (ctx->chunk_ev[i]) cudaEventDestroy(ctx->chunk_ev[i]);
   for (int i = 0; i < 2; ++i) if (ctx->join_ev[i]) cudaEventDestroy(ctx->join_ev[i]);
@@ -293,20 +404,9 @@ int stocs_b200_score_lcp_device(stocs_b200_ctx* ctx, const float* d_T16, int64_t
   if (H < 0 || (H > 0 && (!d_T16 || !d_lcp))) STOCS_FAIL(ctx, STOCS_E_ARG, "score_lcp: bad argument");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-  return stocs_launch_score(ctx, d_T16, H, d_lcp, d_inliers, st, true, 0, nullptr, H > 0 && stocs_host_alias(d_T16));
-}
-
-// Top-32 of the resident lcp array into the page-locked cache, on stream st (no synchronize).
-static int enqueue_resident_topk(stocs_b200_ctx* ctx, int64_t H, cudaStream_t st) {
-  DevBuf& d_top = ctx->pool[POOL_TOPK_RESIDENT];
-  STOCS_CUDA(ctx, d_top.ensure(32 * 12));
-  int64_t* d_idx = d_top.as<int64_t>();
-  float* d_val = (float*)(d_idx + 32);
-  int rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H, 32, 0, d_idx, d_val, st);
-  if (rc) return rc;
-  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_top->idx, d_idx, 32 * 8, cudaMemcpyDeviceToHost, st));
-  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_top->val, d_val, 32 * 4, cudaMemcpyDeviceToHost, st));
-  return STOCS_OK;
+  ScoreRequest rq;
+  rq.time_it = true;
+  return stocs_launch_score(ctx, d_T16, H, d_lcp, d_inliers, st, rq);
 }
 
 int stocs_b200_score_lcp(stocs_b200_ctx* ctx, const float* T16, int64_t H, float* lcp, int32_t* inliers) {
@@ -315,101 +415,9 @@ int stocs_b200_score_lcp(stocs_b200_ctx* ctx, const float* T16, int64_t H, float
   if (H < 0 || (H > 0 && (!T16 || !lcp))) STOCS_FAIL(ctx, STOCS_E_ARG, "score_lcp: bad argument");
   if (H == 0) return STOCS_OK;
   cudaSetDevice(ctx->device);
-  ctx->top_valid = false;
-  ctx->last_T_dev = nullptr;
-  STOCS_CUDA(ctx, ctx->d_lcp.ensure((size_t)H * 4));
-  STOCS_CUDA(ctx, ctx->d_inl.ensure((size_t)H * 4));
-  // Page-locked, device-mapped transforms (cudaHostAlloc / cudaHostRegister, e.g. a pinned torch
-  // tensor) are read by the kernel in place: each warp fetches its 48 B over PCIe while the SM's
-  // other 63 warps compute, so no staging copy and a single launch (one straggler tail instead of
-  // one per chunk).  Measured on S1: 2.98 ms against 2.94 ms with the transforms in HBM; when every
-  // hypothesis is trivially rejected the reads become the bound (1.56 ms per 10^6, 41 GB/s), still
-  // no slower than the staged path.  Results are written to HBM and copied back once: letting the
-  // kernel also write to host memory puts its reads behind the posted writes (3.98 ms).
-  if (const float* d_T = stocs_zero_copy_transforms(T16)) {
-    int rc = stocs_launch_score(ctx, d_T, H, ctx->d_lcp.as<float>(), ctx->d_inl.as<int32_t>(), ctx->stream, true, 0,
-                                nullptr, /*T_in_host_memory=*/true);
-    if (rc != STOCS_OK) return rc;
-    ctx->last_T_dev = d_T;
-    // the top-32 reduction (what stocs_b200_reduce_best returns for the resident array) runs on
-    // the second stream while the copy engine returns the results
-    cudaError_t e = cudaEventRecord(ctx->join_ev[0], ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->aux_stream, ctx->join_ev[0], 0);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(lcp, ctx->d_lcp.p, (size_t)H * 4, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess && inliers)
-      e = cudaMemcpyAsync(inliers, ctx->d_inl.p, (size_t)H * 4, cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) rc = enqueue_resident_topk(ctx, H, ctx->aux_stream);
-    cudaError_t e2 = cudaEventRecord(ctx->join_ev[1], ctx->aux_stream);
-    if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(ctx->stream, ctx->join_ev[1], 0);
-    if (e == cudaSuccess) e = e2;
-    e2 = cudaStreamSynchronize(ctx->stream);
-    if (e == cudaSuccess) e = e2;
-    if (e != cudaSuccess) { ctx->err = std::string("score_lcp: ") + cudaGetErrorString(e); return STOCS_E_CUDA; }
-    if (rc != STOCS_OK) return rc;
-    ctx->last_H = H;
-    ctx->top_valid = true;
-    return STOCS_OK;
-  }
-  // Pageable transforms are staged through HBM in chunks:
-  STOCS_CUDA(ctx, ctx->d_T.ensure((size_t)H * 64));
-  ctx->last_T_dev = ctx->d_T.as<float>();
-  // chunked: the H2D copy of chunk k+1 (copy stream) overlaps the scoring of chunk k.  Chunks grow
-  // geometrically (H/8, H/8, H/4, H/2) so that scoring starts early and most of the work runs in
-  // large launches.  Consecutive chunks alternate between two compute streams, each launch with
-  // its own work counter, so the CTAs of chunk k+1 move in as the straggler warps of chunk k
-  // retire (a launch's tail is 0.1-0.2 ms on the S1 workload); each chunk's results go back on its
-  // own stream behind its kernel.  (H2D from pageable memory is staged by the driver through its
-  // own pinned buffer and returns early; D2H into pageable memory does not -- see below.)
-  std::vector<int64_t> bounds;
-  if (H <= (1 << 16)) {
-    bounds = {0, H};
-  } else {
-    const int64_t e8 = (H + 7) / 8;
-    bounds = {0, e8, 2 * e8, 4 * e8, H};
-    for (auto& b : bounds) if (b > H) b = H;
-  }
-  const int64_t nchunks = (int64_t)bounds.size() - 1;
-  cudaStream_t cs[2] = {ctx->stream, ctx->aux_stream};
-  int rc = STOCS_OK;
-  cudaError_t e = cudaSuccess;
-  if (nchunks > 1) {  // aux stream starts behind whatever is queued on the context stream
-    e = cudaEventRecord(ctx->join_ev[0], ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(ctx->aux_stream, ctx->join_ev[0], 0);
-  }
-  for (int64_t c = 0; c < nchunks && rc == STOCS_OK && e == cudaSuccess; ++c) {
-    const int64_t off = bounds[c], n = bounds[c + 1] - bounds[c];
-    if (n <= 0) continue;
-    cudaStream_t st = cs[c & 1];
-    e = cudaMemcpyAsync(ctx->d_T.as<float>() + off * 16, T16 + off * 16, (size_t)n * 64, cudaMemcpyHostToDevice,
-                        ctx->copy_stream);
-    if (e == cudaSuccess) e = cudaEventRecord(ctx->chunk_ev[c], ctx->copy_stream);
-    if (e == cudaSuccess) e = cudaStreamWaitEvent(st, ctx->chunk_ev[c], 0);
-    if (e != cudaSuccess) break;
-    rc = stocs_launch_score(ctx, ctx->d_T.as<float>() + off * 16, n, ctx->d_lcp.as<float>() + off,
-                            ctx->d_inl.as<int32_t>() + off, st, false, (int)c);
-    if (rc != STOCS_OK) break;
-  }
-  // Result copies are enqueued only after EVERY chunk's H2D copy and kernel: a cudaMemcpyAsync into
-  // pageable memory returns when the copy is done, so issuing it inside the loop above would hold
-  // back the enqueue of chunk k+1's H2D until chunk k's kernel has finished (no overlap at all).
-  for (int64_t c = 0; c < nchunks && rc == STOCS_OK && e == cudaSuccess; ++c) {
-    const int64_t off = bounds[c], n = bounds[c + 1] - bounds[c];
-    if (n <= 0) continue;
-    cudaStream_t st = cs[c & 1];
-    e = cudaMemcpyAsync(lcp + off, ctx->d_lcp.as<float>() + off, (size_t)n * 4, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && inliers)
-      e = cudaMemcpyAsync(inliers + off, ctx->d_inl.as<int32_t>() + off, (size_t)n * 4, cudaMemcpyDeviceToHost, st);
-  }
-  if (nchunks > 1) {  // join: the context stream is the one callers order against
-    cudaError_t e2 = cudaEventRecord(ctx->join_ev[1], ctx->aux_stream);
-    if (e2 == cudaSuccess) e2 = cudaStreamWaitEvent(ctx->stream, ctx->join_ev[1], 0);
-    if (e == cudaSuccess) e = e2;
-  }
-  if (rc == STOCS_OK && e == cudaSuccess) rc = enqueue_resident_topk(ctx, H, ctx->stream);
-  cudaError_t es = cudaStreamSynchronize(ctx->stream);
-  if (e == cudaSuccess) e = es;
-  if (rc == STOCS_OK && e != cudaSuccess) { ctx->err = std::string("score_lcp: ") + cudaGetErrorString(e); rc = STOCS_E_CUDA; }
-  ctx->last_H = H;
+  // the tail is the top-32 of the resident array, what stocs_b200_reduce_best(NULL) returns
+  const int rc = stocs_score_host(ctx, "score_lcp", T16, H, lcp, inliers,
+                                  [ctx, H](cudaStream_t st, const float*) { return enqueue_resident_topk(ctx, H, st); });
   ctx->top_valid = rc == STOCS_OK;
   return rc;
 }
@@ -420,7 +428,10 @@ int stocs_b200_reduce_best_device(stocs_b200_ctx* ctx, const float* d_lcp, int64
   if (!d_lcp || H < 0 || !d_topk_index || !d_topk_lcp) STOCS_FAIL(ctx, STOCS_E_ARG, "reduce_best: bad argument");
   cudaSetDevice(ctx->device);
   cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-  return stocs_launch_topk(ctx, d_lcp, H, K, index_offset, d_topk_index, d_topk_lcp, st);
+  TopkRequest rq;
+  rq.idx = d_topk_index;
+  rq.val = d_topk_lcp;
+  return stocs_launch_topk(ctx, d_lcp, H, K, index_offset, st, rq);
 }
 
 int stocs_b200_reduce_best(stocs_b200_ctx* ctx, const float* lcp, int64_t H, int K, int64_t* best_index,
@@ -429,41 +440,27 @@ int stocs_b200_reduce_best(stocs_b200_ctx* ctx, const float* lcp, int64_t H, int
   if (H < 0 || K < 1 || K > 32) STOCS_FAIL(ctx, STOCS_E_ARG, "reduce_best: bad argument");
   cudaSetDevice(ctx->device);
   cudaStream_t st = ctx->stream;
-  const float* d_src = nullptr;
   if (lcp) {
     ctx->top_valid = false;
     STOCS_CUDA(ctx, ctx->d_lcp.ensure((size_t)(H ? H : 1) * 4));
     if (H) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_lcp.p, lcp, (size_t)H * 4, cudaMemcpyHostToDevice, st));
     ctx->last_H = H;
-    d_src = ctx->d_lcp.as<float>();
-  } else {
-    if (ctx->last_H != H || !ctx->d_lcp.p) STOCS_FAIL(ctx, STOCS_E_STATE, "reduce_best: no resident lcp array of that size");
-    if (ctx->top_valid) {  // score_lcp already reduced this array (top-K is a prefix of top-32)
-      if (best_index) *best_index = ctx->h_top->idx[0];
-      if (best_lcp) *best_lcp = ctx->h_top->val[0];
-      for (int k = 0; k < K; ++k) {
-        if (topk_index) topk_index[k] = ctx->h_top->idx[k];
-        if (topk_lcp) topk_lcp[k] = ctx->h_top->val[k];
-      }
-      return STOCS_OK;
-    }
-    d_src = ctx->d_lcp.as<float>();
+  } else if (ctx->last_H != H || !ctx->d_lcp.p) {
+    STOCS_FAIL(ctx, STOCS_E_STATE, "reduce_best: no resident lcp array of that size");
   }
-  STOCS_CUDA(ctx, ctx->d_tmp2.ensure(32 * 12));
-  int64_t* d_idx = ctx->d_tmp2.as<int64_t>();
-  float* d_val = (float*)(d_idx + 32);
-  int rc = stocs_launch_topk(ctx, d_src, H, K, 0, d_idx, d_val, st);
-  if (rc) return rc;
-  int64_t hidx[32];
-  float hval[32];
-  STOCS_CUDA(ctx, cudaMemcpyAsync(hidx, d_idx, (size_t)K * 8, cudaMemcpyDeviceToHost, st));
-  STOCS_CUDA(ctx, cudaMemcpyAsync(hval, d_val, (size_t)K * 4, cudaMemcpyDeviceToHost, st));
-  STOCS_CUDA(ctx, cudaStreamSynchronize(st));
-  if (best_index) *best_index = hidx[0];
-  if (best_lcp) *best_lcp = hval[0];
+  // both branches reduce ctx->d_lcp; h_top may already hold its top-32 (score_lcp, an earlier call)
+  if (!ctx->top_valid) {
+    int rc = enqueue_resident_topk(ctx, H, st);
+    if (rc) return rc;
+    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
+    ctx->top_valid = true;
+  }
+  // top-K is a prefix of top-32
+  if (best_index) *best_index = ctx->h_top->idx[0];
+  if (best_lcp) *best_lcp = ctx->h_top->val[0];
   for (int k = 0; k < K; ++k) {
-    if (topk_index) topk_index[k] = hidx[k];
-    if (topk_lcp) topk_lcp[k] = hval[k];
+    if (topk_index) topk_index[k] = ctx->h_top->idx[k];
+    if (topk_lcp) topk_lcp[k] = ctx->h_top->val[k];
   }
   return STOCS_OK;
 }
@@ -497,7 +494,9 @@ int stocs_b200_score_counters(stocs_b200_ctx* ctx, const float* d_T16, int64_t H
   unsigned long long* d_cnt = ctx->scratch()->score_counts;
   unsigned long long h[sizeof(DevScratch::score_counts) / 8] = {0};
   STOCS_CUDA(ctx, cudaMemsetAsync(d_cnt, 0, sizeof(h), st));
-  int rc = stocs_launch_score(ctx, d_T16, H, d_lcp.as<float>(), d_inl.as<int32_t>(), st, false, 0, d_cnt);
+  ScoreRequest rq;
+  rq.counters = d_cnt;
+  int rc = stocs_launch_score(ctx, d_T16, H, d_lcp.as<float>(), d_inl.as<int32_t>(), st, rq);
   if (rc) return rc;
   STOCS_CUDA(ctx, cudaMemcpyAsync(h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
   STOCS_CUDA(ctx, cudaStreamSynchronize(st));

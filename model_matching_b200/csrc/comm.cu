@@ -124,13 +124,17 @@ __global__ void __launch_bounds__(1024) merge_records_kernel(const stocs_b200_re
 // cannot enter the top K may be left unscored (lcp 0, see kPrune in score.cu)
 int enqueue_local_topk(stocs_b200_ctx* ctx, const float* d_T, int64_t H_local, int64_t index_offset, int K,
                        float* d_lcp, int32_t* d_inl, stocs_b200_record* d_send, cudaStream_t st, bool time_it, bool prune) {
-  if (H_local > 0) {
-    int rc = stocs_launch_score(ctx, d_T, H_local, d_lcp, d_inl, st, time_it, 0, nullptr, stocs_host_alias(d_T) != nullptr,
-                                nullptr, 0, prune ? K : 0);
-    if (rc) return rc;
-  }
-  // H_local == 0: the top-K kernels run over an empty array and emit K empty records
-  return stocs_launch_topk(ctx, d_lcp, H_local, K, index_offset, nullptr, nullptr, st, d_T, d_inl, d_send);
+  ScoreRequest sq;
+  sq.time_it = time_it;
+  sq.top_K = prune ? K : 0;
+  int rc = stocs_launch_score(ctx, d_T, H_local, d_lcp, d_inl, st, sq);
+  if (rc) return rc;
+  // H_local == 0: nothing is scored, the top-K kernels run over an empty array and emit K empty records
+  TopkRequest tq;
+  tq.T16 = d_T;
+  tq.inl = d_inl;
+  tq.rec = d_send;
+  return stocs_launch_topk(ctx, d_lcp, H_local, K, index_offset, st, tq);
 }
 
 // the buffers of the collective: K local records (POOL_COMM_SEND), nranks*K gathered records
@@ -238,67 +242,26 @@ int stocs_b200_score_sharded(stocs_b200_ctx* ctx, const float* T16_local, int64_
     STOCS_FAIL(ctx, STOCS_E_ARG, "score_sharded: bad argument");
   if (ctx->S <= 0 || ctx->M <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "score_sharded: upload_model and upload_scene first");
   cudaSetDevice(ctx->device);
-  cudaStream_t st = ctx->stream;
-  // 1. the local block through the host-buffer scoring call (page-locked transforms read in place,
-  //    pageable ones staged in overlapped chunks); per-hypothesis results come back as in the
-  //    single-GPU drop-in, into the caller's arrays or into a context-owned page-locked scratch
-  if (H_local > 0 && !lcp_local) {
-    if (ctx->h_pinned_bytes < (size_t)H_local * 4) {
-      if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
-      ctx->h_pinned = nullptr; ctx->h_pinned_bytes = 0;
-      STOCS_CUDA(ctx, cudaHostAlloc(&ctx->h_pinned, (size_t)H_local * 4, cudaHostAllocDefault));
-      ctx->h_pinned_bytes = (size_t)H_local * 4;
-    }
-    lcp_local = (float*)ctx->h_pinned;
-  }
   const int nranks = ctx->comm ? ctx->comm_nranks : 1;
   STOCS_CUDA(ctx, ensure_record_buffers(ctx, K, nranks));
-  DevBuf& b_out = ctx->pool[POOL_COMM_OUT];
-  stocs_b200_record* d_local = nranks > 1 ? ctx->pool[POOL_COMM_SEND].as<stocs_b200_record>() : b_out.as<stocs_b200_record>();
-  // Page-locked, device-mapped transforms: ONE pass with ONE synchronisation.  The kernel reads the
-  // transforms in place over PCIe; then the per-hypothesis results go back on the context stream
-  // while, on the second stream, the K best are packed, all-gathered and merged.  (Going through
-  // stocs_b200_score_lcp first costs its own top-32 reduction and a second synchronisation:
-  // 0.58 -> 0.50 ms per step at 125 000 hypotheses per rank on 8 GPUs.)
-  if (const float* d_T = H_local > 0 ? stocs_zero_copy_transforms(T16_local) : nullptr) {
-    STOCS_CUDA(ctx, ctx->d_lcp.ensure((size_t)H_local * 4));
-    STOCS_CUDA(ctx, ctx->d_inl.ensure((size_t)H_local * 4));
-    ctx->top_valid = false;
-    int rc = stocs_launch_score(ctx, d_T, H_local, ctx->d_lcp.as<float>(), ctx->d_inl.as<int32_t>(), st, true, 0, nullptr, true);
+  stocs_b200_record* d_out = ctx->pool[POOL_COMM_OUT].as<stocs_b200_record>();
+  stocs_b200_record* d_local = nranks > 1 ? ctx->pool[POOL_COMM_SEND].as<stocs_b200_record>() : d_out;
+  // ONE pass with ONE synchronisation: the records are the tail of the host-buffer scoring call --
+  // the K best of the resident results as records, ONE all-gather and the merge, the K merged
+  // records back.  (Scoring through the single-GPU host call first, with its own top-32 reduction
+  // and synchronisation, cost 0.58 against 0.50 ms per step at 125 000 hypotheses per rank on 8 GPUs.)
+  auto tail = [&](cudaStream_t st, const float* d_T) -> int {
+    TopkRequest tq;
+    tq.T16 = d_T;
+    tq.inl = ctx->d_inl.as<int32_t>();
+    tq.rec = d_local;
+    int rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H_local, K, index_offset, st, tq);
+    if (rc == STOCS_OK && nranks > 1) rc = gather_merge_records(ctx, K, d_out, st);
     if (rc) return rc;
-    ctx->last_H = H_local;
-    ctx->last_T_dev = d_T;
-    cudaStream_t aux = ctx->aux_stream;
-    STOCS_CUDA(ctx, cudaEventRecord(ctx->join_ev[0], st));
-    STOCS_CUDA(ctx, cudaStreamWaitEvent(aux, ctx->join_ev[0], 0));
-    STOCS_CUDA(ctx, cudaMemcpyAsync(lcp_local, ctx->d_lcp.p, (size_t)H_local * 4, cudaMemcpyDeviceToHost, st));
-    if (inliers_local)
-      STOCS_CUDA(ctx, cudaMemcpyAsync(inliers_local, ctx->d_inl.p, (size_t)H_local * 4, cudaMemcpyDeviceToHost, st));
-    rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H_local, K, index_offset, nullptr, nullptr, aux, d_T,
-                           ctx->d_inl.as<int32_t>(), d_local);
-    if (rc) return rc;
-    if (nranks > 1) rc = gather_merge_records(ctx, K, b_out.as<stocs_b200_record>(), aux);
-    if (rc) return rc;
-    STOCS_CUDA(ctx, cudaMemcpyAsync(topk_out, b_out.p, (size_t)K * sizeof(stocs_b200_record), cudaMemcpyDeviceToHost, aux));
-    STOCS_CUDA(ctx, cudaEventRecord(ctx->join_ev[1], aux));
-    STOCS_CUDA(ctx, cudaStreamWaitEvent(st, ctx->join_ev[1], 0));
-    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
+    STOCS_CUDA(ctx, cudaMemcpyAsync(topk_out, d_out, (size_t)K * sizeof(stocs_b200_record), cudaMemcpyDeviceToHost, st));
     return STOCS_OK;
-  }
-  if (H_local > 0) {
-    int rc = stocs_b200_score_lcp(ctx, T16_local, H_local, lcp_local, inliers_local);
-    if (rc) return rc;
-  }
-  // 2. K best of the resident results as records, 3. ONE all-gather, 4. merge
-  STOCS_CUDA(ctx, ctx->d_lcp.ensure(4));
-  int rc = stocs_launch_topk(ctx, ctx->d_lcp.as<float>(), H_local, K, index_offset, nullptr, nullptr, st,
-                             H_local > 0 ? ctx->last_T_dev : nullptr, H_local > 0 ? ctx->d_inl.as<int32_t>() : nullptr, d_local);
-  if (rc) return rc;
-  if (nranks > 1) rc = gather_merge_records(ctx, K, b_out.as<stocs_b200_record>(), st);
-  if (rc) return rc;
-  STOCS_CUDA(ctx, cudaMemcpyAsync(topk_out, b_out.p, (size_t)K * sizeof(stocs_b200_record), cudaMemcpyDeviceToHost, st));
-  STOCS_CUDA(ctx, cudaStreamSynchronize(st));
-  return STOCS_OK;
+  };
+  return stocs_score_host(ctx, "score_sharded", T16_local, H_local, lcp_local, inliers_local, tail);
 }
 
 }  // extern "C"

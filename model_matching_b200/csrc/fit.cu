@@ -332,14 +332,23 @@ static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, in
     fit_kernel<<<(unsigned)fit_blocks, 128, 0, st>>>(a);
     tr.mark("pipeline: select + fit");
     // 4. score + 5. best
-    rc = stocs_launch_score(ctx, d_Tc, cap_items, d_lcp, d_inl, st, true, 0, nullptr, false, &d_state->n_items, guess);
+    ScoreRequest sq;
+    sq.time_it = true;
+    sq.d_H = &d_state->n_items;
+    sq.grid_hint = guess;
+    rc = stocs_launch_score(ctx, d_Tc, cap_items, d_lcp, d_inl, st, sq);
     if (rc) return rc;
     long long* d_bi = &ctx->scratch()->pipe_best_idx;
     float* d_bv = &ctx->scratch()->pipe_best_lcp;
     // lists the closing block can scan itself (every online frame) skip the general top-K launch
     const bool small_list = cap_items <= (1ll << 20);
     if (!small_list) {
-      rc = stocs_launch_topk(ctx, d_lcp, cap_items, 1, 0, (int64_t*)d_bi, d_bv, st, nullptr, nullptr, nullptr, &d_state->n_items, guess);
+      TopkRequest tq;
+      tq.idx = (int64_t*)d_bi;
+      tq.val = d_bv;
+      tq.d_H = &d_state->n_items;
+      tq.grid_hint = guess;
+      rc = stocs_launch_topk(ctx, d_lcp, cap_items, 1, 0, st, tq);
       if (rc) return rc;
     }
     pipe_finalize_kernel<<<1, 1024, 0, st>>>(small_list ? d_lcp : nullptr, d_ok, d_valid, n_bases, d_item_base, d_bi, d_bv, d_Tc, d_Tw, d_state);

@@ -206,12 +206,11 @@ extern "C" int stocs_b200_select_above(stocs_b200_ctx* ctx, const float* lcp, in
 }
 
 int stocs_launch_topk(stocs_b200_ctx* ctx, const float* d_lcp, int64_t H, int K, int64_t index_offset,
-                      int64_t* d_idx, float* d_val, cudaStream_t st, const float* d_T16, const int32_t* d_inl,
-                      stocs_b200_record* d_rec, const long long* d_H, long long grid_hint) {
+                      cudaStream_t st, const TopkRequest& rq) {
   if (K < 1 || K > 32) STOCS_FAIL(ctx, STOCS_E_ARG, "reduce_best: K must be in 1..32");
   if (H >= (1ll << 32)) STOCS_FAIL(ctx, STOCS_E_ARG, "reduce_best: H must be < 2^32");
   int blocks = ctx->num_sms * 2;
-  long long need = ((d_H && grid_hint > 0 && grid_hint < H ? grid_hint : H) + 2047) / 2048;   // at least 256 keys per warp: fewer, longer lists for the merge
+  long long need = ((rq.d_H && rq.grid_hint > 0 && rq.grid_hint < H ? rq.grid_hint : H) + 2047) / 2048;   // at least 256 keys per warp: fewer, longer lists for the merge
   if (need < 1) need = 1;
   if (blocks > need) blocks = (int)need;
   // per-stream scratch: launches on the context stream and on its second stream (the host-buffer
@@ -221,7 +220,7 @@ int stocs_launch_topk(stocs_b200_ctx* ctx, const float* d_lcp, int64_t H, int K,
   STOCS_CUDA(ctx, lists.ensure((size_t)blocks * 32 * 8));
   unsigned* ticket = &ctx->scratch()->topk_ticket[which];   // zero at creation, reset by the last CTA
   topk_kernel<<<blocks, 256, 0, st>>>(d_lcp, H, lists.as<unsigned long long>(), ticket, K, index_offset,
-                                      (long long*)d_idx, d_val, d_T16, d_inl, d_rec, d_H);
+                                      (long long*)rq.idx, rq.val, rq.T16, rq.inl, rq.rec, rq.d_H);
   STOCS_CUDA(ctx, cudaGetLastError());
   return STOCS_OK;
 }

@@ -793,10 +793,15 @@ bool stocs_fmad_selftest(stocs_b200_ctx* ctx) {
 }
 
 int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl,
-                       cudaStream_t st, bool time_it, int slot, unsigned long long* d_counters, bool T_in_host_memory,
-                       const long long* d_H, long long grid_hint, int prune_K) {
+                       cudaStream_t st, const ScoreRequest& rq) {
   if (H <= 0) return STOCS_OK;
   if (H >= (1ll << 31)) STOCS_FAIL(ctx, STOCS_E_ARG, "score: at most 2^31-1 hypotheses per call");
+  // the pruned instantiation exists for one launch shape: slot 0, count on the host, no counting
+  if (rq.top_K > 0 && (rq.counters || rq.d_H || rq.slot != 0))
+    STOCS_FAIL(ctx, STOCS_E_ARG, "score: a top-K launch takes no counters, device count or slot");
+  const int slot = rq.slot;
+  unsigned long long* const d_counters = rq.counters;
+  const long long* const d_H = rq.d_H;
   // the kd-tree of a freshly uploaded scene may still be under construction on a host thread: collect
   // it and queue its upload in front of this launch (no-op on every later launch)
   if (ctx->kd_pending) { const int rc = stocs_kd_finish(ctx, st); if (rc) return rc; }
@@ -816,7 +821,7 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   a.T = d_T;
   a.lcp = d_lcp;
   a.inl = d_inl;
-  // slot 0 is the default work counter; launches that may run concurrently (score_lcp's chunks
+  // slot 0 is the default work counter; launches that may run concurrently (staged host-buffer chunks
   // on two streams) take distinct slots.  One tie counter accumulates over all launches.
   DevScratch* scr = ctx->scratch();
   unsigned long long* wctr = &scr->work[slot];
@@ -833,19 +838,19 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   a.dot_thr = ctx->dot_thr;
   a.to_block = 1.0f / (float)(1u << ctx->coarse_shift);
   a.to_cell = (float)(1u << ctx->coarse_shift);
-  // top-K pruning: only for a caller that receives nothing but the K best records (prune_K = K), and
+  // top-K pruning: only for a caller that receives nothing but the K best records (top_K = K), and
   // only on a scene whose class weights are all finite and >= 0 (the bound needs w_max)
   // (and with the lowest bucket edge a normal float, see lcp_bucket)
   unsigned wbits;
   memcpy(&wbits, &ctx->w_max, 4);
   const int key_lo = (int)(wbits >> 19) + 1 - (kBuckets - 1);
-  const bool prune = prune_K > 0 && ctx->prune_ok && key_lo >= 16 && !d_counters && !d_H && slot == 0;
+  const bool prune = rq.top_K > 0 && ctx->prune_ok && key_lo >= 16;
   a.prune = nullptr;
   a.rejected = scr->score_totals.rejected;
   a.w_max = ctx->w_max;
   a.bound_scale = 1.0f + (float)(ctx->M + 2) * 0x1p-23f;   // exact: M + 2 < 2^13
   a.key_lo = (unsigned)key_lo;
-  a.K = prune_K;
+  a.K = rq.top_K;
   if (prune) {
     // [0, 8) work counter, [128, 132) theta bucket, [256, 768) bucket counts: one memset per launch
     DevBuf& b = ctx->pool[POOL_SCORE_PRUNE];
@@ -864,7 +869,7 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   int per_sm = 0;
   STOCS_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kWarps * 32, smem));
   if (per_sm < 1) STOCS_FAIL(ctx, STOCS_E_ARG, "score: model too large for shared memory");
-  long long want = ((d_H && grid_hint > 0 && grid_hint < H ? grid_hint : H) + kWarps - 1) / kWarps;
+  long long want = ((d_H && rq.grid_hint > 0 && rq.grid_hint < H ? rq.grid_hint : H) + kWarps - 1) / kWarps;
   long long grid = (long long)ctx->num_sms * per_sm;
   if (grid > want) grid = want;
   STOCS_CUDA(ctx, cudaMemsetAsync(wctr, 0, prune ? 256 + kBuckets * 4 : 8, st));  // tie counter accumulates
@@ -878,7 +883,7 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   const long long lpt_max = getenv("STOCS_LPT_MAX") ? atoll(getenv("STOCS_LPT_MAX")) : 300000;
   // (not when the transforms are read in place from page-locked host memory: the probe would pull
   // every transform over PCIe a second time -- measured 1.7e9 -> 0.9e9 hypotheses/s end to end on 8 GPUs)
-  if (!no_lpt && !d_counters && !T_in_host_memory && !d_H && H >= 32768 && H <= lpt_max && slot == 0) {
+  if (!no_lpt && !d_counters && !d_H && H >= 32768 && H <= lpt_max && slot == 0 && !stocs_host_alias(d_T)) {
     DevBuf& b_order = ctx->pool[POOL_SCORE_ORDER];
     STOCS_CUDA(ctx, b_order.ensure((size_t)H * 4));
     unsigned* fill = scr->lpt_fill;
@@ -887,7 +892,7 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
     probe_order_kernel<<<(unsigned)((H + 255) / 256), 256, psm, st>>>(a, b_order.as<int>(), fill, 16);
     a.order = b_order.as<int>();
   }
-  if (time_it) {  // next pair of the ring (events are created on first use)
+  if (rq.time_it) {  // next pair of the ring (events are created on first use)
     const int k = (int)(ctx->ev_count % stocs_b200_ctx::kEvRing);
     for (int j = 0; j < 2; ++j)
       if (!ctx->ev_ring[2 * k + j]) STOCS_CUDA(ctx, cudaEventCreate(&ctx->ev_ring[2 * k + j]));
@@ -896,9 +901,9 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
     STOCS_CUDA(ctx, cudaEventRecord(ctx->ev0, st));
   }
   kernel<<<(unsigned)grid, kWarps * 32, smem, st>>>(a);
-  if (time_it) { STOCS_CUDA(ctx, cudaEventRecord(ctx->ev1, st)); ctx->ev_count++; }
+  if (rq.time_it) { STOCS_CUDA(ctx, cudaEventRecord(ctx->ev1, st)); ctx->ev_count++; }
   STOCS_CUDA(ctx, cudaGetLastError());
   ctx->counters[CTR_SCORE_LAUNCHES] += 1;
-  ctx->timing_valid = time_it;
+  ctx->timing_valid = rq.time_it;
   return STOCS_OK;
 }

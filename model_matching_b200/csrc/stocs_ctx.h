@@ -6,6 +6,7 @@
 #include <chrono>
 #include <cstdio>
 #include <cstdlib>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -76,7 +77,7 @@ enum PoolSlot : int {
   // capi.cu: top-32 of the resident lcp array
   POOL_TOPK_RESIDENT = 37,
   // comm.cu: packed 64-byte records (local K, gathered world*K, merged K)
-  POOL_COMM_SEND = 38, POOL_COMM_RECV, POOL_COMM_OUT, POOL_COMM_TOPK,
+  POOL_COMM_SEND = 38, POOL_COMM_RECV, POOL_COMM_OUT,
   // sharded scoring scratch (transforms / lcp / inliers of the local shard)
   POOL_SHARD_T = 42, POOL_SHARD_LCP, POOL_SHARD_INL,
   // score.cu: claim order of the heavy-first schedule (one int per hypothesis of the launch)
@@ -147,8 +148,8 @@ struct stocs_b200_ctx {
   static constexpr int kEvRing = 512;
   cudaEvent_t ev_ring[2 * kEvRing] = {};
   int64_t ev_count = 0;
-  static constexpr int kMaxChunks = 4;    // chunks of score_lcp's geometric plan
-  cudaEvent_t chunk_ev[kMaxChunks] = {};  // H2D-complete events of score_lcp's chunks
+  static constexpr int kMaxChunks = 4;    // chunks of the staged host-buffer scoring plan (stocs_score_host)
+  cudaEvent_t chunk_ev[kMaxChunks] = {};  // H2D-complete events of those chunks
   cudaEvent_t join_ev[2] = {nullptr, nullptr};
   std::string err;
 
@@ -210,8 +211,6 @@ struct stocs_b200_ctx {
   // scratch (d_small: 4 KB, laid out by DevScratch)
   DevBuf d_T, d_lcp, d_inl, d_work, d_tmp, d_tmp2, d_small;
   DevScratch* scratch() const { return d_small.as<DevScratch>(); }
-  void* h_pinned = nullptr;
-  size_t h_pinned_bytes = 0;
 
   // capacities the online stages are enqueued against (entries; grown when a search reports overflow)
   long long cong_cap_codes = 1 << 18, cong_cap_quads = 1 << 21;
@@ -226,10 +225,9 @@ struct stocs_b200_ctx {
   struct KdPending* kd_pending = nullptr;   // kd-tree of the current scene, still being built on a host thread
   cudaEvent_t kd_copy_done = nullptr;       // the staging buffer may be overwritten once this has completed
 
-  // last score call
+  // resident lcp array (d_lcp / d_inl) of the last host-buffer score call or explicit reduce_best
   int64_t last_H = 0;
-  const float* last_T_dev = nullptr;   // device-visible transforms of the last host-buffer score call
-  // top-32 of the resident lcp array, computed by score_lcp behind its result copies
+  // top-32 of the resident lcp array, computed by score_lcp behind its result copies and by reduce_best
   struct TopCache { int64_t idx[32]; float val[32]; };
   TopCache* h_top = nullptr;   // page-locked
   bool top_valid = false;
@@ -245,7 +243,7 @@ struct stocs_b200_ctx {
 // stocs_b200_create zeroes it once.  Fields marked ZERO-RELIANT count on that and are never cleared
 // again; every other field is written by its stage before it is read.
 struct DevScratch {
-  // score.cu: work counter of a scoring launch per slot (slot 0 by default, score_lcp's chunks use
+  // score.cu: work counter of a scoring launch per slot (slot 0 by default, staged host-buffer chunks use
   // their chunk number so that concurrent chunks do not share one); cleared before each launch
   unsigned long long work[stocs_b200_ctx::kMaxChunks];
   // score.cu, ZERO-RELIANT: NN queries resolved by the kd-tree tie path, and top-K hypotheses
@@ -298,12 +296,20 @@ int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4*
                         float* d_out3, float* h_centroid3, float* h_aabb6, const float* h_pos3 = nullptr,
                         float* h_centred3 = nullptr);
 int stocs_pack_scene_attr(stocs_b200_ctx* ctx, const float* d_nrm3, const float* d_cls, int S);
-int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp,
-                       int32_t* d_inl, cudaStream_t st, bool time_it, int slot = 0,
-                       unsigned long long* d_counters = nullptr, bool T_in_host_memory = false,
-                       const long long* d_H = nullptr, long long grid_hint = 0,
-                       int prune_K = 0);  // score.cu (d_H: the count lives on the device, H bounds it, grid_hint sizes
-                                          // the launch; prune_K > 0: only the K best will be read, see kPrune)
+// One scoring launch (score.cu).  The caller states which instantiation it wants: per-hypothesis
+// results (the default), only the K best (top_K = K: hypotheses that provably cannot enter them may
+// be left unscored, lcp 0, see kPrune; slot 0 only, no device count) or counting (counters: the
+// ScoreCounter slots).
+struct ScoreRequest {
+  bool time_it = false;                    // events around the launch (stocs_b200_kernel_ms_stats)
+  int slot = 0;                            // work counter; launches that may run concurrently take distinct slots
+  int top_K = 0;
+  unsigned long long* counters = nullptr;
+  const long long* d_H = nullptr;          // the count lives on the device, H bounds it ...
+  long long grid_hint = 0;                 // ... and grid_hint sizes the launch
+};
+int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl,
+                       cudaStream_t st, const ScoreRequest& rq);
 int stocs_launch_backproject(stocs_b200_ctx* ctx, const uint16_t* d_depth, const uint8_t* d_bgr,
                              int W, int H, float fx, float cx, float fy, float cy, float scale,
                              float* d_xyz, uint32_t* d_rgb, cudaStream_t st);  // backproject.cu
@@ -317,11 +323,30 @@ const void* stocs_host_alias(const void* p);
 const float* stocs_zero_copy_transforms(const float* T16);
 // w_max / prune_ok of the scene from its class weights (capi.cu; every writer of the weights calls it)
 void stocs_set_weight_bound(stocs_b200_ctx* ctx, const float* cls, int S);
-// top-K of a device lcp array (reduce.cu); d_idx/d_val may be NULL when only records are wanted
+// Outputs of one top-K reduction of a device lcp array (reduce.cu): the K best as (index, lcp)
+// pairs (idx and val together) and/or as 64-byte records, which read the scored transforms (T16)
+// and inlier counts (inl, may be NULL) as well
+struct TopkRequest {
+  int64_t* idx = nullptr;
+  float* val = nullptr;
+  const float* T16 = nullptr;
+  const int32_t* inl = nullptr;
+  stocs_b200_record* rec = nullptr;
+  const long long* d_H = nullptr;          // as for ScoreRequest
+  long long grid_hint = 0;
+};
 int stocs_launch_topk(stocs_b200_ctx* ctx, const float* d_lcp, int64_t H, int K, int64_t index_offset,
-                      int64_t* d_idx, float* d_val, cudaStream_t st, const float* d_T16 = nullptr,
-                      const int32_t* d_inl = nullptr, stocs_b200_record* d_rec = nullptr,
-                      const long long* d_H = nullptr, long long grid_hint = 0);   // as for stocs_launch_score
+                      cudaStream_t st, const TopkRequest& rq);
+// Host-buffer scoring (capi.cu; stocs_b200_score_lcp, stocs_b200_score_sharded): scores H host
+// transforms into the resident ctx->d_lcp / d_inl, copies back whichever of lcp / inliers is
+// non-NULL, enqueues tail(stream, device-visible transforms), joins the second stream and
+// synchronises once.  After the first error nothing more is enqueued, but the join and the
+// synchronisation still happen; that first error is returned.  On success the resident array
+// holds H results (last_H); on failure last_H is 0.  H == 0: nothing is scored, the resident
+// state is untouched and only the tail runs, on the context stream.  `who` prefixes error messages.
+using ScoreTail = std::function<int(cudaStream_t, const float*)>;
+int stocs_score_host(stocs_b200_ctx* ctx, const char* who, const float* T16, int64_t H, float* lcp, int32_t* inliers,
+                     const ScoreTail& tail);
 float stocs_angle_threshold_dot();                                         // capi.cu (host)
 
 // STOCS_TRACE=1: wall-clock of each stage of a host-driven sequence on stderr (adds a synchronize
