@@ -223,6 +223,51 @@ int stocs_b200_run_pipeline(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int
 int stocs_b200_run_pipeline_instance(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets,
                                      float dispersion, stocs_b200_pipeline_result* result);
 
+/* ---- f3: greedy pose clustering (clustering::greedy_clustering, src/pose_clustering.cpp:79-122) ----
+ * Keeps the candidates with lcp > acceptable_fraction * best_score (product in binary32), orders them
+ * by lcp descending (equal lcps: index ascending, the shim's std::stable_sort), and walks them in that
+ * order: a candidate is dropped when some already kept pose c gives get_pose_diff(candidate, c) with
+ * rotation < min_angle AND translation < min_distance.  As in the reference the walk stops once MORE
+ * than maximum_pose_count poses are kept, so up to maximum_pose_count + 1 come back.  The pose distance
+ * is csrc/stocs_pose_math.h, which the host shim's get_pose_diff calls too: both keep the same poses.
+ * Runs on the device in one CTA after a device sort; the call synchronises once. */
+typedef struct stocs_b200_cluster_params {
+  float acceptable_fraction;
+  int32_t maximum_pose_count;   /* 0..1023; up to maximum_pose_count + 1 poses are returned (reference break rule) */
+  float min_distance;           /* metres, translation of the world poses */
+  float min_angle;              /* degrees, max Euler angle after symmetry folding */
+  float sym_info[3];            /* per axis: 90, 180, 360 or anything else (no folding), as pose_clustering.cpp:31-48 */
+} stocs_b200_cluster_params;
+
+typedef struct stocs_b200_pose {
+  int64_t index;       /* rank in the list of pushed transforms: the convention of pipeline_result.best_index */
+  float lcp;
+  int32_t base;        /* PoseCandidate::base_index, as pipeline_result.best_base */
+  float T_centred[16];
+  float T_world[16];   /* PoseCandidate::transform: the pose the clustering compares */
+} stocs_b200_pose;     /* 144 bytes */
+
+/* greedy_clustering over H host poses (world, column-major) and their LCPs.  Needs no model or scene.
+ * index_out receives the kept indices in the order they were kept (index_out[0] is the best candidate
+ * when any qualifies), *n_out their number.  STOCS_E_ARG: p or n_out NULL, maximum_pose_count outside
+ * 0..1023, cap < maximum_pose_count + 1 (results are never partial), H outside 0 <= H < 2^31. */
+int stocs_b200_cluster_poses(stocs_b200_ctx* ctx, const float* T16_world, const float* lcp, int64_t H,
+                             float best_score, const stocs_b200_cluster_params* p,
+                             int64_t* index_out, int64_t cap, int64_t* n_out);
+
+/* run_pipeline[_instance] + greedy_clustering of its scored list, best_score = the run's best LCP.
+ * The candidates are the transforms the fit pushed (a failed fit is never a candidate); poses[k].index
+ * is the rank among them, so poses[0] is the result's best pose whenever there is one.  `result` is
+ * what the plain call returns; the clustering is enqueued behind it and the call still synchronises
+ * once.  cap < maximum_pose_count + 1 is STOCS_E_ARG. */
+int stocs_b200_run_pipeline_clustered(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets,
+                                      const stocs_b200_cluster_params* p, stocs_b200_pipeline_result* result,
+                                      stocs_b200_pose* poses, int cap, int* n_poses);
+int stocs_b200_run_pipeline_instance_clustered(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets,
+                                               float dispersion, const stocs_b200_cluster_params* p,
+                                               stocs_b200_pipeline_result* result, stocs_b200_pose* poses,
+                                               int cap, int* n_poses);
+
 /* ---- e: multi-GPU, hypothesis sharding (SURVEY.md section 8e) -------------------------------
  * The reference scores its hypotheses in one sequential loop (src/stocs.cpp:990-998); they are
  * independent, so the list is split into contiguous blocks, one per GPU.  Every GPU holds a replica

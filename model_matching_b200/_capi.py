@@ -25,7 +25,8 @@ SYMBOLS = [
     "stocs_b200_find_congruent", "stocs_b200_fit_transforms", "stocs_b200_score_lcp",
     "stocs_b200_score_lcp_device", "stocs_b200_reduce_best", "stocs_b200_reduce_best_device", "stocs_b200_select_above",
     "stocs_b200_icp_point_to_plane",
-    "stocs_b200_run_pipeline", "stocs_b200_run_pipeline_instance", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
+    "stocs_b200_run_pipeline", "stocs_b200_run_pipeline_instance", "stocs_b200_cluster_poses",
+    "stocs_b200_run_pipeline_clustered", "stocs_b200_run_pipeline_instance_clustered", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
     "stocs_b200_score_counters", "stocs_b200_kernel_ms_stats", "stocs_b200_host_kdtree_order",
     "stocs_b200_debug_angle_estimates",
     "stocs_b200_comm_unique_id", "stocs_b200_comm_init", "stocs_b200_comm_destroy", "stocs_b200_shard_range",
@@ -45,6 +46,17 @@ class PipelineResult(C.Structure):
                 ("n_transforms", C.c_int64), ("best_index", C.c_int64), ("best_lcp", C.c_float),
                 ("best_base", C.c_int32), ("best_T_centred", C.c_float * 16),
                 ("best_T_world", C.c_float * 16)]
+
+
+class ClusterParams(C.Structure):
+    _fields_ = [("acceptable_fraction", C.c_float), ("maximum_pose_count", C.c_int32), ("min_distance", C.c_float),
+                ("min_angle", C.c_float), ("sym_info", C.c_float * 3)]
+
+
+# stocs_b200_pose (include/stocs_b200.h): one pose kept by the clustered pipeline
+POSE = np.dtype([("index", np.int64), ("lcp", np.float32), ("base", np.int32), ("T_centred", np.float32, (16,)),
+                 ("T_world", np.float32, (16,))])
+assert POSE.itemsize == 144
 
 
 def lib():
@@ -92,6 +104,11 @@ def lib():
     L.stocs_b200_icp_point_to_plane.argtypes = [vp, vp, i32, vp, vp, i32, i32, f32, vp, vp, vp, C.POINTER(i32), C.POINTER(i32)]
     L.stocs_b200_run_pipeline.argtypes = [vp, u64, i32, i32, C.POINTER(PipelineResult)]
     L.stocs_b200_run_pipeline_instance.argtypes = [vp, u64, i32, i32, f32, C.POINTER(PipelineResult)]
+    L.stocs_b200_cluster_poses.argtypes = [vp, vp, vp, i64, f32, C.POINTER(ClusterParams), vp, i64, C.POINTER(i64)]
+    L.stocs_b200_run_pipeline_clustered.argtypes = [vp, u64, i32, i32, C.POINTER(ClusterParams), C.POINTER(PipelineResult),
+                                                    vp, i32, C.POINTER(i32)]
+    L.stocs_b200_run_pipeline_instance_clustered.argtypes = [vp, u64, i32, i32, f32, C.POINTER(ClusterParams),
+                                                             C.POINTER(PipelineResult), vp, i32, C.POINTER(i32)]
     L.stocs_b200_get_counters.argtypes = [vp, vp, i32]
     L.stocs_b200_last_kernel_ms.argtypes = [vp, C.POINTER(f32)]
     L.stocs_b200_score_counters.argtypes = [vp, vp, i64, vp, i32]
@@ -133,6 +150,11 @@ def _f32(a, shape=None):
 # stocs_b200_record (include/stocs_b200.h): the 64-byte unit of the multi-GPU all-gather
 RECORD = np.dtype([("lcp", np.float32), ("inliers", np.int32), ("index", np.int64), ("T", np.float32, (12,))])
 assert RECORD.itemsize == 64
+
+
+def _cluster_params(acceptable_fraction, maximum_pose_count, min_distance, min_angle, sym_info=(0, 0, 0)):
+    return ClusterParams(acceptable_fraction, int(maximum_pose_count), min_distance, min_angle,
+                         (C.c_float * 3)(*[float(v) for v in sym_info]))
 
 
 def host_kdtree_order(pos):
@@ -439,6 +461,40 @@ class Context:
         r = PipelineResult()
         self._check(self._L.stocs_b200_run_pipeline_instance(self.h, int(seed), n_bases, max_sets, dispersion, C.byref(r)))
         return r
+
+    # ---- f3: greedy pose clustering
+    def cluster_poses(self, T_world, lcp, best_score, acceptable_fraction, maximum_pose_count, min_distance, min_angle,
+                      sym_info=(0, 0, 0)):
+        """clustering::greedy_clustering on the device -> int64 array of the kept indices, in the order kept
+        (T_world: H world poses, 4x4 row-major or 16 column-major floats each)."""
+        lcp = _f32(lcp, (-1,))
+        T = np.asarray(T_world, np.float32)
+        T = _f32(T.transpose(0, 2, 1) if T.ndim == 3 else T, (-1, 16))
+        assert T.shape[0] == lcp.shape[0]
+        p = _cluster_params(acceptable_fraction, maximum_pose_count, min_distance, min_angle, sym_info)
+        cap = max(int(maximum_pose_count) + 1, 1)
+        out, n = np.empty(cap, np.int64), C.c_int64(0)
+        self._check(self._L.stocs_b200_cluster_poses(self.h, _ptr(T), _ptr(lcp), lcp.shape[0], best_score, C.byref(p),
+                                                      _ptr(out), cap, C.byref(n)))
+        return out[:n.value].copy()
+
+    def run_pipeline_clustered(self, seed, n_bases=100, max_sets=200, **params):
+        """run_pipeline + greedy clustering of its scored list -> (PipelineResult, POSE array).
+        params: acceptable_fraction, maximum_pose_count, min_distance, min_angle, sym_info=(0, 0, 0)"""
+        p = _cluster_params(**params)
+        r, poses, n = PipelineResult(), np.zeros(max(p.maximum_pose_count + 1, 1), POSE), C.c_int32(0)
+        self._check(self._L.stocs_b200_run_pipeline_clustered(self.h, int(seed), n_bases, max_sets, C.byref(p), C.byref(r),
+                                                               _ptr(poses), poses.shape[0], C.byref(n)))
+        return r, poses[:n.value].copy()
+
+    def run_pipeline_instance_clustered(self, seed, n_bases=100, max_sets=200, dispersion=0.9, **params):
+        """run_pipeline_instance + greedy clustering of its scored list -> (PipelineResult, POSE array)"""
+        p = _cluster_params(**params)
+        r, poses, n = PipelineResult(), np.zeros(max(p.maximum_pose_count + 1, 1), POSE), C.c_int32(0)
+        self._check(self._L.stocs_b200_run_pipeline_instance_clustered(self.h, int(seed), n_bases, max_sets, dispersion,
+                                                                        C.byref(p), C.byref(r), _ptr(poses), poses.shape[0],
+                                                                        C.byref(n)))
+        return r, poses[:n.value].copy()
 
     def counters(self):
         c = np.zeros(9, np.int64)

@@ -239,6 +239,7 @@ void stocs_b200_destroy(stocs_b200_ctx* ctx) {
   if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
   if (ctx->h_top) cudaFreeHost(ctx->h_top);
   if (ctx->h_pipe_state) cudaFreeHost(ctx->h_pipe_state);
+  stocs_cluster_free_host(ctx);
   if (ctx->h_index_counts) cudaFreeHost(ctx->h_index_counts);
   if (ctx->h_kd_stage) cudaFreeHost(ctx->h_kd_stage);
   if (ctx->kd_copy_done) cudaEventDestroy(ctx->kd_copy_done);

@@ -263,9 +263,15 @@ int stocs_launch_sample_instance(stocs_b200_ctx* ctx, uint64_t seed, int base_nu
 // coupled: one launch per base, base numbers 1..n_bases).  The whole chain -- bases, congruent sets, item
 // selection, fits, scores, best, result record -- is enqueued back to back against capacities and the
 // host synchronises ONCE, on the 200-byte state record (round 1: six synchronisations per pose).
+// cp != NULL: the greedy clustering of the scored list (cluster.cu) is enqueued behind the result record
+// and its poses come back in the same queue; with cp == NULL nothing of it is enqueued.
 static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets, int mode, float dispersion,
-                             stocs_b200_pipeline_result* result) {
+                             stocs_b200_pipeline_result* result, const stocs_b200_cluster_params* cp = nullptr,
+                             stocs_b200_pose* poses = nullptr, int cap = 0, int* n_poses = nullptr) {
   if (!ctx) return STOCS_E_ARG;
+  if (cp && (!poses || !n_poses)) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline_clustered: bad argument");
+  if (cp && stocs_cluster_check(ctx, cp, cap)) return STOCS_E_ARG;
+  if (n_poses) *n_poses = 0;
   if (ctx->S <= 0 || ctx->M <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "run_pipeline: upload_model and upload_scene first");
   if (n_bases <= 0 || max_sets <= 0 || !result) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline: bad argument");
   if (mode == 1 && n_bases > 255) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline: instance mode numbers its bases 1..255");
@@ -353,6 +359,11 @@ static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, in
     }
     pipe_finalize_kernel<<<1, 1024, 0, st>>>(small_list ? d_lcp : nullptr, d_ok, d_valid, n_bases, d_item_base, d_bi, d_bv, d_Tc, d_Tw, d_state);
     STOCS_CUDA(ctx, cudaGetLastError());
+    if (cp) {
+      const PipeClusterInputs ci = {d_lcp, d_Tc, d_Tw, d_ok, d_valid, d_item_base, cap_items, d_state};
+      rc = stocs_cluster_enqueue_pipeline(ctx, *cp, ci, st);
+      if (rc) return rc;
+    }
     STOCS_CUDA(ctx, cudaMemcpyAsync(&hs, d_state, sizeof(StocsPipeState), cudaMemcpyDeviceToHost, st));
     STOCS_CUDA(ctx, cudaStreamSynchronize(st));
     tr.mark("pipeline: score + best");
@@ -370,6 +381,10 @@ static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, in
     memcpy(result->best_T_centred, hs.best_Tc, 64);
     memcpy(result->best_T_world, hs.best_Tw, 64);
   }
+  if (cp) {
+    memcpy(poses, stocs_cluster_poses_host(ctx), (size_t)hs.n_poses * sizeof(stocs_b200_pose));
+    *n_poses = hs.n_poses;
+  }
   return STOCS_OK;
 }
 
@@ -381,4 +396,21 @@ extern "C" int stocs_b200_run_pipeline(stocs_b200_ctx* ctx, uint64_t seed, int n
 extern "C" int stocs_b200_run_pipeline_instance(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets,
                                                 float dispersion, stocs_b200_pipeline_result* result) {
   return run_pipeline_impl(ctx, seed, n_bases, max_sets, 1, dispersion, result);
+}
+
+extern "C" int stocs_b200_run_pipeline_clustered(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets,
+                                                 const stocs_b200_cluster_params* p, stocs_b200_pipeline_result* result,
+                                                 stocs_b200_pose* poses, int cap, int* n_poses) {
+  if (!ctx) return STOCS_E_ARG;
+  if (!p) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline_clustered: params are NULL");
+  return run_pipeline_impl(ctx, seed, n_bases, max_sets, 0, 0.f, result, p, poses, cap, n_poses);
+}
+
+extern "C" int stocs_b200_run_pipeline_instance_clustered(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets,
+                                                          float dispersion, const stocs_b200_cluster_params* p,
+                                                          stocs_b200_pipeline_result* result, stocs_b200_pose* poses,
+                                                          int cap, int* n_poses) {
+  if (!ctx) return STOCS_E_ARG;
+  if (!p) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline_clustered: params are NULL");
+  return run_pipeline_impl(ctx, seed, n_bases, max_sets, 1, dispersion, result, p, poses, cap, n_poses);
 }

@@ -3,8 +3,8 @@
 // Replaces the argmax loop of stocs_estimator::compute_best_transform (reference
 // src/stocs.cpp:987-1001: FIRST strict maximum wins, index -1 when every score is 0) and produces
 // the K best candidates that feed clustering::greedy_clustering (src/pose_clustering.cpp:79-122).
-// Keys are (lcp bits << 32) | ~index, so a larger key is a larger score or, at equal score, a
-// smaller index.  Each warp keeps a sorted top-32 across its lanes (lane j = j-th best) and
+// Keys are (ordered lcp bits << 32) | ~index, so a larger key is a larger score or, at equal score,
+// a smaller index; key 0 is "no entry" (the low word of a real key is never 0, indices being < 2^32 - 1).  Each warp keeps a sorted top-32 across its lanes (lane j = j-th best) and
 // inserts with one ballot + shuffle per surviving key; a single-warp kernel merges the per-warp
 // lists.  Memory traffic: one read of the LCP array.
 #include <cub/device/device_radix_sort.cuh>
@@ -23,8 +23,19 @@ __device__ __forceinline__ void warp_insert(unsigned long long& mine, unsigned l
   else if (lane > pos) mine = up;
 }
 
+// Order-preserving map of binary32 onto uint32 (sign bit flipped for positives, all bits for
+// negatives), -0.0 folded onto +0.0: the clustering filter `lcp > threshold` admits lcp <= 0 when the
+// threshold is negative, and its `>` holds -0.0 and +0.0 equal, so the index must break that tie.
+__device__ __forceinline__ unsigned ordered_bits(float v) {
+  const unsigned u = __float_as_uint(v == 0.f ? 0.f : v);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float key_lcp(unsigned long long key) {
+  const unsigned o = (unsigned)(key >> 32);
+  return __uint_as_float((o & 0x80000000u) ? (o & 0x7fffffffu) : ~o);
+}
 __device__ __forceinline__ unsigned long long make_key(float v, unsigned long long idx) {
-  return ((unsigned long long)__float_as_uint(v) << 32) | (0xffffffffull - (idx & 0xffffffffull));
+  return ((unsigned long long)ordered_bits(v) << 32) | (0xffffffffull - (idx & 0xffffffffull));
 }
 
 // offer one key per lane to the warp's sorted list
@@ -116,7 +127,7 @@ __global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ lcp
       if (mine == 0ull) { out_idx[lane] = -1; out_lcp[lane] = 0.f; }
       else {
         out_idx[lane] = local + index_offset;
-        out_lcp[lane] = __uint_as_float((unsigned)(mine >> 32));
+        out_lcp[lane] = key_lcp(mine);
       }
     }
     if (rec_out) {
@@ -125,7 +136,7 @@ __global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ lcp
 #pragma unroll
       for (int k = 0; k < 12; ++k) r.T[k] = 0.f;
       if (mine != 0ull) {
-        r.lcp = __uint_as_float((unsigned)(mine >> 32));
+        r.lcp = key_lcp(mine);
         r.inliers = inl ? inl[local] : 0;
         r.index = local + index_offset;
         const float* t = T16 + 16 * local;   // column-major 4x4 -> rows 0..2, row-major
@@ -139,11 +150,19 @@ __global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ lcp
   }
 }
 
-__global__ void above_keys_kernel(const float* __restrict__ lcp, long long H, float thr, unsigned long long* __restrict__ keys) {
+// key of every entry i < H: make_key(lcp[i], i) when lcp[i] > threshold (and > 0 with positive_only,
+// and ok[i] != 0 with ok), 0 otherwise.  The threshold is thr, or thr * *thr_scale computed here when
+// thr_scale is given (a factor times a best score that lives on the device).  H_dev: entries at or
+// beyond the device count get key 0.
+__global__ void above_keys_kernel(const float* __restrict__ lcp, long long H, float thr, const float* __restrict__ thr_scale,
+                                  bool positive_only, const uint8_t* __restrict__ ok, const long long* __restrict__ H_dev,
+                                  unsigned long long* __restrict__ keys) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= H) return;
-  const float v = lcp[i];
-  keys[i] = (v > thr && v > 0.f) ? make_key(v, (unsigned long long)i) : 0ull;
+  if (thr_scale) thr = thr * *thr_scale;
+  const bool in = (!H_dev || i < *H_dev) && (!ok || ok[i]);
+  const float v = in ? lcp[i] : 0.f;
+  keys[i] = (in && v > thr && (!positive_only || v > 0.f)) ? make_key(v, (unsigned long long)i) : 0ull;
 }
 struct NonZero { __device__ bool operator()(unsigned long long k) const { return k != 0ull; } };
 __global__ void unpack_keys_kernel(const unsigned long long* __restrict__ keys, long long n, long long* __restrict__ idx,
@@ -151,7 +170,7 @@ __global__ void unpack_keys_kernel(const unsigned long long* __restrict__ keys, 
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   idx[i] = (long long)(0xffffffffull - (keys[i] & 0xffffffffull));
-  val[i] = __uint_as_float((unsigned)(keys[i] >> 32));
+  val[i] = key_lcp(keys[i]);
 }
 
 }  // namespace
@@ -180,7 +199,8 @@ extern "C" int stocs_b200_select_above(stocs_b200_ctx* ctx, const float* lcp, in
   auto cleanup = [&]() { ka.release(); kb.release(); tmp.release(); cnt.release(); oi.release(); ov.release(); };
 #define SA(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { ctx->err = std::string(#call) + ": " + cudaGetErrorString(_e); cleanup(); return STOCS_E_CUDA; } } while (0)
   SA(ka.ensure((size_t)H * 8)); SA(kb.ensure((size_t)H * 8)); SA(cnt.ensure(16));
-  above_keys_kernel<<<(unsigned)((H + 255) / 256), 256, 0, st>>>(d_src, H, threshold, ka.as<unsigned long long>());
+  above_keys_kernel<<<(unsigned)((H + 255) / 256), 256, 0, st>>>(d_src, H, threshold, nullptr, true, nullptr, nullptr,
+                                                                  ka.as<unsigned long long>());
   size_t tb = 0, tb2 = 0;
   cub::DeviceSelect::If(nullptr, tb, ka.as<unsigned long long>(), kb.as<unsigned long long>(), cnt.as<int>(), (int)H, NonZero(), st);
   cub::DeviceRadixSort::SortKeysDescending(nullptr, tb2, kb.as<unsigned long long>(), ka.as<unsigned long long>(), (int)H, 0, 64, st);
@@ -222,5 +242,23 @@ int stocs_launch_topk(stocs_b200_ctx* ctx, const float* d_lcp, int64_t H, int K,
   topk_kernel<<<blocks, 256, 0, st>>>(d_lcp, H, lists.as<unsigned long long>(), ticket, K, index_offset,
                                       (long long*)rq.idx, rq.val, rq.T16, rq.inl, rq.rec, rq.d_H);
   STOCS_CUDA(ctx, cudaGetLastError());
+  return STOCS_OK;
+}
+
+// The filter + order of clustering::greedy_clustering over a device list, without a host round trip:
+// keys[0..H) = make_key of every entry with (ok[i] and) lcp[i] > thr * *thr_scale (or > thr), sorted
+// descending into keys_out, non-candidates (key 0) last.  tmp / tmp_bytes: cub scratch (query with
+// tmp == NULL: *tmp_bytes is set and nothing is enqueued).
+int stocs_enqueue_cluster_keys(stocs_b200_ctx* ctx, const float* d_lcp, int64_t H, float thr, const float* d_thr_scale,
+                               const uint8_t* d_ok, const long long* d_H, unsigned long long* keys,
+                               unsigned long long* keys_out, void* tmp, size_t* tmp_bytes, cudaStream_t st) {
+  if (!tmp) {
+    STOCS_CUDA(ctx, cub::DeviceRadixSort::SortKeysDescending(nullptr, *tmp_bytes, keys, keys_out, (int)H, 0, 64, st));
+    return STOCS_OK;
+  }
+  if (H == 0) return STOCS_OK;
+  above_keys_kernel<<<(unsigned)((H + 255) / 256), 256, 0, st>>>(d_lcp, H, thr, d_thr_scale, false, d_ok, d_H, keys);
+  STOCS_CUDA(ctx, cudaGetLastError());
+  STOCS_CUDA(ctx, cub::DeviceRadixSort::SortKeysDescending(tmp, *tmp_bytes, keys, keys_out, (int)H, 0, 64, st));
   return STOCS_OK;
 }

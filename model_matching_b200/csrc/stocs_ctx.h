@@ -96,6 +96,8 @@ enum PoolSlot : int {
   POOL_CONG_NEXT = 51, POOL_CONG_BSTART = 52, POOL_CONG_BUCKET = 53,
   // score.cu: work counter, theta and bucket counts of a top-K-pruned scoring launch
   POOL_SCORE_PRUNE = 54,
+  // cluster.cu: sort keys, cub scratch, kept poses (and the uploaded poses of stocs_b200_cluster_poses)
+  POOL_CLUSTER = 55,
   POOL_COUNT = 56
 };
 
@@ -114,7 +116,7 @@ struct StocsPipeState {
   long long best_item, rank_of_best;
   int n_valid, best_base;
   float best_lcp;
-  int pad;
+  int n_poses;                     // poses kept by the clustering of a clustered run (cluster.cu)
   float best_Tc[16], best_Tw[16];
 };
 
@@ -218,6 +220,7 @@ struct stocs_b200_ctx {
   bool cong_bcount_clean = false;      // ... and whether the last search left them zero
   long long pipe_last_items = 0;       // transforms of the previous pipeline run (sizes the next run's grids)
   StocsPipeState* h_pipe_state = nullptr;   // page-locked landing zone of the state record
+  struct ClusterHost* h_cluster = nullptr;  // page-locked landing zone of the clustering results (cluster.cu)
   uint32_t* h_index_counts = nullptr;       // page-locked: list lengths of the scene-index build
   size_t index_counts_clean = 0;            // leading words of pool[POOL_INDEX_COUNTS] known to be zero
   void* h_kd_stage = nullptr;               // page-locked staging of the kd-tree upload (frame-sized scenes)
@@ -348,6 +351,20 @@ using ScoreTail = std::function<int(cudaStream_t, const float*)>;
 int stocs_score_host(stocs_b200_ctx* ctx, const char* who, const float* T16, int64_t H, float* lcp, int32_t* inliers,
                      const ScoreTail& tail);
 float stocs_angle_threshold_dot();                                         // capi.cu (host)
+// Greedy clustering of a pipeline run's scored list (cluster.cu), enqueued behind pipe_finalize_kernel:
+// candidates are the fitted items (ok) below the device count, best score = the state's best_lcp; the
+// kept poses land in ctx->h_cluster and their number in the state record's n_poses.
+struct PipeClusterInputs {
+  const float* lcp; const float* Tc; const float* Tw;
+  const uint8_t* ok; const uint8_t* valid; const int* item_base;
+  long long cap_items;
+  StocsPipeState* d_state;
+};
+int stocs_cluster_check(stocs_b200_ctx* ctx, const stocs_b200_cluster_params* p, int64_t cap);
+int stocs_cluster_enqueue_pipeline(stocs_b200_ctx* ctx, const stocs_b200_cluster_params& p, const PipeClusterInputs& in,
+                                   cudaStream_t st);
+const stocs_b200_pose* stocs_cluster_poses_host(stocs_b200_ctx* ctx);
+void stocs_cluster_free_host(stocs_b200_ctx* ctx);
 
 // STOCS_TRACE=1: wall-clock of each stage of a host-driven sequence on stderr (adds a synchronize
 // per stage, so the total is not the untraced time).

@@ -1,7 +1,9 @@
 // pose_clustering.hpp -- same declarations as the reference's include/pose_clustering.hpp:9-28.
-// greedy_clustering is a faithful host restatement (the pass is serial and tiny: it runs over the
-// few hypotheses that survive `lcp > acceptable_fraction * best_score`; on large hypothesis lists
-// that filter + descending sort is available on the GPU as stocs_b200_select_above).
+// greedy_clustering is a faithful host restatement, one candidate at a time against every kept pose.
+// That suits the shim's few thousand candidates; for the lists the device produces (10^5..10^6 scored
+// hypotheses) the same pass runs on the GPU as stocs_b200_cluster_poses, and the fused pipeline
+// clusters its own scored list (stocs_b200_run_pipeline[_instance]_clustered).  Both keep the same
+// poses: get_pose_diff is csrc/stocs_pose_math.h, which the kernels call too.
 // point_to_plane_icp (pcl::IterativeClosestPointWithNormals in the reference, PCL not being part
 // of the reference tree) runs PCL's published point-to-plane loop on the GPU through
 // stocs_b200_icp_point_to_plane (csrc/icp.cu, arithmetic in csrc/stocs_icp_math.h).
