@@ -69,6 +69,26 @@ int stocs_b200_build_scene_cloud(stocs_b200_ctx* ctx, const uint16_t* depth, con
                                  float class_threshold, float* pos3, float* nrm3, float* rgb3,
                                  int32_t* pixel_rc, float* class_p, float* edge_p, int64_t cap, int64_t* n_out);
 
+/* The scene clouds of n_objects objects of one frame in one call: the back-projection, voxel grid, outlier
+ * removal and depth normals run once, and only the class test runs per object.  class_probs holds
+ * n_objects H*W uint16 maps, object after object; class_thresholds one threshold per object.  The
+ * outputs are those of build_scene_cloud, concatenated: object k's points are rows
+ * [offsets[k], offsets[k+1]) (offsets: n_objects + 1 entries, the CSR of find_congruent), and that slice
+ * is bit-identical, in the same order, to build_scene_cloud on (class_probs[k], class_thresholds[k]).
+ * rgb3 and edge_p may be NULL.  More than cap points in all: STOCS_E_CAPACITY with offsets filled.
+ * STOCS_E_ARG: n_objects outside 1..STOCS_B200_MAX_CLOUD_OBJECTS, class_probs, class_thresholds or
+ * offsets NULL, the argument checks of build_scene_cloud, or a required output NULL while points are
+ * emitted.  Like build_scene_cloud, the call synchronises once when its read-back estimate (from the
+ * previous call) covers the output, twice otherwise.  Device memory per object, held by the context:
+ * one 4-byte flag per pixel plus the 2-byte map (1.8 MB at 640x480), besides the output rows. */
+#define STOCS_B200_MAX_CLOUD_OBJECTS 32
+int stocs_b200_build_scene_clouds(stocs_b200_ctx* ctx, const uint16_t* depth, const uint8_t* bgr,
+                                  const uint16_t* class_probs, const float* class_thresholds, int n_objects,
+                                  const uint8_t* edge, int W, int H, float fx, float cx, float fy, float cy,
+                                  float depth_scale, float voxel_size,
+                                  float* pos3, float* nrm3, float* rgb3, int32_t* pixel_rc, float* class_p,
+                                  float* edge_p, int64_t cap, int64_t* offsets);
+
 /* ---- a2/a11: model and scene upload --------------------------------------------------------
  * upload_model replaces load_object_info's point part (src/stocs.cpp:86-97) and the model half of
  * centroid_shift (src/stocs.cpp:951-962); it also builds the compact own-bin PPF table that

@@ -16,7 +16,8 @@ _LIB = None
 # every symbol include/stocs_b200.h declares (checked by tests/test_abi.py)
 SYMBOLS = [
     "stocs_b200_abi_version", "stocs_b200_create", "stocs_b200_destroy", "stocs_b200_last_error",
-    "stocs_b200_set_params", "stocs_b200_backproject", "stocs_b200_build_scene_cloud", "stocs_b200_upload_model",
+    "stocs_b200_set_params", "stocs_b200_backproject", "stocs_b200_build_scene_cloud", "stocs_b200_build_scene_clouds",
+    "stocs_b200_upload_model",
     "stocs_b200_upload_scene", "stocs_b200_get_centroids", "stocs_b200_get_centred",
     "stocs_b200_ppf_num_pairs", "stocs_b200_ppf_num_expanded_keys", "stocs_b200_ppf_export",
     "stocs_b200_ppf_lookup", "stocs_b200_upload_ppf_table", "stocs_b200_sample_bases",
@@ -80,6 +81,8 @@ def lib():
     L.stocs_b200_backproject.argtypes = [vp, vp, vp, i32, i32, f32, f32, f32, f32, f32, vp, vp]
     L.stocs_b200_build_scene_cloud.argtypes = [vp, vp, vp, vp, vp, i32, i32, f32, f32, f32, f32, f32, f32, f32,
                                                vp, vp, vp, vp, vp, vp, i64, C.POINTER(i64)]
+    L.stocs_b200_build_scene_clouds.argtypes = [vp, vp, vp, vp, vp, i32, vp, i32, i32, f32, f32, f32, f32, f32, f32,
+                                                vp, vp, vp, vp, vp, vp, i64, vp]
     L.stocs_b200_upload_model.argtypes = [vp, vp, vp, i32]
     L.stocs_b200_upload_scene.argtypes = [vp, vp, vp, vp, vp, i32]
     L.stocs_b200_get_centroids.argtypes = [vp, vp, vp]
@@ -247,6 +250,34 @@ class Context:
         k = n.value
         return dict(pos=pos[:k].copy(), nrm=nrm[:k].copy(), rgb=rgb[:k].copy(), pix=pix[:k].copy(), cls=cls[:k].copy(),
                     edge=ep[:k].copy())
+
+    def build_scene_clouds(self, depth, bgr, probs, edge, K, depth_scale, voxel_size, class_thresholds):
+        """The scene clouds of n objects of one frame in one call: probs (n, H, W), class_thresholds a scalar or n
+        values -> n dicts, each equal to build_scene_cloud with that object's map and threshold."""
+        depth = np.ascontiguousarray(depth, np.uint16)
+        H, W = depth.shape
+        bgr = None if bgr is None else np.ascontiguousarray(bgr, np.uint8)
+        probs = np.ascontiguousarray(probs, np.uint16)
+        assert probs.ndim == 3 and probs.shape[1:] == (H, W), "probs must be (n, H, W)"
+        n_obj = probs.shape[0]
+        thr = np.ascontiguousarray(np.broadcast_to(np.asarray(class_thresholds, np.float32), (n_obj,)))
+        edge = None if edge is None else np.ascontiguousarray(edge, np.uint8)
+        offs = np.zeros(n_obj + 1, np.int64)
+        cap = H * W   # one object's bound; a frame with more points in all is run again at its exact size
+        while True:
+            pos, nrm, rgb = (np.empty((cap, 3), np.float32) for _ in range(3))
+            pix = np.empty((cap, 2), np.int32)
+            cls, ep = np.empty(cap, np.float32), np.empty(cap, np.float32)
+            rc = self._L.stocs_b200_build_scene_clouds(self.h, _ptr(depth), _ptr(bgr), _ptr(probs), _ptr(thr), n_obj,
+                                                       _ptr(edge), W, H, K[0], K[1], K[2], K[3], depth_scale, voxel_size,
+                                                       _ptr(pos), _ptr(nrm), _ptr(rgb), _ptr(pix), _ptr(cls), _ptr(ep),
+                                                       cap, _ptr(offs))
+            if rc == -5:  # STOCS_E_CAPACITY: offsets are filled
+                cap = int(offs[-1])
+                continue
+            self._check(rc)
+            return [dict(pos=pos[a:b].copy(), nrm=nrm[a:b].copy(), rgb=rgb[a:b].copy(), pix=pix[a:b].copy(),
+                         cls=cls[a:b].copy(), edge=ep[a:b].copy()) for a, b in zip(offs[:-1], offs[1:])]
 
     # ---- uploads
     def upload_model(self, pos, nrm):

@@ -198,7 +198,7 @@ int stocs_b200_create(stocs_b200_ctx** out, int device) {
             cudaEventCreateWithFlags(&ctx->join_ev[1], cudaEventDisableTiming) == cudaSuccess;
   ok = ok && cudaHostAlloc((void**)&ctx->h_top, sizeof(stocs_b200_ctx::TopCache), cudaHostAllocDefault) == cudaSuccess;
   ok = ok && cudaHostAlloc((void**)&ctx->h_pipe_state, sizeof(StocsPipeState), cudaHostAllocDefault) == cudaSuccess;
-  ok = ok && cudaHostAlloc((void**)&ctx->h_index_counts, 64, cudaHostAllocDefault) == cudaSuccess;
+  ok = ok && cudaHostAlloc((void**)&ctx->h_index_counts, 4 * (8 + 1 + STOCS_B200_MAX_CLOUD_OBJECTS), cudaHostAllocDefault) == cudaSuccess;
   for (int i = 0; ok && i < stocs_b200_ctx::kMaxChunks; ++i)
     ok = cudaEventCreateWithFlags(&ctx->chunk_ev[i], cudaEventDisableTiming) == cudaSuccess;
   if (!ok) { g_create_err = "stream/event creation failed"; delete ctx; return STOCS_E_CUDA; }

@@ -63,7 +63,8 @@ enum PoolSlot : int {
   POOL_CONG_QE, POOL_CONG_QCELL, POOL_CONG_CNT, POOL_CONG_SCAN, POOL_CONG_QOFF, POOL_CONG_QUADS = 11,
   // scene_index.cu (upload_scene): 12..15
   POOL_INDEX_DENSE = 12, POOL_INDEX_MASKS, POOL_INDEX_OCC, POOL_INDEX_OCC_SCAN,
-  // scene_cloud.cu (build_scene_cloud): 12..30
+  // scene_cloud.cu (build_scene_cloud[s]): 12..30; POOL_CLOUD_PROB holds one map per object, POOL_CLOUD_FLAGS
+  // one row flag per (object, pixel)
   POOL_CLOUD_DEPTH = 12, POOL_CLOUD_BGR, POOL_CLOUD_PROB, POOL_CLOUD_EDGE, POOL_CLOUD_XYZ, POOL_CLOUD_KEYS_A,
   POOL_CLOUD_KEYS_B, POOL_CLOUD_IDX_A, POOL_CLOUD_IDX_B, POOL_CLOUD_TMP, POOL_CLOUD_FLAGS, POOL_CLOUD_SCAN,
   POOL_CLOUD_STARTS, POOL_CLOUD_UKEYS, POOL_CLOUD_CENT, POOL_CLOUD_KEEP, POOL_CLOUD_NRM, POOL_CLOUD_RC,
@@ -221,7 +222,8 @@ struct stocs_b200_ctx {
   long long pipe_last_items = 0;       // transforms of the previous pipeline run (sizes the next run's grids)
   StocsPipeState* h_pipe_state = nullptr;   // page-locked landing zone of the state record
   struct ClusterHost* h_cluster = nullptr;  // page-locked landing zone of the clustering results (cluster.cu)
-  uint32_t* h_index_counts = nullptr;       // page-locked: list lengths of the scene-index build
+  uint32_t* h_index_counts = nullptr;       // page-locked: list lengths of the scene-index build [0, 8) and of
+                                            // the scene-cloud build [8, 8 + 1 + STOCS_B200_MAX_CLOUD_OBJECTS)
   size_t index_counts_clean = 0;            // leading words of pool[POOL_INDEX_COUNTS] known to be zero
   void* h_kd_stage = nullptr;               // page-locked staging of the kd-tree upload (frame-sized scenes)
   size_t h_kd_stage_bytes = 0;
@@ -235,6 +237,8 @@ struct stocs_b200_ctx {
   TopCache* h_top = nullptr;   // page-locked
   bool top_valid = false;
   int64_t counters[CTR_COUNT] = {0};
+  // points of the last build_scene_cloud[s] (all objects): with CTR_CLOUD_VOXELS, the next call's read-back estimate
+  long long cloud_last_points = 0;
   bool timing_valid = false;
 
   // multi-GPU (comm.cu): one NCCL communicator per context; ncclComm_t kept opaque here
@@ -276,8 +280,9 @@ struct DevScratch {
   int inst_ids[4];
   float inst_inv[2];
   uint8_t inst_valid;
-  // scene_cloud.cu (build_scene_cloud): first zero-depth pixel, zero-depth pixels, valid pixels, voxels
-  int cloud[4];
+  // scene_cloud.cu (build_scene_clouds): first zero-depth pixel, zero-depth pixels, valid pixels, voxels, then
+  // the end of each object's rows in the concatenated output
+  int cloud[4 + STOCS_B200_MAX_CLOUD_OBJECTS];
 };
 static_assert(sizeof(DevScratch) <= 4096, "DevScratch must fit the 4 KB d_small allocation");
 
