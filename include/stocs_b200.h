@@ -288,6 +288,53 @@ int stocs_b200_run_pipeline_instance_clustered(stocs_b200_ctx* ctx, uint64_t see
                                                stocs_b200_pipeline_result* result, stocs_b200_pose* poses,
                                                int cap, int* n_poses);
 
+/* ---- a15/f3: several objects of one frame, one context per object ------------------------------
+ * A context holds one object's model, PPF table, scene and instance state and shares nothing with other
+ * contexts, so a caller who keeps one context per object also keeps every model resident across frames.
+ * These two calls give K such contexts a frame's work together: every object's work is enqueued on its
+ * own context's stream, stage by stage across the objects, and the host waits once at the end, so the
+ * objects' chains of small launches overlap on the device.  Every object's device buffers are grown before
+ * any object's work is enqueued (growth frees memory, which waits for the whole device).  Each context's work runs under
+ * cudaSetDevice(ctx->device); the contexts may sit on different devices.
+ *
+ * Equivalence: object k's outcome is bit-identical to the single call on ctxs[k] (upload_scene on its
+ * slice; run_pipeline, run_pipeline_instance, run_pipeline_clustered or run_pipeline_instance_clustered
+ * with seeds[k] and cluster[k]), and each context ends in the state that single call leaves: centroid,
+ * centred points, grid, candidate lists, kd-tree, class-weight bound, pixel range, reset instance state,
+ * counters [2], [3] and [6]; instance mode advances each context's prior decay and mask cache.
+ *
+ * Empty slices (an object that is not visible): upload_scenes leaves that context with no scene (counters
+ * [2], [3] and [6] zero) and marks it as holding an empty scene; run_pipelines then returns the no-pose result for it (zeros,
+ * best_index and best_base -1, n_poses 0) and enqueues nothing for it.  The single calls are unchanged:
+ * upload_scene with S = 0 is STOCS_E_ARG, run_pipeline without a scene STOCS_E_STATE.
+ *
+ * Validation happens before anything is enqueued on any context, and a rejected call changes no context:
+ * n_objects < 1, a NULL entry or one context given twice (STOCS_E_ARG; the objects would share a stream
+ * and scratch), NULL required arrays, offsets that do not start at 0 or decrease, a slice over 2^27
+ * points, any argument check of the single call, a context without a model or without any scene (never
+ * uploaded, or its last upload failed: STOCS_E_STATE), in instance mode an edge map or pixel coordinates
+ * missing, in a clustered run a bad parameter record or cap < maximum_pose_count + 1.  The error text
+ * ("<call>: object k: ...") names the object and is set on the failing context and on ctxs[0].
+ *
+ * Errors after validation (a CUDA error, a kernel error, non-finite coordinates found while centring):
+ * the first in object order is returned; every other object completes as its single call would, the
+ * failing context is left as its single call leaves it, and no stream has work pending on return.
+ * An object whose capacities overflow (congruent code/quad buffers, candidate records) is grown and
+ * enqueued again on its own, with the same result.  The input buffers are not referenced after return. */
+
+/* Object k's scene = rows [offsets[k], offsets[k+1]) of the arrays stocs_b200_build_scene_clouds writes
+ * (pos3, nrm3, class_p as class_probability, pixel_rc or NULL); offsets has n_objects + 1 entries. */
+int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const float* pos3, const float* nrm3,
+                             const float* class_probability, const int32_t* pixel_rc, const int64_t* offsets);
+
+/* instance_mode 0 or 1; cluster: NULL (plain run) or n_objects parameter records (sym_info is per
+ * object); results: n_objects records; poses: n_objects * cap records, object k's at poses + k * cap, and
+ * n_poses: n_objects entries (both used by a clustered run only; n_poses is zeroed when given). */
+int stocs_b200_run_pipelines(stocs_b200_ctx* const* ctxs, int n_objects, const uint64_t* seeds, int n_bases,
+                             int max_sets, int instance_mode, float dispersion,
+                             const stocs_b200_cluster_params* cluster, stocs_b200_pipeline_result* results,
+                             stocs_b200_pose* poses, int cap, int* n_poses);
+
 /* ---- e: multi-GPU, hypothesis sharding (SURVEY.md section 8e) -------------------------------
  * The reference scores its hypotheses in one sequential loop (src/stocs.cpp:990-998); they are
  * independent, so the list is split into contiguous blocks, one per GPU.  Every GPU holds a replica

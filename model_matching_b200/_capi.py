@@ -5,6 +5,7 @@ no CPU fallback: importing works without a GPU (so that the symbol table can be 
 creating a Context without a B200 raises, and a missing .so raises at import of `lib()`.
 """
 import ctypes as C
+import itertools
 import os
 
 import numpy as np
@@ -27,7 +28,8 @@ SYMBOLS = [
     "stocs_b200_score_lcp_device", "stocs_b200_reduce_best", "stocs_b200_reduce_best_device", "stocs_b200_select_above",
     "stocs_b200_icp_point_to_plane",
     "stocs_b200_run_pipeline", "stocs_b200_run_pipeline_instance", "stocs_b200_cluster_poses",
-    "stocs_b200_run_pipeline_clustered", "stocs_b200_run_pipeline_instance_clustered", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
+    "stocs_b200_run_pipeline_clustered", "stocs_b200_run_pipeline_instance_clustered",
+    "stocs_b200_upload_scenes", "stocs_b200_run_pipelines", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
     "stocs_b200_score_counters", "stocs_b200_kernel_ms_stats", "stocs_b200_host_kdtree_order",
     "stocs_b200_debug_angle_estimates",
     "stocs_b200_comm_unique_id", "stocs_b200_comm_init", "stocs_b200_comm_destroy", "stocs_b200_shard_range",
@@ -112,6 +114,8 @@ def lib():
                                                     vp, i32, C.POINTER(i32)]
     L.stocs_b200_run_pipeline_instance_clustered.argtypes = [vp, u64, i32, i32, f32, C.POINTER(ClusterParams),
                                                              C.POINTER(PipelineResult), vp, i32, C.POINTER(i32)]
+    L.stocs_b200_upload_scenes.argtypes = [vp, i32, vp, vp, vp, vp, vp]
+    L.stocs_b200_run_pipelines.argtypes = [vp, i32, vp, i32, i32, i32, f32, vp, vp, vp, i32, vp]
     L.stocs_b200_get_counters.argtypes = [vp, vp, i32]
     L.stocs_b200_last_kernel_ms.argtypes = [vp, C.POINTER(f32)]
     L.stocs_b200_score_counters.argtypes = [vp, vp, i64, vp, i32]
@@ -158,6 +162,69 @@ assert RECORD.itemsize == 64
 def _cluster_params(acceptable_fraction, maximum_pose_count, min_distance, min_angle, sym_info=(0, 0, 0)):
     return ClusterParams(acceptable_fraction, int(maximum_pose_count), min_distance, min_angle,
                          (C.c_float * 3)(*[float(v) for v in sym_info]))
+
+
+def _handles(contexts):
+    assert len(contexts) >= 1, "at least one context"
+    return (C.c_void_p * len(contexts))(*[c.h for c in contexts])
+
+
+def _has_scene(ctx):
+    return lib().stocs_b200_get_centroids(ctx.h, _ptr(np.zeros(3, np.float32)), None) == 0
+
+
+def upload_scenes(contexts, clouds):
+    """Object k's cloud (a dict of Context.build_scene_clouds: pos, nrm, cls and optionally pix) to contexts[k],
+    every object in one call (stocs_b200_upload_scenes); an empty cloud leaves its context with an empty scene."""
+    assert len(contexts) == len(clouds), "one cloud per context"
+    n = [len(c["pos"]) for c in clouds]
+    if len({id(c) for c in contexts}) < len(contexts) or any(not c.h for c in contexts) or max(n, default=0) > (1 << 27):
+        raise StocsError("upload_scenes: a context given twice or closed, or a slice over 2^27 points")
+    offs = np.fromiter(itertools.accumulate(n, initial=0), np.int64, len(n) + 1)
+    has_pix = all(c.get("pix") is not None for c in clouds)
+    if len(clouds) == 1:   # one object's arrays are passed as they are
+        c = clouds[0]
+        pos, nrm, cls = _f32(c["pos"], (-1, 3)), _f32(c["nrm"], (-1, 3)), _f32(c["cls"], (-1,))
+        pix = np.ascontiguousarray(c["pix"], np.int32).reshape(-1, 2) if has_pix else None
+    else:                  # the CSR concatenation
+        pos = np.concatenate([_f32(c["pos"], (-1, 3)) for c in clouds])
+        nrm = np.concatenate([_f32(c["nrm"], (-1, 3)) for c in clouds])
+        cls = np.concatenate([_f32(c["cls"], (-1,)) for c in clouds])
+        pix = np.concatenate([np.ascontiguousarray(c["pix"], np.int32).reshape(-1, 2) for c in clouds]) if has_pix else None
+    assert pos.shape == nrm.shape and cls.shape[0] == pos.shape[0]
+    rc = lib().stocs_b200_upload_scenes(_handles(contexts), len(contexts), _ptr(pos), _ptr(nrm), _ptr(cls), _ptr(pix),
+                                        _ptr(offs))
+    err = None
+    try:
+        contexts[0]._check(rc)
+    except StocsError as e:
+        err = e
+    for c, k in zip(contexts, n):
+        # the arguments passed the checks above, so a failure came after validation: the objects that
+        # uploaded hold their slice, the failing one (and any empty slice) holds none
+        c.S = k if err is None or _has_scene(c) else 0
+    if err is not None:
+        raise err
+
+
+def run_pipelines(contexts, seeds, n_bases=100, max_sets=200, instance=False, dispersion=0.9, cluster=None):
+    """run_pipeline[_instance][_clustered] on every context in one call (stocs_b200_run_pipelines), with seeds[k]
+    on contexts[k].  cluster: None, or one dict of cluster parameters per object (acceptable_fraction,
+    maximum_pose_count, min_distance, min_angle, sym_info).  -> [PipelineResult], or [(PipelineResult, POSE array)]."""
+    n = len(contexts)
+    seeds = np.ascontiguousarray(np.asarray(seeds, np.uint64).reshape(n))
+    results = (PipelineResult * n)()
+    if cluster is None:
+        contexts[0]._check(lib().stocs_b200_run_pipelines(_handles(contexts), n, _ptr(seeds), n_bases, max_sets, int(instance),
+                                                          dispersion, None, results, None, 0, None))
+        return list(results)
+    assert len(cluster) == n, "one cluster parameter record per object"
+    params = (ClusterParams * n)(*[_cluster_params(**p) for p in cluster])
+    cap = max(max(p.maximum_pose_count for p in params) + 1, 1)
+    poses, n_poses = np.zeros((n, cap), POSE), np.zeros(n, np.int32)
+    contexts[0]._check(lib().stocs_b200_run_pipelines(_handles(contexts), n, _ptr(seeds), n_bases, max_sets, int(instance),
+                                                      dispersion, params, results, _ptr(poses), cap, _ptr(n_poses)))
+    return [(results[k], poses[k, :n_poses[k]].copy()) for k in range(n)]
 
 
 def host_kdtree_order(pos):

@@ -328,32 +328,25 @@ int stocs_b200_upload_model(stocs_b200_ctx* ctx, const float* pos3, const float*
   return stocs_build_ppf_table(ctx);
 }
 
-int stocs_b200_upload_scene(stocs_b200_ctx* ctx, const float* pos3, const float* nrm3,
-                            const float* class_probability, const int32_t* pixel_rc, int S) {
-  if (!ctx) return STOCS_E_ARG;
-  if (!pos3 || !nrm3 || !class_probability || S <= 0) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: bad argument");
-  if (S > (1 << 27)) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: at most 2^27 scene points are supported");
+}  // extern "C"
+
+// First step of an upload: replaces the scene and grows every buffer the upload uses, with the host
+// work (centring, pixel range, class-weight bound, kd-tree thread start) but nothing enqueued, so that
+// the growth of several objects' buffers happens before any object's kernels are queued.  The caller has
+// checked the arguments.
+static int scene_upload_plan(stocs_b200_ctx* ctx, const float* pos3, const float* class_probability,
+                             const int32_t* pixel_rc, int S) {
   cudaSetDevice(ctx->device);
   cudaStream_t st = ctx->stream;
   // The previous scene is invalid from here on; S is committed only when the new index is complete,
   // so an early error return cannot leave S > 0 describing buffers that were half replaced.
   ctx->S = 0;
+  ctx->scene_empty = false;
   ctx->S_pending = S;
   stocs_kd_finish(ctx, st, false);   // a kd-tree still being built belongs to the scene this call replaces
-  // attributes: d_tmp = nrm3 | cls
-  STOCS_CUDA(ctx, ctx->d_tmp.ensure((size_t)S * 16));
-  float* d_n = ctx->d_tmp.as<float>();
-  float* d_c = d_n + (size_t)S * 3;
-  STOCS_CUDA(ctx, cudaMemcpyAsync(d_n, nrm3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
-  STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, class_probability, (size_t)S * 4, cudaMemcpyHostToDevice, st));
-  int rc = stocs_pack_scene_attr(ctx, d_n, d_c, S);
-  if (rc) { ctx->S_pending = 0; return rc; }
-  // (no synchronisation: the position upload below re-uses d_tmp in stream order, and the H2D copies
-  // of pageable host memory have consumed their source buffers when cudaMemcpyAsync returns)
+  STOCS_CUDA(ctx, ctx->d_tmp.ensure((size_t)S * 16));   // nrm3 | cls, then pos3
+  STOCS_CUDA(ctx, ctx->d_sattr.ensure((size_t)S * 16));
   STOCS_CUDA(ctx, ctx->d_spix.ensure((size_t)S * 8));
-  if (pixel_rc) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_spix.p, pixel_rc, (size_t)S * 8, cudaMemcpyHostToDevice, st));
-  else STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_spix.p, 0, (size_t)S * 8, st));
-  ctx->has_pixels = pixel_rc != nullptr;
   stocs_set_weight_bound(ctx, class_probability, S);
   ctx->pix_min[0] = ctx->pix_min[1] = 0; ctx->pix_max[0] = ctx->pix_max[1] = 0;
   if (pixel_rc) {  // range of the pixel coordinates: instance sampling indexes images with them
@@ -365,16 +358,120 @@ int stocs_b200_upload_scene(stocs_b200_ctx* ctx, const float* pos3, const float*
         if (v > ctx->pix_max[k]) ctx->pix_max[k] = v;
       }
   }
+  ctx->h_pos_pending = getenv("STOCS_DEVICE_CENTROID") ? nullptr : pos3;
+  if (!ctx->h_pos_pending)   // the device centring of the plan reads the positions from d_tmp
+    STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_tmp.p, pos3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
+  return stocs_index_plan(ctx);
+}
+
+// Second step: the uploads and kernels, up to the index build's two length copies; no synchronisation.
+static int scene_upload_enqueue(stocs_b200_ctx* ctx, const float* pos3, const float* nrm3, const float* class_probability,
+                                const int32_t* pixel_rc, int S) {
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = ctx->stream;
+  float* d_n = ctx->d_tmp.as<float>();
+  float* d_c = d_n + (size_t)S * 3;
+  STOCS_CUDA(ctx, cudaMemcpyAsync(d_n, nrm3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
+  STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, class_probability, (size_t)S * 4, cudaMemcpyHostToDevice, st));
+  int rc = stocs_pack_scene_attr(ctx, d_n, d_c, S);
+  if (rc) return rc;
+  // (no synchronisation: the position upload below re-uses d_tmp in stream order, and the H2D copies
+  // of pageable host memory have consumed their source buffers when cudaMemcpyAsync returns)
+  if (pixel_rc) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_spix.p, pixel_rc, (size_t)S * 8, cudaMemcpyHostToDevice, st));
+  else STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_spix.p, 0, (size_t)S * 8, st));
+  ctx->has_pixels = pixel_rc != nullptr;
   if (ctx->d_inst_state.p)  // a new scene starts with empty previous_segment / segmentation_buffer
     STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_inst_state.p, 0, (size_t)ctx->img_w * ctx->img_h * 3, st));
-  // positions -> centre -> index
-  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_tmp.p, pos3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
-  ctx->h_pos_pending = getenv("STOCS_DEVICE_CENTROID") ? nullptr : pos3;
-  rc = stocs_build_scene_index(ctx);
-  ctx->h_pos_pending = nullptr;
+  // positions -> centre -> index (the device-centroid path has centred them in the plan)
+  if (ctx->h_pos_pending) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_tmp.p, pos3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
+  return stocs_index_enqueue(ctx);
+}
+
+// Second half: completes the index build begun with status rc (or only drains the stream after a failed
+// begin) and commits S on success.
+static int scene_upload_end(stocs_b200_ctx* ctx, int rc) {
+  cudaSetDevice(ctx->device);
+  if (rc == STOCS_OK) rc = stocs_index_complete(ctx);
+  else cudaStreamSynchronize(ctx->stream);   // nothing of a failed upload stays queued
+  ctx->S = rc ? 0 : ctx->S_pending;
   ctx->S_pending = 0;
-  if (rc) { ctx->S = 0; return rc; }
-  ctx->S = S;
+  ctx->h_pos_pending = nullptr;
+  return rc;
+}
+
+// Validation shared by the calls over several contexts: n_objects >= 1, no NULL entry, no context twice
+// (two objects would share a stream and scratch).
+int stocs_batch_check(stocs_b200_ctx* const* ctxs, int n_objects, const char* who) {
+  if (!ctxs || n_objects < 1 || !ctxs[0]) return STOCS_E_ARG;   // no context to hold the message
+  for (int k = 0; k < n_objects; ++k) {
+    if (!ctxs[k]) return stocs_batch_fail(ctxs, k, STOCS_E_ARG, who, "context is NULL");
+    for (int j = 0; j < k; ++j)
+      if (ctxs[j] == ctxs[k])
+        return stocs_batch_fail(ctxs, k, STOCS_E_ARG, who, "same context as object " + std::to_string(j));
+  }
+  return STOCS_OK;
+}
+
+int stocs_batch_fail(stocs_b200_ctx* const* ctxs, int k, int code, const char* who, const std::string& msg) {
+  const std::string text = std::string(who) + (k >= 0 ? ": object " + std::to_string(k) + ": " : ": ") + msg;
+  if (k >= 0 && ctxs[k]) ctxs[k]->err = text;
+  ctxs[0]->err = text;
+  return code;
+}
+
+extern "C" {
+
+int stocs_b200_upload_scene(stocs_b200_ctx* ctx, const float* pos3, const float* nrm3,
+                            const float* class_probability, const int32_t* pixel_rc, int S) {
+  if (!ctx) return STOCS_E_ARG;
+  if (!pos3 || !nrm3 || !class_probability || S <= 0) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: bad argument");
+  if (S > (1 << 27)) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: at most 2^27 scene points are supported");
+  int rc = scene_upload_plan(ctx, pos3, class_probability, pixel_rc, S);
+  if (rc == STOCS_OK) rc = scene_upload_enqueue(ctx, pos3, nrm3, class_probability, pixel_rc, S);
+  return scene_upload_end(ctx, rc);
+}
+
+// Every object's buffers are grown before any object's work is enqueued, and every object's work is
+// enqueued before any is waited for: the host waits once per context, at the end.
+int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const float* pos3, const float* nrm3,
+                             const float* class_probability, const int32_t* pixel_rc, const int64_t* offsets) {
+  const char* who = "upload_scenes";
+  int rc = stocs_batch_check(ctxs, n_objects, who);
+  if (rc) return rc;
+  if (!pos3 || !nrm3 || !class_probability || !offsets) return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, "bad argument");
+  if (offsets[0] != 0) return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, "offsets[0] must be 0");
+  for (int k = 0; k < n_objects; ++k) {
+    const int64_t S = offsets[k + 1] - offsets[k];
+    if (S < 0) return stocs_batch_fail(ctxs, k, STOCS_E_ARG, who, "offsets decrease");
+    if (S > (1 << 27)) return stocs_batch_fail(ctxs, k, STOCS_E_ARG, who, "at most 2^27 scene points are supported");
+  }
+  std::vector<int> status(n_objects, STOCS_OK);
+  for (int k = 0; k < n_objects; ++k) {   // every object's host work and buffer growth first ...
+    stocs_b200_ctx* ctx = ctxs[k];
+    const int64_t o = offsets[k];
+    const int S = (int)(offsets[k + 1] - o);
+    if (S == 0) {   // an object that is not visible: no scene, nothing enqueued
+      cudaSetDevice(ctx->device);
+      ctx->S = 0;
+      stocs_kd_finish(ctx, ctx->stream, false);
+      ctx->scene_empty = true;
+      ctx->ncand = 0;
+      ctx->counters[CTR_GRID_CELLS] = ctx->counters[CTR_CANDIDATES] = ctx->counters[CTR_OCCUPIED_CELLS] = 0;
+      continue;
+    }
+    status[k] = scene_upload_plan(ctx, pos3 + 3 * o, class_probability + o, pixel_rc ? pixel_rc + 2 * o : nullptr, S);
+  }
+  for (int k = 0; k < n_objects; ++k) {   // ... then every object's uploads and kernels
+    const int64_t o = offsets[k];
+    const int S = (int)(offsets[k + 1] - o);
+    if (S > 0 && status[k] == STOCS_OK)
+      status[k] = scene_upload_enqueue(ctxs[k], pos3 + 3 * o, nrm3 + 3 * o, class_probability + o,
+                                       pixel_rc ? pixel_rc + 2 * o : nullptr, S);
+  }
+  for (int k = 0; k < n_objects; ++k)
+    if (offsets[k + 1] > offsets[k]) status[k] = scene_upload_end(ctxs[k], status[k]);
+  for (int k = 0; k < n_objects; ++k)
+    if (status[k]) return stocs_batch_fail(ctxs, k, status[k], who, ctxs[k]->err);
   return STOCS_OK;
 }
 

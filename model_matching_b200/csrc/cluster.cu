@@ -213,6 +213,11 @@ int stocs_cluster_enqueue_pipeline(stocs_b200_ctx* ctx, const stocs_b200_cluster
   return STOCS_OK;
 }
 
+int stocs_cluster_reserve(stocs_b200_ctx* ctx, long long cap_items) {
+  ClusterScratch s;
+  return cluster_scratch(ctx, cap_items, false, ctx->stream, s);
+}
+
 const stocs_b200_pose* stocs_cluster_poses_host(stocs_b200_ctx* ctx) { return ctx->h_cluster->poses; }
 
 void stocs_cluster_free_host(stocs_b200_ctx* ctx) {

@@ -497,18 +497,19 @@ static ModelNorm model_norm(const stocs_b200_ctx* ctx) {
 //   d_state: the run's StocsPipeState (the CALLER zeroes it); this search fills need_codes, need_quads,
 //            totalP, total, total_quads and may raise overflow bits 1 / 2 / 4
 //   d_quad_off: n_bases + 1 offsets into the quad buffer ctx->pool[POOL_CONG_QUADS]
-// Buffers are sized by ctx->cong_cap_codes / cong_cap_quads; stocs_congruent_grow() raises them from a
-// state record that came back with overflow set.
-int stocs_congruent_enqueue(stocs_b200_ctx* ctx, int n_bases, const int* d_base_idx4, const float* d_inv2,
-                            const uint8_t* d_valid, StocsPipeState* d_state, long long* d_quad_off, cudaStream_t st) {
-  if (n_bases <= 0) return STOCS_OK;
-  const PpfView v = stocs_ppf_view(ctx);
+// Sizes of one congruent-set search against the context's capacities.
+struct CongSizes { size_t cap, capq, table_size; int table_bits, end_bit; size_t tb, tb2, tb3; };
+
+#define CG(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { ctx->err = std::string(#call) + ": " + cudaGetErrorString(_e); return STOCS_E_CUDA; } } while (0)
+// Grows every buffer of a search over n_bases bases; enqueues nothing.
+static int cong_reserve(stocs_b200_ctx* ctx, int n_bases, CongSizes& z) {
+  cudaStream_t st = ctx->stream;   // (the cub size queries below enqueue nothing)
   DevBuf &d_info = ctx->pool[POOL_CONG_INFO], &d_seg = ctx->pool[POOL_CONG_SEG], &d_codes_a = ctx->pool[POOL_CONG_CODES_A], &d_codes_b = ctx->pool[POOL_CONG_CODES_B], &d_tmp = ctx->pool[POOL_CONG_TMP],
          &d_pe = ctx->pool[POOL_CONG_PE], &d_qe = ctx->pool[POOL_CONG_QE], &d_qcell = ctx->pool[POOL_CONG_QCELL], &d_cnt = ctx->pool[POOL_CONG_CNT], &d_scan = ctx->pool[POOL_CONG_SCAN],
          &quads_buf = ctx->pool[POOL_CONG_QUADS], &d_bcount = ctx->pool[POOL_CONG_HEAD], &d_cone = ctx->pool[POOL_CONG_CONE],
          &d_qslot = ctx->pool[POOL_CONG_NEXT], &d_bstart = ctx->pool[POOL_CONG_BSTART], &d_bucket = ctx->pool[POOL_CONG_BUCKET];
-#define CG(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { ctx->err = std::string(#call) + ": " + cudaGetErrorString(_e); return STOCS_E_CUDA; } } while (0)
   const size_t cap = (size_t)ctx->cong_cap_codes, capq = (size_t)ctx->cong_cap_quads;
+  z.cap = cap; z.capq = capq;
   CG(d_info.ensure((size_t)n_bases * sizeof(BaseInfo)));
   CG(d_seg.ensure(((size_t)2 * n_bases + 1) * 4));
   CG(d_codes_a.ensure(cap * 4));
@@ -522,9 +523,8 @@ int stocs_congruent_enqueue(stocs_b200_ctx* ctx, int n_bases, const int* d_base_
   int table_bits = 10;
   while (table_bits < 31 && ((size_t)1 << table_bits) < 2 * cap) ++table_bits;
   const size_t table_size = (size_t)1 << table_bits;
-  // bucket counters: every search leaves them zero (cong_scatter_kernel), so they are cleared only when
-  // the buffer is new -- or after a search that did not run to its end
-  const bool fresh = d_bcount.bytes < (table_size + 1) * 4 || ctx->cong_table_size != (long long)table_size || !ctx->cong_bcount_clean;
+  z.table_bits = table_bits; z.table_size = table_size;
+  if (d_bcount.bytes < (table_size + 1) * 4) ctx->cong_bcount_clean = false;   // a new buffer holds no zeroed counters
   CG(d_bcount.ensure((table_size + 1) * 4));
   CG(d_bstart.ensure((table_size + 1) * 4));
   CG(d_bucket.ensure(cap * 8));
@@ -533,12 +533,40 @@ int stocs_congruent_enqueue(stocs_b200_ctx* ctx, int n_bases, const int* d_base_
   // (id1 << 16) | id2 with ids < M: the bits above 16 + ceil(log2 M) are zero
   int end_bit = 17;
   while (end_bit < 32 && (1 << (end_bit - 16)) < ctx->M) ++end_bit;
+  z.end_bit = end_bit;
   size_t tb = 0, tb2 = 0, tb3 = 0;
   cub::DeviceSegmentedRadixSort::SortKeys(nullptr, tb, d_codes_a.as<uint32_t>(), d_codes_b.as<uint32_t>(), (int)cap,
                                           2 * n_bases, d_seg.as<uint32_t>(), d_seg.as<uint32_t>() + 1, 0, end_bit, st);
   cub::DeviceScan::ExclusiveSum(nullptr, tb2, d_cnt.as<uint32_t>(), d_scan.as<uint32_t>(), (int)(cap + 1), st);
   cub::DeviceScan::ExclusiveSum(nullptr, tb3, d_bcount.as<uint32_t>(), d_bstart.as<uint32_t>(), (int)(table_size + 1), st);
   CG(d_tmp.ensure(std::max(tb, std::max(tb2, tb3))));
+  z.tb = tb; z.tb2 = tb2; z.tb3 = tb3;
+  return STOCS_OK;
+}
+
+int stocs_congruent_reserve(stocs_b200_ctx* ctx, int n_bases) {
+  CongSizes z;
+  return n_bases > 0 ? cong_reserve(ctx, n_bases, z) : STOCS_OK;
+}
+
+// Buffers are sized by ctx->cong_cap_codes / cong_cap_quads; stocs_congruent_grow() raises them from a
+// state record that came back with overflow set.
+int stocs_congruent_enqueue(stocs_b200_ctx* ctx, int n_bases, const int* d_base_idx4, const float* d_inv2,
+                            const uint8_t* d_valid, StocsPipeState* d_state, long long* d_quad_off, cudaStream_t st) {
+  if (n_bases <= 0) return STOCS_OK;
+  const PpfView v = stocs_ppf_view(ctx);
+  DevBuf &d_info = ctx->pool[POOL_CONG_INFO], &d_seg = ctx->pool[POOL_CONG_SEG], &d_codes_a = ctx->pool[POOL_CONG_CODES_A], &d_codes_b = ctx->pool[POOL_CONG_CODES_B], &d_tmp = ctx->pool[POOL_CONG_TMP],
+         &d_pe = ctx->pool[POOL_CONG_PE], &d_qe = ctx->pool[POOL_CONG_QE], &d_qcell = ctx->pool[POOL_CONG_QCELL], &d_cnt = ctx->pool[POOL_CONG_CNT], &d_scan = ctx->pool[POOL_CONG_SCAN],
+         &quads_buf = ctx->pool[POOL_CONG_QUADS], &d_bcount = ctx->pool[POOL_CONG_HEAD], &d_cone = ctx->pool[POOL_CONG_CONE],
+         &d_qslot = ctx->pool[POOL_CONG_NEXT], &d_bstart = ctx->pool[POOL_CONG_BSTART], &d_bucket = ctx->pool[POOL_CONG_BUCKET];
+  CongSizes z;
+  if (const int rc = cong_reserve(ctx, n_bases, z)) return rc;
+  const size_t cap = z.cap, capq = z.capq, table_size = z.table_size;
+  size_t tb = z.tb, tb2 = z.tb2, tb3 = z.tb3;   // (cub takes them by reference)
+  const int table_bits = z.table_bits, end_bit = z.end_bit;
+  // bucket counters: every search leaves them zero (cong_scatter_kernel), so they are cleared only when
+  // the buffer is new -- or after a search that did not run to its end
+  const bool fresh = ctx->cong_table_size != (long long)table_size || !ctx->cong_bcount_clean;
   if (fresh) CG(cudaMemsetAsync(d_bcount.p, 0, (table_size + 1) * 4, st));
   ctx->cong_table_size = (long long)table_size;
   ctx->cong_bcount_clean = false;   // until the whole search has been enqueued

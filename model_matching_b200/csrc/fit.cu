@@ -20,6 +20,7 @@ int stocs_launch_sample(stocs_b200_ctx* ctx, uint64_t seed, uint32_t first_base_
 int stocs_congruent_enqueue(stocs_b200_ctx* ctx, int n_bases, const int* d_base_idx4, const float* d_inv2,
                             const uint8_t* d_valid, StocsPipeState* d_state, long long* d_quad_off, cudaStream_t st);  // congruent.cu
 bool stocs_congruent_grow(stocs_b200_ctx* ctx, const StocsPipeState& s);
+int stocs_congruent_reserve(stocs_b200_ctx* ctx, int n_bases);   // congruent.cu: its buffers, nothing enqueued
 
 namespace {
 
@@ -259,117 +260,196 @@ extern "C" int stocs_b200_fit_transforms(stocs_b200_ctx* ctx, int64_t n, const i
 int stocs_launch_sample_instance(stocs_b200_ctx* ctx, uint64_t seed, int base_num, float dispersion, int* d_ids,
                                  float* d_inv, uint8_t* d_valid, cudaStream_t st);  // sample_instance.cu
 
-// mode 0: class-mode bases (independent, one launch for all); mode 1: instance-mode bases (sequentially
-// coupled: one launch per base, base numbers 1..n_bases).  The whole chain -- bases, congruent sets, item
-// selection, fits, scores, best, result record -- is enqueued back to back against capacities and the
-// host synchronises ONCE, on the 200-byte state record (round 1: six synchronisations per pose).
-// cp != NULL: the greedy clustering of the scored list (cluster.cu) is enqueued behind the result record
-// and its poses come back in the same queue; with cp == NULL nothing of it is enqueued.
-static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets, int mode, float dispersion,
-                             stocs_b200_pipeline_result* result, const stocs_b200_cluster_params* cp = nullptr,
-                             stocs_b200_pose* poses = nullptr, int cap = 0, int* n_poses = nullptr) {
-  if (!ctx) return STOCS_E_ARG;
+// One object of a pipeline call: the four single entry points run one, stocs_b200_run_pipelines one per
+// context.  mode 0: class-mode bases (independent, one launch for all); mode 1: instance-mode bases
+// (sequentially coupled: one launch per base, base numbers 1..n_bases).  The whole chain -- bases,
+// congruent sets, item selection, fits, scores, best, result record -- is enqueued back to back against
+// capacities and the host synchronises ONCE, on the 200-byte state record (round 1: six synchronisations
+// per pose).  cp != NULL: the greedy clustering of the scored list (cluster.cu) is enqueued behind the
+// result record and its poses come back in the same queue; with cp == NULL nothing of it is enqueued.
+struct PipeJob {
+  stocs_b200_ctx* ctx;
+  uint64_t seed;
+  const stocs_b200_cluster_params* cp;
+  stocs_b200_pipeline_result* result;
+  stocs_b200_pose* poses;
+  int* n_poses;
+  StageTrace tr;
+  int rc = STOCS_OK;
+  int attempt = 0;
+  bool queued = false;   // work is enqueued whose state record has not been read
+  // buffers of the current attempt
+  int* d_ids = nullptr; float* d_inv = nullptr; uint8_t* d_valid = nullptr;
+  StocsPipeState* d_state = nullptr; long long *d_qoff = nullptr, *d_ioff = nullptr;
+  long long cap_items = 0, guess = 0;
+  int* d_item_base = nullptr;
+  float *d_Tc = nullptr, *d_Tw = nullptr, *d_lcp = nullptr;
+  int* d_inl = nullptr; uint8_t* d_ok = nullptr;
+  PipeJob(stocs_b200_ctx* c, uint64_t s, const stocs_b200_cluster_params* p, stocs_b200_pipeline_result* r,
+          stocs_b200_pose* po, int* np)
+      : ctx(c), seed(s), cp(p), result(r), poses(po), n_poses(np), tr(c->stream) {}
+};
+
+// Every argument and state check of a run, before anything is enqueued.  empty_ok: a context that
+// upload_scenes gave an empty slice passes (it gets the no-pose result and no work).
+static int pipe_check(stocs_b200_ctx* ctx, int n_bases, int max_sets, int mode, const stocs_b200_pipeline_result* result,
+                      const stocs_b200_cluster_params* cp, const stocs_b200_pose* poses, int cap, int* n_poses, bool empty_ok) {
   if (cp && (!poses || !n_poses)) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline_clustered: bad argument");
   if (cp && stocs_cluster_check(ctx, cp, cap)) return STOCS_E_ARG;
   if (n_poses) *n_poses = 0;
-  if (ctx->S <= 0 || ctx->M <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "run_pipeline: upload_model and upload_scene first");
+  const bool empty = empty_ok && ctx->scene_empty && ctx->M > 0;
+  if (!empty && (ctx->S <= 0 || ctx->M <= 0)) STOCS_FAIL(ctx, STOCS_E_STATE, "run_pipeline: upload_model and upload_scene first");
   if (n_bases <= 0 || max_sets <= 0 || !result) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline: bad argument");
   if (mode == 1 && n_bases > 255) STOCS_FAIL(ctx, STOCS_E_ARG, "run_pipeline: instance mode numbers its bases 1..255");
-  cudaSetDevice(ctx->device);
-  cudaStream_t st = ctx->stream;
-  StageTrace tr(st);
+  if (mode == 1 && !empty) return stocs_instance_check(ctx);
+  return STOCS_OK;
+}
+
+static void no_pose(stocs_b200_pipeline_result* result) {
   memset(result, 0, sizeof(*result));
   result->best_index = -1;
   result->best_base = -1;
-  // 1. bases (rejected ones keep their slot, flagged in d_valid: every later stage skips them, so the
-  // order of the valid bases -- base_set of the reference driver -- is preserved without compaction)
-  DevBuf& d_bases = ctx->pool[POOL_PIPE_BASES];
-  STOCS_CUDA(ctx, d_bases.ensure((size_t)n_bases * 25 + 64));
-  int* d_ids = d_bases.as<int>();
-  float* d_inv = (float*)(d_ids + 4 * (size_t)n_bases);
-  uint8_t* d_valid = (uint8_t*)(d_inv + 2 * (size_t)n_bases);
+}
+
+// transforms a run can fit: at most max_sets per base, and no more than the quad capacity
+static long long pipe_cap_items(const stocs_b200_ctx* ctx, int n_bases, int max_sets) {
+  const long long cap_items = (long long)n_bases * max_sets;
+  return cap_items > ctx->cong_cap_quads ? ctx->cong_cap_quads : cap_items;
+}
+
+// Grows every buffer one attempt of a run uses, enqueueing nothing.  pipe_run calls it for every object
+// before any object's work is enqueued: DevBuf growth frees the old allocation, and cudaFree waits for
+// the whole device, which would drain the other objects' queued work.  (The kd-tree buffers of the first
+// scoring launch are grown by the scene upload, stocs_index_plan.)
+static int pipe_reserve(stocs_b200_ctx* ctx, int n_bases, int max_sets, int mode, bool clustered) {
+  STOCS_CUDA(ctx, ctx->pool[POOL_PIPE_BASES].ensure((size_t)n_bases * 25 + 64));
+  STOCS_CUDA(ctx, ctx->pool[POOL_PIPE_STATE].ensure(sizeof(StocsPipeState)));
+  STOCS_CUDA(ctx, ctx->pool[POOL_PIPE_OFF].ensure((size_t)(n_bases + 1) * 16));
+  // d_work: the samplers' survivor bitmaps (sample.cu, sample_instance.cu) and the lists of the general
+  // top-K launch (reduce.cu, lists longer than the closing block scans)
+  const size_t words = ((size_t)ctx->S + 31) / 32;
+  size_t work = mode == 0 ? (size_t)ctx->num_sms * 4 * words * 4 : words * 8;
+  const long long cap_items = pipe_cap_items(ctx, n_bases, max_sets);
+  if (cap_items > (1ll << 20)) work = std::max(work, (size_t)ctx->num_sms * 2 * 32 * 8);
+  STOCS_CUDA(ctx, ctx->d_work.ensure(work));
+  if (const int rc = stocs_congruent_reserve(ctx, n_bases)) return rc;
+  STOCS_CUDA(ctx, ctx->pool[POOL_PIPE_ITEMS].ensure((size_t)cap_items * 12));
+  STOCS_CUDA(ctx, ctx->pool[POOL_PIPE_FIT].ensure((size_t)cap_items * (64 + 64 + 1 + 4 + 4) + 1024));
+  if (clustered && cap_items < (1ll << 31)) return stocs_cluster_reserve(ctx, cap_items);
+  return STOCS_OK;
+}
+
+// 1. bases (rejected ones keep their slot, flagged in d_valid: every later stage skips them, so the
+// order of the valid bases -- base_set of the reference driver -- is preserved without compaction)
+static int pipe_sample(PipeJob& j, int n_bases, int mode, float dispersion) {
+  stocs_b200_ctx* ctx = j.ctx;
+  cudaStream_t st = ctx->stream;
+  j.d_ids = ctx->pool[POOL_PIPE_BASES].as<int>();
+  j.d_inv = (float*)(j.d_ids + 4 * (size_t)n_bases);
+  j.d_valid = (uint8_t*)(j.d_inv + 2 * (size_t)n_bases);
   int rc = STOCS_OK;
   if (mode == 0) {
-    rc = stocs_launch_sample(ctx, seed, 0, n_bases, d_ids, d_inv, d_valid, st);
+    rc = stocs_launch_sample(ctx, j.seed, 0, n_bases, j.d_ids, j.d_inv, j.d_valid, st);
   } else {
-    STOCS_CUDA(ctx, cudaMemsetAsync(d_valid, 0, (size_t)n_bases, st));
+    STOCS_CUDA(ctx, cudaMemsetAsync(j.d_valid, 0, (size_t)n_bases, st));
     for (int b = 0; b < n_bases && rc == STOCS_OK; ++b)
-      rc = stocs_launch_sample_instance(ctx, seed, b + 1, dispersion, d_ids + 4 * (size_t)b, d_inv + 2 * (size_t)b, d_valid + b, st);
+      rc = stocs_launch_sample_instance(ctx, j.seed, b + 1, dispersion, j.d_ids + 4 * (size_t)b, j.d_inv + 2 * (size_t)b,
+                                        j.d_valid + b, st);
   }
   if (rc) return rc;
-  tr.mark("pipeline: sample bases");
-  DevBuf &d_off = ctx->pool[POOL_PIPE_OFF], &d_items = ctx->pool[POOL_PIPE_ITEMS], &d_fit = ctx->pool[POOL_PIPE_FIT];
-  STOCS_CUDA(ctx, ctx->pool[POOL_PIPE_STATE].ensure(sizeof(StocsPipeState)));
-  StocsPipeState* d_state = ctx->pool[POOL_PIPE_STATE].as<StocsPipeState>();
-  STOCS_CUDA(ctx, d_off.ensure((size_t)(n_bases + 1) * 16));
-  long long* d_qoff = d_off.as<long long>();
-  long long* d_ioff = d_qoff + (n_bases + 1);
-  StocsPipeState& hs = *ctx->h_pipe_state;
-  for (int attempt = 0;; ++attempt) {
-    STOCS_CUDA(ctx, cudaMemsetAsync(d_state, 0, sizeof(StocsPipeState), st));
-    // 2. congruent sets
-    rc = stocs_congruent_enqueue(ctx, n_bases, d_ids, d_inv, d_valid, d_state, d_qoff, st);
+  j.tr.mark("pipeline: sample bases");
+  j.d_state = ctx->pool[POOL_PIPE_STATE].as<StocsPipeState>();
+  j.d_qoff = ctx->pool[POOL_PIPE_OFF].as<long long>();
+  j.d_ioff = j.d_qoff + (n_bases + 1);
+  return STOCS_OK;
+}
+
+// 2. congruent sets, 3. item selection and fits (one attempt; run again after a capacity overflow)
+static int pipe_front(PipeJob& j, int n_bases, int max_sets) {
+  stocs_b200_ctx* ctx = j.ctx;
+  cudaStream_t st = ctx->stream;
+  STOCS_CUDA(ctx, cudaMemsetAsync(j.d_state, 0, sizeof(StocsPipeState), st));
+  int rc = stocs_congruent_enqueue(ctx, n_bases, j.d_ids, j.d_inv, j.d_valid, j.d_state, j.d_qoff, st);
+  if (rc) return rc;
+  j.tr.mark("pipeline: congruent sets");
+  const long long cap_items = pipe_cap_items(ctx, n_bases, max_sets);
+  j.cap_items = cap_items;
+  pipe_item_offsets_kernel<<<1, 256, 0, st>>>(j.d_qoff, n_bases, max_sets, j.d_ioff, j.d_state);
+  DevBuf &d_items = ctx->pool[POOL_PIPE_ITEMS], &d_fit = ctx->pool[POOL_PIPE_FIT];   // (grown by pipe_reserve)
+  long long* d_item_quad = d_items.as<long long>();
+  j.d_item_base = (int*)(d_item_quad + cap_items);
+  select_items_kernel<<<n_bases, 128, 0, st>>>(j.d_qoff, j.d_ioff, n_bases, max_sets, j.d_item_base, d_item_quad);
+  j.d_Tc = d_fit.as<float>();
+  j.d_Tw = j.d_Tc + 16 * (size_t)cap_items;
+  j.d_lcp = j.d_Tw + 16 * (size_t)cap_items;
+  j.d_inl = (int*)(j.d_lcp + cap_items);
+  j.d_ok = (uint8_t*)(j.d_inl + cap_items);
+  FitArgs a;
+  fill_fit_args(ctx, a);
+  a.base_idx4 = j.d_ids; a.quads4 = ctx->pool[POOL_CONG_QUADS].as<int>(); a.item_base = j.d_item_base; a.item_quad = d_item_quad;
+  a.Tc = j.d_Tc; a.Tw = j.d_Tw; a.ok = j.d_ok; a.n = 0; a.n_dev = &j.d_state->n_items;
+  // grids follow the previous run's item count (any grid is correct: the kernels stride / claim up to the device count)
+  long long guess = ctx->pipe_last_items > 0 ? ctx->pipe_last_items + ctx->pipe_last_items / 4 : 4096;
+  if (guess > cap_items) guess = cap_items;
+  if (guess < 1) guess = 1;
+  j.guess = guess;
+  long long fit_blocks = (guess + 127) / 128;
+  if (fit_blocks > (long long)ctx->num_sms * 16) fit_blocks = (long long)ctx->num_sms * 16;
+  fit_kernel<<<(unsigned)fit_blocks, 128, 0, st>>>(a);
+  j.tr.mark("pipeline: select + fit");
+  return STOCS_OK;
+}
+
+// 4. score, 5. best, the optional clustering and the state record's copy to the host.  The first scoring
+// launch after an upload joins that scene's kd-tree thread (stocs_kd_finish), which is why a call over
+// several objects enqueues every object's front half before any back half.
+static int pipe_back(PipeJob& j, int n_bases) {
+  stocs_b200_ctx* ctx = j.ctx;
+  cudaStream_t st = ctx->stream;
+  ScoreRequest sq;
+  sq.time_it = true;
+  sq.d_H = &j.d_state->n_items;
+  sq.grid_hint = j.guess;
+  int rc = stocs_launch_score(ctx, j.d_Tc, j.cap_items, j.d_lcp, j.d_inl, st, sq);
+  if (rc) return rc;
+  long long* d_bi = &ctx->scratch()->pipe_best_idx;
+  float* d_bv = &ctx->scratch()->pipe_best_lcp;
+  // lists the closing block can scan itself (every online frame) skip the general top-K launch
+  const bool small_list = j.cap_items <= (1ll << 20);
+  if (!small_list) {
+    TopkRequest tq;
+    tq.idx = (int64_t*)d_bi;
+    tq.val = d_bv;
+    tq.d_H = &j.d_state->n_items;
+    tq.grid_hint = j.guess;
+    rc = stocs_launch_topk(ctx, j.d_lcp, j.cap_items, 1, 0, st, tq);
     if (rc) return rc;
-    tr.mark("pipeline: congruent sets");
-    // 3. at most max_sets transforms per base; the count is bounded by both n_bases * max_sets and the quad capacity
-    long long cap_items = (long long)n_bases * max_sets;
-    if (cap_items > ctx->cong_cap_quads) cap_items = ctx->cong_cap_quads;
-    pipe_item_offsets_kernel<<<1, 256, 0, st>>>(d_qoff, n_bases, max_sets, d_ioff, d_state);
-    STOCS_CUDA(ctx, d_items.ensure((size_t)cap_items * 12));
-    long long* d_item_quad = d_items.as<long long>();
-    int* d_item_base = (int*)(d_item_quad + cap_items);
-    select_items_kernel<<<n_bases, 128, 0, st>>>(d_qoff, d_ioff, n_bases, max_sets, d_item_base, d_item_quad);
-    STOCS_CUDA(ctx, d_fit.ensure((size_t)cap_items * (64 + 64 + 1 + 4 + 4) + 1024));
-    float* d_Tc = d_fit.as<float>();
-    float* d_Tw = d_Tc + 16 * (size_t)cap_items;
-    float* d_lcp = d_Tw + 16 * (size_t)cap_items;
-    int* d_inl = (int*)(d_lcp + cap_items);
-    uint8_t* d_ok = (uint8_t*)(d_inl + cap_items);
-    FitArgs a;
-    fill_fit_args(ctx, a);
-    a.base_idx4 = d_ids; a.quads4 = ctx->pool[POOL_CONG_QUADS].as<int>(); a.item_base = d_item_base; a.item_quad = d_item_quad;
-    a.Tc = d_Tc; a.Tw = d_Tw; a.ok = d_ok; a.n = 0; a.n_dev = &d_state->n_items;
-    // grids follow the previous run's item count (any grid is correct: the kernels stride / claim up to the device count)
-    long long guess = ctx->pipe_last_items > 0 ? ctx->pipe_last_items + ctx->pipe_last_items / 4 : 4096;
-    if (guess > cap_items) guess = cap_items;
-    if (guess < 1) guess = 1;
-    long long fit_blocks = (guess + 127) / 128;
-    if (fit_blocks > (long long)ctx->num_sms * 16) fit_blocks = (long long)ctx->num_sms * 16;
-    fit_kernel<<<(unsigned)fit_blocks, 128, 0, st>>>(a);
-    tr.mark("pipeline: select + fit");
-    // 4. score + 5. best
-    ScoreRequest sq;
-    sq.time_it = true;
-    sq.d_H = &d_state->n_items;
-    sq.grid_hint = guess;
-    rc = stocs_launch_score(ctx, d_Tc, cap_items, d_lcp, d_inl, st, sq);
-    if (rc) return rc;
-    long long* d_bi = &ctx->scratch()->pipe_best_idx;
-    float* d_bv = &ctx->scratch()->pipe_best_lcp;
-    // lists the closing block can scan itself (every online frame) skip the general top-K launch
-    const bool small_list = cap_items <= (1ll << 20);
-    if (!small_list) {
-      TopkRequest tq;
-      tq.idx = (int64_t*)d_bi;
-      tq.val = d_bv;
-      tq.d_H = &d_state->n_items;
-      tq.grid_hint = guess;
-      rc = stocs_launch_topk(ctx, d_lcp, cap_items, 1, 0, st, tq);
-      if (rc) return rc;
-    }
-    pipe_finalize_kernel<<<1, 1024, 0, st>>>(small_list ? d_lcp : nullptr, d_ok, d_valid, n_bases, d_item_base, d_bi, d_bv, d_Tc, d_Tw, d_state);
-    STOCS_CUDA(ctx, cudaGetLastError());
-    if (cp) {
-      const PipeClusterInputs ci = {d_lcp, d_Tc, d_Tw, d_ok, d_valid, d_item_base, cap_items, d_state};
-      rc = stocs_cluster_enqueue_pipeline(ctx, *cp, ci, st);
-      if (rc) return rc;
-    }
-    STOCS_CUDA(ctx, cudaMemcpyAsync(&hs, d_state, sizeof(StocsPipeState), cudaMemcpyDeviceToHost, st));
-    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
-    tr.mark("pipeline: score + best");
-    if (!hs.overflow) break;
-    if (!stocs_congruent_grow(ctx, hs) || attempt >= 2) STOCS_FAIL(ctx, STOCS_E_ARG, "find_congruent: pair lists too long");
   }
+  pipe_finalize_kernel<<<1, 1024, 0, st>>>(small_list ? j.d_lcp : nullptr, j.d_ok, j.d_valid, n_bases, j.d_item_base, d_bi, d_bv,
+                                           j.d_Tc, j.d_Tw, j.d_state);
+  STOCS_CUDA(ctx, cudaGetLastError());
+  if (j.cp) {
+    const PipeClusterInputs ci = {j.d_lcp, j.d_Tc, j.d_Tw, j.d_ok, j.d_valid, j.d_item_base, j.cap_items, j.d_state};
+    rc = stocs_cluster_enqueue_pipeline(ctx, *j.cp, ci, st);
+    if (rc) return rc;
+  }
+  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_pipe_state, j.d_state, sizeof(StocsPipeState), cudaMemcpyDeviceToHost, st));
+  return STOCS_OK;
+}
+
+// After the synchronisation: an attempt whose lists outgrew the capacities grows them and is marked for
+// another attempt; otherwise the state record fills the result and the poses.
+static int pipe_collect(PipeJob& j) {
+  stocs_b200_ctx* ctx = j.ctx;
+  const StocsPipeState& hs = *ctx->h_pipe_state;
+  j.tr.mark("pipeline: score + best");
+  if (hs.overflow) {
+    if (!stocs_congruent_grow(ctx, hs) || j.attempt >= 2) STOCS_FAIL(ctx, STOCS_E_ARG, "find_congruent: pair lists too long");
+    ++j.attempt;
+    j.queued = true;
+    return STOCS_OK;
+  }
+  stocs_b200_pipeline_result* result = j.result;
   ctx->pipe_last_items = hs.n_items;
   result->n_valid_bases = hs.n_valid;
   result->n_congruent_sets = (long long)hs.total_quads;
@@ -381,10 +461,91 @@ static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, in
     memcpy(result->best_T_centred, hs.best_Tc, 64);
     memcpy(result->best_T_world, hs.best_Tw, 64);
   }
-  if (cp) {
-    memcpy(poses, stocs_cluster_poses_host(ctx), (size_t)hs.n_poses * sizeof(stocs_b200_pose));
-    *n_poses = hs.n_poses;
+  if (j.cp) {
+    memcpy(j.poses, stocs_cluster_poses_host(ctx), (size_t)hs.n_poses * sizeof(stocs_b200_pose));
+    *j.n_poses = hs.n_poses;
   }
+  return STOCS_OK;
+}
+
+// Runs validated jobs stage by stage across objects: every object's bases, then every object's front half,
+// then every back half, then one wait per stream.  An object whose capacities overflowed is grown and
+// enqueued again alone; an object that failed enqueues nothing more, the others complete.  No stream is
+// left with work pending on return.
+static void pipe_run(std::vector<PipeJob>& jobs, int n_bases, int max_sets, int mode, float dispersion) {
+  for (PipeJob& j : jobs) {   // every object's buffer growth before any object's work is enqueued
+    cudaSetDevice(j.ctx->device);
+    no_pose(j.result);
+    j.rc = pipe_reserve(j.ctx, n_bases, max_sets, mode, j.cp != nullptr);
+  }
+  for (PipeJob& j : jobs) {
+    cudaSetDevice(j.ctx->device);
+    if (!j.rc) j.rc = pipe_sample(j, n_bases, mode, dispersion);
+    j.queued = true;
+  }
+  for (bool any = true; any;) {
+    for (PipeJob& j : jobs)   // an attempt after an overflow: only that object grows, the others have finished
+      if (j.queued && !j.rc && j.attempt > 0) { cudaSetDevice(j.ctx->device); j.rc = pipe_reserve(j.ctx, n_bases, max_sets, mode, j.cp != nullptr); }
+    for (PipeJob& j : jobs)
+      if (j.queued && !j.rc) { cudaSetDevice(j.ctx->device); j.rc = pipe_front(j, n_bases, max_sets); }
+    for (PipeJob& j : jobs)
+      if (j.queued && !j.rc) { cudaSetDevice(j.ctx->device); j.rc = pipe_back(j, n_bases); }
+    any = false;
+    for (PipeJob& j : jobs) {
+      if (!j.queued) continue;
+      j.queued = false;
+      cudaSetDevice(j.ctx->device);
+      const cudaError_t e = cudaStreamSynchronize(j.ctx->stream);
+      if (!j.rc && e != cudaSuccess) {
+        j.ctx->err = std::string("cudaStreamSynchronize(st): ") + cudaGetErrorString(e);
+        j.rc = STOCS_E_CUDA;
+      }
+      if (!j.rc) j.rc = pipe_collect(j);
+      any = any || j.queued;
+    }
+  }
+}
+
+static int run_pipeline_impl(stocs_b200_ctx* ctx, uint64_t seed, int n_bases, int max_sets, int mode, float dispersion,
+                             stocs_b200_pipeline_result* result, const stocs_b200_cluster_params* cp = nullptr,
+                             stocs_b200_pose* poses = nullptr, int cap = 0, int* n_poses = nullptr) {
+  if (!ctx) return STOCS_E_ARG;
+  if (const int rc = pipe_check(ctx, n_bases, max_sets, mode, result, cp, poses, cap, n_poses, false)) return rc;
+  std::vector<PipeJob> jobs;
+  jobs.emplace_back(ctx, seed, cp, result, poses, n_poses);
+  pipe_run(jobs, n_bases, max_sets, mode, dispersion);
+  return jobs[0].rc;
+}
+
+extern "C" int stocs_b200_run_pipelines(stocs_b200_ctx* const* ctxs, int n_objects, const uint64_t* seeds, int n_bases,
+                                        int max_sets, int instance_mode, float dispersion,
+                                        const stocs_b200_cluster_params* cluster, stocs_b200_pipeline_result* results,
+                                        stocs_b200_pose* poses, int cap, int* n_poses) {
+  const char* who = "run_pipelines";
+  if (const int rc = stocs_batch_check(ctxs, n_objects, who)) return rc;
+  if (!seeds || !results) return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, "bad argument");
+  if (instance_mode != 0 && instance_mode != 1) return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, "instance_mode must be 0 or 1");
+  for (int k = 0; k < n_objects; ++k) {
+    stocs_b200_ctx* ctx = ctxs[k];
+    const int rc = pipe_check(ctx, n_bases, max_sets, instance_mode, results + k, cluster ? cluster + k : nullptr,
+                              cluster && poses ? poses + (size_t)k * cap : nullptr, cap, n_poses ? n_poses + k : nullptr, true);
+    if (rc) return stocs_batch_fail(ctxs, k, rc, who, ctx->err);
+  }
+  std::vector<PipeJob> jobs;
+  jobs.reserve(n_objects);
+  for (int k = 0; k < n_objects; ++k) {
+    stocs_b200_ctx* ctx = ctxs[k];
+    if (ctx->S <= 0) { no_pose(results + k); continue; }   // empty slice of upload_scenes: no pose, no work
+    jobs.emplace_back(ctx, seeds[k], cluster ? cluster + k : nullptr, results + k, cluster ? poses + (size_t)k * cap : nullptr,
+                      cluster ? n_poses + k : nullptr);
+  }
+  pipe_run(jobs, n_bases, max_sets, instance_mode, dispersion);
+  for (const PipeJob& j : jobs)
+    if (j.rc) {
+      int k = 0;
+      while (ctxs[k] != j.ctx) ++k;
+      return stocs_batch_fail(ctxs, k, j.rc, who, j.ctx->err);
+    }
   return STOCS_OK;
 }
 

@@ -313,13 +313,18 @@ int stocs_b200_upload_edge_map(stocs_b200_ctx* ctx, const uint8_t* edge, int W, 
 // (d_ids 4 ints, d_inv 2 floats, d_valid 1 byte); mask and segment bits stay in ctx buffers.  No
 // synchronisation: the sequential coupling between bases (prior decay, cached masks) lives in device
 // state and is ordered by the stream, so a whole sequence can be enqueued back to back.
-int stocs_launch_sample_instance(stocs_b200_ctx* ctx, uint64_t seed, int base_num, float dispersion, int* d_ids,
-                                 float* d_inv, uint8_t* d_valid, cudaStream_t st) {
+int stocs_instance_check(stocs_b200_ctx* ctx) {
   if (ctx->S <= 0 || ctx->M <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "sample_instance_base: upload_model and upload_scene first");
   if (ctx->img_w <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "sample_instance_base: upload_edge_map first");
   if (!ctx->has_pixels) STOCS_FAIL(ctx, STOCS_E_STATE, "sample_instance_base: upload_scene was called without pixel coordinates");
   if (ctx->pix_min[0] < 0 || ctx->pix_min[1] < 0 || ctx->pix_max[0] >= ctx->img_h || ctx->pix_max[1] >= ctx->img_w)
     STOCS_FAIL(ctx, STOCS_E_ARG, "sample_instance_base: scene pixel coordinates fall outside the edge map");
+  return STOCS_OK;
+}
+
+int stocs_launch_sample_instance(stocs_b200_ctx* ctx, uint64_t seed, int base_num, float dispersion, int* d_ids,
+                                 float* d_inv, uint8_t* d_valid, cudaStream_t st) {
+  if (const int rc = stocs_instance_check(ctx)) return rc;
   if (base_num < 1 || base_num > 255) STOCS_FAIL(ctx, STOCS_E_ARG, "sample_instance_base: base_num must be 1..255");
   const size_t n = (size_t)ctx->img_w * ctx->img_h;
   InstArgs a;

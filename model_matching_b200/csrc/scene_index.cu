@@ -159,7 +159,7 @@ __global__ void grid_fill_kernel(const float4* __restrict__ pts, int n, GridDesc
     if (!near_cell(g, p, r * r, x, y, z)) continue;
     const size_t cell = cell_number(g, x, y, z);
     const uint32_t slot = cell_start[cell] + atomicSub(&remaining[cell], 1u) - 1u;
-    if (slot < cap) cand[slot] = p;   // (the buffer is sized before the total is known; see stocs_build_scene_index)
+    if (slot < cap) cand[slot] = p;   // (the buffer is sized before the total is known; see stocs_index_enqueue)
   }
 }
 
@@ -407,37 +407,43 @@ static int kd_start(stocs_b200_ctx* ctx, int S) {
   return STOCS_OK;
 }
 
+// Reference centroid of n host points into ctx->h_centroid_stage, their centred copy and bounding box
+// (min xyz, max xyz; min x NaN when a coordinate is not finite).
+static void host_centre(stocs_b200_ctx* ctx, const float* h_pos3, int n, float* h_centred3, float* h_aabb6) {
+  float sx = 0.f, sy = 0.f, sz = 0.f;   // same order, same binary32 adds as the kernel (no contraction: no multiply)
+  for (int i = 0; i < n; ++i) { sx += h_pos3[3 * (size_t)i]; sy += h_pos3[3 * (size_t)i + 1]; sz += h_pos3[3 * (size_t)i + 2]; }
+  ctx->h_centroid_stage[0] = sx / (float)n; ctx->h_centroid_stage[1] = sy / (float)n; ctx->h_centroid_stage[2] = sz / (float)n;
+  if (!h_centred3) return;
+  // The host has everything the callers wait for: centroid, centred copy (one binary32 subtraction per
+  // coordinate, the same operation as centre_pack_kernel) and bounding box.
+  const float cx = ctx->h_centroid_stage[0], cy = ctx->h_centroid_stage[1], cz = ctx->h_centroid_stage[2];
+  float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+  bool finite = true;
+  for (int i = 0; i < n; ++i) {
+    const float v[3] = {h_pos3[3 * (size_t)i] - cx, h_pos3[3 * (size_t)i + 1] - cy, h_pos3[3 * (size_t)i + 2] - cz};
+    for (int k = 0; k < 3; ++k) {
+      h_centred3[3 * (size_t)i + k] = v[k];
+      if (v[k] < mn[k]) mn[k] = v[k];
+      if (v[k] > mx[k]) mx[k] = v[k];
+      finite = finite && std::isfinite(v[k]);
+    }
+  }
+  if (!finite) mn[0] = NAN;   // callers test the box
+  if (h_aabb6) for (int k = 0; k < 3; ++k) { h_aabb6[k] = mn[k]; h_aabb6[3 + k] = mx[k]; }
+}
+
 int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4* d_out4,
                         float* d_out3, float* h_centroid3, float* h_aabb6, const float* h_pos3, float* h_centred3) {
   cudaStream_t st = ctx->stream;
   float* d_c = ctx->scratch()->centroid;
   int* d_aabb = ctx->scratch()->aabb;
   if (h_pos3) {
-    float sx = 0.f, sy = 0.f, sz = 0.f;   // same order, same binary32 adds as the kernel (no contraction: no multiply)
-    for (int i = 0; i < n; ++i) { sx += h_pos3[3 * (size_t)i]; sy += h_pos3[3 * (size_t)i + 1]; sz += h_pos3[3 * (size_t)i + 2]; }
-    ctx->h_centroid_stage[0] = sx / (float)n; ctx->h_centroid_stage[1] = sy / (float)n; ctx->h_centroid_stage[2] = sz / (float)n;
+    host_centre(ctx, h_pos3, n, h_centred3, h_aabb6);
     STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, ctx->h_centroid_stage, 12, cudaMemcpyHostToDevice, st));
-    if (h_centred3) {
-      // The host has everything the callers wait for: centroid, centred copy (one binary32
-      // subtraction per coordinate, the same operation as centre_pack_kernel) and bounding box.
-      // The device centres its own copy concurrently; nothing is read back, no synchronisation.
-      const float cx = ctx->h_centroid_stage[0], cy = ctx->h_centroid_stage[1], cz = ctx->h_centroid_stage[2];
-      float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
-      bool finite = true;
-      for (int i = 0; i < n; ++i) {
-        const float v[3] = {h_pos3[3 * (size_t)i] - cx, h_pos3[3 * (size_t)i + 1] - cy, h_pos3[3 * (size_t)i + 2] - cz};
-        for (int k = 0; k < 3; ++k) {
-          h_centred3[3 * (size_t)i + k] = v[k];
-          if (v[k] < mn[k]) mn[k] = v[k];
-          if (v[k] > mx[k]) mx[k] = v[k];
-          finite = finite && std::isfinite(v[k]);
-        }
-      }
-      if (!finite) mn[0] = NAN;   // callers test the box
+    if (h_centred3) {   // the device centres its own copy concurrently; nothing is read back, no synchronisation
       centre_pack_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_pos3, n, d_c, d_out4, d_out3, nullptr);
       STOCS_CUDA(ctx, cudaGetLastError());
       for (int k = 0; k < 3; ++k) h_centroid3[k] = ctx->h_centroid_stage[k];
-      if (h_aabb6) for (int k = 0; k < 3; ++k) { h_aabb6[k] = mn[k]; h_aabb6[3 + k] = mx[k]; }
       return STOCS_OK;
     }
   } else {
@@ -456,21 +462,96 @@ int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4*
   return STOCS_OK;
 }
 
-int stocs_build_scene_index(stocs_b200_ctx* ctx) {
-  // expects ctx->d_tmp = raw pos3 (S*3 floats)
+// One pass of the index kernels against the capacity in ctx->index_build, ending in the two length
+// copies; no synchronisation.
+static int index_enqueue_attempt(stocs_b200_ctx* ctx) {
+  const int S = ctx->S_pending;
+  const GridDesc& g = ctx->grid;
+  const IndexBuild& ib = ctx->index_build;
+  cudaStream_t st = ctx->stream;
+  const size_t nc1 = ib.nc1, cap = ib.cap;
+  const int nb = (S + 255) / 256;
+  uint32_t* counts = ctx->pool[POOL_INDEX_COUNTS].as<uint32_t>();
+  uint32_t* dense_start = ctx->pool[POOL_INDEX_DENSE].as<uint32_t>();
+  DevBuf &d_masks = ctx->pool[POOL_INDEX_MASKS], &d_occ = ctx->pool[POOL_INDEX_OCC], &d_occ_scan = ctx->pool[POOL_INDEX_OCC_SCAN];
+  uint32_t* h_counts = ctx->h_index_counts;   // page-locked: {candidate records, occupied cells}
+  const size_t starts_cap = (cap < (size_t)g.ncells ? cap : (size_t)g.ncells) + 1;
+  size_t tmp_bytes = ib.tmp_bytes, tmp_bytes2 = ib.tmp_bytes2;
+  const unsigned bb = (g.nbricks + 127) / 128;
+  STOCS_CUDA(ctx, ctx->d_cand.ensure(cap * 16));
+  STOCS_CUDA(ctx, ctx->d_cell_start.ensure(starts_cap * 4));
+  if (ctx->index_counts_clean < nc1) STOCS_CUDA(ctx, cudaMemsetAsync(counts, 0, nc1 * 4, st));
+  ctx->index_counts_clean = 0;   // dirty until this attempt's fill pass has run to completion
+  if (S <= (1 << 18)) grid_count_kernel<32><<<(unsigned)(((size_t)S * 32 + 255) / 256), 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, ib.r, counts);
+  else grid_count_kernel<1><<<nb, 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, ib.r, counts);
+  cub::DeviceScan::ExclusiveSum(ctx->d_tmp2.p, tmp_bytes, counts, dense_start, (int)nc1, st);
+  STOCS_CUDA(ctx, cudaMemcpyAsync(&h_counts[0], dense_start + g.ncells, 4, cudaMemcpyDeviceToHost, st));
+  if (S <= (1 << 18)) grid_fill_kernel<32><<<(unsigned)(((size_t)S * 32 + 255) / 256), 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, ib.r, dense_start, counts, ctx->d_cand.as<float4>(), (uint32_t)cap);
+  else grid_fill_kernel<1><<<nb, 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, ib.r, dense_start, counts, ctx->d_cand.as<float4>(), (uint32_t)cap);
+  // brick table + compact starts
+  STOCS_CUDA(ctx, cudaMemsetAsync(d_occ.p, 0, (size_t)(g.nbricks + 1) * 4, st));
+  brick_mask_kernel<<<(unsigned)(((size_t)g.nbricks + 255) / 256), 256, 0, st>>>(dense_start, g.nbricks, d_masks.as<unsigned long long>(),
+                                                                                d_occ.as<uint32_t>(), ctx->d_brick_occ.as<uint32_t>());
+  cub::DeviceScan::ExclusiveSum(ctx->d_tmp2.p, tmp_bytes2, d_occ.as<uint32_t>(), d_occ_scan.as<uint32_t>(), (int)(g.nbricks + 1), st);
+  STOCS_CUDA(ctx, cudaMemcpyAsync(&h_counts[1], d_occ_scan.as<uint32_t>() + g.nbricks, 4, cudaMemcpyDeviceToHost, st));
+  STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_coarse.p, 0, (size_t)ctx->coarse_words * 4, st));
+  brick_table_kernel<<<bb, 128, 0, st>>>(dense_start, d_masks.as<unsigned long long>(), d_occ_scan.as<uint32_t>(), g.nbricks,
+                                         dense_start + g.ncells, (uint32_t)starts_cap, ctx->d_bricks.as<uint4>(),
+                                         ctx->d_cell_start.as<uint32_t>(), ctx->d_coarse.as<uint32_t>(), g, ctx->coarse_shift,
+                                         ctx->coarse_nx + 1, ctx->coarse_ny + 1);
+  STOCS_CUDA(ctx, cudaGetLastError());
+  return STOCS_OK;
+}
+
+// Second half of the index build: waits for the pass stocs_index_enqueue queued, and when the candidate
+// records did not fit, grows the buffers and runs the pass once more.
+int stocs_index_complete(stocs_b200_ctx* ctx) {
+  cudaStream_t st = ctx->stream;
+  StageTrace tr(st);
+  uint32_t total = 0, n_occ = 0;
+  for (int attempt = 0;; ++attempt) {
+    if (attempt > 0) {
+      const int rc = index_enqueue_attempt(ctx);
+      if (rc) return rc;
+    }
+    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
+    ctx->index_counts_clean = ctx->index_build.nc1;
+    total = ctx->h_index_counts[0]; n_occ = ctx->h_index_counts[1];
+    if ((size_t)total <= ctx->index_build.cap) break;
+    if (attempt >= 1) STOCS_FAIL(ctx, STOCS_E_CUDA, "upload_scene: candidate buffer sizing failed");
+    ctx->index_build.cap = (size_t)total + 1024;
+  }
+  ctx->ncand = total;
+  ctx->counters[CTR_OCCUPIED_CELLS] = n_occ;
+  tr.mark("index build");
+  ctx->counters[CTR_GRID_CELLS] = ctx->grid.ncells;
+  ctx->counters[CTR_CANDIDATES] = total;
+  return STOCS_OK;
+}
+
+// First step of an index build, before any of it is enqueued: centre the points, start the kd-tree
+// thread, lay out the grid and grow every buffer the build uses, so that no allocation happens between
+// the kernels of several objects' uploads.  The centring runs on the host from ctx->h_pos_pending; without
+// it (STOCS_DEVICE_CENTROID) the positions are already in ctx->d_tmp and this waits for the device kernels.
+int stocs_index_plan(stocs_b200_ctx* ctx) {
   const int S = ctx->S_pending;   // committed to ctx->S by upload_scene once the index is complete
   cudaStream_t st = ctx->stream;
   StageTrace tr(st);
   STOCS_CUDA(ctx, ctx->d_spos4.ensure((size_t)S * 16));
   STOCS_CUDA(ctx, ctx->d_tmp2.ensure((size_t)S * 12));
-  int nb = (S + 255) / 256;
+  // the kd-tree upload of the first scoring launch (stocs_kd_finish): S points, and at most S + 3 nodes
+  // (every inner node below the root holds more than 64 points, at most S / 65 of them on each of <= 31 levels)
+  STOCS_CUDA(ctx, ctx->d_kd_pts.ensure((size_t)S * 16));
+  STOCS_CUDA(ctx, ctx->d_kd_nodes.ensure(((size_t)S + 3) * sizeof(KdNodeDev)));
   float aabb[6];
   ctx->h_spos.resize((size_t)S * 3);
-  int rc = stocs_centre_points(ctx, ctx->d_tmp.as<float>(), S, ctx->d_spos4.as<float4>(),
-                               ctx->h_pos_pending ? nullptr : ctx->d_tmp2.as<float>(), ctx->cs, aabb, ctx->h_pos_pending,
-                               ctx->h_pos_pending ? ctx->h_spos.data() : nullptr);
-  if (rc) return rc;
-  if (!ctx->h_pos_pending) {   // device-only path: centred points and box come back from the kernels
+  if (ctx->h_pos_pending) {
+    host_centre(ctx, ctx->h_pos_pending, S, ctx->h_spos.data(), aabb);
+    memcpy(ctx->cs, ctx->h_centroid_stage, 12);
+  } else {   // device-only path: centred points and box come back from the kernels
+    int rc = stocs_centre_points(ctx, ctx->d_tmp.as<float>(), S, ctx->d_spos4.as<float4>(), ctx->d_tmp2.as<float>(), ctx->cs,
+                                 aabb);
+    if (rc) return rc;
     STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_spos.data(), ctx->d_tmp2.p, (size_t)S * 12, cudaMemcpyDeviceToHost, st));
     STOCS_CUDA(ctx, cudaStreamSynchronize(st));
   }
@@ -479,6 +560,7 @@ int stocs_build_scene_index(stocs_b200_ctx* ctx) {
   for (int k = 0; k < 3; ++k)
     if (!(mn[k] <= mx[k]) || !std::isfinite(mn[k]) || !std::isfinite(mx[k]))
       STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: scene contains non-finite coordinates");
+  int rc = STOCS_OK;
 
   // the reference kd-tree (exact-tie resolution in the scoring kernel): host work on the centred
   // points, started here on a host thread and collected by the first scoring launch
@@ -584,50 +666,28 @@ int stocs_build_scene_index(stocs_b200_ctx* ctx) {
   if (cap < ctx->d_cand.bytes / 16) cap = ctx->d_cand.bytes / 16;
   if (const char* e = getenv("STOCS_CAND_CAP")) { const long long v = atoll(e); if (v >= 1) cap = (size_t)v; }   // tests: force the retry
   if (cap > 0xfffffff0u) cap = 0xfffffff0u;
-  const unsigned bb = (g.nbricks + 127) / 128;
-  uint32_t* h_counts = ctx->h_index_counts;   // page-locked: {candidate records, occupied cells}
-  uint32_t total = 0, n_occ = 0;
-  for (int attempt = 0;; ++attempt) {
-    const size_t starts_cap = (cap < (size_t)g.ncells ? cap : (size_t)g.ncells) + 1;
-    STOCS_CUDA(ctx, ctx->d_cand.ensure(cap * 16));
-    STOCS_CUDA(ctx, ctx->d_cell_start.ensure(starts_cap * 4));
-    if (ctx->index_counts_clean < nc1) STOCS_CUDA(ctx, cudaMemsetAsync(counts, 0, nc1 * 4, st));
-    ctx->index_counts_clean = 0;   // dirty until this attempt's fill pass has run to completion
-    if (S <= (1 << 18)) grid_count_kernel<32><<<(unsigned)(((size_t)S * 32 + 255) / 256), 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, r, counts);
-    else grid_count_kernel<1><<<nb, 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, r, counts);
-    cub::DeviceScan::ExclusiveSum(ctx->d_tmp2.p, tmp_bytes, counts, dense_start, (int)nc1, st);
-    STOCS_CUDA(ctx, cudaMemcpyAsync(&h_counts[0], dense_start + g.ncells, 4, cudaMemcpyDeviceToHost, st));
-    if (S <= (1 << 18)) grid_fill_kernel<32><<<(unsigned)(((size_t)S * 32 + 255) / 256), 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, r, dense_start, counts, ctx->d_cand.as<float4>(), (uint32_t)cap);
-    else grid_fill_kernel<1><<<nb, 256, 0, st>>>(ctx->d_spos4.as<float4>(), S, g, r, dense_start, counts, ctx->d_cand.as<float4>(), (uint32_t)cap);
-    // brick table + compact starts
-    STOCS_CUDA(ctx, cudaMemsetAsync(d_occ.p, 0, (size_t)(g.nbricks + 1) * 4, st));
-    brick_mask_kernel<<<(unsigned)(((size_t)g.nbricks + 255) / 256), 256, 0, st>>>(dense_start, g.nbricks, d_masks.as<unsigned long long>(),
-                                                                                  d_occ.as<uint32_t>(), ctx->d_brick_occ.as<uint32_t>());
-    cub::DeviceScan::ExclusiveSum(ctx->d_tmp2.p, tmp_bytes2, d_occ.as<uint32_t>(), d_occ_scan.as<uint32_t>(), (int)(g.nbricks + 1), st);
-    STOCS_CUDA(ctx, cudaMemcpyAsync(&h_counts[1], d_occ_scan.as<uint32_t>() + g.nbricks, 4, cudaMemcpyDeviceToHost, st));
-    STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_coarse.p, 0, (size_t)ctx->coarse_words * 4, st));
-    brick_table_kernel<<<bb, 128, 0, st>>>(dense_start, d_masks.as<unsigned long long>(), d_occ_scan.as<uint32_t>(), g.nbricks,
-                                           dense_start + g.ncells, (uint32_t)starts_cap, ctx->d_bricks.as<uint4>(),
-                                           ctx->d_cell_start.as<uint32_t>(), ctx->d_coarse.as<uint32_t>(), g, cshift, cnx + 1, cny + 1);
-    STOCS_CUDA(ctx, cudaGetLastError());
-    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
-    ctx->index_counts_clean = nc1;
-    total = h_counts[0]; n_occ = h_counts[1];
-    if ((size_t)total <= cap) break;
-    if (attempt >= 1) STOCS_FAIL(ctx, STOCS_E_CUDA, "upload_scene: candidate buffer sizing failed");
-    cap = (size_t)total + 1024;
-  }
-  ctx->ncand = total;
-  ctx->counters[CTR_OCCUPIED_CELLS] = n_occ;
-  tr.mark("index build");
-  ctx->counters[CTR_GRID_CELLS] = g.ncells;
-  ctx->counters[CTR_CANDIDATES] = total;
+  ctx->index_build = IndexBuild{r, cap, nc1, tmp_bytes, tmp_bytes2};
+  STOCS_CUDA(ctx, ctx->d_cand.ensure(cap * 16));
+  STOCS_CUDA(ctx, ctx->d_cell_start.ensure(((cap < (size_t)g.ncells ? cap : (size_t)g.ncells) + 1) * 4));
   return STOCS_OK;
 }
 
-// used by upload_scene in capi.cu
+// Second step: the device centring (host path: the centroid the plan computed; positions in ctx->d_tmp)
+// and one pass of the index kernels, ending in the two length copies; no synchronisation.
+int stocs_index_enqueue(stocs_b200_ctx* ctx) {
+  if (ctx->h_pos_pending) {
+    cudaStream_t st = ctx->stream;
+    const int S = ctx->S_pending;
+    float* d_c = ctx->scratch()->centroid;
+    STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, ctx->h_centroid_stage, 12, cudaMemcpyHostToDevice, st));
+    centre_pack_kernel<<<(S + 255) / 256, 256, 0, st>>>(ctx->d_tmp.as<float>(), S, d_c, ctx->d_spos4.as<float4>(), nullptr, nullptr);
+    STOCS_CUDA(ctx, cudaGetLastError());
+  }
+  return index_enqueue_attempt(ctx);
+}
+
+// used by upload_scene in capi.cu (ctx->d_sattr holds S records)
 int stocs_pack_scene_attr(stocs_b200_ctx* ctx, const float* d_nrm3, const float* d_cls, int S) {
-  STOCS_CUDA(ctx, ctx->d_sattr.ensure((size_t)S * 16));
   pack_attr_kernel<<<(S + 255) / 256, 256, 0, ctx->stream>>>(d_nrm3, d_cls, S, ctx->d_sattr.as<float4>());
   STOCS_CUDA(ctx, cudaGetLastError());
   return STOCS_OK;

@@ -47,6 +47,14 @@ struct GridDesc {
   uint32_t ncells;    // nbricks * 64 (brick-major numbering)
 };
 
+// Parameters of a scene-index build between its enqueue and its completion (scene_index.cu)
+struct IndexBuild {
+  float r;                   // dilation radius of the candidate lists
+  size_t cap;                // candidate records the buffers are sized for
+  size_t nc1;                // cells + 1
+  size_t tmp_bytes, tmp_bytes2;   // cub scratch of the two scans
+};
+
 struct PpfTableDesc {
   int n1, na;          // bins along the distance axis / each angle axis
   int tr, rot;
@@ -173,6 +181,8 @@ struct stocs_b200_ctx {
   int S = 0;
   int S_pending = 0;                   // size of the scene being uploaded (S is committed on success)
   const float* h_pos_pending = nullptr;  // its positions in the caller's host buffer (valid during upload_scene only)
+  bool scene_empty = false;            // S == 0 because upload_scenes gave this context an empty slice
+  IndexBuild index_build{};            // the index build in flight (stocs_index_enqueue -> stocs_index_complete)
   float h_centroid_stage[4] = {0, 0, 0, 0};  // source of the 12-byte centroid upload (must outlive the async copy)
   float cs[3] = {0, 0, 0};
   std::vector<float> h_spos;           // centred positions (S*3)
@@ -299,7 +309,13 @@ static_assert(sizeof(DevScratch) <= 4096, "DevScratch must fit the 4 KB d_small 
   do { (ctx)->err = (msg); return (code); } while (0)
 
 // kernels / stages implemented in the other translation units
-int stocs_build_scene_index(stocs_b200_ctx* ctx);                         // scene_index.cu
+// scene index of ctx->S_pending points (scene_index.cu), in three steps: plan (centre, start the kd-tree
+// thread, lay out the grid, grow every buffer; nothing enqueued), enqueue (device centring of the positions
+// in ctx->d_tmp, the index kernels and their two length copies), complete (wait, grow and run again if the
+// candidate records did not fit, commit the counters)
+int stocs_index_plan(stocs_b200_ctx* ctx);
+int stocs_index_enqueue(stocs_b200_ctx* ctx);
+int stocs_index_complete(stocs_b200_ctx* ctx);
 int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4* d_out4,
                         float* d_out3, float* h_centroid3, float* h_aabb6, const float* h_pos3 = nullptr,
                         float* h_centred3 = nullptr);
@@ -366,8 +382,17 @@ struct PipeClusterInputs {
   StocsPipeState* d_state;
 };
 int stocs_cluster_check(stocs_b200_ctx* ctx, const stocs_b200_cluster_params* p, int64_t cap);
+// Calls over one context per object (capi.cu): stocs_batch_check rejects n_objects < 1, a NULL entry and
+// a context given twice; stocs_batch_fail sets "who: object k: msg" on ctxs[k] and ctxs[0] (k < 0: on
+// ctxs[0] only, without an object) and returns code.
+int stocs_batch_check(stocs_b200_ctx* const* ctxs, int n_objects, const char* who);
+int stocs_batch_fail(stocs_b200_ctx* const* ctxs, int k, int code, const char* who, const std::string& msg);
+// the context can run instance-mode sampling: edge map, pixel coordinates inside it (sample_instance.cu)
+int stocs_instance_check(stocs_b200_ctx* ctx);
 int stocs_cluster_enqueue_pipeline(stocs_b200_ctx* ctx, const stocs_b200_cluster_params& p, const PipeClusterInputs& in,
                                    cudaStream_t st);
+// grows the scratch of stocs_cluster_enqueue_pipeline over cap_items items; enqueues nothing
+int stocs_cluster_reserve(stocs_b200_ctx* ctx, long long cap_items);
 const stocs_b200_pose* stocs_cluster_poses_host(stocs_b200_ctx* ctx);
 void stocs_cluster_free_host(stocs_b200_ctx* ctx);
 
