@@ -89,6 +89,30 @@ int stocs_b200_build_scene_clouds(stocs_b200_ctx* ctx, const uint16_t* depth, co
                                   float* pos3, float* nrm3, float* rgb3, int32_t* pixel_rc, float* class_p,
                                   float* edge_p, int64_t cap, int64_t* offsets);
 
+/* The same from a frame already in GPU memory (e.g. a segmentation network's output), with the same stages, output
+ * order, CSR offsets (a host array), capacity rule and STOCS_E_CAPACITY with offsets filled.  Every image and output
+ * pointer is device memory on the context's device; d_bgr, d_edge, d_rgb3 and d_edge_p may be NULL.  d_class_maps is
+ * a host array of n_objects device pointers, each to a row-major W*H map of map_type; entries may repeat, so the
+ * channels of a [C,H,W] tensor can be passed in any order without a copy.
+ *   STOCS_B200_MAP_U16: uint16, converted as build_scene_clouds does, (float)((double)(float)v * (1.0/10000));
+ *   STOCS_B200_MAP_F32: float, used as given; the class test is p == p && !(p < threshold), so a NaN never passes,
+ *   and a float map holding the exact uint16 conversion gives bit-identical output.
+ * stream (a cudaStream_t of the context's device; NULL is its default stream): the call's work is ordered after
+ * what the caller has queued on it so far.  The call synchronises once and reads back only the voxel count and the
+ * object ends; on return the outputs are complete, and rows past offsets[n_objects] are not written.  The context's
+ * read-back estimate afterwards is what build_scene_clouds leaves.  STOCS_E_ARG, before anything
+ * is enqueued: the checks of build_scene_clouds, an unknown map_type, a NULL map entry, or a pointer that is not
+ * device memory on the context's device (the message names the argument).  Nothing of the frame or the cloud
+ * crosses PCIe. */
+enum { STOCS_B200_MAP_U16 = 0, STOCS_B200_MAP_F32 = 1 };
+int stocs_b200_build_scene_clouds_device(
+    stocs_b200_ctx* ctx, const uint16_t* d_depth, const uint8_t* d_bgr,
+    const void* const* d_class_maps, int map_type, const float* class_thresholds, int n_objects,
+    const uint8_t* d_edge, int W, int H, float fx, float cx, float fy, float cy,
+    float depth_scale, float voxel_size,
+    float* d_pos3, float* d_nrm3, float* d_rgb3, int32_t* d_pixel_rc, float* d_class_p, float* d_edge_p,
+    int64_t cap, int64_t* offsets, void* stream);
+
 /* ---- a2/a11: model and scene upload --------------------------------------------------------
  * upload_model replaces load_object_info's point part (src/stocs.cpp:86-97) and the model half of
  * centroid_shift (src/stocs.cpp:951-962); it also builds the compact own-bin PPF table that
@@ -326,6 +350,17 @@ int stocs_b200_run_pipeline_instance_clustered(stocs_b200_ctx* ctx, uint64_t see
  * (pos3, nrm3, class_p as class_probability, pixel_rc or NULL); offsets has n_objects + 1 entries. */
 int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const float* pos3, const float* nrm3,
                              const float* class_probability, const int32_t* pixel_rc, const int64_t* offsets);
+
+/* upload_scenes, word for word, from device arrays, e.g. the outputs of build_scene_clouds_device: the arrays are
+ * device memory on any device (a context on another device copies its slice with cudaMemcpyPeerAsync); offsets is a
+ * host array.  The positions, class weights and pixel coordinates of each slice are copied once into page-locked
+ * memory the context owns (the centroid, pixel range, class-weight bound and kd-tree are host work); everything else
+ * moves device to device.  d_nrm3, d_class_probability and d_pixel_rc (may be NULL) are on the device of d_pos3; a
+ * pointer that is not device memory is STOCS_E_ARG.  stream (a cudaStream_t of that device; NULL is its default
+ * stream): the call's work is ordered after what the caller has queued on it so far. */
+int stocs_b200_upload_scenes_device(stocs_b200_ctx* const* ctxs, int n_objects, const float* d_pos3,
+                                    const float* d_nrm3, const float* d_class_probability, const int32_t* d_pixel_rc,
+                                    const int64_t* offsets, void* stream);
 
 /* instance_mode 0 or 1; cluster: NULL (plain run) or n_objects parameter records (sym_info is per
  * object); results: n_objects records; poses: n_objects * cap records, object k's at poses + k * cap, and

@@ -18,7 +18,7 @@ _LIB = None
 SYMBOLS = [
     "stocs_b200_abi_version", "stocs_b200_create", "stocs_b200_destroy", "stocs_b200_last_error",
     "stocs_b200_set_params", "stocs_b200_backproject", "stocs_b200_build_scene_cloud", "stocs_b200_build_scene_clouds",
-    "stocs_b200_upload_model",
+    "stocs_b200_build_scene_clouds_device", "stocs_b200_upload_model",
     "stocs_b200_upload_scene", "stocs_b200_get_centroids", "stocs_b200_get_centred",
     "stocs_b200_ppf_num_pairs", "stocs_b200_ppf_num_expanded_keys", "stocs_b200_ppf_export",
     "stocs_b200_ppf_lookup", "stocs_b200_upload_ppf_table", "stocs_b200_sample_bases",
@@ -29,7 +29,7 @@ SYMBOLS = [
     "stocs_b200_icp_point_to_plane",
     "stocs_b200_run_pipeline", "stocs_b200_run_pipeline_instance", "stocs_b200_cluster_poses",
     "stocs_b200_run_pipeline_clustered", "stocs_b200_run_pipeline_instance_clustered",
-    "stocs_b200_upload_scenes", "stocs_b200_run_pipelines", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
+    "stocs_b200_upload_scenes", "stocs_b200_upload_scenes_device", "stocs_b200_run_pipelines", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
     "stocs_b200_score_counters", "stocs_b200_kernel_ms_stats", "stocs_b200_host_kdtree_order",
     "stocs_b200_debug_angle_estimates",
     "stocs_b200_comm_unique_id", "stocs_b200_comm_init", "stocs_b200_comm_destroy", "stocs_b200_shard_range",
@@ -85,6 +85,8 @@ def lib():
                                                vp, vp, vp, vp, vp, vp, i64, C.POINTER(i64)]
     L.stocs_b200_build_scene_clouds.argtypes = [vp, vp, vp, vp, vp, i32, vp, i32, i32, f32, f32, f32, f32, f32, f32,
                                                 vp, vp, vp, vp, vp, vp, i64, vp]
+    L.stocs_b200_build_scene_clouds_device.argtypes = [vp, vp, vp, vp, i32, vp, i32, vp, i32, i32, f32, f32, f32, f32, f32,
+                                                       f32, vp, vp, vp, vp, vp, vp, i64, vp, vp]
     L.stocs_b200_upload_model.argtypes = [vp, vp, vp, i32]
     L.stocs_b200_upload_scene.argtypes = [vp, vp, vp, vp, vp, i32]
     L.stocs_b200_get_centroids.argtypes = [vp, vp, vp]
@@ -115,6 +117,7 @@ def lib():
     L.stocs_b200_run_pipeline_instance_clustered.argtypes = [vp, u64, i32, i32, f32, C.POINTER(ClusterParams),
                                                              C.POINTER(PipelineResult), vp, i32, C.POINTER(i32)]
     L.stocs_b200_upload_scenes.argtypes = [vp, i32, vp, vp, vp, vp, vp]
+    L.stocs_b200_upload_scenes_device.argtypes = [vp, i32, vp, vp, vp, vp, vp, vp]
     L.stocs_b200_run_pipelines.argtypes = [vp, i32, vp, i32, i32, i32, f32, vp, vp, vp, i32, vp]
     L.stocs_b200_get_counters.argtypes = [vp, vp, i32]
     L.stocs_b200_last_kernel_ms.argtypes = [vp, C.POINTER(f32)]
@@ -173,27 +176,59 @@ def _has_scene(ctx):
     return lib().stocs_b200_get_centroids(ctx.h, _ptr(np.zeros(3, np.float32)), None) == 0
 
 
+def _csr_device(clouds, key, cols, dtype, offs):
+    """The CSR array of one key of CUDA-tensor clouds -> (device pointer, tensor to keep alive): the slices' own
+    buffer when they are consecutive views of it (the outputs of Context.build_scene_clouds_device), else their
+    concatenation."""
+    import torch
+    parts = [c[key] for c in clouds]
+    used = [(p, int(o)) for p, o in zip(parts, offs[:-1]) if p.numel()]
+    row = cols * torch.empty(0, dtype=dtype).element_size()
+    if used and all(p.dtype == dtype and p.is_contiguous() and p.device == used[0][0].device for p, _ in used):
+        base = used[0][0].data_ptr() - used[0][1] * row
+        if all(p.data_ptr() == base + o * row for p, o in used):
+            return base, None
+    dev = parts[0].device
+    cat = torch.cat([p.reshape(-1, cols).to(dev, dtype) for p in parts]) if used else torch.zeros((1, cols), dtype=dtype, device=dev)
+    return cat.data_ptr(), cat
+
+
+def _upload_scenes_device(contexts, clouds, offs, has_pix):
+    import torch
+    arrays = [_csr_device(clouds, "pos", 3, torch.float32, offs), _csr_device(clouds, "nrm", 3, torch.float32, offs),
+              _csr_device(clouds, "cls", 1, torch.float32, offs)]
+    arrays.append(_csr_device(clouds, "pix", 2, torch.int32, offs) if has_pix else (None, None))
+    stream = torch.cuda.current_stream(clouds[0]["pos"].device).cuda_stream
+    return lib().stocs_b200_upload_scenes_device(_handles(contexts), len(contexts), *[a[0] for a in arrays], _ptr(offs),
+                                                 stream)
+
+
 def upload_scenes(contexts, clouds):
     """Object k's cloud (a dict of Context.build_scene_clouds: pos, nrm, cls and optionally pix) to contexts[k],
-    every object in one call (stocs_b200_upload_scenes); an empty cloud leaves its context with an empty scene."""
+    every object in one call (stocs_b200_upload_scenes); an empty cloud leaves its context with an empty scene.
+    Clouds of torch CUDA tensors (Context.build_scene_clouds_device) go to stocs_b200_upload_scenes_device, ordered
+    after torch's current stream; views of one output buffer are passed without a copy."""
     assert len(contexts) == len(clouds), "one cloud per context"
     n = [len(c["pos"]) for c in clouds]
     if len({id(c) for c in contexts}) < len(contexts) or any(not c.h for c in contexts) or max(n, default=0) > (1 << 27):
         raise StocsError("upload_scenes: a context given twice or closed, or a slice over 2^27 points")
     offs = np.fromiter(itertools.accumulate(n, initial=0), np.int64, len(n) + 1)
     has_pix = all(c.get("pix") is not None for c in clouds)
-    if len(clouds) == 1:   # one object's arrays are passed as they are
-        c = clouds[0]
-        pos, nrm, cls = _f32(c["pos"], (-1, 3)), _f32(c["nrm"], (-1, 3)), _f32(c["cls"], (-1,))
-        pix = np.ascontiguousarray(c["pix"], np.int32).reshape(-1, 2) if has_pix else None
-    else:                  # the CSR concatenation
-        pos = np.concatenate([_f32(c["pos"], (-1, 3)) for c in clouds])
-        nrm = np.concatenate([_f32(c["nrm"], (-1, 3)) for c in clouds])
-        cls = np.concatenate([_f32(c["cls"], (-1,)) for c in clouds])
-        pix = np.concatenate([np.ascontiguousarray(c["pix"], np.int32).reshape(-1, 2) for c in clouds]) if has_pix else None
-    assert pos.shape == nrm.shape and cls.shape[0] == pos.shape[0]
-    rc = lib().stocs_b200_upload_scenes(_handles(contexts), len(contexts), _ptr(pos), _ptr(nrm), _ptr(cls), _ptr(pix),
-                                        _ptr(offs))
+    if getattr(clouds[0]["pos"], "is_cuda", False):
+        rc = _upload_scenes_device(contexts, clouds, offs, has_pix)
+    else:
+        if len(clouds) == 1:   # one object's arrays are passed as they are
+            c = clouds[0]
+            pos, nrm, cls = _f32(c["pos"], (-1, 3)), _f32(c["nrm"], (-1, 3)), _f32(c["cls"], (-1,))
+            pix = np.ascontiguousarray(c["pix"], np.int32).reshape(-1, 2) if has_pix else None
+        else:                  # the CSR concatenation
+            pos = np.concatenate([_f32(c["pos"], (-1, 3)) for c in clouds])
+            nrm = np.concatenate([_f32(c["nrm"], (-1, 3)) for c in clouds])
+            cls = np.concatenate([_f32(c["cls"], (-1,)) for c in clouds])
+            pix = np.concatenate([np.ascontiguousarray(c["pix"], np.int32).reshape(-1, 2) for c in clouds]) if has_pix else None
+        assert pos.shape == nrm.shape and cls.shape[0] == pos.shape[0]
+        rc = lib().stocs_b200_upload_scenes(_handles(contexts), len(contexts), _ptr(pos), _ptr(nrm), _ptr(cls), _ptr(pix),
+                                            _ptr(offs))
     err = None
     try:
         contexts[0]._check(rc)
@@ -345,6 +380,58 @@ class Context:
             self._check(rc)
             return [dict(pos=pos[a:b].copy(), nrm=nrm[a:b].copy(), rgb=rgb[a:b].copy(), pix=pix[a:b].copy(),
                          cls=cls[a:b].copy(), edge=ep[a:b].copy()) for a, b in zip(offs[:-1], offs[1:])]
+
+    def build_scene_clouds_device(self, depth, bgr, maps, edge, K, depth_scale, voxel_size, class_thresholds, cap=None,
+                                  stream=None):
+        """build_scene_clouds from a frame already on this context's GPU (stocs_b200_build_scene_clouds_device).  torch
+        CUDA tensors: depth [H, W] and maps 2-byte (read as uint16), bgr [H, W, 3] and edge [H, W] uint8 or None; maps
+        is a [n, H, W] tensor or a list of n [H, W] tensors, all float32 (used as given) or all 2-byte (converted as
+        build_scene_clouds does), and may repeat.  stream (torch.cuda.Stream or a raw handle; default: torch's current
+        stream) is the one the inputs were written on.  -> n dicts of CUDA tensor views (pos nrm rgb pix cls edge),
+        shaped as build_scene_clouds returns them; cap: rows of the output buffers (default H * W, grown to the
+        frame's size when more are needed)."""
+        import torch
+        two_byte = (torch.uint16, torch.int16)
+
+        def image(t, name, dtypes):
+            if t is None:
+                return None
+            if not (isinstance(t, torch.Tensor) and t.is_cuda and t.dtype in dtypes):
+                raise StocsError(f"build_scene_clouds_device: {name} must be a CUDA tensor of {dtypes}")
+            return t.contiguous()
+
+        depth = image(depth, "depth", two_byte)
+        H, W = depth.shape
+        bgr, edge = image(bgr, "bgr", (torch.uint8,)), image(edge, "edge", (torch.uint8,))
+        maps = [image(m, "maps", two_byte + (torch.float32,)) for m in maps]
+        if len({m.dtype == torch.float32 for m in maps}) != 1 or any(tuple(m.shape) != (H, W) for m in maps):
+            raise StocsError("build_scene_clouds_device: maps must be [H, W] each, all float32 or all 2-byte")
+        n_obj = len(maps)
+        map_type = 1 if maps[0].dtype == torch.float32 else 0   # STOCS_B200_MAP_F32 / _U16
+        table = (C.c_void_p * n_obj)(*[m.data_ptr() for m in maps])
+        thr = np.ascontiguousarray(np.broadcast_to(np.asarray(class_thresholds, np.float32), (n_obj,)))
+        if stream is None:
+            stream = torch.cuda.current_stream(depth.device)
+        stream = getattr(stream, "cuda_stream", stream)
+        dev = torch.device("cuda", self.device)
+        offs = np.zeros(n_obj + 1, np.int64)
+        cap = H * W if cap is None else int(cap)
+        while True:
+            c = max(cap, 1)
+            pos, nrm, rgb = (torch.empty((c, 3), dtype=torch.float32, device=dev) for _ in range(3))
+            pix = torch.empty((c, 2), dtype=torch.int32, device=dev)
+            cls, ep = torch.empty(c, dtype=torch.float32, device=dev), torch.empty(c, dtype=torch.float32, device=dev)
+            ptr = [None if t is None else t.data_ptr() for t in (depth, bgr)]
+            rc = self._L.stocs_b200_build_scene_clouds_device(
+                self.h, ptr[0], ptr[1], table, map_type, _ptr(thr), n_obj, None if edge is None else edge.data_ptr(), W, H,
+                K[0], K[1], K[2], K[3], depth_scale, voxel_size, pos.data_ptr(), nrm.data_ptr(), rgb.data_ptr(),
+                pix.data_ptr(), cls.data_ptr(), ep.data_ptr(), cap, _ptr(offs), stream)
+            if rc == -5:  # STOCS_E_CAPACITY: offsets are filled
+                cap = int(offs[-1])
+                continue
+            self._check(rc)
+            return [dict(pos=pos[a:b], nrm=nrm[a:b], rgb=rgb[a:b], pix=pix[a:b], cls=cls[a:b], edge=ep[a:b])
+                    for a, b in zip(offs[:-1], offs[1:])]
 
     # ---- uploads
     def upload_model(self, pos, nrm):

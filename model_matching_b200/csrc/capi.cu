@@ -7,6 +7,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <utility>
 
 #include "stocs_ctx.h"
 
@@ -32,6 +33,14 @@ const void* stocs_host_alias(const void* p) {
   cudaPointerAttributes pa{};
   if (cudaPointerGetAttributes(&pa, p) != cudaSuccess) { cudaGetLastError(); return nullptr; }
   return pa.type == cudaMemoryTypeHost ? pa.devicePointer : nullptr;
+}
+
+bool stocs_device_memory(const void* p, int device, int* owner) {
+  cudaPointerAttributes pa{};
+  if (!p || cudaPointerGetAttributes(&pa, p) != cudaSuccess) { cudaGetLastError(); return false; }
+  if (pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) return false;
+  if (owner) *owner = pa.device;
+  return device < 0 || pa.device == device;
 }
 
 // The host-buffer scoring calls read page-locked transforms in place through their device alias;
@@ -242,6 +251,7 @@ void stocs_b200_destroy(stocs_b200_ctx* ctx) {
   stocs_cluster_free_host(ctx);
   if (ctx->h_index_counts) cudaFreeHost(ctx->h_index_counts);
   if (ctx->h_kd_stage) cudaFreeHost(ctx->h_kd_stage);
+  if (ctx->h_scene_stage) cudaFreeHost(ctx->h_scene_stage);
   if (ctx->kd_copy_done) cudaEventDestroy(ctx->kd_copy_done);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -364,26 +374,27 @@ static int scene_upload_plan(stocs_b200_ctx* ctx, const float* pos3, const float
   return stocs_index_plan(ctx);
 }
 
-// Second step: the uploads and kernels, up to the index build's two length copies; no synchronisation.
+// Second step: the uploads and kernels, up to the index build's two length copies; no synchronisation.  The
+// arrays are copied with `kind`: host arrays (upload_scene[s]) or device arrays on the context's device.
 static int scene_upload_enqueue(stocs_b200_ctx* ctx, const float* pos3, const float* nrm3, const float* class_probability,
-                                const int32_t* pixel_rc, int S) {
+                                const int32_t* pixel_rc, int S, cudaMemcpyKind kind) {
   cudaSetDevice(ctx->device);
   cudaStream_t st = ctx->stream;
   float* d_n = ctx->d_tmp.as<float>();
   float* d_c = d_n + (size_t)S * 3;
-  STOCS_CUDA(ctx, cudaMemcpyAsync(d_n, nrm3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
-  STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, class_probability, (size_t)S * 4, cudaMemcpyHostToDevice, st));
+  STOCS_CUDA(ctx, cudaMemcpyAsync(d_n, nrm3, (size_t)S * 12, kind, st));
+  STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, class_probability, (size_t)S * 4, kind, st));
   int rc = stocs_pack_scene_attr(ctx, d_n, d_c, S);
   if (rc) return rc;
   // (no synchronisation: the position upload below re-uses d_tmp in stream order, and the H2D copies
   // of pageable host memory have consumed their source buffers when cudaMemcpyAsync returns)
-  if (pixel_rc) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_spix.p, pixel_rc, (size_t)S * 8, cudaMemcpyHostToDevice, st));
+  if (pixel_rc) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_spix.p, pixel_rc, (size_t)S * 8, kind, st));
   else STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_spix.p, 0, (size_t)S * 8, st));
   ctx->has_pixels = pixel_rc != nullptr;
   if (ctx->d_inst_state.p)  // a new scene starts with empty previous_segment / segmentation_buffer
     STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_inst_state.p, 0, (size_t)ctx->img_w * ctx->img_h * 3, st));
   // positions -> centre -> index (the device-centroid path has centred them in the plan)
-  if (ctx->h_pos_pending) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_tmp.p, pos3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
+  if (ctx->h_pos_pending) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_tmp.p, pos3, (size_t)S * 12, kind, st));
   return stocs_index_enqueue(ctx);
 }
 
@@ -427,15 +438,18 @@ int stocs_b200_upload_scene(stocs_b200_ctx* ctx, const float* pos3, const float*
   if (!pos3 || !nrm3 || !class_probability || S <= 0) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: bad argument");
   if (S > (1 << 27)) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: at most 2^27 scene points are supported");
   int rc = scene_upload_plan(ctx, pos3, class_probability, pixel_rc, S);
-  if (rc == STOCS_OK) rc = scene_upload_enqueue(ctx, pos3, nrm3, class_probability, pixel_rc, S);
+  if (rc == STOCS_OK) rc = scene_upload_enqueue(ctx, pos3, nrm3, class_probability, pixel_rc, S, cudaMemcpyHostToDevice);
   return scene_upload_end(ctx, rc);
 }
 
-// Every object's buffers are grown before any object's work is enqueued, and every object's work is
-// enqueued before any is waited for: the host waits once per context, at the end.
-int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const float* pos3, const float* nrm3,
-                             const float* class_probability, const int32_t* pixel_rc, const int64_t* offsets) {
-  const char* who = "upload_scenes";
+}  // extern "C"
+
+// One object's slice of the CSR arrays of an upload over several contexts (pix may be NULL)
+struct SceneSlice { const float* pos3; const float* nrm3; const float* cls; const int32_t* pix; };
+
+// The checks upload_scenes and upload_scenes_device share, on the arguments they both take.
+static int upload_scenes_check(stocs_b200_ctx* const* ctxs, int n_objects, const char* who, const float* pos3,
+                               const float* nrm3, const float* class_probability, const int64_t* offsets) {
   int rc = stocs_batch_check(ctxs, n_objects, who);
   if (rc) return rc;
   if (!pos3 || !nrm3 || !class_probability || !offsets) return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, "bad argument");
@@ -445,11 +459,17 @@ int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const f
     if (S < 0) return stocs_batch_fail(ctxs, k, STOCS_E_ARG, who, "offsets decrease");
     if (S > (1 << 27)) return stocs_batch_fail(ctxs, k, STOCS_E_ARG, who, "at most 2^27 scene points are supported");
   }
-  std::vector<int> status(n_objects, STOCS_OK);
+  return STOCS_OK;
+}
+
+// Every object's buffers are grown before any object's work is enqueued, and every object's work is
+// enqueued before any is waited for: the host waits once per context, at the end.  Object k's host work reads
+// host[k]; its uploads copy dev[k] with `kind`.  An object whose status is already an error is only ended.
+static int upload_slices(stocs_b200_ctx* const* ctxs, int n_objects, const char* who, const int64_t* offsets,
+                         const SceneSlice* host, const SceneSlice* dev, cudaMemcpyKind kind, std::vector<int>& status) {
   for (int k = 0; k < n_objects; ++k) {   // every object's host work and buffer growth first ...
     stocs_b200_ctx* ctx = ctxs[k];
-    const int64_t o = offsets[k];
-    const int S = (int)(offsets[k + 1] - o);
+    const int S = (int)(offsets[k + 1] - offsets[k]);
     if (S == 0) {   // an object that is not visible: no scene, nothing enqueued
       cudaSetDevice(ctx->device);
       ctx->S = 0;
@@ -459,20 +479,108 @@ int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const f
       ctx->counters[CTR_GRID_CELLS] = ctx->counters[CTR_CANDIDATES] = ctx->counters[CTR_OCCUPIED_CELLS] = 0;
       continue;
     }
-    status[k] = scene_upload_plan(ctx, pos3 + 3 * o, class_probability + o, pixel_rc ? pixel_rc + 2 * o : nullptr, S);
+    if (status[k] == STOCS_OK) status[k] = scene_upload_plan(ctx, host[k].pos3, host[k].cls, host[k].pix, S);
   }
   for (int k = 0; k < n_objects; ++k) {   // ... then every object's uploads and kernels
-    const int64_t o = offsets[k];
-    const int S = (int)(offsets[k + 1] - o);
+    const int S = (int)(offsets[k + 1] - offsets[k]);
     if (S > 0 && status[k] == STOCS_OK)
-      status[k] = scene_upload_enqueue(ctxs[k], pos3 + 3 * o, nrm3 + 3 * o, class_probability + o,
-                                       pixel_rc ? pixel_rc + 2 * o : nullptr, S);
+      status[k] = scene_upload_enqueue(ctxs[k], dev[k].pos3, dev[k].nrm3, dev[k].cls, dev[k].pix, S, kind);
   }
   for (int k = 0; k < n_objects; ++k)
     if (offsets[k + 1] > offsets[k]) status[k] = scene_upload_end(ctxs[k], status[k]);
   for (int k = 0; k < n_objects; ++k)
     if (status[k]) return stocs_batch_fail(ctxs, k, status[k], who, ctxs[k]->err);
   return STOCS_OK;
+}
+
+extern "C" {
+
+int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const float* pos3, const float* nrm3,
+                             const float* class_probability, const int32_t* pixel_rc, const int64_t* offsets) {
+  const char* who = "upload_scenes";
+  int rc = upload_scenes_check(ctxs, n_objects, who, pos3, nrm3, class_probability, offsets);
+  if (rc) return rc;
+  std::vector<SceneSlice> slices(n_objects);
+  for (int k = 0; k < n_objects; ++k) {
+    const int64_t o = offsets[k];
+    slices[k] = SceneSlice{pos3 + 3 * o, nrm3 + 3 * o, class_probability + o, pixel_rc ? pixel_rc + 2 * o : nullptr};
+  }
+  std::vector<int> status(n_objects, STOCS_OK);
+  return upload_slices(ctxs, n_objects, who, offsets, slices.data(), slices.data(), cudaMemcpyHostToDevice, status);
+}
+
+// The slices' positions, class weights and pixels are staged into each context's page-locked memory (a context on
+// another device first copies its slice to its own device), the host waits once per context, and the host plan of
+// upload_scenes runs on the staged copies; the kernels' inputs are copied device to device.
+int stocs_b200_upload_scenes_device(stocs_b200_ctx* const* ctxs, int n_objects, const float* d_pos3, const float* d_nrm3,
+                                    const float* d_class_probability, const int32_t* d_pixel_rc, const int64_t* offsets,
+                                    void* stream) {
+  const char* who = "upload_scenes_device";
+  int rc = upload_scenes_check(ctxs, n_objects, who, d_pos3, d_nrm3, d_class_probability, offsets);
+  if (rc) return rc;
+  int src_dev = -1;
+  if (!stocs_device_memory(d_pos3, -1, &src_dev)) return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, "d_pos3 is not device memory");
+  const std::pair<const void*, const char*> others[] = {{d_nrm3, "d_nrm3"}, {d_class_probability, "d_class_probability"},
+                                                        {d_pixel_rc, "d_pixel_rc"}};
+  for (const auto& a : others)
+    if (a.first && !stocs_device_memory(a.first, src_dev))
+      return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, std::string(a.second) + " is not device memory on the device of d_pos3");
+  std::vector<int> status(n_objects, STOCS_OK);
+  std::vector<SceneSlice> host(n_objects), dev(n_objects);
+  auto fail = [&](int k, cudaError_t e, const char* what) {
+    if (e == cudaSuccess || status[k]) return;
+    ctxs[k]->err = std::string(what) + ": " + cudaGetErrorString(e);
+    status[k] = STOCS_E_CUDA;
+  };
+  for (int k = 0; k < n_objects; ++k) {   // growth first: page-locked staging, and the device copy of a foreign slice
+    stocs_b200_ctx* ctx = ctxs[k];
+    const size_t S = (size_t)(offsets[k + 1] - offsets[k]);
+    if (S == 0) continue;
+    cudaSetDevice(ctx->device);
+    if (ctx->h_scene_stage_bytes < S * 24) {
+      if (ctx->h_scene_stage) cudaFreeHost(ctx->h_scene_stage);
+      ctx->h_scene_stage = nullptr; ctx->h_scene_stage_bytes = 0;
+      fail(k, cudaHostAlloc(&ctx->h_scene_stage, S * 24, cudaHostAllocDefault), "cudaHostAlloc");
+      if (!status[k]) ctx->h_scene_stage_bytes = S * 24;
+    }
+    if (ctx->device != src_dev) fail(k, ctx->pool[POOL_SCENE_PEER].ensure(S * 36), "peer copy buffer");
+  }
+  CallerEvent producer;
+  const cudaError_t ev = producer.record(stream, src_dev);
+  for (int k = 0; k < n_objects; ++k) {   // then every object's copies ...
+    stocs_b200_ctx* ctx = ctxs[k];
+    const int64_t o = offsets[k];
+    const size_t S = (size_t)(offsets[k + 1] - o);
+    if (S == 0) continue;
+    fail(k, ev, "cudaEventRecord on the caller's stream");
+    if (status[k]) continue;
+    cudaSetDevice(ctx->device);
+    cudaStream_t st = ctx->stream;
+    fail(k, producer.wait(st), "cudaStreamWaitEvent");
+    SceneSlice d{d_pos3 + 3 * o, d_nrm3 + 3 * o, d_class_probability + o, d_pixel_rc ? d_pixel_rc + 2 * o : nullptr};
+    if (ctx->device != src_dev) {   // the slice moves to this context's device first
+      float* p = ctx->pool[POOL_SCENE_PEER].as<float>();
+      const SceneSlice local{p, p + 3 * S, p + 6 * S, d.pix ? (const int32_t*)(p + 7 * S) : nullptr};
+      fail(k, cudaMemcpyPeerAsync((void*)local.pos3, ctx->device, d.pos3, src_dev, S * 12, st), "cudaMemcpyPeerAsync");
+      fail(k, cudaMemcpyPeerAsync((void*)local.nrm3, ctx->device, d.nrm3, src_dev, S * 12, st), "cudaMemcpyPeerAsync");
+      fail(k, cudaMemcpyPeerAsync((void*)local.cls, ctx->device, d.cls, src_dev, S * 4, st), "cudaMemcpyPeerAsync");
+      if (d.pix) fail(k, cudaMemcpyPeerAsync((void*)local.pix, ctx->device, d.pix, src_dev, S * 8, st), "cudaMemcpyPeerAsync");
+      d = local;
+    }
+    dev[k] = d;
+    float* h = (float*)ctx->h_scene_stage;   // pos3 | cls | pix
+    host[k] = SceneSlice{h, nullptr, h + 3 * S, d.pix ? (const int32_t*)(h + 4 * S) : nullptr};
+    fail(k, cudaMemcpyAsync((void*)host[k].pos3, d.pos3, S * 12, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
+    fail(k, cudaMemcpyAsync((void*)host[k].cls, d.cls, S * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
+    if (d.pix) fail(k, cudaMemcpyAsync((void*)host[k].pix, d.pix, S * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
+  }
+  for (int k = 0; k < n_objects; ++k)     // ... one wait per context ...
+    if (offsets[k + 1] > offsets[k]) {
+      cudaSetDevice(ctxs[k]->device);
+      fail(k, cudaStreamSynchronize(ctxs[k]->stream), "cudaStreamSynchronize");
+    }
+  // ... and the plan, uploads and index builds of upload_scenes
+  return upload_slices(ctxs, n_objects, who, offsets, host.data(), dev.data(), cudaMemcpyDeviceToDevice, status);
 }
 
 int stocs_b200_get_centroids(stocs_b200_ctx* ctx, float* scene3, float* model3) {

@@ -20,6 +20,7 @@
 
 #include <algorithm>
 #include <cmath>
+#include <utility>
 
 #include "stocs_ctx.h"
 #include "stocs_scene_math.h"
@@ -136,7 +137,8 @@ __global__ void outlier_kernel(const float4* __restrict__ cent, const unsigned l
 // exactly when its entry and the next one differ, and entry k * (n + 1) + n ends object k's rows.
 struct FilterArgs {
   const float4* cent; const int* keep; const int* nvox_p; int n; int n_obj; int out_cap;
-  const uint16_t* depth; const uint8_t* bgr; const uint16_t* prob; const uint8_t* edge;   // prob: n_obj maps of n
+  const uint16_t* depth; const uint8_t* bgr; const uint8_t* edge;
+  const void* map[STOCS_B200_MAX_CLOUD_OBJECTS];   // object k's W*H map, of the kernel's map type; entries may repeat
   int W, H; float fx, cx, fy, cy;
   float class_threshold[STOCS_B200_MAX_CLOUD_OBJECTS];
   int* rows;       // n_obj * (n + 1)
@@ -144,12 +146,16 @@ struct FilterArgs {
   int* rc;         // nvox * 2
 };
 
+// MAP_U16: the reference's conversion of the 16-bit map; MAP_F32: the value as given
+template <int MT>
 __device__ __forceinline__ float class_probability_at(const FilterArgs& a, int k, size_t px) {
-  return (float)((double)(float)a.prob[(size_t)k * a.n + px] * (1.0 / 10000));
+  if (MT == STOCS_B200_MAP_F32) return ((const float*)a.map[k])[px];
+  return (float)((double)(float)((const uint16_t*)a.map[k])[px] * (1.0 / 10000));
 }
 
 // src/rgbd.cpp:238-279 per centroid: everything but the class test is the same for every object, and the
-// normal is computed once, when some object passes
+// normal is computed once, when some object passes.  A NaN probability never passes (a u16 map has none).
+template <int MT>
 __global__ void filter_kernel(const __grid_constant__ FilterArgs a) {
   const int v = blockIdx.x * blockDim.x + threadIdx.x;
   if (v > a.n) return;
@@ -161,8 +167,10 @@ __global__ void filter_kernel(const __grid_constant__ FilterArgs a) {
       reproject(p.x, p.y, p.z, a.fx, a.cx, a.fy, a.cy, &row, &col);
       if (row >= 0 && row < a.H && col >= 0 && col < a.W) {  // the reference indexes unchecked here
         const size_t px = (size_t)row * a.W + col;
-        for (int k = 0; k < a.n_obj; ++k)
-          if (!(class_probability_at(a, k, px) < a.class_threshold[k])) pass |= 1u << k;
+        for (int k = 0; k < a.n_obj; ++k) {
+          const float p = class_probability_at<MT>(a, k, px);
+          if (p == p && !(p < a.class_threshold[k])) pass |= 1u << k;
+        }
         if (pass) {
           float n[3];
           linemod_normal_at(a.depth, a.W, a.H, row, col, a.fx, a.cx, a.fy, a.cy, n);
@@ -181,6 +189,7 @@ __global__ void filter_kernel(const __grid_constant__ FilterArgs a) {
 }
 
 // after the scan: ends[k] = end of object k's rows; every emitted (object, centroid) pair to its row
+template <int MT>
 __global__ void emit_kernel(const __grid_constant__ FilterArgs a, int* __restrict__ ends, float* __restrict__ pos3,
                             float* __restrict__ nrm3, float* __restrict__ rgb3, int* __restrict__ pix2,
                             float* __restrict__ cls, float* __restrict__ edgep) {
@@ -207,32 +216,44 @@ __global__ void emit_kernel(const __grid_constant__ FilterArgs a, int* __restric
     nrm3[3 * (size_t)o] = n.x; nrm3[3 * (size_t)o + 1] = n.y; nrm3[3 * (size_t)o + 2] = n.z;
     if (rgb3) { rgb3[3 * (size_t)o] = r; rgb3[3 * (size_t)o + 1] = g; rgb3[3 * (size_t)o + 2] = b; }
     pix2[2 * (size_t)o] = row; pix2[2 * (size_t)o + 1] = col;
-    cls[o] = class_probability_at(a, k, px);
+    cls[o] = class_probability_at<MT>(a, k, px);
     if (edgep) edgep[o] = e;
   }
 }
 
-// stocs_b200_build_scene_cloud is the one-object case of stocs_b200_build_scene_clouds; `who` prefixes the
-// error messages.
-int build_scene_clouds(stocs_b200_ctx* ctx, const char* who, const uint16_t* depth, const uint8_t* bgr,
-                       const uint16_t* class_probs, const float* class_thresholds, int n_objects, const uint8_t* edge,
-                       int W, int H, float fx, float cx, float fy, float cy, float depth_scale, float voxel_size,
-                       float* pos3, float* nrm3, float* rgb3, int32_t* pixel_rc, float* class_p, float* edge_p,
-                       int64_t cap, int64_t* offsets) {
+// One frame as the shared stages read it: images and maps in device memory on the context's device
+struct CloudFrame {
+  const uint16_t* depth; const uint8_t* bgr; const uint8_t* edge;   // bgr, edge may be NULL
+  const void* const* maps; int map_type;                            // n_objects W*H maps of map_type
+  const float* thresholds; int n_objects;
+  int W, H; float fx, cx, fy, cy, depth_scale, voxel_size;
+};
+
+// Where emit_kernel writes the rows: room for out_cap of them (0: nothing is written; rgb, edge may be NULL)
+struct CloudRows { float* pos; float* nrm; float* rgb; int* pix; float* cls; float* edge; long long out_cap; };
+
+#define SC(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { ctx->err = std::string(#call) + ": " + cudaGetErrorString(_e); return STOCS_E_CUDA; } } while (0)
+
+// The argument checks both front ends share; zeroes offsets once they pass.
+int cloud_check(stocs_b200_ctx* ctx, const char* who, const void* depth, const void* maps, const float* class_thresholds,
+                int n_objects, int W, int H, float voxel_size, int64_t cap, int64_t* offsets) {
   // every (object, pixel) entry of the scan and every output row is an int
   const long long rows_needed = (long long)n_objects * ((long long)W * H + 1);
-  if (!depth || !class_probs || !class_thresholds || !offsets || n_objects < 1 || n_objects > STOCS_B200_MAX_CLOUD_OBJECTS ||
+  if (!depth || !maps || !class_thresholds || !offsets || n_objects < 1 || n_objects > STOCS_B200_MAX_CLOUD_OBJECTS ||
       W <= 0 || H <= 0 || rows_needed > 0x7fffffffll - 1024 || !(voxel_size > 0) || cap < 0)
     STOCS_FAIL(ctx, STOCS_E_ARG, std::string(who) + ": bad argument");
   for (int k = 0; k <= n_objects; ++k) offsets[k] = 0;
-  cudaSetDevice(ctx->device);
+  return STOCS_OK;
+}
+
+// The device side of both front ends, on the context stream: back-projection -> voxel keys -> sort -> centroids ->
+// outliers -> filter -> scan -> emit into `out`, then the copy of the voxel count and every object's end into
+// ctx->h_index_counts + 8.  No synchronisation.
+int cloud_enqueue(stocs_b200_ctx* ctx, const CloudFrame& f, const CloudRows& out) {
   cudaStream_t st = ctx->stream;
-  const int n = W * H;
+  const int n = f.W * f.H;
   const int nb = (n + 255) / 256;
-  DevBuf& d_depth = ctx->pool[POOL_CLOUD_DEPTH];
-  DevBuf& d_bgr = ctx->pool[POOL_CLOUD_BGR];
-  DevBuf& d_prob = ctx->pool[POOL_CLOUD_PROB];
-  DevBuf& d_edge = ctx->pool[POOL_CLOUD_EDGE];
+  const int n_objects = f.n_objects;
   DevBuf& d_xyz = ctx->pool[POOL_CLOUD_XYZ];
   DevBuf& d_keys_a = ctx->pool[POOL_CLOUD_KEYS_A];
   DevBuf& d_keys_b = ctx->pool[POOL_CLOUD_KEYS_B];
@@ -247,22 +268,16 @@ int build_scene_clouds(stocs_b200_ctx* ctx, const char* who, const uint16_t* dep
   DevBuf& d_keep = ctx->pool[POOL_CLOUD_KEEP];
   DevBuf& d_nrm = ctx->pool[POOL_CLOUD_NRM];
   DevBuf& d_rc = ctx->pool[POOL_CLOUD_RC];
-  DevBuf& d_out = ctx->pool[POOL_CLOUD_OUT];
-#define SC(call) do { cudaError_t _e = (call); if (_e != cudaSuccess) { ctx->err = std::string(#call) + ": " + cudaGetErrorString(_e); return STOCS_E_CUDA; } } while (0)
-  SC(d_depth.ensure((size_t)n * 2)); SC(d_prob.ensure((size_t)n_objects * n * 2)); SC(d_xyz.ensure((size_t)n * 12));
-  SC(cudaMemcpyAsync(d_depth.p, depth, (size_t)n * 2, cudaMemcpyHostToDevice, st));
-  SC(cudaMemcpyAsync(d_prob.p, class_probs, (size_t)n_objects * n * 2, cudaMemcpyHostToDevice, st));
-  if (bgr) { SC(d_bgr.ensure((size_t)n * 3)); SC(cudaMemcpyAsync(d_bgr.p, bgr, (size_t)n * 3, cudaMemcpyHostToDevice, st)); }
-  if (edge) { SC(d_edge.ensure((size_t)n)); SC(cudaMemcpyAsync(d_edge.p, edge, (size_t)n, cudaMemcpyHostToDevice, st)); }
-  int rc = stocs_launch_backproject(ctx, d_depth.as<uint16_t>(), nullptr, W, H, fx, cx, fy, cy, depth_scale, d_xyz.as<float>(), nullptr, st);
+  SC(d_xyz.ensure((size_t)n * 12));
+  int rc = stocs_launch_backproject(ctx, f.depth, nullptr, f.W, f.H, f.fx, f.cx, f.fy, f.cy, f.depth_scale, d_xyz.as<float>(), nullptr, st);
   if (rc) return rc;
   // device counters: first_zero, n_zero, n_valid, n_vox, then the end of each object's rows (emit_kernel)
   int* d_cnt = ctx->scratch()->cloud;
   int init[3] = {0x7fffffff, 0, 0};
   SC(cudaMemcpyAsync(d_cnt, init, 12, cudaMemcpyHostToDevice, st));
-  first_zero_kernel<<<nb, 256, 0, st>>>(d_depth.as<uint16_t>(), n, d_cnt, d_cnt + 1);
+  first_zero_kernel<<<nb, 256, 0, st>>>(f.depth, n, d_cnt, d_cnt + 1);
   SC(d_keys_a.ensure((size_t)n * 8)); SC(d_keys_b.ensure((size_t)n * 8)); SC(d_idx_a.ensure((size_t)n * 4)); SC(d_idx_b.ensure((size_t)n * 4));
-  voxel_keys_kernel<<<nb, 256, 0, st>>>(d_xyz.as<float>(), d_depth.as<uint16_t>(), n, 1.0f / voxel_size, d_cnt,
+  voxel_keys_kernel<<<nb, 256, 0, st>>>(d_xyz.as<float>(), f.depth, n, 1.0f / f.voxel_size, d_cnt,
                                         d_keys_a.as<unsigned long long>(), d_idx_a.as<int>(), d_cnt + 2);
   size_t tb = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, tb, d_keys_a.as<unsigned long long>(), d_keys_b.as<unsigned long long>(), d_idx_a.as<int>(),
@@ -288,30 +303,75 @@ int build_scene_clouds(stocs_b200_ctx* ctx, const char* who, const uint16_t* dep
   voxel_starts_kernel<<<nb, 256, 0, st>>>(keys, d_flags.as<int>(), d_scan.as<int>(), d_nvalid, d_starts.as<int>(),
                                           d_ukeys.as<unsigned long long>(), d_nvox);
   const int nxb = (n + 127) / 128;
-  centroid_kernel<<<nxb, 128, 0, st>>>(d_xyz.as<float>(), d_depth.as<uint16_t>(), idx, d_starts.as<int>(), d_nvox, d_nvalid, d_cnt,
+  centroid_kernel<<<nxb, 128, 0, st>>>(d_xyz.as<float>(), f.depth, idx, d_starts.as<int>(), d_nvox, d_nvalid, d_cnt,
                                        d_cnt + 1, d_cent.as<float4>());
   // src/rgbd.cpp:234: setRadiusSearch(double(2*voxel_size) + 0.005); the search compares squared
   // distances with float(radius * radius) (pcl::KdTreeFLANN::radiusSearch)
-  const double radius = (double)(2 * voxel_size) + 0.005;
+  const double radius = (double)(2 * f.voxel_size) + 0.005;
   const float r2 = (float)(radius * radius);
-  const int reach = (int)std::ceil(radius / (double)voxel_size) + 1;
+  const int reach = (int)std::ceil(radius / (double)f.voxel_size) + 1;
   outlier_kernel<<<nxb, 128, 0, st>>>(d_cent.as<float4>(), d_ukeys.as<unsigned long long>(), d_nvox, r2, reach, 10, d_keep.as<int>());
   // one flag per (object, centroid), scanned in place into output rows (see FilterArgs)
-  const long long out_cap = cap < (long long)n_objects * n ? cap : (long long)n_objects * n;
   FilterArgs fa;
   fa.cent = d_cent.as<float4>(); fa.keep = d_keep.as<int>(); fa.nvox_p = d_nvox; fa.n = n; fa.n_obj = n_objects;
-  fa.out_cap = (int)out_cap;
-  fa.depth = d_depth.as<uint16_t>();
-  fa.bgr = bgr ? d_bgr.as<uint8_t>() : nullptr; fa.prob = d_prob.as<uint16_t>(); fa.edge = edge ? d_edge.as<uint8_t>() : nullptr;
-  fa.W = W; fa.H = H; fa.fx = fx; fa.cx = cx; fa.fy = fy; fa.cy = cy;
-  for (int k = 0; k < STOCS_B200_MAX_CLOUD_OBJECTS; ++k) fa.class_threshold[k] = k < n_objects ? class_thresholds[k] : 0.f;
+  fa.out_cap = (int)out.out_cap;
+  fa.depth = f.depth; fa.bgr = f.bgr; fa.edge = f.edge;
+  fa.W = f.W; fa.H = f.H; fa.fx = f.fx; fa.cx = f.cx; fa.fy = f.fy; fa.cy = f.cy;
+  for (int k = 0; k < STOCS_B200_MAX_CLOUD_OBJECTS; ++k) {
+    fa.map[k] = k < n_objects ? f.maps[k] : nullptr;
+    fa.class_threshold[k] = k < n_objects ? f.thresholds[k] : 0.f;
+  }
   fa.rows = d_flags.as<int>(); fa.nrm = d_nrm.as<float>(); fa.rc = d_rc.as<int>();
-  filter_kernel<<<(n + 1 + 127) / 128, 128, 0, st>>>(fa);
+  const bool f32 = f.map_type == STOCS_B200_MAP_F32;
+  if (f32) filter_kernel<STOCS_B200_MAP_F32><<<(n + 1 + 127) / 128, 128, 0, st>>>(fa);
+  else filter_kernel<STOCS_B200_MAP_U16><<<(n + 1 + 127) / 128, 128, 0, st>>>(fa);
   size_t tb3 = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, tb3, fa.rows, n_rows, st);
   SC(d_tmp.ensure(tb3));
   cub::DeviceScan::ExclusiveSum(d_tmp.p, tb3, fa.rows, n_rows, st);
+  int* d_ends = d_cnt + 4;
+  if (f32) emit_kernel<STOCS_B200_MAP_F32><<<nxb, 128, 0, st>>>(fa, d_ends, out.pos, out.nrm, out.rgb, out.pix, out.cls, out.edge);
+  else emit_kernel<STOCS_B200_MAP_U16><<<nxb, 128, 0, st>>>(fa, d_ends, out.pos, out.nrm, out.rgb, out.pix, out.cls, out.edge);
+  SC(cudaGetLastError());
+  // page-locked: {voxels, end of object 0, .., end of object K-1}
+  SC(cudaMemcpyAsync(ctx->h_index_counts + 8, d_nvox, (size_t)(1 + n_objects) * 4, cudaMemcpyDeviceToHost, st));
+  return STOCS_OK;
+}
+
+// After the synchronisation: offsets and the context's read-back estimate from the lengths cloud_enqueue copied;
+// returns the number of rows.
+long long cloud_commit(stocs_b200_ctx* ctx, int n_objects, int64_t* offsets) {
+  const uint32_t* h_len = ctx->h_index_counts + 8;
+  for (int k = 0; k < n_objects; ++k) offsets[k + 1] = (int64_t)h_len[1 + k];
+  ctx->counters[CTR_CLOUD_VOXELS] = (long long)h_len[0];
+  ctx->cloud_last_points = offsets[n_objects];
+  return offsets[n_objects];
+}
+
+// Host front end: stages the images and n_objects uint16 maps into the pool, runs the shared stages into the pool's
+// output rows and fetches them.  stocs_b200_build_scene_cloud is its one-object case; `who` prefixes the error messages.
+int build_scene_clouds(stocs_b200_ctx* ctx, const char* who, const uint16_t* depth, const uint8_t* bgr,
+                       const uint16_t* class_probs, const float* class_thresholds, int n_objects, const uint8_t* edge,
+                       int W, int H, float fx, float cx, float fy, float cy, float depth_scale, float voxel_size,
+                       float* pos3, float* nrm3, float* rgb3, int32_t* pixel_rc, float* class_p, float* edge_p,
+                       int64_t cap, int64_t* offsets) {
+  int rc = cloud_check(ctx, who, depth, class_probs, class_thresholds, n_objects, W, H, voxel_size, cap, offsets);
+  if (rc) return rc;
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = ctx->stream;
+  const int n = W * H;
+  DevBuf& d_depth = ctx->pool[POOL_CLOUD_DEPTH];
+  DevBuf& d_bgr = ctx->pool[POOL_CLOUD_BGR];
+  DevBuf& d_prob = ctx->pool[POOL_CLOUD_PROB];
+  DevBuf& d_edge = ctx->pool[POOL_CLOUD_EDGE];
+  DevBuf& d_out = ctx->pool[POOL_CLOUD_OUT];
+  SC(d_depth.ensure((size_t)n * 2)); SC(d_prob.ensure((size_t)n_objects * n * 2));
+  SC(cudaMemcpyAsync(d_depth.p, depth, (size_t)n * 2, cudaMemcpyHostToDevice, st));
+  SC(cudaMemcpyAsync(d_prob.p, class_probs, (size_t)n_objects * n * 2, cudaMemcpyHostToDevice, st));
+  if (bgr) { SC(d_bgr.ensure((size_t)n * 3)); SC(cudaMemcpyAsync(d_bgr.p, bgr, (size_t)n * 3, cudaMemcpyHostToDevice, st)); }
+  if (edge) { SC(d_edge.ensure((size_t)n)); SC(cudaMemcpyAsync(d_edge.p, edge, (size_t)n, cudaMemcpyHostToDevice, st)); }
   // out: pos3 | nrm3 | rgb3 | pix2 | cls | edge, each with room for out_cap points
+  const long long out_cap = cap < (long long)n_objects * n ? cap : (long long)n_objects * n;
   const size_t oc = (size_t)(out_cap > 0 ? out_cap : 1);
   SC(d_out.ensure(oc * (12 + 12 + 12 + 8 + 4 + 4)));
   float* o_pos = d_out.as<float>();
@@ -320,14 +380,14 @@ int build_scene_clouds(stocs_b200_ctx* ctx, const char* who, const uint16_t* dep
   int* o_pix = (int*)(o_rgb + 3 * oc);
   float* o_cls = (float*)(o_pix + 2 * oc);
   float* o_edge = o_cls + oc;
-  int* d_ends = d_cnt + 4;
-  emit_kernel<<<nxb, 128, 0, st>>>(fa, d_ends, o_pos, o_nrm, o_rgb, o_pix, o_cls, o_edge);
-  SC(cudaGetLastError());
-  // read-back: the voxel count and every object's end, and -- in the same queue, before anything is
-  // known -- as many points as the previous call's estimate below; a frame that emits more fetches the
-  // rest afterwards
-  uint32_t* h_len = ctx->h_index_counts + 8;   // page-locked: {voxels, end of object 0, .., end of object K-1}
-  SC(cudaMemcpyAsync(h_len, d_nvox, (size_t)(1 + n_objects) * 4, cudaMemcpyDeviceToHost, st));
+  const void* maps[STOCS_B200_MAX_CLOUD_OBJECTS];
+  for (int k = 0; k < n_objects; ++k) maps[k] = d_prob.as<uint16_t>() + (size_t)k * n;
+  const CloudFrame f{d_depth.as<uint16_t>(), bgr ? d_bgr.as<uint8_t>() : nullptr, edge ? d_edge.as<uint8_t>() : nullptr,
+                     maps, STOCS_B200_MAP_U16, class_thresholds, n_objects, W, H, fx, cx, fy, cy, depth_scale, voxel_size};
+  rc = cloud_enqueue(ctx, f, CloudRows{o_pos, o_nrm, o_rgb, o_pix, o_cls, o_edge, out_cap});
+  if (rc) return rc;
+  // in the same queue as the lengths, before anything is known: as many points as the previous call's estimate
+  // below; a frame that emits more fetches the rest afterwards
   const bool have_out = pos3 && nrm3 && pixel_rc && class_p;
   // the previous voxel count bounds what one object of a frame like the previous one emits; with several
   // objects, the previous call's points plus that much again
@@ -346,18 +406,13 @@ int build_scene_clouds(stocs_b200_ctx* ctx, const char* who, const uint16_t* dep
   };
   if (guess > 0) SC(fetch(0, guess));
   SC(cudaStreamSynchronize(st));
-  const long long nvox = (long long)h_len[0];
-  for (int k = 0; k < n_objects; ++k) offsets[k + 1] = (int64_t)h_len[1 + k];
-  const long long n_emit = offsets[n_objects];
-  ctx->counters[CTR_CLOUD_VOXELS] = nvox;
-  ctx->cloud_last_points = n_emit;
+  const long long n_emit = cloud_commit(ctx, n_objects, offsets);
   if (n_emit > cap) STOCS_FAIL(ctx, STOCS_E_CAPACITY, std::string(who) + ": output capacity too small");
   if (n_emit > 0 && !have_out) STOCS_FAIL(ctx, STOCS_E_ARG, std::string(who) + ": output pointer is NULL");
   if (n_emit > guess) {
     SC(fetch(guess, n_emit));
     SC(cudaStreamSynchronize(st));
   }
-#undef SC
   return STOCS_OK;
 }
 
@@ -372,6 +427,50 @@ extern "C" int stocs_b200_build_scene_clouds(stocs_b200_ctx* ctx, const uint16_t
   return build_scene_clouds(ctx, "build_scene_clouds", depth, bgr, class_probs, class_thresholds, n_objects, edge, W, H, fx,
                             cx, fy, cy, depth_scale, voxel_size, pos3, nrm3, rgb3, pixel_rc, class_p, edge_p, cap, offsets);
 }
+
+// Device front end: the shared stages read the caller's images and maps and emit straight into the caller's rows;
+// only the lengths come back to the host.
+extern "C" int stocs_b200_build_scene_clouds_device(
+    stocs_b200_ctx* ctx, const uint16_t* d_depth, const uint8_t* d_bgr, const void* const* d_class_maps, int map_type,
+    const float* class_thresholds, int n_objects, const uint8_t* d_edge, int W, int H, float fx, float cx, float fy,
+    float cy, float depth_scale, float voxel_size, float* d_pos3, float* d_nrm3, float* d_rgb3, int32_t* d_pixel_rc,
+    float* d_class_p, float* d_edge_p, int64_t cap, int64_t* offsets, void* stream) {
+  if (!ctx) return STOCS_E_ARG;
+  const std::string who = "build_scene_clouds_device";
+  int rc = cloud_check(ctx, who.c_str(), d_depth, d_class_maps, class_thresholds, n_objects, W, H, voxel_size, cap, offsets);
+  if (rc) return rc;
+  if (map_type != STOCS_B200_MAP_U16 && map_type != STOCS_B200_MAP_F32) STOCS_FAIL(ctx, STOCS_E_ARG, who + ": unknown map_type");
+  const std::pair<const void*, const char*> ptrs[] = {{d_depth, "d_depth"}, {d_bgr, "d_bgr"}, {d_edge, "d_edge"},
+                                                      {d_pos3, "d_pos3"}, {d_nrm3, "d_nrm3"}, {d_rgb3, "d_rgb3"},
+                                                      {d_pixel_rc, "d_pixel_rc"}, {d_class_p, "d_class_p"}, {d_edge_p, "d_edge_p"}};
+  const std::string where = " is not device memory on device " + std::to_string(ctx->device);
+  for (const auto& p : ptrs)
+    if (p.first && !stocs_device_memory(p.first, ctx->device)) STOCS_FAIL(ctx, STOCS_E_ARG, who + ": " + p.second + where);
+  for (int k = 0; k < n_objects; ++k) {
+    const std::string name = who + ": d_class_maps[" + std::to_string(k) + "]";
+    if (!d_class_maps[k]) STOCS_FAIL(ctx, STOCS_E_ARG, name + " is NULL");
+    if (!stocs_device_memory(d_class_maps[k], ctx->device)) STOCS_FAIL(ctx, STOCS_E_ARG, name + where);
+  }
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = ctx->stream;
+  const long long n = (long long)W * H;
+  const bool have_out = d_pos3 && d_nrm3 && d_pixel_rc && d_class_p;
+  const long long out_cap = !have_out ? 0 : cap < n_objects * n ? cap : n_objects * n;
+  CallerEvent producer;
+  SC(producer.record(stream, ctx->device));
+  SC(producer.wait(st));
+  const CloudFrame f{d_depth, d_bgr, d_edge, d_class_maps, map_type, class_thresholds, n_objects, W, H, fx, cx, fy, cy,
+                     depth_scale, voxel_size};
+  rc = cloud_enqueue(ctx, f, CloudRows{d_pos3, d_nrm3, d_rgb3, d_pixel_rc, d_class_p, d_edge_p, out_cap});
+  const cudaError_t e = cudaStreamSynchronize(st);   // nothing stays queued, also after an error
+  if (rc) return rc;
+  SC(e);
+  const long long n_emit = cloud_commit(ctx, n_objects, offsets);
+  if (n_emit > cap) STOCS_FAIL(ctx, STOCS_E_CAPACITY, who + ": output capacity too small");
+  if (n_emit > 0 && !have_out) STOCS_FAIL(ctx, STOCS_E_ARG, who + ": output pointer is NULL");
+  return STOCS_OK;
+}
+#undef SC
 
 extern "C" int stocs_b200_build_scene_cloud(stocs_b200_ctx* ctx, const uint16_t* depth, const uint8_t* bgr,
                                             const uint16_t* class_prob, const uint8_t* edge, int W, int H, float fx,

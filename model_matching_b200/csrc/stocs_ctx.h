@@ -107,7 +107,9 @@ enum PoolSlot : int {
   POOL_SCORE_PRUNE = 54,
   // cluster.cu: sort keys, cub scratch, kept poses (and the uploaded poses of stocs_b200_cluster_poses)
   POOL_CLUSTER = 55,
-  POOL_COUNT = 56
+  // capi.cu (upload_scenes_device): a slice held on another device, copied to this one (pos3 | nrm3 | cls | pix)
+  POOL_SCENE_PEER = 56,
+  POOL_COUNT = 57
 };
 
 // Device scalars of one congruent-set search (congruent.cu) and of the pipeline run around it (fit.cu).
@@ -237,6 +239,8 @@ struct stocs_b200_ctx {
   size_t index_counts_clean = 0;            // leading words of pool[POOL_INDEX_COUNTS] known to be zero
   void* h_kd_stage = nullptr;               // page-locked staging of the kd-tree upload (frame-sized scenes)
   size_t h_kd_stage_bytes = 0;
+  void* h_scene_stage = nullptr;            // page-locked: positions | class weights | pixels of an upload_scenes_device slice
+  size_t h_scene_stage_bytes = 0;
   struct KdPending* kd_pending = nullptr;   // kd-tree of the current scene, still being built on a host thread
   cudaEvent_t kd_copy_done = nullptr;       // the staging buffer may be overwritten once this has completed
 
@@ -342,6 +346,29 @@ int stocs_kd_finish(stocs_b200_ctx* ctx, cudaStream_t st, bool upload = true);  
 bool stocs_fmad_selftest(stocs_b200_ctx* ctx);                             // score.cu
 // device alias of page-locked host memory, NULL for any other pointer (capi.cu)
 const void* stocs_host_alias(const void* p);
+// p is device memory (cudaMalloc'd or managed) on `device`, or on any device when device < 0; its device goes to
+// *owner (capi.cu)
+bool stocs_device_memory(const void* p, int device, int* owner = nullptr);
+// The calls that read a caller's device buffers order their work after what the caller has queued on its stream
+// so far: an event recorded there (a stream of `device`; NULL is that device's default stream, as everywhere in
+// CUDA, and torch's default stream), which context streams wait for.
+struct CallerEvent {
+  cudaEvent_t ev = nullptr;
+  cudaError_t record(void* stream, int device) {
+    int cur = 0;
+    cudaError_t e = cudaGetDevice(&cur);
+    if (e == cudaSuccess) e = cudaSetDevice(device);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
+    if (e == cudaSuccess) e = cudaEventRecord(ev, stream ? (cudaStream_t)stream : cudaStreamLegacy);
+    cudaSetDevice(cur);
+    return e;
+  }
+  cudaError_t wait(cudaStream_t st) const { return cudaStreamWaitEvent(st, ev, 0); }
+  CallerEvent() = default;
+  CallerEvent(const CallerEvent&) = delete;
+  CallerEvent& operator=(const CallerEvent&) = delete;
+  ~CallerEvent() { if (ev) cudaEventDestroy(ev); }   // released once recorded work completes
+};
 // device alias through which a host-buffer scoring call reads its transforms in place, NULL when
 // they are staged instead: pageable memory, or STOCS_NO_ZERO_COPY set (capi.cu)
 const float* stocs_zero_copy_transforms(const float* T16);
