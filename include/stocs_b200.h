@@ -448,6 +448,12 @@ int stocs_b200_get_counters(stocs_b200_ctx* ctx, int64_t* counters, int n);
  * bench.py derives SURVEY.md section 8(d)'s data-dependent byte figure from these. */
 int stocs_b200_score_counters(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int64_t* counters,
                               int n);
+/* Test hook: the coarse-survivor count of each of H device-resident transforms, as the device top-K
+ * path computes it to order its claims: model points whose block of the coarse occupancy map is
+ * occupied (counters[1] of score_counters on that one transform, for a finite transform and |M| a
+ * multiple of 32), or |M| for a transform whose grid map is not finite or too large to evaluate
+ * without overflow.  counts: H host int32. */
+int stocs_b200_debug_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts);
 /* name + average duration (ms, CUDA events on the context stream) of the dominant kernel of the
  * most recent score call; used by bench.py for the roofline line. */
 int stocs_b200_last_kernel_ms(stocs_b200_ctx* ctx, float* ms);

@@ -335,6 +335,9 @@ int stocs_b200_upload_model(stocs_b200_ctx* ctx, const float* pos3, const float*
   STOCS_CUDA(ctx, cudaStreamSynchronize(st));
   ctx->M = M;
   ctx->Mpad = Mpad;
+  float amax = 0.f;   // (std::max keeps a NaN that is already there)
+  for (float c : ctx->h_mpos) amax = std::isfinite(c) ? std::max(amax, std::fabs(c)) : NAN;
+  ctx->model_abs_max = amax;
   return stocs_build_ppf_table(ctx);
 }
 
@@ -709,6 +712,21 @@ int stocs_b200_score_counters(stocs_b200_ctx* ctx, const float* d_T16, int64_t H
   int64_t out[9] = {H * (int64_t)ctx->M, (int64_t)h[0], (int64_t)h[1], (int64_t)h[2], (int64_t)h[3],
                     (int64_t)h[4], (int64_t)h[5], (int64_t)h[6], H};
   for (int i = 0; i < n && i < 9; ++i) counters[i] = out[i];
+  return STOCS_OK;
+}
+
+int stocs_b200_debug_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts) {
+  if (!ctx) return STOCS_E_ARG;
+  if (ctx->S <= 0 || ctx->M <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "survivor_counts: upload_model and upload_scene first");
+  if (H <= 0 || H >= (1ll << 31) || !d_T16 || !counts) STOCS_FAIL(ctx, STOCS_E_ARG, "survivor_counts: bad argument");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = ctx->stream;
+  DevBuf& d_ns = ctx->pool[POOL_SCORE_NS];
+  STOCS_CUDA(ctx, d_ns.ensure((size_t)H * 4));
+  int rc = stocs_survivor_counts(ctx, d_T16, H, d_ns.as<unsigned>(), st);
+  if (rc) return rc;
+  STOCS_CUDA(ctx, cudaMemcpyAsync(counts, d_ns.p, (size_t)H * 4, cudaMemcpyDeviceToHost, st));
+  STOCS_CUDA(ctx, cudaStreamSynchronize(st));
   return STOCS_OK;
 }
 

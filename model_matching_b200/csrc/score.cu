@@ -28,7 +28,11 @@
 // All memory-dependent steps are batched 32 wide, so the latency chain
 // brick -> offsets -> candidates -> attributes is paid once per drain, not once per model point.
 // The top-K instantiation (kPrune) also skips every hypothesis whose LCP provably stays below a
-// value K other hypotheses of the launch reach: see prune_reject / prune_publish.
+// value K other hypotheses of the launch reach: see prune_reject / prune_publish.  A large top-K launch
+// first counts every hypothesis's coarse survivors and claims in descending count, so that it can stop
+// at the first claim the bound rejects: see survivor_count_kernel.
+#include <algorithm>
+#include <cmath>
 #include <cstring>
 
 #include "stocs_ctx.h"
@@ -63,6 +67,9 @@ struct ScoreArgs {
   unsigned long long* tie_counter;
   unsigned long long* cnt;   // counting variant only (stocs_b200_score_counters): see ScoreCounter
   const int* __restrict__ order;   // claim number -> hypothesis (heavy-first schedule, see probe_order_kernel) or NULL
+  // kPrune: claim number -> {hypothesis, coarse survivors}, survivors non-increasing (survivor_count_kernel,
+  // rank_scatter_kernel), or NULL
+  const uint2* __restrict__ ranked;
   // top-K pruning (kPrune only, see prune_publish): theta bucket + histogram of this launch, the
   // context's two rejection counters, and the scene's bound constants
   unsigned* prune;                 // [0] theta bucket, [kBucketBase..] per-bucket counts; zeroed with the work counter
@@ -324,12 +331,18 @@ __device__ __forceinline__ void drain_queue(const ScoreArgs& a, WarpQueue& q, in
 }
 
 // next unit of work (lane 0 only): a claim number from the global counter, mapped through the
-// heavy-first order when there is one; any value >= H ends the warp
-__device__ __forceinline__ int claim_hypothesis(const ScoreArgs& a) {
+// heavy-first order or the descending-survivor order when there is one (the latter also gives the
+// hypothesis's coarse survivors in *ns); any value >= H ends the warp
+__device__ __forceinline__ int claim_hypothesis(const ScoreArgs& a, int* ns) {
   const unsigned long long c = atomicAdd(a.work_counter, 1ull);
   // (the online pipeline keeps its transform count on the device: H is then only an upper bound)
   const unsigned long long lim = a.H_dev ? (unsigned long long)__ldg(a.H_dev) : (unsigned long long)a.H;
   if (c >= lim) return 0x7fffffff;
+  if (a.ranked) {
+    const uint2 e = __ldg(a.ranked + c);
+    *ns = (int)e.y;
+    return (int)e.x;
+  }
   return a.order ? __ldg(a.order + c) : (int)c;
 }
 
@@ -442,9 +455,25 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) score_lcp_kernel(Scor
   // than it saves: 2.63 / 2.76 ms against 2.58 ms.)
   // (claimed index broadcast by redux for the same reason: h stays in a uniform register)
   int h = 0;
-  if (lane == 0) h = claim_hypothesis(a);
+  // (kPrune with a survivor order: lane 0 leaves the claim's coarse survivors in q.later, which is free
+  // until loop 1b; a register carried across the loop would cost the 32-register budget spills)
+  if (lane == 0) h = claim_hypothesis(a, &q.later);
   h = (int)__reduce_max_sync(0xffffffffu, (unsigned)h);
   while (h < a.H) {
+    if (kPrune && a.ranked) {
+      // Claims come in non-increasing survivor count and theta only grows, so once the count rejects a
+      // claim it rejects every later one: this warp stops, and the work counter jumps to H so that the
+      // other warps stop after the claim they hold.  Whoever makes the jump counts the claims that will
+      // never be handed out; every claim handed out is counted by the warp that holds it.
+      const int nsc = (int)__reduce_max_sync(0xffffffffu, lane == 0 ? (unsigned)q.later : 0u);
+      if (prune_reject(a, 0.f, nsc, theta_M(a, theta_bucket(a, lane)))) {
+        if (lane == 0) {
+          const unsigned long long handed = atomicMax(a.work_counter, (unsigned long long)a.H);
+          q.rej[0] += 1u + (handed < (unsigned long long)a.H ? (unsigned)((unsigned long long)a.H - handed) : 0u);
+        }
+        break;
+      }
+    }
     // lanes 0..11 fetch the 3x4 transform (column-major 4x4: element (r,c) at c*4+r) and publish
     // it, with its grid-coordinate version G = inv_cell * (T - origin), to the warp's shared slot
     if (lane < 12) {
@@ -702,8 +731,9 @@ __global__ void __launch_bounds__(kWarps * 32, kMinBlocks) score_lcp_kernel(Scor
         if (a.inl) a.inl[h] = 0;
       }
     }
+    __syncwarp();   // (the claim overwrites q.later, which this hypothesis's lanes read)
     h = 0;
-    if (lane == 0) h = claim_hypothesis(a);
+    if (lane == 0) h = claim_hypothesis(a, &q.later);
     h = (int)__reduce_max_sync(0xffffffffu, (unsigned)h);
     __syncwarp();
   }
@@ -777,6 +807,185 @@ __global__ void __launch_bounds__(256) probe_order_kernel(ScoreArgs a, int* __re
   }
 }
 
+// ---- Survivor order of a top-K launch (kPrune, above the heavy-first range) -------------------------
+// survivor_count_kernel computes, for every hypothesis, the count loop 1 would compute: model points
+// (index < M) whose coarse block has its bit set, with the same grid-block map G and the same
+// __fmaf_rn chain.  rank_scatter_kernel turns the counts into a claim order with the count
+// non-increasing; the scorer claims in that order and stops at the first claim the bound rejects
+// (see the top of score_lcp_kernel's loop).  The K best records do not depend on the claim order.
+//
+// Layout for throughput (this kernel is not held to the scorer's 32 registers): a warp takes 32
+// hypotheses and holds 256 model points in registers at a time, 8 per lane as float2 pairs, lane l
+// taking points l, l+32, ..., so that for one hypothesis the warp tests 32 consecutive points per
+// step as loop 1 does.  The hypothesis's G rows come from shared memory by broadcast once per 256
+// points; the only other shared access is the bitmap word.  Two points per instruction: __ffma2_rn
+// (FFMA2) rounds each half exactly as __fmaf_rn.  Floor and clamp: v + 2^23 rounded down (FADD2.RM)
+// holds floor(v) in its low mantissa bits for 0 <= v < 2^23, and bits - 0x4B000000 clamped to n (one
+// VIADDMNMX) is then floor(v); every other finite or infinite v -- negative, >= 2^23 -- lands on n, the
+// always-empty border block, as F2I.FLOOR + the unsigned clamp does.  Only NaN differs (F2I gives 0).
+// So a hypothesis whose G rows are below g_lim = 2^120 / max(1, max |model coordinate|) in magnitude --
+// no product or sum of the chain can then overflow, so no NaN can arise -- gets exactly loop 1's count;
+// any other one (non-finite or huge transform entries) gets M, which never rejects.
+constexpr int kPfWarps = 8;          // warps per CTA
+constexpr int kPfPairs = 4;          // float2 pairs per coordinate per lane: 256 model points per warp pass
+constexpr int kPruneHist = 1024;     // byte offset of the survivor histogram in POOL_SCORE_PRUNE
+
+__global__ void __launch_bounds__(kPfWarps * 32) survivor_count_kernel(ScoreArgs a, unsigned* __restrict__ ns,
+                                                                      unsigned* __restrict__ hist, float g_lim) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  uint32_t* s_coarse = reinterpret_cast<uint32_t*>(smem_raw);
+  float4* s_G = reinterpret_cast<float4*>(s_coarse + ((a.coarse_words + 3) & ~3));   // [warp][hypothesis][row]
+  unsigned* s_hist = reinterpret_cast<unsigned*>(s_G + kPfWarps * 32 * 3);            // M + 1 bins
+  const int M = a.M;
+  for (int i = threadIdx.x; i < a.coarse_words; i += blockDim.x) s_coarse[i] = a.coarse[i];
+  for (int i = threadIdx.x; i <= M; i += blockDim.x) s_hist[i] = 0u;
+  __syncthreads();
+  const int warp = threadIdx.x >> 5;
+  const unsigned lane = lane_id();
+  float4* G = s_G + warp * 32 * 3;
+  const float4* mp = reinterpret_cast<const float4*>(a.model);
+  const unsigned nx = (unsigned)a.coarse_nx, ny = (unsigned)a.coarse_ny, nz = (unsigned)a.coarse_nz;
+  const unsigned sx = (unsigned)a.coarse_sx, sy = (unsigned)a.coarse_sy;
+  const float2 k23 = make_float2(8388608.f, 8388608.f);
+  for (long long base = ((long long)blockIdx.x * kPfWarps + warp) * 32; base < a.H;
+       base += (long long)gridDim.x * kPfWarps * 32) {
+    const long long h = base + lane;
+    bool safe = false;
+    if (h < a.H) {
+      float g[12];
+      const float* t = a.T + 16 * (size_t)h;
+      safe = true;
+#pragma unroll
+      for (int c = 0; c < 4; ++c)
+#pragma unroll
+        for (int rr = 0; rr < 3; ++rr) {
+          const float v = __ldg(t + c * 4 + rr);
+          const float o = (rr == 0) ? a.g.ox : (rr == 1 ? a.g.oy : a.g.oz);
+          g[rr * 4 + c] = ((c == 3) ? (v - o) * a.g.inv_cell : v * a.g.inv_cell) * a.to_block;
+          safe = safe && fabsf(g[rr * 4 + c]) < g_lim;
+        }
+#pragma unroll
+      for (int rr = 0; rr < 3; ++rr) G[lane * 3 + rr] = make_float4(g[rr * 4], g[rr * 4 + 1], g[rr * 4 + 2], g[rr * 4 + 3]);
+    }
+    const unsigned safe_m = __ballot_sync(0xffffffffu, safe);
+    __syncwarp();
+    unsigned cnt = 0;   // lane t: survivors of hypothesis base + t
+    for (int s0 = 0; s0 < M; s0 += 64 * kPfPairs) {
+      float2 x[kPfPairs], y[kPfPairs], z[kPfPairs];
+#pragma unroll
+      for (int k = 0; k < kPfPairs; ++k) {
+        const int p0 = s0 + 64 * k + (int)lane, p1 = p0 + 32;
+        const float4 m0 = p0 < M ? __ldg(mp + p0) : make_float4(NAN, NAN, NAN, 0.f);
+        const float4 m1 = p1 < M ? __ldg(mp + p1) : make_float4(NAN, NAN, NAN, 0.f);
+        x[k] = make_float2(m0.x, m1.x); y[k] = make_float2(m0.y, m1.y); z[k] = make_float2(m0.z, m1.z);
+      }
+      for (int t = 0; t < 32; ++t) {
+        if (!((safe_m >> t) & 1u)) continue;   // warp-uniform
+        const float4 r0 = G[t * 3], r1 = G[t * 3 + 1], r2 = G[t * 3 + 2];
+        unsigned n = 0;
+#pragma unroll
+        for (int k = 0; k < kPfPairs; ++k) {
+          float2 fx = __ffma2_rn(make_float2(r0.x, r0.x), x[k], __ffma2_rn(make_float2(r0.y, r0.y), y[k],
+                                 __ffma2_rn(make_float2(r0.z, r0.z), z[k], make_float2(r0.w, r0.w))));
+          float2 fy = __ffma2_rn(make_float2(r1.x, r1.x), x[k], __ffma2_rn(make_float2(r1.y, r1.y), y[k],
+                                 __ffma2_rn(make_float2(r1.z, r1.z), z[k], make_float2(r1.w, r1.w))));
+          float2 fz = __ffma2_rn(make_float2(r2.x, r2.x), x[k], __ffma2_rn(make_float2(r2.y, r2.y), y[k],
+                                 __ffma2_rn(make_float2(r2.z, r2.z), z[k], make_float2(r2.w, r2.w))));
+          fx = __fadd2_rd(fx, k23); fy = __fadd2_rd(fy, k23); fz = __fadd2_rd(fz, k23);
+          const unsigned c0 = (min(__float_as_uint(fz.x) - 0x4B000000u, nz) * sy + min(__float_as_uint(fy.x) - 0x4B000000u, ny)) * sx +
+                              min(__float_as_uint(fx.x) - 0x4B000000u, nx);
+          const unsigned c1 = (min(__float_as_uint(fz.y) - 0x4B000000u, nz) * sy + min(__float_as_uint(fy.y) - 0x4B000000u, ny)) * sx +
+                              min(__float_as_uint(fx.y) - 0x4B000000u, nx);
+          n += ((s_coarse[c0 >> 5] >> (c0 & 31u)) & 1u) + ((s_coarse[c1 >> 5] >> (c1 & 31u)) & 1u);
+        }
+        const unsigned r = __reduce_add_sync(0xffffffffu, n);
+        if (lane == (unsigned)t) cnt += r;
+      }
+    }
+    if (h < a.H) {
+      const unsigned v = safe ? cnt : (unsigned)M;
+      ns[h] = v;
+      a.lcp[h] = 0.f;   // what a hypothesis the scorer never claims keeps: topk_kernel ignores it
+      if (a.inl) a.inl[h] = 0;
+      atomicAdd(s_hist + v, 1u);
+    }
+    __syncwarp();
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i <= M; i += blockDim.x)
+    if (s_hist[i]) atomicAdd(hist + i, s_hist[i]);
+}
+
+// Counting sort of the counts, descending: every CTA scans the histogram itself (M + 1 bins), then
+// places chunks of kRsChunk hypotheses, reserving each bin's slots of a chunk with one global atomic.
+// Order inside a bin is not fixed (it needs no stability: the records do not depend on the order).
+constexpr int kRsThreads = 1024, kRsItems = 4, kRsChunk = kRsThreads * kRsItems;
+__global__ void __launch_bounds__(kRsThreads) rank_scatter_kernel(const unsigned* __restrict__ ns, long long H, int M,
+                                                                  const unsigned* __restrict__ hist, unsigned* __restrict__ fill,
+                                                                  uint2* __restrict__ ranked) {
+  extern __shared__ unsigned s_rs[];
+  unsigned* s_base = s_rs;             // bin v starts at the hypotheses with a count above v
+  unsigned* s_cnt = s_rs + (M + 1);    // per chunk: bin's hypotheses, then the chunk's first slot in it
+  __shared__ unsigned s_warp[kRsThreads / 32];
+  const int tid = threadIdx.x;
+  const unsigned lane = lane_id();
+  const int nb = M + 1, per = (nb + kRsThreads - 1) / kRsThreads;
+  // exclusive scan over the bins from the top: thread tid takes bins M - tid*per, ... downwards
+  unsigned sum = 0;
+  for (int j = 0; j < per; ++j) { const int v = M - (tid * per + j); if (v >= 0) sum += __ldg(hist + v); }
+  unsigned incl = sum;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const unsigned up = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= (unsigned)o) incl += up;
+  }
+  if (lane == 31) s_warp[tid >> 5] = incl;
+  __syncthreads();
+  if (tid < 32) {
+    unsigned w = s_warp[tid], wi = w;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const unsigned up = __shfl_up_sync(0xffffffffu, wi, o);
+      if (tid >= o) wi += up;
+    }
+    s_warp[tid] = wi - w;
+  }
+  __syncthreads();
+  unsigned run = s_warp[tid >> 5] + incl - sum;
+  for (int j = 0; j < per; ++j) {
+    const int v = M - (tid * per + j);
+    if (v >= 0) { s_base[v] = run; run += __ldg(hist + v); }
+  }
+  for (long long c0 = (long long)blockIdx.x * kRsChunk; c0 < H; c0 += (long long)gridDim.x * kRsChunk) {
+    for (int v = tid; v < nb; v += kRsThreads) s_cnt[v] = 0u;
+    __syncthreads();
+    unsigned val[kRsItems], rank[kRsItems];
+#pragma unroll
+    for (int j = 0; j < kRsItems; ++j) {
+      const long long h = c0 + j * kRsThreads + tid;
+      val[j] = h < H ? __ldg(ns + h) : 0xffffffffu;
+      // warp-aggregated: one shared atomic per distinct count of the warp
+      const unsigned peers = __match_any_sync(0xffffffffu, val[j]);
+      const unsigned leader = __ffs(peers) - 1;
+      unsigned first = 0;
+      if (lane == leader && val[j] != 0xffffffffu) first = atomicAdd(s_cnt + val[j], (unsigned)__popc(peers));
+      rank[j] = __shfl_sync(0xffffffffu, first, leader) + __popc(peers & lanemask_lt());
+    }
+    __syncthreads();
+    for (int v = tid; v < nb; v += kRsThreads) {
+      const unsigned n = s_cnt[v];
+      if (n) s_cnt[v] = s_base[v] + atomicAdd(fill + v, n);
+    }
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < kRsItems; ++j) {
+      const long long h = c0 + j * kRsThreads + tid;
+      if (h < H) ranked[s_cnt[val[j]] + rank[j]] = make_uint2((unsigned)h, val[j]);
+    }
+    __syncthreads();
+  }
+}
+
 __global__ void fmad_selftest_kernel(float a, float b, float c, float* out) { out[0] = a * b + c; }
 
 }  // namespace
@@ -792,20 +1001,12 @@ bool stocs_fmad_selftest(stocs_b200_ctx* ctx) {
   return hres == 0.0f;
 }
 
-int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl,
-                       cudaStream_t st, const ScoreRequest& rq) {
-  if (H <= 0) return STOCS_OK;
-  if (H >= (1ll << 31)) STOCS_FAIL(ctx, STOCS_E_ARG, "score: at most 2^31-1 hypotheses per call");
-  // the pruned instantiation exists for one launch shape: slot 0, count on the host, no counting
-  if (rq.top_K > 0 && (rq.counters || rq.d_H || rq.slot != 0))
-    STOCS_FAIL(ctx, STOCS_E_ARG, "score: a top-K launch takes no counters, device count or slot");
-  const int slot = rq.slot;
-  unsigned long long* const d_counters = rq.counters;
-  const long long* const d_H = rq.d_H;
-  // the kd-tree of a freshly uploaded scene may still be under construction on a host thread: collect
-  // it and queue its upload in front of this launch (no-op on every later launch)
-  if (ctx->kd_pending) { const int rc = stocs_kd_finish(ctx, st); if (rc) return rc; }
+namespace {
+
+// the scene, model and transform fields of a launch (work distribution and pruning are the caller's)
+ScoreArgs score_args(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl) {
   ScoreArgs a;
+  memset(&a, 0, sizeof(a));
   a.bricks = ctx->d_bricks.as<uint4>();
   a.coarse = ctx->d_coarse.as<uint32_t>();
   a.brick_occ = ctx->d_brick_occ.as<uint32_t>();
@@ -821,16 +1022,7 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   a.T = d_T;
   a.lcp = d_lcp;
   a.inl = d_inl;
-  // slot 0 is the default work counter; launches that may run concurrently (staged host-buffer chunks
-  // on two streams) take distinct slots.  One tie counter accumulates over all launches.
-  DevScratch* scr = ctx->scratch();
-  unsigned long long* wctr = &scr->work[slot];
-  a.work_counter = wctr;
-  a.tie_counter = &scr->score_totals.ties;
-  a.cnt = d_counters;
-  a.order = nullptr;
   a.H = H;
-  a.H_dev = d_H;
   a.g = ctx->grid;
   a.M = ctx->M;
   a.Mpad = ctx->Mpad;
@@ -838,6 +1030,49 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   a.dot_thr = ctx->dot_thr;
   a.to_block = 1.0f / (float)(1u << ctx->coarse_shift);
   a.to_cell = (float)(1u << ctx->coarse_shift);
+  return a;
+}
+
+// survivor_count_kernel over the launch of a: ns[h] for every hypothesis, lcp (and inliers) 0, and the
+// counts' histogram added into hist (M + 1 bins)
+int enqueue_survivor_counts(stocs_b200_ctx* ctx, const ScoreArgs& a, unsigned* ns, unsigned* hist, cudaStream_t st) {
+  // bound on the grid-map entries below which loop 1's chain cannot overflow (see survivor_count_kernel)
+  const float g_lim = std::isfinite(ctx->model_abs_max) ? 0x1p120f / std::max(1.0f, ctx->model_abs_max) : 0.f;
+  const size_t smem = (size_t)((a.coarse_words + 3) & ~3) * 4 + (size_t)kPfWarps * 32 * 3 * 16 + (size_t)(a.M + 1) * 4;
+  STOCS_CUDA(ctx, cudaFuncSetAttribute(survivor_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int per_sm = 0;
+  STOCS_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, survivor_count_kernel, kPfWarps * 32, smem));
+  if (per_sm < 1) STOCS_FAIL(ctx, STOCS_E_ARG, "score: coarse map too large for the survivor count");
+  const long long tiles = (a.H + kPfWarps * 32 - 1) / (kPfWarps * 32);
+  const long long grid = std::min(tiles, (long long)ctx->num_sms * per_sm);
+  survivor_count_kernel<<<(unsigned)grid, kPfWarps * 32, smem, st>>>(a, ns, hist, g_lim);
+  return STOCS_OK;
+}
+
+}  // namespace
+
+int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl,
+                       cudaStream_t st, const ScoreRequest& rq) {
+  if (H <= 0) return STOCS_OK;
+  if (H >= (1ll << 31)) STOCS_FAIL(ctx, STOCS_E_ARG, "score: at most 2^31-1 hypotheses per call");
+  // the pruned instantiation exists for one launch shape: slot 0, count on the host, no counting
+  if (rq.top_K > 0 && (rq.counters || rq.d_H || rq.slot != 0))
+    STOCS_FAIL(ctx, STOCS_E_ARG, "score: a top-K launch takes no counters, device count or slot");
+  const int slot = rq.slot;
+  unsigned long long* const d_counters = rq.counters;
+  const long long* const d_H = rq.d_H;
+  // the kd-tree of a freshly uploaded scene may still be under construction on a host thread: collect
+  // it and queue its upload in front of this launch (no-op on every later launch)
+  if (ctx->kd_pending) { const int rc = stocs_kd_finish(ctx, st); if (rc) return rc; }
+  ScoreArgs a = score_args(ctx, d_T, H, d_lcp, d_inl);
+  // slot 0 is the default work counter; launches that may run concurrently (staged host-buffer chunks
+  // on two streams) take distinct slots.  One tie counter accumulates over all launches.
+  DevScratch* scr = ctx->scratch();
+  unsigned long long* wctr = &scr->work[slot];
+  a.work_counter = wctr;
+  a.tie_counter = &scr->score_totals.ties;
+  a.cnt = d_counters;
+  a.H_dev = d_H;
   // top-K pruning: only for a caller that receives nothing but the K best records (top_K = K), and
   // only on a scene whose class weights are all finite and >= 0 (the bound needs w_max)
   // (and with the lowest bucket edge a normal float, see lcp_bucket)
@@ -845,19 +1080,36 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   memcpy(&wbits, &ctx->w_max, 4);
   const int key_lo = (int)(wbits >> 19) + 1 - (kBuckets - 1);
   const bool prune = rq.top_K > 0 && ctx->prune_ok && key_lo >= 16;
-  a.prune = nullptr;
   a.rejected = scr->score_totals.rejected;
   a.w_max = ctx->w_max;
   a.bound_scale = 1.0f + (float)(ctx->M + 2) * 0x1p-23f;   // exact: M + 2 < 2^13
   a.key_lo = (unsigned)key_lo;
   a.K = rq.top_K;
+  // Heavy-first schedule for MID-SIZE launches only.  Measured on B200 (S1 hypotheses, kernel + probe):
+  // 125 000 hypotheses (the per-GPU share of the named config on 8 GPUs) 0.347 -> 0.312 ms; 10^6
+  // hypotheses 2.100 -> 2.139 ms (the probe costs 64 us per 10^6, the tail it removes is ~0.09 ms
+  // whatever the size), and on the all-fitted S1-fit list the heavy-first order itself slows the
+  // kernel by 2 % (3.622 -> 3.692 ms).  Small launches (the online pipeline's ~1 000 hypotheses)
+  // cannot spare one more launch.  STOCS_NO_LPT=1 switches it off, STOCS_LPT_MAX overrides the bound.
+  const bool no_lpt = getenv("STOCS_NO_LPT") != nullptr;
+  const long long lpt_max = getenv("STOCS_LPT_MAX") ? atoll(getenv("STOCS_LPT_MAX")) : 300000;
+  // A top-K launch above that range counts every hypothesis's coarse survivors first and claims in
+  // descending count (survivor_count_kernel): B200, S1 call 1.100 -> 0.822 ms; at 125 000 hypotheses
+  // the two extra launches cost more than they save (0.294 -> 0.312 ms), so there the heavy-first order
+  // stays.  Not when the transforms are read in place from page-locked host memory: the count would
+  // pull every transform over PCIe a second time.
+  const bool ranked = prune && H > lpt_max && !stocs_host_alias(d_T);
+  // [0, 8) work counter, [128, 132) theta bucket, [256, 768) bucket counts, and with the survivor order
+  // from kPruneHist the survivor histogram and the bins' fill counters (M + 1 each): one memset per launch
+  const size_t prune_bytes = ranked ? kPruneHist + (size_t)(ctx->M + 1) * 8 : 256 + kBuckets * 4;
+  unsigned* hist = nullptr;
   if (prune) {
-    // [0, 8) work counter, [128, 132) theta bucket, [256, 768) bucket counts: one memset per launch
     DevBuf& b = ctx->pool[POOL_SCORE_PRUNE];
-    STOCS_CUDA(ctx, b.ensure(256 + kBuckets * 4));
+    STOCS_CUDA(ctx, b.ensure(prune_bytes));
     wctr = b.as<unsigned long long>();
     a.work_counter = wctr;
     a.prune = (unsigned*)(b.as<char>() + 128);
+    hist = (unsigned*)(b.as<char>() + kPruneHist);
   }
   size_t smem = (size_t)kModelFloats * ctx->Mpad * 4 + (size_t)((a.coarse_words + 3) & ~3) * 4 +
                 (size_t)kWarps * (sizeof(WarpQueue) + (prune ? (size_t)(ctx->Mpad / 32) * 4 : 0));   // + survivor masks
@@ -872,18 +1124,11 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   long long want = ((d_H && rq.grid_hint > 0 && rq.grid_hint < H ? rq.grid_hint : H) + kWarps - 1) / kWarps;
   long long grid = (long long)ctx->num_sms * per_sm;
   if (grid > want) grid = want;
-  STOCS_CUDA(ctx, cudaMemsetAsync(wctr, 0, prune ? 256 + kBuckets * 4 : 8, st));  // tie counter accumulates
-  // Heavy-first schedule for MID-SIZE launches only.  Measured on B200 (S1 hypotheses, kernel + probe):
-  // 125 000 hypotheses (the per-GPU share of the named config on 8 GPUs) 0.347 -> 0.312 ms; 10^6
-  // hypotheses 2.100 -> 2.139 ms (the probe costs 64 us per 10^6, the tail it removes is ~0.09 ms
-  // whatever the size), and on the all-fitted S1-fit list the heavy-first order itself slows the
-  // kernel by 2 % (3.622 -> 3.692 ms).  Small launches (the online pipeline's ~1 000 hypotheses)
-  // cannot spare one more launch.  STOCS_NO_LPT=1 switches it off, STOCS_LPT_MAX overrides the bound.
-  const bool no_lpt = getenv("STOCS_NO_LPT") != nullptr;
-  const long long lpt_max = getenv("STOCS_LPT_MAX") ? atoll(getenv("STOCS_LPT_MAX")) : 300000;
-  // (not when the transforms are read in place from page-locked host memory: the probe would pull
+  STOCS_CUDA(ctx, cudaMemsetAsync(wctr, 0, prune ? prune_bytes : 8, st));  // tie counter accumulates
+  // (heavy-first: not when the transforms are read in place from page-locked host memory: the probe would pull
   // every transform over PCIe a second time -- measured 1.7e9 -> 0.9e9 hypotheses/s end to end on 8 GPUs)
-  if (!no_lpt && !d_counters && !d_H && H >= 32768 && H <= lpt_max && slot == 0 && !stocs_host_alias(d_T)) {
+  // (a top-K launch that takes the survivor order claims in that order instead)
+  if (!no_lpt && !ranked && !d_counters && !d_H && H >= 32768 && H <= lpt_max && slot == 0 && !stocs_host_alias(d_T)) {
     DevBuf& b_order = ctx->pool[POOL_SCORE_ORDER];
     STOCS_CUDA(ctx, b_order.ensure((size_t)H * 4));
     unsigned* fill = scr->lpt_fill;
@@ -900,10 +1145,33 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
     ctx->ev1 = ctx->ev_ring[2 * k + 1];
     STOCS_CUDA(ctx, cudaEventRecord(ctx->ev0, st));
   }
+  if (ranked) {   // (inside the timed window: the count and the sort are part of the scoring work)
+    DevBuf &b_ns = ctx->pool[POOL_SCORE_NS], &b_ranked = ctx->pool[POOL_SCORE_ORDER];
+    STOCS_CUDA(ctx, b_ns.ensure((size_t)H * 4));
+    STOCS_CUDA(ctx, b_ranked.ensure((size_t)H * 8));
+    const int rc = enqueue_survivor_counts(ctx, a, b_ns.as<unsigned>(), hist, st);
+    if (rc) return rc;
+    const size_t rs_smem = (size_t)(ctx->M + 1) * 8;
+    STOCS_CUDA(ctx, cudaFuncSetAttribute(rank_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem));
+    const long long rs_grid = std::min((long long)(H + kRsChunk - 1) / kRsChunk, (long long)ctx->num_sms);
+    rank_scatter_kernel<<<(unsigned)rs_grid, kRsThreads, rs_smem, st>>>(b_ns.as<unsigned>(), H, ctx->M, hist,
+                                                                         hist + ctx->M + 1, b_ranked.as<uint2>());
+    a.ranked = b_ranked.as<uint2>();
+  }
   kernel<<<(unsigned)grid, kWarps * 32, smem, st>>>(a);
   if (rq.time_it) { STOCS_CUDA(ctx, cudaEventRecord(ctx->ev1, st)); ctx->ev_count++; }
   STOCS_CUDA(ctx, cudaGetLastError());
   ctx->counters[CTR_SCORE_LAUNCHES] += 1;
   ctx->timing_valid = rq.time_it;
   return STOCS_OK;
+}
+
+// coarse-survivor count of every hypothesis, as the top-K path's survivor order computes it (test hook)
+int stocs_survivor_counts(stocs_b200_ctx* ctx, const float* d_T, int64_t H, unsigned* d_ns, cudaStream_t st) {
+  if (ctx->kd_pending) { const int rc = stocs_kd_finish(ctx, st); if (rc) return rc; }
+  DevBuf &b_lcp = ctx->pool[POOL_SHARD_LCP], &b_hist = ctx->pool[POOL_SCORE_PRUNE];
+  STOCS_CUDA(ctx, b_lcp.ensure((size_t)H * 4));
+  STOCS_CUDA(ctx, b_hist.ensure((size_t)(ctx->M + 1) * 4));
+  STOCS_CUDA(ctx, cudaMemsetAsync(b_hist.p, 0, (size_t)(ctx->M + 1) * 4, st));
+  return enqueue_survivor_counts(ctx, score_args(ctx, d_T, H, b_lcp.as<float>(), nullptr), d_ns, b_hist.as<unsigned>(), st);
 }

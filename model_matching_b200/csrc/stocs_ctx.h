@@ -89,7 +89,8 @@ enum PoolSlot : int {
   POOL_COMM_SEND = 38, POOL_COMM_RECV, POOL_COMM_OUT,
   // sharded scoring scratch (transforms / lcp / inliers of the local shard)
   POOL_SHARD_T = 42, POOL_SHARD_LCP, POOL_SHARD_INL,
-  // score.cu: claim order of the heavy-first schedule (one int per hypothesis of the launch)
+  // score.cu: claim order of the heavy-first schedule (one int per hypothesis of the launch), or of a
+  // top-K launch in descending coarse-survivor count (one {hypothesis, count} uint2 per hypothesis)
   POOL_SCORE_ORDER = 45,
   // reduce.cu: per-CTA top-32 lists of reductions launched on the context's second stream
   POOL_TOPK_LISTS_AUX = 46,
@@ -109,7 +110,9 @@ enum PoolSlot : int {
   POOL_CLUSTER = 55,
   // capi.cu (upload_scenes_device): a slice held on another device, copied to this one (pos3 | nrm3 | cls | pix)
   POOL_SCENE_PEER = 56,
-  POOL_COUNT = 57
+  // score.cu: coarse-survivor count of every hypothesis of a top-K launch (survivor_count_kernel)
+  POOL_SCORE_NS = 57,
+  POOL_COUNT = 58
 };
 
 // Device scalars of one congruent-set search (congruent.cu) and of the pipeline run around it (fit.cu).
@@ -173,6 +176,7 @@ struct stocs_b200_ctx {
 
   // model (centred)
   int M = 0, Mpad = 0;
+  float model_abs_max = 0.f;           // largest |coordinate| of the centred model (NaN if one is not finite)
   float cm[3] = {0, 0, 0};
   std::vector<float> h_mpos, h_mnrm;  // centred positions, normals (M*3)
   DevBuf d_model;                      // 8*Mpad floats: float4 positions, then float4 normals
@@ -338,6 +342,9 @@ struct ScoreRequest {
 };
 int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl,
                        cudaStream_t st, const ScoreRequest& rq);
+// coarse-survivor count of each of H device transforms into d_ns, as a large top-K launch orders its
+// claims by it (score.cu; enqueued on st, lcp written to scratch)
+int stocs_survivor_counts(stocs_b200_ctx* ctx, const float* d_T, int64_t H, unsigned* d_ns, cudaStream_t st);
 int stocs_launch_backproject(stocs_b200_ctx* ctx, const uint16_t* d_depth, const uint8_t* d_bgr,
                              int W, int H, float fx, float cx, float fy, float cy, float scale,
                              float* d_xyz, uint32_t* d_rgb, cudaStream_t st);  // backproject.cu
