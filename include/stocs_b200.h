@@ -123,7 +123,8 @@ int stocs_b200_build_scene_clouds_device(
  * distance ties the way kdtree.h:416-428 does).  pixel_rc may be NULL.
  * upload_scene returns when the grid index is complete; the kd-tree (host work) is finished on a
  * host thread and collected by the first scoring launch that follows, or by the next upload_scene /
- * destroy.  The input buffers are not referenced after the call returns. */
+ * destroy.  (upload_scenes_device builds it on the device instead, on the context's copy stream, and
+ * the same calls wait for it.)  The input buffers are not referenced after the call returns. */
 int stocs_b200_upload_model(stocs_b200_ctx* ctx, const float* pos3, const float* nrm3, int M);
 int stocs_b200_upload_scene(stocs_b200_ctx* ctx, const float* pos3, const float* nrm3,
                             const float* class_probability, const int32_t* pixel_rc, int S);
@@ -353,9 +354,11 @@ int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const f
 
 /* upload_scenes, word for word, from device arrays, e.g. the outputs of build_scene_clouds_device: the arrays are
  * device memory on any device (a context on another device copies its slice with cudaMemcpyPeerAsync); offsets is a
- * host array.  The positions, class weights and pixel coordinates of each slice are copied once into page-locked
- * memory the context owns (the centroid, pixel range, class-weight bound and kd-tree are host work); everything else
- * moves device to device.  d_nrm3, d_class_probability and d_pixel_rc (may be NULL) are on the device of d_pos3; a
+ * host array.  Nothing scene-sized crosses to the host: the centroid, box, class-weight bound and pixel range of
+ * each slice are reduced on the device and come back as one 64-byte record per context (the host lays out the
+ * grid from it), the index build returns its two list lengths as upload_scenes does, and the reference kd-tree is
+ * built on the device beside the index build and joined by the first scoring launch.  Everything else moves
+ * device to device.  d_nrm3, d_class_probability and d_pixel_rc (may be NULL) are on the device of d_pos3; a
  * pointer that is not device memory is STOCS_E_ARG.  stream (a cudaStream_t of that device; NULL is its default
  * stream): the call's work is ordered after what the caller has queued on it so far. */
 int stocs_b200_upload_scenes_device(stocs_b200_ctx* const* ctxs, int n_objects, const float* d_pos3,
@@ -468,6 +471,13 @@ int stocs_b200_kernel_ms_stats(stocs_b200_ctx* ctx, int reset, int32_t* n_launch
  * in leaf order plus the node count.  The build's partition is a branch-free rewrite of the reference's
  * loop; the CPU tests compare its output with the oracle's literal restatement. */
 int stocs_b200_host_kdtree_order(const float* pos3, int n, int32_t* leaf_order, int32_t* n_nodes);
+/* Test hook: the same kd-tree over n finite host points (taken as given, not centred), built on the context's
+ * device as upload_scenes_device builds it (on_device != 0) or on the host as upload_scene builds it.  leaf_order:
+ * n original indices in leaf order; n_nodes: node count; nodes_out (may be NULL, 3 * (n + 3) entries): every node
+ * in pre-order from the root, first child first, as (leaf, bits of the split value, split axis or leaf size), so
+ * that two builds can be compared whatever their node numbering.  The context's scene is not touched. */
+int stocs_b200_debug_kdtree(stocs_b200_ctx* ctx, const float* pos3, int n, int on_device, int32_t* leaf_order,
+                            int32_t* n_nodes, int32_t* nodes_out);
 /* Test hook: the samplers decide the integer part of a PPF angle (int(atan2(y, x) * 180 / M_PI)) and the
  * side of 30 degrees an internal angle lies on from fp32 estimates whenever those are safely away from
  * the deciding thresholds, and by the pinned binary64 evaluation otherwise.  For n pairs (y, x) this

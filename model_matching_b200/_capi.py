@@ -30,7 +30,7 @@ SYMBOLS = [
     "stocs_b200_run_pipeline", "stocs_b200_run_pipeline_instance", "stocs_b200_cluster_poses",
     "stocs_b200_run_pipeline_clustered", "stocs_b200_run_pipeline_instance_clustered",
     "stocs_b200_upload_scenes", "stocs_b200_upload_scenes_device", "stocs_b200_run_pipelines", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
-    "stocs_b200_score_counters", "stocs_b200_kernel_ms_stats", "stocs_b200_host_kdtree_order",
+    "stocs_b200_score_counters", "stocs_b200_kernel_ms_stats", "stocs_b200_host_kdtree_order", "stocs_b200_debug_kdtree",
     "stocs_b200_debug_angle_estimates", "stocs_b200_debug_survivor_counts",
     "stocs_b200_comm_unique_id", "stocs_b200_comm_init", "stocs_b200_comm_destroy", "stocs_b200_shard_range",
     "stocs_b200_score_sharded_device", "stocs_b200_score_sharded",
@@ -124,6 +124,7 @@ def lib():
     L.stocs_b200_score_counters.argtypes = [vp, vp, i64, vp, i32]
     L.stocs_b200_kernel_ms_stats.argtypes = [vp, i32, C.POINTER(i32), C.POINTER(f32), C.POINTER(f32)]
     L.stocs_b200_host_kdtree_order.argtypes = [vp, i32, vp, C.POINTER(i32)]
+    L.stocs_b200_debug_kdtree.argtypes = [vp, vp, i32, i32, vp, C.POINTER(i32), vp]
     L.stocs_b200_debug_angle_estimates.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
     L.stocs_b200_debug_survivor_counts.argtypes = [vp, vp, i64, vp]
     L.stocs_b200_comm_unique_id.argtypes = [vp]
@@ -721,6 +722,16 @@ class Context:
         ns = np.empty(H, np.int32)
         self._check(self._L.stocs_b200_debug_survivor_counts(self.h, dT_ptr, H, _ptr(ns)))
         return ns
+
+    def debug_kdtree(self, pos, on_device):
+        """the reference kd-tree over pos as built on the device (on_device) or on the host (test hook, see
+        include/stocs_b200.h) -> (leaf order, node count, int32 [nodes, 3] pre-order dump)"""
+        pos = _f32(pos, (-1, 3))
+        n = pos.shape[0]
+        order, nn, nodes = np.empty(n, np.int32), C.c_int32(0), np.empty((n + 3, 3), np.int32)
+        self._check(self._L.stocs_b200_debug_kdtree(self.h, _ptr(pos), n, int(bool(on_device)), _ptr(order), C.byref(nn),
+                                                    _ptr(nodes)))
+        return order, nn.value, nodes[:nn.value].copy()
 
     def last_kernel_ms(self):
         ms = C.c_float(0)

@@ -208,6 +208,7 @@ int stocs_b200_create(stocs_b200_ctx** out, int device) {
   ok = ok && cudaHostAlloc((void**)&ctx->h_top, sizeof(stocs_b200_ctx::TopCache), cudaHostAllocDefault) == cudaSuccess;
   ok = ok && cudaHostAlloc((void**)&ctx->h_pipe_state, sizeof(StocsPipeState), cudaHostAllocDefault) == cudaSuccess;
   ok = ok && cudaHostAlloc((void**)&ctx->h_index_counts, 4 * (8 + 1 + STOCS_B200_MAX_CLOUD_OBJECTS), cudaHostAllocDefault) == cudaSuccess;
+  ok = ok && cudaHostAlloc((void**)&ctx->h_plan, sizeof(ScenePlan), cudaHostAllocDefault) == cudaSuccess;
   for (int i = 0; ok && i < stocs_b200_ctx::kMaxChunks; ++i)
     ok = cudaEventCreateWithFlags(&ctx->chunk_ev[i], cudaEventDisableTiming) == cudaSuccess;
   if (!ok) { g_create_err = "stream/event creation failed"; delete ctx; return STOCS_E_CUDA; }
@@ -236,7 +237,7 @@ void stocs_b200_destroy(stocs_b200_ctx* ctx) {
   if (ctx->stream) cudaStreamSynchronize(ctx->stream);
   stocs_b200_comm_destroy(ctx);
   DevBuf* bufs[] = {&ctx->d_model, &ctx->d_mpos4, &ctx->d_mnrm4, &ctx->d_spos4, &ctx->d_sattr, &ctx->d_spix,
-                    &ctx->d_coarse, &ctx->d_brick_occ, &ctx->d_bricks, &ctx->d_cell_start, &ctx->d_cand, &ctx->d_kd_nodes, &ctx->d_kd_pts, &ctx->d_ppf_bin_start,
+                    &ctx->d_coarse, &ctx->d_brick_occ, &ctx->d_bricks, &ctx->d_cell_start, &ctx->d_cand, &ctx->d_kd_nodes, &ctx->d_kd_pts, &ctx->d_kd_build, &ctx->d_ppf_bin_start,
                     &ctx->d_ppf_pairs, &ctx->d_ppf_keybits, &ctx->d_T, &ctx->d_lcp, &ctx->d_inl, &ctx->d_work,
                     &ctx->d_tmp, &ctx->d_tmp2, &ctx->d_small, &ctx->d_edge, &ctx->d_inst_state, &ctx->d_mask_store,
                     &ctx->d_frontier};
@@ -251,7 +252,7 @@ void stocs_b200_destroy(stocs_b200_ctx* ctx) {
   stocs_cluster_free_host(ctx);
   if (ctx->h_index_counts) cudaFreeHost(ctx->h_index_counts);
   if (ctx->h_kd_stage) cudaFreeHost(ctx->h_kd_stage);
-  if (ctx->h_scene_stage) cudaFreeHost(ctx->h_scene_stage);
+  if (ctx->h_plan) cudaFreeHost(ctx->h_plan);
   if (ctx->kd_copy_done) cudaEventDestroy(ctx->kd_copy_done);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -312,8 +313,7 @@ int stocs_b200_upload_model(stocs_b200_ctx* ctx, const float* pos3, const float*
   STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_tmp.p, pos3, (size_t)M * 12, cudaMemcpyHostToDevice, st));
   // centroid, centred copy and box on the host (see stocs_centre_points); the device centres its own copy
   ctx->h_mpos.resize((size_t)M * 3);
-  int rc = stocs_centre_points(ctx, ctx->d_tmp.as<float>(), M, ctx->d_mpos4.as<float4>(), nullptr, ctx->cm, nullptr, pos3,
-                               ctx->h_mpos.data());
+  int rc = stocs_centre_points(ctx, ctx->d_tmp.as<float>(), M, ctx->d_mpos4.as<float4>(), ctx->cm, pos3, ctx->h_mpos.data());
   if (rc) return rc;
   ctx->h_mnrm.assign(nrm3, nrm3 + (size_t)M * 3);
   const int Mpad = ((M + 63) / 64) * 64;  // the scoring kernel consumes 64 points per iteration
@@ -343,12 +343,13 @@ int stocs_b200_upload_model(stocs_b200_ctx* ctx, const float* pos3, const float*
 
 }  // extern "C"
 
-// First step of an upload: replaces the scene and grows every buffer the upload uses, with the host
-// work (centring, pixel range, class-weight bound, kd-tree thread start) but nothing enqueued, so that
-// the growth of several objects' buffers happens before any object's kernels are queued.  The caller has
-// checked the arguments.
+// First step of an upload: replaces the scene and grows every buffer the upload uses, with nothing enqueued,
+// so that the growth of several objects' buffers happens before any object's kernels are queued.  Arrays in
+// host memory (kind cudaMemcpyHostToDevice) are planned on the host here: centring, pixel range, class-weight
+// bound, kd-tree thread start.  Arrays in device memory -- and host arrays with STOCS_DEVICE_CENTROID set --
+// are planned on the device by the next two steps.  The caller has checked the arguments.
 static int scene_upload_plan(stocs_b200_ctx* ctx, const float* pos3, const float* class_probability,
-                             const int32_t* pixel_rc, int S) {
+                             const int32_t* pixel_rc, int S, cudaMemcpyKind kind) {
   cudaSetDevice(ctx->device);
   cudaStream_t st = ctx->stream;
   // The previous scene is invalid from here on; S is committed only when the new index is complete,
@@ -360,24 +361,50 @@ static int scene_upload_plan(stocs_b200_ctx* ctx, const float* pos3, const float
   STOCS_CUDA(ctx, ctx->d_tmp.ensure((size_t)S * 16));   // nrm3 | cls, then pos3
   STOCS_CUDA(ctx, ctx->d_sattr.ensure((size_t)S * 16));
   STOCS_CUDA(ctx, ctx->d_spix.ensure((size_t)S * 8));
-  stocs_set_weight_bound(ctx, class_probability, S);
-  ctx->pix_min[0] = ctx->pix_min[1] = 0; ctx->pix_max[0] = ctx->pix_max[1] = 0;
-  if (pixel_rc) {  // range of the pixel coordinates: instance sampling indexes images with them
-    ctx->pix_min[0] = ctx->pix_max[0] = pixel_rc[0]; ctx->pix_min[1] = ctx->pix_max[1] = pixel_rc[1];
-    for (int i = 0; i < S; ++i)
-      for (int k = 0; k < 2; ++k) {
-        const int v = pixel_rc[2 * (size_t)i + k];
-        if (v < ctx->pix_min[k]) ctx->pix_min[k] = v;
-        if (v > ctx->pix_max[k]) ctx->pix_max[k] = v;
-      }
+  ctx->h_pos_pending = nullptr;
+  if (kind == cudaMemcpyHostToDevice && !getenv("STOCS_DEVICE_CENTROID")) {
+    stocs_set_weight_bound(ctx, class_probability, S);
+    ctx->pix_min[0] = ctx->pix_min[1] = 0; ctx->pix_max[0] = ctx->pix_max[1] = 0;
+    if (pixel_rc) {  // range of the pixel coordinates: instance sampling indexes images with them
+      ctx->pix_min[0] = ctx->pix_max[0] = pixel_rc[0]; ctx->pix_min[1] = ctx->pix_max[1] = pixel_rc[1];
+      for (int i = 0; i < S; ++i)
+        for (int k = 0; k < 2; ++k) {
+          const int v = pixel_rc[2 * (size_t)i + k];
+          if (v < ctx->pix_min[k]) ctx->pix_min[k] = v;
+          if (v > ctx->pix_max[k]) ctx->pix_max[k] = v;
+        }
+    }
+    ctx->h_pos_pending = pos3;
   }
-  ctx->h_pos_pending = getenv("STOCS_DEVICE_CENTROID") ? nullptr : pos3;
-  if (!ctx->h_pos_pending)   // the device centring of the plan reads the positions from d_tmp
-    STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_tmp.p, pos3, (size_t)S * 12, cudaMemcpyHostToDevice, st));
   return stocs_index_plan(ctx);
 }
 
-// Second step: the uploads and kernels, up to the index build's two length copies; no synchronisation.  The
+// Second step of a scene planned on the device: its positions, class weights and pixels (host arrays are
+// copied to d_tmp | d_spix first) are reduced to the record stocs_index_plan_finish waits for.
+static int scene_upload_centre(stocs_b200_ctx* ctx, const float* pos3, const float* class_probability,
+                               const int32_t* pixel_rc, int S, cudaMemcpyKind kind) {
+  if (!ctx->plan_on_device) return STOCS_OK;
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = ctx->stream;
+  if (kind == cudaMemcpyHostToDevice) {
+    float* d = ctx->d_tmp.as<float>();
+    STOCS_CUDA(ctx, cudaMemcpyAsync(d, pos3, (size_t)S * 12, kind, st));
+    STOCS_CUDA(ctx, cudaMemcpyAsync(d + 3 * (size_t)S, class_probability, (size_t)S * 4, kind, st));
+    if (pixel_rc) STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_spix.p, pixel_rc, (size_t)S * 8, kind, st));
+    pos3 = d;
+    class_probability = d + 3 * (size_t)S;
+    pixel_rc = pixel_rc ? ctx->d_spix.as<int32_t>() : nullptr;
+  }
+  return stocs_index_centre_device(ctx, pos3, class_probability, pixel_rc);
+}
+
+// Third step of a scene planned on the device: one wait for its record, then the grid layout.
+static int scene_upload_plan_finish(stocs_b200_ctx* ctx) {
+  cudaSetDevice(ctx->device);
+  return stocs_index_plan_finish(ctx);
+}
+
+// Last enqueue step: the uploads and kernels, up to the index build's two length copies; no synchronisation.  The
 // arrays are copied with `kind`: host arrays (upload_scene[s]) or device arrays on the context's device.
 static int scene_upload_enqueue(stocs_b200_ctx* ctx, const float* pos3, const float* nrm3, const float* class_probability,
                                 const int32_t* pixel_rc, int S, cudaMemcpyKind kind) {
@@ -405,8 +432,12 @@ static int scene_upload_enqueue(stocs_b200_ctx* ctx, const float* pos3, const fl
 // begin) and commits S on success.
 static int scene_upload_end(stocs_b200_ctx* ctx, int rc) {
   cudaSetDevice(ctx->device);
+  ctx->plan_on_device = false;
   if (rc == STOCS_OK) rc = stocs_index_complete(ctx);
-  else cudaStreamSynchronize(ctx->stream);   // nothing of a failed upload stays queued
+  if (rc) {   // nothing of a failed upload stays queued, a device kd-tree build included
+    stocs_kd_finish(ctx, ctx->stream, false);
+    cudaStreamSynchronize(ctx->stream);
+  }
   ctx->S = rc ? 0 : ctx->S_pending;
   ctx->S_pending = 0;
   ctx->h_pos_pending = nullptr;
@@ -440,8 +471,11 @@ int stocs_b200_upload_scene(stocs_b200_ctx* ctx, const float* pos3, const float*
   if (!ctx) return STOCS_E_ARG;
   if (!pos3 || !nrm3 || !class_probability || S <= 0) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: bad argument");
   if (S > (1 << 27)) STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: at most 2^27 scene points are supported");
-  int rc = scene_upload_plan(ctx, pos3, class_probability, pixel_rc, S);
-  if (rc == STOCS_OK) rc = scene_upload_enqueue(ctx, pos3, nrm3, class_probability, pixel_rc, S, cudaMemcpyHostToDevice);
+  const cudaMemcpyKind kind = cudaMemcpyHostToDevice;
+  int rc = scene_upload_plan(ctx, pos3, class_probability, pixel_rc, S, kind);
+  if (rc == STOCS_OK) rc = scene_upload_centre(ctx, pos3, class_probability, pixel_rc, S, kind);
+  if (rc == STOCS_OK) rc = scene_upload_plan_finish(ctx);
+  if (rc == STOCS_OK) rc = scene_upload_enqueue(ctx, pos3, nrm3, class_probability, pixel_rc, S, kind);
   return scene_upload_end(ctx, rc);
 }
 
@@ -466,10 +500,12 @@ static int upload_scenes_check(stocs_b200_ctx* const* ctxs, int n_objects, const
 }
 
 // Every object's buffers are grown before any object's work is enqueued, and every object's work is
-// enqueued before any is waited for: the host waits once per context, at the end.  Object k's host work reads
-// host[k]; its uploads copy dev[k] with `kind`.  An object whose status is already an error is only ended.
+// enqueued before any is waited for.  Slices copied with `kind` cudaMemcpyHostToDevice are planned on the host
+// and waited for once per context, at the end; slices in device memory are planned on the device, with one more
+// wait per context for the plan's record before the index builds are enqueued.  An object whose status is
+// already an error is only ended.
 static int upload_slices(stocs_b200_ctx* const* ctxs, int n_objects, const char* who, const int64_t* offsets,
-                         const SceneSlice* host, const SceneSlice* dev, cudaMemcpyKind kind, std::vector<int>& status) {
+                         const SceneSlice* sl, cudaMemcpyKind kind, std::vector<int>& status) {
   for (int k = 0; k < n_objects; ++k) {   // every object's host work and buffer growth first ...
     stocs_b200_ctx* ctx = ctxs[k];
     const int S = (int)(offsets[k + 1] - offsets[k]);
@@ -482,12 +518,18 @@ static int upload_slices(stocs_b200_ctx* const* ctxs, int n_objects, const char*
       ctx->counters[CTR_GRID_CELLS] = ctx->counters[CTR_CANDIDATES] = ctx->counters[CTR_OCCUPIED_CELLS] = 0;
       continue;
     }
-    if (status[k] == STOCS_OK) status[k] = scene_upload_plan(ctx, host[k].pos3, host[k].cls, host[k].pix, S);
+    if (status[k] == STOCS_OK) status[k] = scene_upload_plan(ctx, sl[k].pos3, sl[k].cls, sl[k].pix, S, kind);
   }
+  for (int k = 0; k < n_objects; ++k) {   // ... then every device plan ...
+    const int S = (int)(offsets[k + 1] - offsets[k]);
+    if (S > 0 && status[k] == STOCS_OK) status[k] = scene_upload_centre(ctxs[k], sl[k].pos3, sl[k].cls, sl[k].pix, S, kind);
+  }
+  for (int k = 0; k < n_objects; ++k)     // ... one wait for each plan's record ...
+    if (offsets[k + 1] > offsets[k] && status[k] == STOCS_OK) status[k] = scene_upload_plan_finish(ctxs[k]);
   for (int k = 0; k < n_objects; ++k) {   // ... then every object's uploads and kernels
     const int S = (int)(offsets[k + 1] - offsets[k]);
     if (S > 0 && status[k] == STOCS_OK)
-      status[k] = scene_upload_enqueue(ctxs[k], dev[k].pos3, dev[k].nrm3, dev[k].cls, dev[k].pix, S, kind);
+      status[k] = scene_upload_enqueue(ctxs[k], sl[k].pos3, sl[k].nrm3, sl[k].cls, sl[k].pix, S, kind);
   }
   for (int k = 0; k < n_objects; ++k)
     if (offsets[k + 1] > offsets[k]) status[k] = scene_upload_end(ctxs[k], status[k]);
@@ -509,12 +551,11 @@ int stocs_b200_upload_scenes(stocs_b200_ctx* const* ctxs, int n_objects, const f
     slices[k] = SceneSlice{pos3 + 3 * o, nrm3 + 3 * o, class_probability + o, pixel_rc ? pixel_rc + 2 * o : nullptr};
   }
   std::vector<int> status(n_objects, STOCS_OK);
-  return upload_slices(ctxs, n_objects, who, offsets, slices.data(), slices.data(), cudaMemcpyHostToDevice, status);
+  return upload_slices(ctxs, n_objects, who, offsets, slices.data(), cudaMemcpyHostToDevice, status);
 }
 
-// The slices' positions, class weights and pixels are staged into each context's page-locked memory (a context on
-// another device first copies its slice to its own device), the host waits once per context, and the host plan of
-// upload_scenes runs on the staged copies; the kernels' inputs are copied device to device.
+// A context on another device first copies its slice to its own device; the plan, uploads and index builds of
+// upload_scenes then run from device memory, planned on the device.
 int stocs_b200_upload_scenes_device(stocs_b200_ctx* const* ctxs, int n_objects, const float* d_pos3, const float* d_nrm3,
                                     const float* d_class_probability, const int32_t* d_pixel_rc, const int64_t* offsets,
                                     void* stream) {
@@ -529,28 +570,22 @@ int stocs_b200_upload_scenes_device(stocs_b200_ctx* const* ctxs, int n_objects, 
     if (a.first && !stocs_device_memory(a.first, src_dev))
       return stocs_batch_fail(ctxs, -1, STOCS_E_ARG, who, std::string(a.second) + " is not device memory on the device of d_pos3");
   std::vector<int> status(n_objects, STOCS_OK);
-  std::vector<SceneSlice> host(n_objects), dev(n_objects);
+  std::vector<SceneSlice> dev(n_objects);
   auto fail = [&](int k, cudaError_t e, const char* what) {
     if (e == cudaSuccess || status[k]) return;
     ctxs[k]->err = std::string(what) + ": " + cudaGetErrorString(e);
     status[k] = STOCS_E_CUDA;
   };
-  for (int k = 0; k < n_objects; ++k) {   // growth first: page-locked staging, and the device copy of a foreign slice
+  for (int k = 0; k < n_objects; ++k) {   // growth first: the device copy of a foreign slice
     stocs_b200_ctx* ctx = ctxs[k];
     const size_t S = (size_t)(offsets[k + 1] - offsets[k]);
-    if (S == 0) continue;
+    if (S == 0 || ctx->device == src_dev) continue;
     cudaSetDevice(ctx->device);
-    if (ctx->h_scene_stage_bytes < S * 24) {
-      if (ctx->h_scene_stage) cudaFreeHost(ctx->h_scene_stage);
-      ctx->h_scene_stage = nullptr; ctx->h_scene_stage_bytes = 0;
-      fail(k, cudaHostAlloc(&ctx->h_scene_stage, S * 24, cudaHostAllocDefault), "cudaHostAlloc");
-      if (!status[k]) ctx->h_scene_stage_bytes = S * 24;
-    }
-    if (ctx->device != src_dev) fail(k, ctx->pool[POOL_SCENE_PEER].ensure(S * 36), "peer copy buffer");
+    fail(k, ctx->pool[POOL_SCENE_PEER].ensure(S * 36), "peer copy buffer");
   }
   CallerEvent producer;
   const cudaError_t ev = producer.record(stream, src_dev);
-  for (int k = 0; k < n_objects; ++k) {   // then every object's copies ...
+  for (int k = 0; k < n_objects; ++k) {   // then every object's wait for the caller and peer copies ...
     stocs_b200_ctx* ctx = ctxs[k];
     const int64_t o = offsets[k];
     const size_t S = (size_t)(offsets[k + 1] - o);
@@ -571,19 +606,9 @@ int stocs_b200_upload_scenes_device(stocs_b200_ctx* const* ctxs, int n_objects, 
       d = local;
     }
     dev[k] = d;
-    float* h = (float*)ctx->h_scene_stage;   // pos3 | cls | pix
-    host[k] = SceneSlice{h, nullptr, h + 3 * S, d.pix ? (const int32_t*)(h + 4 * S) : nullptr};
-    fail(k, cudaMemcpyAsync((void*)host[k].pos3, d.pos3, S * 12, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
-    fail(k, cudaMemcpyAsync((void*)host[k].cls, d.cls, S * 4, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
-    if (d.pix) fail(k, cudaMemcpyAsync((void*)host[k].pix, d.pix, S * 8, cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync");
   }
-  for (int k = 0; k < n_objects; ++k)     // ... one wait per context ...
-    if (offsets[k + 1] > offsets[k]) {
-      cudaSetDevice(ctxs[k]->device);
-      fail(k, cudaStreamSynchronize(ctxs[k]->stream), "cudaStreamSynchronize");
-    }
   // ... and the plan, uploads and index builds of upload_scenes
-  return upload_slices(ctxs, n_objects, who, offsets, host.data(), dev.data(), cudaMemcpyDeviceToDevice, status);
+  return upload_slices(ctxs, n_objects, who, offsets, dev.data(), cudaMemcpyDeviceToDevice, status);
 }
 
 int stocs_b200_get_centroids(stocs_b200_ctx* ctx, float* scene3, float* model3) {
@@ -597,7 +622,14 @@ int stocs_b200_get_centred(stocs_b200_ctx* ctx, float* scene_pos3, float* model_
   if (!ctx) return STOCS_E_ARG;
   if (scene_pos3) {
     if (ctx->S <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "no scene");
-    memcpy(scene_pos3, ctx->h_spos.data(), (size_t)ctx->S * 12);
+    // read from the device: a scene uploaded from device memory has no host copy
+    cudaSetDevice(ctx->device);
+    std::vector<float4> p((size_t)ctx->S);
+    STOCS_CUDA(ctx, cudaMemcpyAsync(p.data(), ctx->d_spos4.p, (size_t)ctx->S * 16, cudaMemcpyDeviceToHost, ctx->stream));
+    STOCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    for (int i = 0; i < ctx->S; ++i) {
+      scene_pos3[3 * (size_t)i] = p[i].x; scene_pos3[3 * (size_t)i + 1] = p[i].y; scene_pos3[3 * (size_t)i + 2] = p[i].z;
+    }
   }
   if (model_pos3) {
     if (ctx->M <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "no model");

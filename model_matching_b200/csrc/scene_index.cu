@@ -10,9 +10,10 @@
 // reads is a dense voxel grid whose cells carry eps-DILATED candidate lists: cell C lists every
 // scene point within eps (plus a rounding margin) of C's box, so an exact radius-eps query reads
 // ONE cell descriptor and one contiguous run of float4 candidates.  The reference kd-tree
-// (kdtree.h:355-370,522-641) is also built -- on the host, once per frame -- and uploaded; the
-// scoring kernel walks it only when two candidates are at exactly the same squared distance, to
-// reproduce the reference's traversal-order tie rule (kdtree.h:416-428).
+// (kdtree.h:355-370,522-641) is also built once per frame -- on a host thread for a scene given in host
+// memory, on the device for one given in device memory; the scoring kernel walks it only when two
+// candidates are at exactly the same squared distance, to reproduce the reference's traversal-order
+// tie rule (kdtree.h:416-428).
 #include <cub/device/device_scan.cuh>
 
 #include <cstdio>
@@ -30,18 +31,28 @@
 namespace {
 
 // Sequential fp32 centroid in index order (src/stocs.cpp:945-956).  The sums are order
-// dependent, so the chain is serial: 256 threads stage 2048-point chunks into shared memory with
-// coalesced loads and lanes 0..2 of warp 0 run the three dependent add chains out of it.
+// dependent, so the chain is serial: lanes 0..2 of warp 0 run the three dependent add chains out of
+// shared memory while warps 1..7 stage the next 1024-point chunk into the other buffer with coalesced
+// loads (a full chunk's adds are unrolled so that their loads issue ahead of the chain).
 __global__ void centroid_seq_kernel(const float* __restrict__ pos3, int n, float* __restrict__ out3) {
-  constexpr int CH = 2048;
-  __shared__ float buf[CH * 3];
+  constexpr int CH = 1024;
+  __shared__ float buf[2][CH * 3];
   float acc = 0.f;
-  for (int base = 0; base < n; base += CH) {
-    int cnt = min(CH, n - base);
-    for (int t = threadIdx.x; t < cnt * 3; t += blockDim.x) buf[t] = pos3[(size_t)base * 3 + t];
-    __syncthreads();
-    if (threadIdx.x < 3) {
-      for (int i = 0; i < cnt; ++i) acc += buf[i * 3 + threadIdx.x];
+  for (int t = threadIdx.x; t < min(CH, n) * 3; t += blockDim.x) buf[0][t] = pos3[t];
+  __syncthreads();
+  for (int base = 0, c = 0; base < n; base += CH, ++c) {
+    const int cnt = min(CH, n - base);
+    if (threadIdx.x >= 32) {
+      const int nb = base + CH, ncnt = min(CH, n - nb);
+      for (int t = threadIdx.x - 32; t < ncnt * 3; t += blockDim.x - 32) buf[(c + 1) & 1][t] = pos3[(size_t)nb * 3 + t];
+    } else if (threadIdx.x < 3) {
+      const float* b = buf[c & 1] + threadIdx.x;
+      if (cnt == CH) {
+#pragma unroll 32
+        for (int i = 0; i < CH; ++i) acc += b[i * 3];
+      } else {
+        for (int i = 0; i < cnt; ++i) acc += b[i * 3];
+      }
     }
     __syncthreads();
   }
@@ -86,6 +97,193 @@ __global__ void pack_attr_kernel(const float* __restrict__ nrm3, const float* __
                                  float4* __restrict__ out) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = make_float4(nrm3[3 * (size_t)i], nrm3[3 * (size_t)i + 1], nrm3[3 * (size_t)i + 2], cls[i]);
+}
+
+// Device plan of a scene in device memory: the record starts as the identity of every reduction below
+__global__ void plan_init_kernel(ScenePlan* p) {
+  const int t = threadIdx.x;
+  if (t < 3) { p->aabb[t] = INT_MAX; p->aabb[3 + t] = INT_MIN; }
+  if (t < 2) { p->pix_min[t] = INT_MAX; p->pix_max[t] = INT_MIN; }
+  if (t == 0) { p->wbits = 0; p->first_bad = INT_MAX; }
+}
+
+// first class weight that is negative, NaN or infinite (stocs_set_weight_bound stops there), and the
+// (row, col) range of the pixel coordinates (pix may be NULL)
+__global__ void plan_bounds_kernel(const float* __restrict__ cls, const int32_t* __restrict__ pix, int n,
+                                   ScenePlan* __restrict__ p) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  int bad = INT_MAX, mn[2] = {INT_MAX, INT_MAX}, mx[2] = {INT_MIN, INT_MIN};
+  if (i < n) {
+    const float w = cls[i];
+    if (!(w >= 0.f && w <= FLT_MAX)) bad = i;
+    if (pix) for (int k = 0; k < 2; ++k) mn[k] = mx[k] = pix[2 * (size_t)i + k];
+  }
+  bad = __reduce_min_sync(0xffffffffu, bad);
+  if ((threadIdx.x & 31) == 0 && bad != INT_MAX) atomicMin(&p->first_bad, bad);
+  if (pix)
+    for (int k = 0; k < 2; ++k) {
+      const int a = __reduce_min_sync(0xffffffffu, mn[k]), b = __reduce_max_sync(0xffffffffu, mx[k]);
+      if ((threadIdx.x & 31) == 0) { atomicMin(&p->pix_min[k], a); atomicMax(&p->pix_max[k], b); }
+    }
+}
+
+// largest class weight before the first bad one.  Those weights are in [0, FLT_MAX], where the bit
+// patterns order as the values do (-0 reads as INT_MIN and loses to the initial +0, as on the host).
+__global__ void plan_weight_max_kernel(const float* __restrict__ cls, int n, ScenePlan* __restrict__ p) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int m = __reduce_max_sync(0xffffffffu, (i < n && i < p->first_bad) ? __float_as_int(cls[i]) : 0);
+  if ((threadIdx.x & 31) == 0 && m > 0) atomicMax(&p->wbits, m);
+}
+
+// ---- the reference kd-tree on the device -------------------------------------------------------------
+// Level-synchronous: one launch per level (at most 32, the depth cap), one CTA per node of the level's
+// frontier.  Per node, exactly KdBuild::build below: box (min / max are exact in any order), axis of the
+// largest half-extent with strict > in x, y, z order, split value in binary32 without contraction, and
+// the reference's partition -- the k-th element >= sv of [start, mid) swaps with the k-th element < sv
+// counted from the end of [mid, end), mid = start + #{c < sv} -- as a count, a scan that lists the left
+// misplaced positions, and a reverse scan that swaps each right misplaced element with its partner.
+// Node numbers differ from the host build's (children are allocated by an atomic counter); tree shape,
+// split values and leaf point order do not.
+struct KdJob { uint32_t node, start, end, pad; };
+constexpr int kKdThreads = 512;
+constexpr int kKdCounters = 64;   // [0] nodes allocated, [L] nodes of level L's frontier (L = 1..32)
+
+__global__ void kd_init_kernel(int* __restrict__ ctr, KdJob* __restrict__ front, int n) {
+  const int t = threadIdx.x;
+  if (t < kKdCounters) ctr[t] = t <= 1 ? 1 : 0;
+  if (t == 0) front[0] = KdJob{0u, 0u, (uint32_t)n, 0u};
+}
+
+// exclusive prefix of a 0/1 flag over the CTA in thread order; *total: the CTA's sum
+__device__ __forceinline__ int kd_scan(bool flag, int* s_warp, int* total) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const unsigned b = __ballot_sync(0xffffffffu, flag);
+  if (lane == 0) s_warp[warp] = __popc(b);
+  __syncthreads();
+  int off = 0, tot = 0;
+#pragma unroll
+  for (int w = 0; w < kKdThreads / 32; ++w) { const int c = s_warp[w]; off += w < warp ? c : 0; tot += c; }
+  __syncthreads();
+  *total = tot;
+  return off + __popc(b & ((1u << lane) - 1u));
+}
+
+__device__ __forceinline__ float kd_comp(float4 p, int d) { return d == 0 ? p.x : (d == 1 ? p.y : p.z); }
+
+__global__ void __launch_bounds__(kKdThreads) kd_level_kernel(float4* pts, KdNodeDev* __restrict__ nodes,
+                                                               int* __restrict__ ctr, const KdJob* __restrict__ in,
+                                                               KdJob* __restrict__ out, uint32_t* lpos, int level) {
+  __shared__ float s_box[6][kKdThreads / 32];
+  __shared__ int s_warp[kKdThreads / 32];
+  __shared__ float s_sv;
+  __shared__ int s_dim;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int njobs = ctr[level];
+  for (int j = blockIdx.x; j < njobs; j += gridDim.x) {
+    const KdJob job = in[j];
+    const float big = FLT_MAX / 2;   // the host build's initial box
+    float b[6] = {big, big, big, -big, -big, -big};
+    for (uint32_t i = job.start + threadIdx.x; i < job.end; i += kKdThreads) {
+      const float4 p = pts[i];
+      b[0] = fminf(b[0], p.x); b[1] = fminf(b[1], p.y); b[2] = fminf(b[2], p.z);
+      b[3] = fmaxf(b[3], p.x); b[4] = fmaxf(b[4], p.y); b[5] = fmaxf(b[5], p.z);
+    }
+#pragma unroll
+    for (int k = 0; k < 6; ++k) {
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float v = __shfl_xor_sync(0xffffffffu, b[k], o);
+        b[k] = k < 3 ? fminf(b[k], v) : fmaxf(b[k], v);
+      }
+      if (lane == 0) s_box[k][warp] = b[k];
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      float mn[3], mx[3];
+      for (int k = 0; k < 3; ++k) {
+        mn[k] = s_box[k][0]; mx[k] = s_box[3 + k][0];
+        for (int w = 1; w < kKdThreads / 32; ++w) { mn[k] = fminf(mn[k], s_box[k][w]); mx[k] = fmaxf(mx[k], s_box[3 + k][w]); }
+      }
+      float hd[3];
+      for (int k = 0; k < 3; ++k) hd[k] = __fmul_rn(0.5f, __fsub_rn(mx[k], mn[k]));
+      int dim = 0;
+      if (hd[1] > hd[dim]) dim = 1;
+      if (hd[2] > hd[dim]) dim = 2;
+      s_dim = dim;
+      s_sv = __fadd_rn(mn[dim], __fdiv_rn(__fsub_rn(mx[dim], mn[dim]), 2.0f));
+    }
+    __syncthreads();
+    const int dim = s_dim;
+    const float sv = s_sv;
+    int below = 0;
+    for (uint32_t i = job.start + threadIdx.x; i < job.end; i += kKdThreads) below += kd_comp(pts[i], dim) < sv ? 1 : 0;
+    below = __reduce_add_sync(0xffffffffu, below);
+    if (lane == 0) s_warp[warp] = below;
+    __syncthreads();
+    int nbelow = 0;
+    for (int w = 0; w < kKdThreads / 32; ++w) nbelow += s_warp[w];
+    __syncthreads();
+    const uint32_t mid = job.start + (uint32_t)nbelow;
+    // left misplaced positions, in increasing order, into lpos[start + k]
+    int run = 0;
+    for (uint32_t base = job.start; base < mid; base += kKdThreads) {
+      const uint32_t i = base + threadIdx.x;
+      const bool f = i < mid && !(kd_comp(pts[i], dim) < sv);
+      int tot;
+      const int k = run + kd_scan(f, s_warp, &tot);
+      if (f) lpos[job.start + k] = i;
+      run += tot;
+    }
+    __syncthreads();
+    // right misplaced positions, counted from the end: the k-th swaps with lpos[start + k]
+    run = 0;
+    for (uint32_t base = 0; base < job.end - mid; base += kKdThreads) {
+      const uint32_t r = base + threadIdx.x;
+      const uint32_t i = job.end - 1 - r;
+      const bool f = r < job.end - mid && kd_comp(pts[i], dim) < sv;
+      int tot;
+      const int k = run + kd_scan(f, s_warp, &tot);
+      if (f) {
+        const uint32_t l = lpos[job.start + k];
+        const float4 a = pts[l];
+        pts[l] = pts[i];
+        pts[i] = a;
+      }
+      run += tot;
+    }
+    if (threadIdx.x == 0) {
+      const uint32_t first = (uint32_t)atomicAdd(&ctr[0], 2);
+      nodes[job.node] = KdNodeDev{sv, first, (uint32_t)dim, 0u};
+      const uint32_t lo[2] = {job.start, mid}, hi[2] = {mid, job.end};
+      for (int c = 0; c < 2; ++c) {
+        const uint32_t cnt = hi[c] - lo[c];
+        if (cnt <= 64u || level >= 32) nodes[first + c] = KdNodeDev{0.f, lo[c], cnt, 1u};
+        else out[atomicAdd(&ctr[level + 1], 1)] = KdJob{first + (uint32_t)c, lo[c], hi[c], 0u};
+      }
+    }
+    __syncthreads();
+  }
+}
+
+// scratch of a device build over n points: counters | two frontiers (a level holds at most n / 65 nodes
+// of more than 64 points each, the root level one) | the left misplaced positions of every node
+size_t kd_frontier_cap(int n) { return (size_t)n / 65 + 1; }
+size_t kd_scratch_bytes(int n) { return kKdCounters * 4 + 2 * kd_frontier_cap(n) * sizeof(KdJob) + (size_t)n * 4; }
+
+// Builds the tree over the n points of pts ({x, y, z, bits(original index)}, reordered in place into leaf
+// order) into nodes (at most n + 3); enqueued on st, no synchronisation.
+cudaError_t kd_build_enqueue(float4* pts, KdNodeDev* nodes, void* scratch, int n, cudaStream_t st) {
+  int* ctr = (int*)scratch;
+  const size_t F = kd_frontier_cap(n);
+  KdJob* front[2] = {(KdJob*)((char*)scratch + kKdCounters * 4), (KdJob*)((char*)scratch + kKdCounters * 4) + F};
+  uint32_t* lpos = (uint32_t*)(front[1] + F);
+  kd_init_kernel<<<1, kKdCounters, 0, st>>>(ctr, front[0], n);
+  for (int level = 1; level <= 32; ++level) {
+    const size_t width = std::min<size_t>((size_t)1 << std::min(level - 1, 20), F);
+    kd_level_kernel<<<(unsigned)width, kKdThreads, 0, st>>>(pts, nodes, ctr, front[(level - 1) & 1], front[level & 1],
+                                                            lpos, level);
+  }
+  return cudaGetLastError();
 }
 
 // Cells are numbered brick-major: 4x4x4 bricks, 64 consecutive cell numbers per brick, so that a
@@ -313,18 +511,18 @@ struct KdBuild {
 
 }  // namespace
 
-// Centre n points with the reference's sequential fp32 centroid; optional float4 / float3 device
-// outputs, centroid and AABB (min xyz, max xyz of the centred points) returned to the host.
-// h_pos3 (optional): the same points in host memory.  The centroid is an ORDER-DEPENDENT serial fp32
-// sum (src/stocs.cpp:945-956), i.e. three dependent add chains of length n: one SM needs 5.5 ms for
-// 2^20 points, a host core ~1.3 ms, and the host runs it while the H2D copy of the points is still in
-// flight.  Without host data the single-CTA kernel does the same sum on the device.
+// The centroid is an ORDER-DEPENDENT serial fp32 sum (src/stocs.cpp:945-956), i.e. three dependent add
+// chains of length n: one SM needs 5.5 ms for 2^20 points, a host core ~1.3 ms.  Points in host memory
+// are summed on the host while their H2D copy is in flight; points in device memory by the single-CTA
+// centroid_seq_kernel.
 // The reference kd-tree serves one purpose on the device: resolving EXACT distance ties in the scoring
-// kernel.  Nothing before the first scoring launch needs it, so upload_scene starts its build (host
-// work on the centred points, ~0.3 ms for a 13 000-point frame) on a host thread and returns once the
-// grid index is complete; the first scoring launch -- in the online pipeline that is after base
-// sampling, congruent sets and fits have been enqueued -- joins the thread and queues the upload in
-// front of its kernel (stocs_kd_finish).  A new scene or the context's destruction joins it too.
+// kernel.  Nothing before the first scoring launch needs it, so upload_scene starts its build and returns
+// once the grid index is complete; the first scoring launch -- in the online pipeline that is after base
+// sampling, congruent sets and fits have been enqueued -- joins it (stocs_kd_finish).  A scene from host
+// memory is built by a host thread on the host's centred copy (~0.3 ms for a 13 000-point frame), which
+// the first scoring launch joins before it queues the upload in front of its kernel.  A scene from device
+// memory is built by kd_build_enqueue on the context's copy stream, beside the index build; the first
+// scoring launch waits for it through kd_copy_done.  A new scene or the context's destruction joins it too.
 struct KdPending {
   std::thread th;
   KdBuild kb;
@@ -332,6 +530,7 @@ struct KdPending {
   float4* pts = nullptr;                 // leaf-ordered points {x, y, z, bits(index)}: page-locked staging or `pageable`
   std::vector<float4> pageable;
   bool failed = false;
+  bool on_device = false;                // built by kd_build_enqueue into d_kd_nodes / d_kd_pts; kd_copy_done follows it
 };
 
 extern "C" int stocs_b200_host_kdtree_order(const float* pos3, int n, int32_t* leaf_order, int32_t* n_nodes) {
@@ -343,12 +542,65 @@ extern "C" int stocs_b200_host_kdtree_order(const float* pos3, int n, int32_t* l
   return STOCS_OK;
 }
 
+extern "C" int stocs_b200_debug_kdtree(stocs_b200_ctx* ctx, const float* pos3, int n, int on_device, int32_t* leaf_order,
+                                       int32_t* n_nodes, int32_t* nodes_out) {
+  if (!ctx) return STOCS_E_ARG;
+  if (!pos3 || n <= 0 || !leaf_order) STOCS_FAIL(ctx, STOCS_E_ARG, "debug_kdtree: bad argument");
+  std::vector<float4> pts((size_t)n);
+  std::vector<KdNodeDev> nodes;
+  if (on_device) {
+    cudaSetDevice(ctx->device);
+    cudaStream_t st = ctx->stream;
+    for (int i = 0; i < n; ++i) { float w; memcpy(&w, &i, 4); pts[i] = make_float4(pos3[3 * (size_t)i], pos3[3 * (size_t)i + 1], pos3[3 * (size_t)i + 2], w); }
+    DevBuf d_pts, d_nodes, d_scratch;   // the context's own tree stays untouched
+    struct Release { DevBuf* b[3]; ~Release() { for (DevBuf* x : b) x->release(); } } rel{{&d_pts, &d_nodes, &d_scratch}};
+    STOCS_CUDA(ctx, d_pts.ensure((size_t)n * 16));
+    STOCS_CUDA(ctx, d_nodes.ensure(((size_t)n + 3) * sizeof(KdNodeDev)));
+    STOCS_CUDA(ctx, d_scratch.ensure(kd_scratch_bytes(n)));
+    STOCS_CUDA(ctx, cudaMemcpyAsync(d_pts.p, pts.data(), (size_t)n * 16, cudaMemcpyHostToDevice, st));
+    STOCS_CUDA(ctx, kd_build_enqueue(d_pts.as<float4>(), d_nodes.as<KdNodeDev>(), d_scratch.p, n, st));
+    int used = 0;
+    STOCS_CUDA(ctx, cudaMemcpyAsync(&used, d_scratch.p, 4, cudaMemcpyDeviceToHost, st));
+    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
+    nodes.resize((size_t)used);
+    STOCS_CUDA(ctx, cudaMemcpyAsync(nodes.data(), d_nodes.p, (size_t)used * sizeof(KdNodeDev), cudaMemcpyDeviceToHost, st));
+    STOCS_CUDA(ctx, cudaMemcpyAsync(pts.data(), d_pts.p, (size_t)n * 16, cudaMemcpyDeviceToHost, st));
+    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
+    for (int i = 0; i < n; ++i) memcpy(&leaf_order[i], &pts[i].w, 4);
+  } else {
+    KdBuild kb;
+    kb.build(pos3, n);
+    for (int i = 0; i < n; ++i) leaf_order[i] = kb.idx[i];
+    nodes = kb.nodes;
+  }
+  if (n_nodes) *n_nodes = (int32_t)nodes.size();
+  if (nodes_out) {   // pre-order from the root, first child before second: independent of the node numbering
+    std::vector<uint32_t> todo{0u};
+    size_t k = 0;
+    while (!todo.empty()) {
+      const KdNodeDev nd = nodes[todo.back()];
+      todo.pop_back();
+      int32_t split;
+      memcpy(&split, &nd.split, 4);
+      nodes_out[3 * k] = (int32_t)nd.leaf; nodes_out[3 * k + 1] = split; nodes_out[3 * k + 2] = (int32_t)nd.dim_or_size;
+      ++k;
+      if (!nd.leaf) { todo.push_back(nd.first_or_start + 1); todo.push_back(nd.first_or_start); }
+    }
+  }
+  return STOCS_OK;
+}
+
 int stocs_kd_finish(stocs_b200_ctx* ctx, cudaStream_t st, bool upload) {
   KdPending* kp = ctx->kd_pending;
   if (!kp) return STOCS_OK;
   if (kp->th.joinable()) kp->th.join();
   ctx->kd_pending = nullptr;
   struct Deleter { KdPending* p; ~Deleter() { delete p; } } del{kp};
+  if (kp->on_device) {   // whatever next reads or rewrites the tree on these streams comes after the build
+    for (cudaStream_t s : {st, ctx->stream, ctx->aux_stream})
+      if (s) STOCS_CUDA(ctx, cudaStreamWaitEvent(s, ctx->kd_copy_done, 0));
+    return STOCS_OK;
+  }
   if (!upload) return STOCS_OK;
   if (kp->failed) STOCS_FAIL(ctx, STOCS_E_CUDA, "upload_scene: kd-tree construction failed (out of host memory)");
   const size_t node_bytes = kp->kb.nodes.size() * sizeof(KdNodeDev), pts_bytes = (size_t)kp->S * 16;
@@ -407,6 +659,24 @@ static int kd_start(stocs_b200_ctx* ctx, int S) {
   return STOCS_OK;
 }
 
+// Device build of the kd-tree over the S centred points in d_spos4, on the copy stream; kd_copy_done marks
+// its end (the buffers are grown by stocs_index_plan).  It needs no event from the context stream:
+// stocs_index_plan_finish synchronised that stream after the centring, before anything that reads d_spos4 or
+// the old tree could still be queued there.
+static int kd_start_device(stocs_b200_ctx* ctx, int S) {
+  KdPending* kp = new (std::nothrow) KdPending();
+  if (!kp) STOCS_FAIL(ctx, STOCS_E_CUDA, "upload_scene: out of host memory");
+  kp->S = S;
+  kp->on_device = true;
+  ctx->kd_pending = kp;
+  cudaStream_t side = ctx->copy_stream;
+  if (!ctx->kd_copy_done) STOCS_CUDA(ctx, cudaEventCreateWithFlags(&ctx->kd_copy_done, cudaEventDisableTiming));
+  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->d_kd_pts.p, ctx->d_spos4.p, (size_t)S * 16, cudaMemcpyDeviceToDevice, side));
+  STOCS_CUDA(ctx, kd_build_enqueue(ctx->d_kd_pts.as<float4>(), ctx->d_kd_nodes.as<KdNodeDev>(), ctx->d_kd_build.p, S, side));
+  STOCS_CUDA(ctx, cudaEventRecord(ctx->kd_copy_done, side));
+  return STOCS_OK;
+}
+
 // Reference centroid of n host points into ctx->h_centroid_stage, their centred copy and bounding box
 // (min xyz, max xyz; min x NaN when a coordinate is not finite).
 static void host_centre(stocs_b200_ctx* ctx, const float* h_pos3, int n, float* h_centred3, float* h_aabb6) {
@@ -432,33 +702,16 @@ static void host_centre(stocs_b200_ctx* ctx, const float* h_pos3, int n, float* 
   if (h_aabb6) for (int k = 0; k < 3; ++k) { h_aabb6[k] = mn[k]; h_aabb6[3 + k] = mx[k]; }
 }
 
-int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4* d_out4,
-                        float* d_out3, float* h_centroid3, float* h_aabb6, const float* h_pos3, float* h_centred3) {
+int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4* d_out4, float* h_centroid3,
+                        const float* h_pos3, float* h_centred3) {
   cudaStream_t st = ctx->stream;
-  float* d_c = ctx->scratch()->centroid;
-  int* d_aabb = ctx->scratch()->aabb;
-  if (h_pos3) {
-    host_centre(ctx, h_pos3, n, h_centred3, h_aabb6);
-    STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, ctx->h_centroid_stage, 12, cudaMemcpyHostToDevice, st));
-    if (h_centred3) {   // the device centres its own copy concurrently; nothing is read back, no synchronisation
-      centre_pack_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_pos3, n, d_c, d_out4, d_out3, nullptr);
-      STOCS_CUDA(ctx, cudaGetLastError());
-      for (int k = 0; k < 3; ++k) h_centroid3[k] = ctx->h_centroid_stage[k];
-      return STOCS_OK;
-    }
-  } else {
-    centroid_seq_kernel<<<1, 256, 0, st>>>(d_pos3, n, d_c);
-  }
-  int init[6] = {INT_MAX, INT_MAX, INT_MAX, INT_MIN, INT_MIN, INT_MIN};
-  STOCS_CUDA(ctx, cudaMemcpyAsync(d_aabb, init, sizeof(init), cudaMemcpyHostToDevice, st));
-  centre_pack_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_pos3, n, d_c, d_out4, d_out3, d_aabb);
+  float* d_c = ctx->scratch()->plan.centroid;
+  host_centre(ctx, h_pos3, n, h_centred3, nullptr);
+  STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, ctx->h_centroid_stage, 12, cudaMemcpyHostToDevice, st));
+  // the device centres its own copy concurrently; nothing is read back, no synchronisation
+  centre_pack_kernel<<<(n + 255) / 256, 256, 0, st>>>(d_pos3, n, d_c, d_out4, nullptr, nullptr);
   STOCS_CUDA(ctx, cudaGetLastError());
-  int haabb[6];
-  STOCS_CUDA(ctx, cudaMemcpyAsync(h_centroid3, d_c, 12, cudaMemcpyDeviceToHost, st));
-  STOCS_CUDA(ctx, cudaMemcpyAsync(haabb, d_aabb, 24, cudaMemcpyDeviceToHost, st));
-  STOCS_CUDA(ctx, cudaStreamSynchronize(st));
-  if (h_aabb6)
-    for (int k = 0; k < 6; ++k) h_aabb6[k] = ord2f(haabb[k]);
+  for (int k = 0; k < 3; ++k) h_centroid3[k] = ctx->h_centroid_stage[k];
   return STOCS_OK;
 }
 
@@ -529,43 +782,87 @@ int stocs_index_complete(stocs_b200_ctx* ctx) {
   return STOCS_OK;
 }
 
-// First step of an index build, before any of it is enqueued: centre the points, start the kd-tree
-// thread, lay out the grid and grow every buffer the build uses, so that no allocation happens between
-// the kernels of several objects' uploads.  The centring runs on the host from ctx->h_pos_pending; without
-// it (STOCS_DEVICE_CENTROID) the positions are already in ctx->d_tmp and this waits for the device kernels.
+static int index_layout(stocs_b200_ctx* ctx, const float* aabb);
+
+// First step of an index build, before any of it is enqueued: grow every buffer the build uses, so that no
+// allocation happens between the kernels of several objects' uploads.  With ctx->h_pos_pending (a scene in
+// host memory) this also centres the points on the host, starts the kd-tree thread and lays out the grid.
+// Without it the centring is device work that stocs_index_centre_device enqueues, and stocs_index_plan_finish
+// lays out the grid from what the device reports.
 int stocs_index_plan(stocs_b200_ctx* ctx) {
   const int S = ctx->S_pending;   // committed to ctx->S by upload_scene once the index is complete
-  cudaStream_t st = ctx->stream;
-  StageTrace tr(st);
+  StageTrace tr(ctx->stream);
   STOCS_CUDA(ctx, ctx->d_spos4.ensure((size_t)S * 16));
-  STOCS_CUDA(ctx, ctx->d_tmp2.ensure((size_t)S * 12));
-  // the kd-tree upload of the first scoring launch (stocs_kd_finish): S points, and at most S + 3 nodes
+  // the kd-tree of the first scoring launch (stocs_kd_finish): S points, and at most S + 3 nodes
   // (every inner node below the root holds more than 64 points, at most S / 65 of them on each of <= 31 levels)
   STOCS_CUDA(ctx, ctx->d_kd_pts.ensure((size_t)S * 16));
   STOCS_CUDA(ctx, ctx->d_kd_nodes.ensure(((size_t)S + 3) * sizeof(KdNodeDev)));
+  if (!ctx->h_pos_pending) {
+    STOCS_CUDA(ctx, ctx->d_kd_build.ensure(kd_scratch_bytes(S)));
+    ctx->plan_on_device = true;
+    return STOCS_OK;
+  }
   float aabb[6];
   ctx->h_spos.resize((size_t)S * 3);
-  if (ctx->h_pos_pending) {
-    host_centre(ctx, ctx->h_pos_pending, S, ctx->h_spos.data(), aabb);
-    memcpy(ctx->cs, ctx->h_centroid_stage, 12);
-  } else {   // device-only path: centred points and box come back from the kernels
-    int rc = stocs_centre_points(ctx, ctx->d_tmp.as<float>(), S, ctx->d_spos4.as<float4>(), ctx->d_tmp2.as<float>(), ctx->cs,
-                                 aabb);
-    if (rc) return rc;
-    STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_spos.data(), ctx->d_tmp2.p, (size_t)S * 12, cudaMemcpyDeviceToHost, st));
-    STOCS_CUDA(ctx, cudaStreamSynchronize(st));
-  }
-  tr.mark("centre + copy back");
+  host_centre(ctx, ctx->h_pos_pending, S, ctx->h_spos.data(), aabb);
+  memcpy(ctx->cs, ctx->h_centroid_stage, 12);
+  tr.mark("centre");
+  return index_layout(ctx, aabb);
+}
+
+// Device half of the plan of a scene in device memory (on the context's device): the reference centroid,
+// the centred points into d_spos4 with their box, the class-weight bound and the pixel range (d_pix may be
+// NULL), reduced into one ScenePlan record and copied to ctx->h_plan; no synchronisation.
+int stocs_index_centre_device(stocs_b200_ctx* ctx, const float* d_pos3, const float* d_cls, const int32_t* d_pix) {
+  const int S = ctx->S_pending;
+  cudaStream_t st = ctx->stream;
+  ScenePlan* p = &ctx->scratch()->plan;
+  const unsigned nb = (unsigned)((S + 255) / 256);
+  plan_init_kernel<<<1, 32, 0, st>>>(p);
+  centroid_seq_kernel<<<1, 256, 0, st>>>(d_pos3, S, p->centroid);
+  centre_pack_kernel<<<nb, 256, 0, st>>>(d_pos3, S, p->centroid, ctx->d_spos4.as<float4>(), nullptr, p->aabb);
+  plan_bounds_kernel<<<nb, 256, 0, st>>>(d_cls, d_pix, S, p);
+  plan_weight_max_kernel<<<nb, 256, 0, st>>>(d_cls, S, p);
+  STOCS_CUDA(ctx, cudaGetLastError());
+  STOCS_CUDA(ctx, cudaMemcpyAsync(ctx->h_plan, p, sizeof(ScenePlan), cudaMemcpyDeviceToHost, st));
+  return STOCS_OK;
+}
+
+// Waits for the record of stocs_index_centre_device and takes from it what the host needs: centroid,
+// class-weight bound (stocs_set_weight_bound's semantics), pixel range (0 without pixels) and the box the
+// grid is laid out over.  No-op for a scene planned on the host.
+int stocs_index_plan_finish(stocs_b200_ctx* ctx) {
+  if (!ctx->plan_on_device) return STOCS_OK;
+  ctx->plan_on_device = false;
+  STOCS_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  const ScenePlan& p = *ctx->h_plan;
+  memcpy(ctx->cs, p.centroid, 12);
+  memcpy(&ctx->w_max, &p.wbits, 4);
+  ctx->prune_ok = p.first_bad == INT_MAX;
+  const bool pix = p.pix_min[0] <= p.pix_max[0];
+  for (int k = 0; k < 2; ++k) { ctx->pix_min[k] = pix ? p.pix_min[k] : 0; ctx->pix_max[k] = pix ? p.pix_max[k] : 0; }
+  float aabb[6];
+  for (int k = 0; k < 6; ++k) aabb[k] = ord2f(p.aabb[k]);
+  return index_layout(ctx, aabb);
+}
+
+// The rest of the plan, from the box of the centred points (min xyz, max xyz): lay out the grid and grow its
+// buffers; the host path also starts the kd-tree thread here.
+static int index_layout(stocs_b200_ctx* ctx, const float* aabb) {
+  const int S = ctx->S_pending;
+  cudaStream_t st = ctx->stream;
   float mn[3] = {aabb[0], aabb[1], aabb[2]}, mx[3] = {aabb[3], aabb[4], aabb[5]};
   for (int k = 0; k < 3; ++k)
     if (!(mn[k] <= mx[k]) || !std::isfinite(mn[k]) || !std::isfinite(mx[k]))
       STOCS_FAIL(ctx, STOCS_E_ARG, "upload_scene: scene contains non-finite coordinates");
   int rc = STOCS_OK;
 
-  // the reference kd-tree (exact-tie resolution in the scoring kernel): host work on the centred
-  // points, started here on a host thread and collected by the first scoring launch
-  rc = kd_start(ctx, S);
-  if (rc) return rc;
+  // the reference kd-tree (exact-tie resolution in the scoring kernel) of a scene in host memory: host
+  // work on the centred points, started here on a host thread and collected by the first scoring launch
+  if (ctx->h_pos_pending) {
+    rc = kd_start(ctx, S);
+    if (rc) return rc;
+  }
 
   // grid geometry.  Cell edge in units of eps, measured on B200 with the S1 workload (10^6
   // hypotheses, all bit-identical): 2.0 -> 4.3 ms, 1.0 -> 2.93 ms, 0.6 -> 2.73 ms, 0.5 -> 2.64 ms,
@@ -672,18 +969,22 @@ int stocs_index_plan(stocs_b200_ctx* ctx) {
   return STOCS_OK;
 }
 
-// Second step: the device centring (host path: the centroid the plan computed; positions in ctx->d_tmp)
-// and one pass of the index kernels, ending in the two length copies; no synchronisation.
+// Second step: the device centring of a host scene (the centroid the plan computed; positions in ctx->d_tmp),
+// or the device kd-tree build of a device scene (centred by stocs_index_centre_device), and one pass of the
+// index kernels, ending in the two length copies; no synchronisation.
 int stocs_index_enqueue(stocs_b200_ctx* ctx) {
+  const int S = ctx->S_pending;
   if (ctx->h_pos_pending) {
     cudaStream_t st = ctx->stream;
-    const int S = ctx->S_pending;
-    float* d_c = ctx->scratch()->centroid;
+    float* d_c = ctx->scratch()->plan.centroid;
     STOCS_CUDA(ctx, cudaMemcpyAsync(d_c, ctx->h_centroid_stage, 12, cudaMemcpyHostToDevice, st));
     centre_pack_kernel<<<(S + 255) / 256, 256, 0, st>>>(ctx->d_tmp.as<float>(), S, d_c, ctx->d_spos4.as<float4>(), nullptr, nullptr);
     STOCS_CUDA(ctx, cudaGetLastError());
+    return index_enqueue_attempt(ctx);
   }
-  return index_enqueue_attempt(ctx);
+  // the index kernels first: the kd-tree's launches are enqueued while they run
+  const int rc = index_enqueue_attempt(ctx);
+  return rc ? rc : kd_start_device(ctx, S);
 }
 
 // used by upload_scene in capi.cu (ctx->d_sattr holds S records)

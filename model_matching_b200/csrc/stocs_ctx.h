@@ -153,6 +153,17 @@ enum CtxCounter : int {
 
 struct DevScratch;
 
+// What the device tells the host about a scene in device memory before its index is laid out
+// (stocs_index_centre_device): one 64-byte record, reduced in DevScratch::plan and copied to ctx->h_plan.
+struct ScenePlan {
+  float centroid[4];
+  int aabb[6];                  // box of the centred points as ordered ints (min xyz, max xyz)
+  int wbits;                    // bits of the largest class weight before first_bad
+  int first_bad;                // first class weight that is negative, NaN or infinite; INT_MAX: none
+  int pix_min[2], pix_max[2];   // (row, col) range; min > max: no pixel coordinates
+};
+static_assert(sizeof(ScenePlan) == 64, "ScenePlan is one 64-byte read-back");
+
 struct stocs_b200_ctx {
   int device = 0;
   int num_sms = 0;
@@ -191,7 +202,8 @@ struct stocs_b200_ctx {
   IndexBuild index_build{};            // the index build in flight (stocs_index_enqueue -> stocs_index_complete)
   float h_centroid_stage[4] = {0, 0, 0, 0};  // source of the 12-byte centroid upload (must outlive the async copy)
   float cs[3] = {0, 0, 0};
-  std::vector<float> h_spos;           // centred positions (S*3)
+  std::vector<float> h_spos;           // centred positions (S*3) of a scene from host memory: the kd-tree thread's input
+  bool plan_on_device = false;         // the scene is planned on the device (between stocs_index_plan and _finish)
   DevBuf d_spos4;                      // float4 (x,y,z,bits(idx))
   DevBuf d_sattr;                      // float4 (nx,ny,nz,class probability)
   DevBuf d_spix;                       // int2 (row, col)
@@ -211,6 +223,7 @@ struct stocs_b200_ctx {
   DevBuf d_cand;                       // float4 (x,y,z,bits(idx)) replicated per dilated cell
   int64_t ncand = 0;
   DevBuf d_kd_nodes, d_kd_pts;         // reference kd-tree for exact-tie resolution
+  DevBuf d_kd_build;                   // scratch of its device build (in use until kd_copy_done, across calls)
   int kd_nodes = 0;
 
   // PPF table
@@ -243,10 +256,9 @@ struct stocs_b200_ctx {
   size_t index_counts_clean = 0;            // leading words of pool[POOL_INDEX_COUNTS] known to be zero
   void* h_kd_stage = nullptr;               // page-locked staging of the kd-tree upload (frame-sized scenes)
   size_t h_kd_stage_bytes = 0;
-  void* h_scene_stage = nullptr;            // page-locked: positions | class weights | pixels of an upload_scenes_device slice
-  size_t h_scene_stage_bytes = 0;
-  struct KdPending* kd_pending = nullptr;   // kd-tree of the current scene, still being built on a host thread
-  cudaEvent_t kd_copy_done = nullptr;       // the staging buffer may be overwritten once this has completed
+  ScenePlan* h_plan = nullptr;              // page-locked landing zone of a device plan's record
+  struct KdPending* kd_pending = nullptr;   // kd-tree of the current scene, still being built (host thread or device)
+  cudaEvent_t kd_copy_done = nullptr;       // the staging buffer may be overwritten / the device build is complete
 
   // resident lcp array (d_lcp / d_inl) of the last host-buffer score call or explicit reduce_best
   int64_t last_H = 0;
@@ -284,9 +296,8 @@ struct DevScratch {
   unsigned lpt_fill[2];
   // score.cu (stocs_fmad_selftest): written after the creation memset, so shared with no other field
   float fmad_selftest;
-  // scene_index.cu (stocs_centre_points): centroid, and the bounding box as ordered ints (min xyz, max xyz)
-  float centroid[4];
-  int aabb[6];
+  // scene_index.cu: centroid of stocs_centre_points; the device plan of a scene (stocs_index_centre_device)
+  ScenePlan plan;
   // ppf_table.cu: occupied keys of the table build, entries of a lookup, entries an upload rejected
   unsigned long long ppf_nkeys;
   long long ppf_lookup_n;
@@ -317,16 +328,21 @@ static_assert(sizeof(DevScratch) <= 4096, "DevScratch must fit the 4 KB d_small 
   do { (ctx)->err = (msg); return (code); } while (0)
 
 // kernels / stages implemented in the other translation units
-// scene index of ctx->S_pending points (scene_index.cu), in three steps: plan (centre, start the kd-tree
-// thread, lay out the grid, grow every buffer; nothing enqueued), enqueue (device centring of the positions
-// in ctx->d_tmp, the index kernels and their two length copies), complete (wait, grow and run again if the
-// candidate records did not fit, commit the counters)
+// scene index of ctx->S_pending points (scene_index.cu), in three steps: plan (grow every buffer; for a scene
+// in host memory also centre on the host, start the kd-tree thread and lay out the grid; nothing enqueued),
+// enqueue (device centring of host positions in ctx->d_tmp or the device kd-tree build, the index kernels and
+// their two length copies), complete (wait, grow and run again if the candidate records did not fit, commit
+// the counters).  A scene in device memory is planned between the first two: centre_device enqueues the
+// centring and the plan record's copy, plan_finish waits for it and lays out the grid.
 int stocs_index_plan(stocs_b200_ctx* ctx);
+int stocs_index_centre_device(stocs_b200_ctx* ctx, const float* d_pos3, const float* d_cls, const int32_t* d_pix);
+int stocs_index_plan_finish(stocs_b200_ctx* ctx);
 int stocs_index_enqueue(stocs_b200_ctx* ctx);
 int stocs_index_complete(stocs_b200_ctx* ctx);
-int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4* d_out4,
-                        float* d_out3, float* h_centroid3, float* h_aabb6, const float* h_pos3 = nullptr,
-                        float* h_centred3 = nullptr);
+// reference centroid of n host points (h_pos3) into h_centroid3, their centred copy into h_centred3, and the
+// same centring on the device of their copy d_pos3 into d_out4 (enqueued, no synchronisation)
+int stocs_centre_points(stocs_b200_ctx* ctx, const float* d_pos3, int n, float4* d_out4, float* h_centroid3,
+                        const float* h_pos3, float* h_centred3);
 int stocs_pack_scene_attr(stocs_b200_ctx* ctx, const float* d_nrm3, const float* d_cls, int S);
 // One scoring launch (score.cu).  The caller states which instantiation it wants: per-hypothesis
 // results (the default), only the K best (top_K = K: hypotheses that provably cannot enter them may
