@@ -437,7 +437,9 @@ int stocs_b200_group_score_best(stocs_b200_group* g, const float* T16, int64_t H
  * over the lifetime of the context; [2] grid cells and [3] replicated candidate records of the
  * current scene index; [4] / [5] hypotheses the device top-K path (score_sharded_device,
  * group_score_best without per-hypothesis outputs) left unscored because they provably cannot
- * enter the top K, rejected after the coarse test / before a queue drain, accumulated over the
+ * enter the top K, rejected on the prefilter count (a launch of more than 300 000 hypotheses: the
+ * survivor count on the fine occupancy map; otherwise loop 1's coarse count) / before a queue drain,
+ * accumulated over the
  * lifetime of the context; [6] and [7] are internal; [8] hypotheses of the same path rejected
  * after the brick-bit refinement of the coarse survivors, which runs between the two, accumulated
  * likewise. */
@@ -457,6 +459,13 @@ int stocs_b200_score_counters(stocs_b200_ctx* ctx, const float* d_T16, int64_t H
  * multiple of 32), or |M| for a transform whose grid map is not finite or too large to evaluate
  * without overflow.  counts: H host int32. */
 int stocs_b200_debug_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts);
+/* Test hook: the count a top-K launch of more than 300 000 hypotheses actually orders and stops its claims
+ * by: the same test on the scene's fine occupancy map (blocks of 2^fine_shift cells per axis, at most
+ * the coarse map's 2^coarse_shift).  For a transform whose grid map is below the overflow limit at both
+ * scales it is at most the coarse count and at least the transform's inlier count.  fine_shift (optional):
+ * 2 host int32, {fine_shift, coarse_shift} of the current scene. */
+int stocs_b200_debug_fine_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts,
+                                          int32_t* fine_shift);
 /* name + average duration (ms, CUDA events on the context stream) of the dominant kernel of the
  * most recent score call; used by bench.py for the roofline line. */
 int stocs_b200_last_kernel_ms(stocs_b200_ctx* ctx, float* ms);

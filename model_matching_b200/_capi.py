@@ -31,7 +31,7 @@ SYMBOLS = [
     "stocs_b200_run_pipeline_clustered", "stocs_b200_run_pipeline_instance_clustered",
     "stocs_b200_upload_scenes", "stocs_b200_upload_scenes_device", "stocs_b200_run_pipelines", "stocs_b200_get_counters", "stocs_b200_last_kernel_ms",
     "stocs_b200_score_counters", "stocs_b200_kernel_ms_stats", "stocs_b200_host_kdtree_order", "stocs_b200_debug_kdtree",
-    "stocs_b200_debug_angle_estimates", "stocs_b200_debug_survivor_counts",
+    "stocs_b200_debug_angle_estimates", "stocs_b200_debug_survivor_counts", "stocs_b200_debug_fine_survivor_counts",
     "stocs_b200_comm_unique_id", "stocs_b200_comm_init", "stocs_b200_comm_destroy", "stocs_b200_shard_range",
     "stocs_b200_score_sharded_device", "stocs_b200_score_sharded",
     "stocs_b200_group_create", "stocs_b200_group_destroy", "stocs_b200_group_size", "stocs_b200_group_ctx",
@@ -127,6 +127,7 @@ def lib():
     L.stocs_b200_debug_kdtree.argtypes = [vp, vp, i32, i32, vp, C.POINTER(i32), vp]
     L.stocs_b200_debug_angle_estimates.argtypes = [vp, vp, vp, i64, vp, vp, vp, vp, vp, vp]
     L.stocs_b200_debug_survivor_counts.argtypes = [vp, vp, i64, vp]
+    L.stocs_b200_debug_fine_survivor_counts.argtypes = [vp, vp, i64, vp, vp]
     L.stocs_b200_comm_unique_id.argtypes = [vp]
     L.stocs_b200_comm_init.argtypes = [vp, vp, i32, i32]
     L.stocs_b200_comm_destroy.argtypes = [vp]
@@ -716,12 +717,17 @@ class Context:
                                                              _ptr(pf), _ptr(bf), _ptr(bp)))
         return {"est": est, "pinned": pin, "fast_floor": ff, "pinned_floor": pf, "below30_fast": bf, "below30_pinned": bp}
 
-    def debug_survivor_counts(self, dT_ptr, H):
-        """coarse-survivor count of each of H device transforms, as the top-K path orders its claims by it
-        (test hook, see include/stocs_b200.h) -> int32 array"""
+    def debug_survivor_counts(self, dT_ptr, H, fine=False):
+        """survivor count of each of H device transforms (test hook, see include/stocs_b200.h) -> int32
+        array: loop 1's count on the coarse map, or with fine=True the count on the fine map that a large
+        top-K launch orders and stops its claims by, returned with (fine_shift, coarse_shift)"""
         ns = np.empty(H, np.int32)
-        self._check(self._L.stocs_b200_debug_survivor_counts(self.h, dT_ptr, H, _ptr(ns)))
-        return ns
+        if not fine:
+            self._check(self._L.stocs_b200_debug_survivor_counts(self.h, dT_ptr, H, _ptr(ns)))
+            return ns
+        shifts = np.zeros(2, np.int32)
+        self._check(self._L.stocs_b200_debug_fine_survivor_counts(self.h, dT_ptr, H, _ptr(ns), _ptr(shifts)))
+        return ns, (int(shifts[0]), int(shifts[1]))
 
     def debug_kdtree(self, pos, on_device):
         """the reference kd-tree over pos as built on the device (on_device) or on the host (test hook, see

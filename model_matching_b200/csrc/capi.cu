@@ -237,7 +237,7 @@ void stocs_b200_destroy(stocs_b200_ctx* ctx) {
   if (ctx->stream) cudaStreamSynchronize(ctx->stream);
   stocs_b200_comm_destroy(ctx);
   DevBuf* bufs[] = {&ctx->d_model, &ctx->d_mpos4, &ctx->d_mnrm4, &ctx->d_spos4, &ctx->d_sattr, &ctx->d_spix,
-                    &ctx->d_coarse, &ctx->d_brick_occ, &ctx->d_bricks, &ctx->d_cell_start, &ctx->d_cand, &ctx->d_kd_nodes, &ctx->d_kd_pts, &ctx->d_kd_build, &ctx->d_ppf_bin_start,
+                    &ctx->d_coarse, &ctx->d_fine, &ctx->d_brick_occ, &ctx->d_bricks, &ctx->d_cell_start, &ctx->d_cand, &ctx->d_kd_nodes, &ctx->d_kd_pts, &ctx->d_kd_build, &ctx->d_ppf_bin_start,
                     &ctx->d_ppf_pairs, &ctx->d_ppf_keybits, &ctx->d_T, &ctx->d_lcp, &ctx->d_inl, &ctx->d_work,
                     &ctx->d_tmp, &ctx->d_tmp2, &ctx->d_small, &ctx->d_edge, &ctx->d_inst_state, &ctx->d_mask_store,
                     &ctx->d_frontier};
@@ -747,7 +747,7 @@ int stocs_b200_score_counters(stocs_b200_ctx* ctx, const float* d_T16, int64_t H
   return STOCS_OK;
 }
 
-int stocs_b200_debug_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts) {
+static int debug_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts, bool fine) {
   if (!ctx) return STOCS_E_ARG;
   if (ctx->S <= 0 || ctx->M <= 0) STOCS_FAIL(ctx, STOCS_E_STATE, "survivor_counts: upload_model and upload_scene first");
   if (H <= 0 || H >= (1ll << 31) || !d_T16 || !counts) STOCS_FAIL(ctx, STOCS_E_ARG, "survivor_counts: bad argument");
@@ -755,11 +755,22 @@ int stocs_b200_debug_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, in
   cudaStream_t st = ctx->stream;
   DevBuf& d_ns = ctx->pool[POOL_SCORE_NS];
   STOCS_CUDA(ctx, d_ns.ensure((size_t)H * 4));
-  int rc = stocs_survivor_counts(ctx, d_T16, H, d_ns.as<unsigned>(), st);
+  int rc = stocs_survivor_counts(ctx, d_T16, H, d_ns.as<unsigned>(), st, fine);
   if (rc) return rc;
   STOCS_CUDA(ctx, cudaMemcpyAsync(counts, d_ns.p, (size_t)H * 4, cudaMemcpyDeviceToHost, st));
   STOCS_CUDA(ctx, cudaStreamSynchronize(st));
   return STOCS_OK;
+}
+
+int stocs_b200_debug_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts) {
+  return debug_survivor_counts(ctx, d_T16, H, counts, false);
+}
+
+int stocs_b200_debug_fine_survivor_counts(stocs_b200_ctx* ctx, const float* d_T16, int64_t H, int32_t* counts,
+                                          int32_t* fine_shift) {
+  const int rc = debug_survivor_counts(ctx, d_T16, H, counts, true);
+  if (rc == STOCS_OK && fine_shift) fine_shift[0] = ctx->fine_shift, fine_shift[1] = ctx->coarse_shift;
+  return rc;
 }
 
 int stocs_b200_kernel_ms_stats(stocs_b200_ctx* ctx, int reset, int32_t* n_launches, float* mean_ms, float* max_ms) {

@@ -401,7 +401,8 @@ __global__ void brick_table_kernel(const uint32_t* __restrict__ cell_start, cons
                                    const uint32_t* __restrict__ occ_scan, uint32_t nbricks,
                                    const uint32_t* __restrict__ total_cand, uint32_t starts_cap,
                                    uint4* __restrict__ bricks, uint32_t* __restrict__ starts,
-                                   uint32_t* __restrict__ coarse, GridDesc g, int cshift, int csx, int csy) {
+                                   uint32_t* __restrict__ coarse, GridDesc g, int cshift, int csx, int csy,
+                                   uint32_t* __restrict__ fine, int fshift, int fsx, int fsy) {
   const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= nbricks) return;
   const unsigned long long m = masks[b];
@@ -410,6 +411,11 @@ __global__ void brick_table_kernel(const uint32_t* __restrict__ cell_start, cons
     const int s = cshift - 2;
     const uint32_t cidx = (uint32_t)(((bz >> s) * csy + (by >> s)) * csx + (bx >> s));  // strides = blocks + 1
     atomicOr(&coarse[cidx >> 5], 1u << (cidx & 31));
+    if (fine) {  // and the fine block (2^fshift cells per axis, 2 <= fshift < cshift)
+      const int f = fshift - 2;
+      const uint32_t fidx = (uint32_t)(((bz >> f) * fsy + (by >> f)) * fsx + (bx >> f));
+      atomicOr(&fine[fidx >> 5], 1u << (fidx & 31));
+    }
   }
   const uint32_t base = occ_scan[b];
   bricks[b] = make_uint4((uint32_t)m, (uint32_t)(m >> 32), base, 0u);
@@ -748,10 +754,13 @@ static int index_enqueue_attempt(stocs_b200_ctx* ctx) {
   cub::DeviceScan::ExclusiveSum(ctx->d_tmp2.p, tmp_bytes2, d_occ.as<uint32_t>(), d_occ_scan.as<uint32_t>(), (int)(g.nbricks + 1), st);
   STOCS_CUDA(ctx, cudaMemcpyAsync(&h_counts[1], d_occ_scan.as<uint32_t>() + g.nbricks, 4, cudaMemcpyDeviceToHost, st));
   STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_coarse.p, 0, (size_t)ctx->coarse_words * 4, st));
+  const bool two_maps = ctx->fine_shift < ctx->coarse_shift;
+  if (two_maps) STOCS_CUDA(ctx, cudaMemsetAsync(ctx->d_fine.p, 0, (size_t)ctx->fine_words * 4, st));
   brick_table_kernel<<<bb, 128, 0, st>>>(dense_start, d_masks.as<unsigned long long>(), d_occ_scan.as<uint32_t>(), g.nbricks,
                                          dense_start + g.ncells, (uint32_t)starts_cap, ctx->d_bricks.as<uint4>(),
                                          ctx->d_cell_start.as<uint32_t>(), ctx->d_coarse.as<uint32_t>(), g, ctx->coarse_shift,
-                                         ctx->coarse_nx + 1, ctx->coarse_ny + 1);
+                                         ctx->coarse_nx + 1, ctx->coarse_ny + 1, two_maps ? ctx->d_fine.as<uint32_t>() : nullptr,
+                                         ctx->fine_shift, ctx->fine_nx + 1, ctx->fine_ny + 1);
   STOCS_CUDA(ctx, cudaGetLastError());
   return STOCS_OK;
 }
@@ -953,6 +962,20 @@ static int index_layout(stocs_b200_ctx* ctx, const float* aabb) {
   ctx->coarse_shift = cshift; ctx->coarse_nx = cnx; ctx->coarse_ny = cny; ctx->coarse_nz = cnz;
   ctx->coarse_words = (int)(((size_t)(cnx + 1) * (cny + 1) * (cnz + 1) + 31) / 32);
   STOCS_CUDA(ctx, ctx->d_coarse.ensure((size_t)ctx->coarse_words * 4));
+  // Fine occupancy map, for the top-K survivor count only (survivor_count_kernel, score.cu): the same
+  // map at the smallest block shift >= 2 whose bitmap, border blocks included, fits 80 KB.  The count
+  // kernel's CTA (16 warps) stages the map beside 24 KB of transforms and a histogram of M + 1 bins, and
+  // two such CTAs per SM need <= 113 KB each: 80 KB leaves room for models of up to ~2 000 points.  (S1:
+  // 40 mm coarse blocks, 9 KB; 20 mm fine blocks, 69 KB.)  The grid is padded to whole coarse blocks, so
+  // fine blocks tile it exactly.  When nothing finer fits, the count reads the coarse map.
+  // STOCS_FINE_BITS overrides the budget (tuning knob).
+  size_t fine_bits = 80 * 1024 * 8;
+  if (const char* e = getenv("STOCS_FINE_BITS")) { long v = atol(e); if (v >= 0 && v <= 160 * 1024 * 8) fine_bits = (size_t)v; }
+  int fshift = 2;
+  while (fshift < cshift && (size_t)((g.nx >> fshift) + 1) * ((g.ny >> fshift) + 1) * ((g.nz >> fshift) + 1) > fine_bits) ++fshift;
+  ctx->fine_shift = fshift; ctx->fine_nx = g.nx >> fshift; ctx->fine_ny = g.ny >> fshift; ctx->fine_nz = g.nz >> fshift;
+  ctx->fine_words = (int)(((size_t)(ctx->fine_nx + 1) * (ctx->fine_ny + 1) * (ctx->fine_nz + 1) + 31) / 32);
+  if (fshift < cshift) STOCS_CUDA(ctx, ctx->d_fine.ensure((size_t)ctx->fine_words * 4));
   size_t tmp_bytes = 0, tmp_bytes2 = 0;
   cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes, counts, dense_start, (int)nc1, st);
   cub::DeviceScan::ExclusiveSum(nullptr, tmp_bytes2, d_occ.as<uint32_t>(), d_occ_scan.as<uint32_t>(), (int)(g.nbricks + 1), st);

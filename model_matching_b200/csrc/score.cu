@@ -54,6 +54,10 @@ struct ScoreArgs {
   int coarse_words;                      // words of `coarse` (always staged in shared memory, <= 16 KB)
   int coarse_shift, coarse_nx, coarse_ny, coarse_nz;  // real blocks per axis; index n* is the empty border block
   int coarse_sx, coarse_sy;                           // row / slab strides of the map = blocks + 1
+  // the fine map (survivor_count_kernel only): blocks of 2^fine_shift cells, fine_shift <= coarse_shift;
+  // == coarse when fine_shift == coarse_shift
+  const uint32_t* __restrict__ fine;
+  int fine_words, fine_shift, fine_nx, fine_ny, fine_nz, fine_sx, fine_sy;
   const uint32_t* __restrict__ starts;
   const float4* __restrict__ cand;
   const float4* __restrict__ sattr;
@@ -808,45 +812,65 @@ __global__ void __launch_bounds__(256) probe_order_kernel(ScoreArgs a, int* __re
 }
 
 // ---- Survivor order of a top-K launch (kPrune, above the heavy-first range) -------------------------
-// survivor_count_kernel computes, for every hypothesis, the count loop 1 would compute: model points
-// (index < M) whose coarse block has its bit set, with the same grid-block map G and the same
+// survivor_count_kernel computes, for every hypothesis, the count of model points (index < M) whose
+// block of an occupancy map has its bit set, with loop 1's grid-block map G (coarse scale) and loop 1's
 // __fmaf_rn chain.  rank_scatter_kernel turns the counts into a claim order with the count
 // non-increasing; the scorer claims in that order and stops at the first claim the bound rejects
 // (see the top of score_lcp_kernel's loop).  The K best records do not depend on the claim order.
+//
+// The map is the FINE one (blocks of 2^fine_shift = 2^(coarse_shift - d) cells): the chain's result v
+// is in coarse-block units, and the fine block is floor(2^d v).  visit() takes its cell as
+// floor(2^coarse_shift v) from the same v, and nested floors by powers of two give cell >> fine_shift ==
+// floor(2^d v): the cell lies inside that fine block.  A point whose fine block is empty therefore finds
+// an empty cell and queues nothing, and the fine count bounds the hypothesis's inliers as loop 1's count
+// does; every fine bit implies its coarse block's bit, so it is never above loop 1's count.  (S1: the
+// 40 mm coarse map leaves ~11 % of the hypotheses to claim, the 20 mm fine map ~2 %.)  With d = 0 (the
+// test hook for loop 1's count, or a scene with no finer map) the kernel computes loop 1's count exactly.
 //
 // Layout for throughput (this kernel is not held to the scorer's 32 registers): a warp takes 32
 // hypotheses and holds 256 model points in registers at a time, 8 per lane as float2 pairs, lane l
 // taking points l, l+32, ..., so that for one hypothesis the warp tests 32 consecutive points per
 // step as loop 1 does.  The hypothesis's G rows come from shared memory by broadcast once per 256
 // points; the only other shared access is the bitmap word.  Two points per instruction: __ffma2_rn
-// (FFMA2) rounds each half exactly as __fmaf_rn.  Floor and clamp: v + 2^23 rounded down (FADD2.RM)
-// holds floor(v) in its low mantissa bits for 0 <= v < 2^23, and bits - 0x4B000000 clamped to n (one
-// VIADDMNMX) is then floor(v); every other finite or infinite v -- negative, >= 2^23 -- lands on n, the
-// always-empty border block, as F2I.FLOOR + the unsigned clamp does.  Only NaN differs (F2I gives 0).
-// So a hypothesis whose G rows are below g_lim = 2^120 / max(1, max |model coordinate|) in magnitude --
-// no product or sum of the chain can then overflow, so no NaN can arise -- gets exactly loop 1's count;
-// any other one (non-finite or huge transform entries) gets M, which never rejects.
-constexpr int kPfWarps = 8;          // warps per CTA
+// (FFMA2) rounds each half exactly as __fmaf_rn.  Floor and clamp: 2^d v + 2^23 rounded down (one
+// FFMA2.RM; 2^d v is exact, so it is rounded once) holds floor(2^d v) in its low mantissa bits for
+// 0 <= 2^d v < 2^23, and bits - 0x4B000000 clamped to n (one VIADDMNMX) is then floor(2^d v); every other
+// finite or infinite value -- negative, >= 2^23 -- lands on n, the always-empty border block, as F2I.FLOOR
+// + the unsigned clamp does.  Only NaN differs (F2I gives 0).  So a hypothesis whose G rows are below
+// g_lim = 2^(120-d) / max(1, max |model coordinate|) in magnitude -- no product or sum of the chain, nor
+// 2^d v, can then overflow, so no NaN can arise -- gets exactly the count; any other one (non-finite or
+// huge transform entries) gets M, which never rejects.
+// CTA shape: 16 warps with the map, 24 KB of G rows and the histogram in shared memory; two CTAs per SM
+// (32 warps, 64 registers) for maps up to 80 KB and models up to ~2 000 points (see the index build).
+constexpr int kPfWarps = 16;         // warps per CTA
 constexpr int kPfPairs = 4;          // float2 pairs per coordinate per lane: 256 model points per warp pass
 constexpr int kPruneHist = 1024;     // byte offset of the survivor histogram in POOL_SCORE_PRUNE
 
-__global__ void __launch_bounds__(kPfWarps * 32) survivor_count_kernel(ScoreArgs a, unsigned* __restrict__ ns,
-                                                                      unsigned* __restrict__ hist, float g_lim) {
+// the occupancy map a survivor count tests against: real blocks per axis (index n = the border block),
+// strides, and the scale 2^d from loop 1's coarse-block coordinates to its blocks
+struct PfMap {
+  const uint32_t* __restrict__ bits;
+  int words;
+  unsigned nx, ny, nz, sx, sy;
+  float scale;
+};
+
+__global__ void __launch_bounds__(kPfWarps * 32, 2) survivor_count_kernel(ScoreArgs a, PfMap map, unsigned* __restrict__ ns,
+                                                                         unsigned* __restrict__ hist, float g_lim) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  uint32_t* s_coarse = reinterpret_cast<uint32_t*>(smem_raw);
-  float4* s_G = reinterpret_cast<float4*>(s_coarse + ((a.coarse_words + 3) & ~3));   // [warp][hypothesis][row]
-  unsigned* s_hist = reinterpret_cast<unsigned*>(s_G + kPfWarps * 32 * 3);            // M + 1 bins
+  uint32_t* s_map = reinterpret_cast<uint32_t*>(smem_raw);
+  float4* s_G = reinterpret_cast<float4*>(s_map + ((map.words + 3) & ~3));   // [warp][hypothesis][row]
+  unsigned* s_hist = reinterpret_cast<unsigned*>(s_G + kPfWarps * 32 * 3);   // M + 1 bins
   const int M = a.M;
-  for (int i = threadIdx.x; i < a.coarse_words; i += blockDim.x) s_coarse[i] = a.coarse[i];
+  for (int i = threadIdx.x; i < map.words; i += blockDim.x) s_map[i] = map.bits[i];
   for (int i = threadIdx.x; i <= M; i += blockDim.x) s_hist[i] = 0u;
   __syncthreads();
   const int warp = threadIdx.x >> 5;
   const unsigned lane = lane_id();
   float4* G = s_G + warp * 32 * 3;
   const float4* mp = reinterpret_cast<const float4*>(a.model);
-  const unsigned nx = (unsigned)a.coarse_nx, ny = (unsigned)a.coarse_ny, nz = (unsigned)a.coarse_nz;
-  const unsigned sx = (unsigned)a.coarse_sx, sy = (unsigned)a.coarse_sy;
-  const float2 k23 = make_float2(8388608.f, 8388608.f);
+  const unsigned nx = map.nx, ny = map.ny, nz = map.nz, sx = map.sx, sy = map.sy;
+  const float2 k23 = make_float2(8388608.f, 8388608.f), sc = make_float2(map.scale, map.scale);
   for (long long base = ((long long)blockIdx.x * kPfWarps + warp) * 32; base < a.H;
        base += (long long)gridDim.x * kPfWarps * 32) {
     const long long h = base + lane;
@@ -891,12 +915,12 @@ __global__ void __launch_bounds__(kPfWarps * 32) survivor_count_kernel(ScoreArgs
                                  __ffma2_rn(make_float2(r1.z, r1.z), z[k], make_float2(r1.w, r1.w))));
           float2 fz = __ffma2_rn(make_float2(r2.x, r2.x), x[k], __ffma2_rn(make_float2(r2.y, r2.y), y[k],
                                  __ffma2_rn(make_float2(r2.z, r2.z), z[k], make_float2(r2.w, r2.w))));
-          fx = __fadd2_rd(fx, k23); fy = __fadd2_rd(fy, k23); fz = __fadd2_rd(fz, k23);
+          fx = __ffma2_rd(fx, sc, k23); fy = __ffma2_rd(fy, sc, k23); fz = __ffma2_rd(fz, sc, k23);
           const unsigned c0 = (min(__float_as_uint(fz.x) - 0x4B000000u, nz) * sy + min(__float_as_uint(fy.x) - 0x4B000000u, ny)) * sx +
                               min(__float_as_uint(fx.x) - 0x4B000000u, nx);
           const unsigned c1 = (min(__float_as_uint(fz.y) - 0x4B000000u, nz) * sy + min(__float_as_uint(fy.y) - 0x4B000000u, ny)) * sx +
                               min(__float_as_uint(fx.y) - 0x4B000000u, nx);
-          n += ((s_coarse[c0 >> 5] >> (c0 & 31u)) & 1u) + ((s_coarse[c1 >> 5] >> (c1 & 31u)) & 1u);
+          n += ((s_map[c0 >> 5] >> (c0 & 31u)) & 1u) + ((s_map[c1 >> 5] >> (c1 & 31u)) & 1u);
         }
         const unsigned r = __reduce_add_sync(0xffffffffu, n);
         if (lane == (unsigned)t) cnt += r;
@@ -1013,6 +1037,10 @@ ScoreArgs score_args(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_
   a.coarse_words = ctx->coarse_words;
   a.coarse_shift = ctx->coarse_shift; a.coarse_nx = ctx->coarse_nx; a.coarse_ny = ctx->coarse_ny; a.coarse_nz = ctx->coarse_nz;
   a.coarse_sx = ctx->coarse_nx + 1; a.coarse_sy = ctx->coarse_ny + 1;
+  a.fine = ctx->fine_shift < ctx->coarse_shift ? ctx->d_fine.as<uint32_t>() : a.coarse;
+  a.fine_words = ctx->fine_words;
+  a.fine_shift = ctx->fine_shift; a.fine_nx = ctx->fine_nx; a.fine_ny = ctx->fine_ny; a.fine_nz = ctx->fine_nz;
+  a.fine_sx = ctx->fine_nx + 1; a.fine_sy = ctx->fine_ny + 1;
   a.starts = ctx->d_cell_start.as<uint32_t>();
   a.cand = ctx->d_cand.as<float4>();
   a.sattr = ctx->d_sattr.as<float4>();
@@ -1033,19 +1061,29 @@ ScoreArgs score_args(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_
   return a;
 }
 
-// survivor_count_kernel over the launch of a: ns[h] for every hypothesis, lcp (and inliers) 0, and the
-// counts' histogram added into hist (M + 1 bins)
-int enqueue_survivor_counts(stocs_b200_ctx* ctx, const ScoreArgs& a, unsigned* ns, unsigned* hist, cudaStream_t st) {
-  // bound on the grid-map entries below which loop 1's chain cannot overflow (see survivor_count_kernel)
-  const float g_lim = std::isfinite(ctx->model_abs_max) ? 0x1p120f / std::max(1.0f, ctx->model_abs_max) : 0.f;
-  const size_t smem = (size_t)((a.coarse_words + 3) & ~3) * 4 + (size_t)kPfWarps * 32 * 3 * 16 + (size_t)(a.M + 1) * 4;
+// survivor_count_kernel over the launch of a, on the fine map (fine) or the coarse one: ns[h] for every
+// hypothesis, lcp (and inliers) 0, and the counts' histogram added into hist (M + 1 bins)
+int enqueue_survivor_counts(stocs_b200_ctx* ctx, const ScoreArgs& a, unsigned* ns, unsigned* hist, cudaStream_t st,
+                            bool fine) {
+  PfMap map;
+  if (fine) {
+    map = PfMap{a.fine, a.fine_words, (unsigned)a.fine_nx, (unsigned)a.fine_ny, (unsigned)a.fine_nz,
+                (unsigned)a.fine_sx, (unsigned)a.fine_sy, (float)(1u << (a.coarse_shift - a.fine_shift))};
+  } else {
+    map = PfMap{a.coarse, a.coarse_words, (unsigned)a.coarse_nx, (unsigned)a.coarse_ny, (unsigned)a.coarse_nz,
+                (unsigned)a.coarse_sx, (unsigned)a.coarse_sy, 1.0f};
+  }
+  // bound on the grid-map entries below which the chain, and 2^d times its result, cannot overflow (see
+  // survivor_count_kernel)
+  const float g_lim = std::isfinite(ctx->model_abs_max) ? 0x1p120f / std::max(1.0f, ctx->model_abs_max) / map.scale : 0.f;
+  const size_t smem = (size_t)((map.words + 3) & ~3) * 4 + (size_t)kPfWarps * 32 * 3 * 16 + (size_t)(a.M + 1) * 4;
   STOCS_CUDA(ctx, cudaFuncSetAttribute(survivor_count_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int per_sm = 0;
   STOCS_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, survivor_count_kernel, kPfWarps * 32, smem));
-  if (per_sm < 1) STOCS_FAIL(ctx, STOCS_E_ARG, "score: coarse map too large for the survivor count");
+  if (per_sm < 1) STOCS_FAIL(ctx, STOCS_E_ARG, "score: occupancy map too large for the survivor count");
   const long long tiles = (a.H + kPfWarps * 32 - 1) / (kPfWarps * 32);
   const long long grid = std::min(tiles, (long long)ctx->num_sms * per_sm);
-  survivor_count_kernel<<<(unsigned)grid, kPfWarps * 32, smem, st>>>(a, ns, hist, g_lim);
+  survivor_count_kernel<<<(unsigned)grid, kPfWarps * 32, smem, st>>>(a, map, ns, hist, g_lim);
   return STOCS_OK;
 }
 
@@ -1093,10 +1131,11 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   // cannot spare one more launch.  STOCS_NO_LPT=1 switches it off, STOCS_LPT_MAX overrides the bound.
   const bool no_lpt = getenv("STOCS_NO_LPT") != nullptr;
   const long long lpt_max = getenv("STOCS_LPT_MAX") ? atoll(getenv("STOCS_LPT_MAX")) : 300000;
-  // A top-K launch above that range counts every hypothesis's coarse survivors first and claims in
-  // descending count (survivor_count_kernel): B200, S1 call 1.100 -> 0.822 ms; at 125 000 hypotheses
-  // the two extra launches cost more than they save (0.294 -> 0.312 ms), so there the heavy-first order
-  // stays.  Not when the transforms are read in place from page-locked host memory: the count would
+  // A top-K launch above that range counts every hypothesis's survivors first and claims in
+  // descending count (survivor_count_kernel): B200, S1 call 1.100 -> 0.822 ms, and 0.823 -> 0.773 ms
+  // with the count on the fine map; at 125 000 hypotheses the two extra launches cost more than they
+  // save (0.294 -> 0.312 ms on the coarse map, 0.291 -> 0.322 ms on the fine one), so there the
+  // heavy-first order stays.  Not when the transforms are read in place from page-locked host memory: the count would
   // pull every transform over PCIe a second time.
   const bool ranked = prune && H > lpt_max && !stocs_host_alias(d_T);
   // [0, 8) work counter, [128, 132) theta bucket, [256, 768) bucket counts, and with the survivor order
@@ -1149,7 +1188,7 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
     DevBuf &b_ns = ctx->pool[POOL_SCORE_NS], &b_ranked = ctx->pool[POOL_SCORE_ORDER];
     STOCS_CUDA(ctx, b_ns.ensure((size_t)H * 4));
     STOCS_CUDA(ctx, b_ranked.ensure((size_t)H * 8));
-    const int rc = enqueue_survivor_counts(ctx, a, b_ns.as<unsigned>(), hist, st);
+    const int rc = enqueue_survivor_counts(ctx, a, b_ns.as<unsigned>(), hist, st, true);
     if (rc) return rc;
     const size_t rs_smem = (size_t)(ctx->M + 1) * 8;
     STOCS_CUDA(ctx, cudaFuncSetAttribute(rank_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem));
@@ -1166,12 +1205,14 @@ int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* 
   return STOCS_OK;
 }
 
-// coarse-survivor count of every hypothesis, as the top-K path's survivor order computes it (test hook)
-int stocs_survivor_counts(stocs_b200_ctx* ctx, const float* d_T, int64_t H, unsigned* d_ns, cudaStream_t st) {
+// survivor count of every hypothesis on the fine map, as the top-K path's survivor order computes it, or
+// on the coarse map, as loop 1 does (test hooks)
+int stocs_survivor_counts(stocs_b200_ctx* ctx, const float* d_T, int64_t H, unsigned* d_ns, cudaStream_t st, bool fine) {
   if (ctx->kd_pending) { const int rc = stocs_kd_finish(ctx, st); if (rc) return rc; }
   DevBuf &b_lcp = ctx->pool[POOL_SHARD_LCP], &b_hist = ctx->pool[POOL_SCORE_PRUNE];
   STOCS_CUDA(ctx, b_lcp.ensure((size_t)H * 4));
   STOCS_CUDA(ctx, b_hist.ensure((size_t)(ctx->M + 1) * 4));
   STOCS_CUDA(ctx, cudaMemsetAsync(b_hist.p, 0, (size_t)(ctx->M + 1) * 4, st));
-  return enqueue_survivor_counts(ctx, score_args(ctx, d_T, H, b_lcp.as<float>(), nullptr), d_ns, b_hist.as<unsigned>(), st);
+  return enqueue_survivor_counts(ctx, score_args(ctx, d_T, H, b_lcp.as<float>(), nullptr), d_ns, b_hist.as<unsigned>(), st,
+                                 fine);
 }

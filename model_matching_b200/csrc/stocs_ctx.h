@@ -90,7 +90,7 @@ enum PoolSlot : int {
   // sharded scoring scratch (transforms / lcp / inliers of the local shard)
   POOL_SHARD_T = 42, POOL_SHARD_LCP, POOL_SHARD_INL,
   // score.cu: claim order of the heavy-first schedule (one int per hypothesis of the launch), or of a
-  // top-K launch in descending coarse-survivor count (one {hypothesis, count} uint2 per hypothesis)
+  // top-K launch in descending survivor count (one {hypothesis, count} uint2 per hypothesis)
   POOL_SCORE_ORDER = 45,
   // reduce.cu: per-CTA top-32 lists of reductions launched on the context's second stream
   POOL_TOPK_LISTS_AUX = 46,
@@ -110,7 +110,7 @@ enum PoolSlot : int {
   POOL_CLUSTER = 55,
   // capi.cu (upload_scenes_device): a slice held on another device, copied to this one (pos3 | nrm3 | cls | pix)
   POOL_SCENE_PEER = 56,
-  // score.cu: coarse-survivor count of every hypothesis of a top-K launch (survivor_count_kernel)
+  // score.cu: survivor count of every hypothesis of a top-K launch (survivor_count_kernel, fine map)
   POOL_SCORE_NS = 57,
   POOL_COUNT = 58
 };
@@ -141,7 +141,7 @@ enum CtxCounter : int {
   CTR_TIES,                 // NN queries resolved by the kd-tree tie path (DevScratch::score_totals)
   CTR_GRID_CELLS,           // grid cells of the current scene index
   CTR_CANDIDATES,           // replicated candidate records of the current scene index
-  CTR_REJECTED_LOOP1,       // top-K hypotheses rejected after the coarse test (DevScratch::score_totals)
+  CTR_REJECTED_LOOP1,       // top-K hypotheses rejected on the prefilter count: fine-map survivor count or loop 1 (DevScratch::score_totals)
   CTR_REJECTED_DRAIN,       // top-K hypotheses rejected before a queue drain (DevScratch::score_totals)
   CTR_OCCUPIED_CELLS,       // occupied cells of the current scene index
   // STATE, not a diagnostic: voxels of the last build_scene_cloud, which the next call takes as its
@@ -218,7 +218,11 @@ struct stocs_b200_ctx {
   DevBuf d_brick_occ;                  // 1 bit per brick: brick has an occupied cell
   DevBuf d_coarse;                     // 1 bit per block of 2^coarse_shift cells/axis (>= brick): block has an occupied cell
   int coarse_shift = 2, coarse_nx = 0, coarse_ny = 0, coarse_nz = 0, coarse_words = 0;
-  DevBuf d_bricks;                     // uint4 {mask lo, mask hi, first occupied-cell rank, 0} per brick
+  // the same map at blocks of 2^fine_shift cells/axis (2 <= fine_shift <= coarse_shift), for the top-K
+  // survivor count only; fine_shift == coarse_shift: no second map, d_fine is unused and the count reads d_coarse
+  DevBuf d_fine;
+  int fine_shift = 2, fine_nx = 0, fine_ny = 0, fine_nz = 0, fine_words = 0;
+  DevBuf d_bricks;                    // uint4 {mask lo, mask hi, first occupied-cell rank, 0} per brick
   DevBuf d_cell_start;                 // uint32[occupied cells + 1]: candidate offsets
   DevBuf d_cand;                       // float4 (x,y,z,bits(idx)) replicated per dilated cell
   int64_t ncand = 0;
@@ -284,7 +288,7 @@ struct DevScratch {
   // their chunk number so that concurrent chunks do not share one); cleared before each launch
   unsigned long long work[stocs_b200_ctx::kMaxChunks];
   // score.cu, ZERO-RELIANT: NN queries resolved by the kd-tree tie path, and top-K hypotheses
-  // rejected after the coarse test / before a drain / after the brick-bit refinement, accumulated
+  // rejected on the prefilter count / before a drain / after the brick-bit refinement, accumulated
   // over the context's lifetime; stocs_b200_get_counters reads the four in one copy
   struct ScoreTotals { unsigned long long ties, rejected[3]; } score_totals;
   // capi.cu (stocs_b200_score_counters): the counting variant's ScoreCounter slots (score.cu)
@@ -358,9 +362,10 @@ struct ScoreRequest {
 };
 int stocs_launch_score(stocs_b200_ctx* ctx, const float* d_T, int64_t H, float* d_lcp, int32_t* d_inl,
                        cudaStream_t st, const ScoreRequest& rq);
-// coarse-survivor count of each of H device transforms into d_ns, as a large top-K launch orders its
-// claims by it (score.cu; enqueued on st, lcp written to scratch)
-int stocs_survivor_counts(stocs_b200_ctx* ctx, const float* d_T, int64_t H, unsigned* d_ns, cudaStream_t st);
+// survivor count of each of H device transforms into d_ns (score.cu; enqueued on st, lcp written to
+// scratch): on the fine map as a large top-K launch orders its claims by it (fine), or on the coarse map
+// as loop 1 counts (!fine)
+int stocs_survivor_counts(stocs_b200_ctx* ctx, const float* d_T, int64_t H, unsigned* d_ns, cudaStream_t st, bool fine);
 int stocs_launch_backproject(stocs_b200_ctx* ctx, const uint16_t* d_depth, const uint8_t* d_bgr,
                              int W, int H, float fx, float cx, float fy, float cy, float scale,
                              float* d_xyz, uint32_t* d_rgb, cudaStream_t st);  // backproject.cu
